@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- acquisition cells/s of the B200 engine on BASELINE.json's workloads.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (front end + PRN x Doppler x code-phase search + best-Doppler pick) over one
 batch of synthetic captures.
@@ -24,6 +24,8 @@ records are gathered with NCCL inside the timed region.
   cpu_baseline  BASELINE.md rows B1 (literal search.cpp, one core) and B2 (forked over all cores) plus the OpenMP
              oracle port, on a bounded sample of the same captures (N = 1, rank 0)
 `--impl reference` times the reference's own CPU path on the same workload instead (see reference_arm()).
+`--dump-outputs DIR` writes the records the last timed step of each workload returned (dump_records()); the inputs are
+generated from fixed seeds, so two builds run with the same arguments can be compared record for record.
 """
 import argparse
 import json
@@ -120,6 +122,13 @@ class ClockSampler:
                 "power_w": statistics.median([r[1][2] for r in use]),
                 "reasons": sorted(reasons), "samples": len(use), "samples_in_timed_region": len(inside),
                 "samples_total": len(rows), "period_ms": 20}
+
+
+def dump_records(out_dir, name, rec):
+    """One workload's records as DIR/<name>_<field>.npy, float64 (exact for every field: int32 and float32)."""
+    os.makedirs(out_dir, exist_ok=True)
+    for f in rec.dtype.names:
+        np.save(os.path.join(out_dir, "%s_%s.npy" % (name, f)), np.ascontiguousarray(rec[f], np.float64))
 
 
 # ------------------------------------------------------------------------------------------ workload description
@@ -499,6 +508,8 @@ def main():
     ap.add_argument("--no-configs", action="store_true", help="headline only (skip the cfg1..cfg4 entries)")
     ap.add_argument("--only", default="", help="comma list of the cfg1..cfg4 entries to run (default: all)")
     ap.add_argument("--no-cufft", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the records of each workload's last timed step "
+                    "as DIR/<workload>_<field>.npy (float64)")
     args = ap.parse_args()
     if args.impl == "reference":
         return reference_arm(args)
@@ -552,6 +563,8 @@ def main():
     launches_timed = launches * args.steps // (args.steps + args.warmup)
     value = cells_total / (ms_per_step * 1e-3)
     dev_records = fm.d_all.cpu().numpy().copy()
+    if args.dump_outputs and rank == 0:
+        dump_records(args.dump_outputs, HEADLINE, fm._unpad(dev_records, fm.n_sel).reshape(n_total, fm.n_sel))
     # per-kernel durations (CUDA events between the kernels on the launching stream), same window of clock samples
     eng.set_profiling(True)
     kern_ms = []
@@ -585,7 +598,7 @@ def main():
         kw = scenarios.params_kw(cfg)
         e = eng if cfg == "cfg1" else F.AcqEngine(tb, F.default_params(**kw), device=local)
         cap = single_capture(cfg)
-        steps_c = max(args.steps, 100) if cfg != "cfg2" else args.steps
+        steps_c = args.steps
         cells_c, tiles_c = e.cells_per_search(), e.tiles_per_search()
         ent = {"cells_per_step": cells_c, "tiles_per_step": tiles_c, "steps": steps_c}
         if world == 1:
@@ -608,7 +621,7 @@ def main():
             ent["sharding"] = "single GPU"
             e.set_profiling(True)
             km = []
-            for _ in range(10):
+            for _ in range(min(steps_c, 10)):
                 flush.fill_(1)
                 e.search_device(d_in.data_ptr(), d_out.data_ptr(), 1, stream_ptr=stream.cuda_stream)
                 km.append(e.kernel_ms())
@@ -629,12 +642,14 @@ def main():
                                   world, min(sf.counts), max(sf.counts))
             e.set_profiling(True)
             km = []
-            for _ in range(10):
+            for _ in range(min(steps_c, 10)):
                 flush.fill_(1)
                 sf.search_resident()
                 km.append(e.kernel_ms())
             T.barrier()
             e.set_profiling(False)
+        if args.dump_outputs and rank == 0:
+            dump_records(args.dump_outputs, cfg, nrec)
         thr = kw.get("thr_e1b", 16.0) if cfg.startswith("cfg3") else kw.get("thr_l1", 16.0)
         ent.update({"value": cells_c / (ms * 1e-3), "unit": UNIT, "ms_per_step": ms, "tiles_per_s": tiles_c / (ms * 1e-3),
                     "kernel_ms": {k: statistics.mean(x[k] for x in km) for k in km[0]},

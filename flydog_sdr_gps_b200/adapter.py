@@ -1,7 +1,7 @@
 """ctypes driver of integration/_build/libsearch_gpu.so: the reference-side adapter (integration/search_gpu.cpp -- the
 six Search* entry points of gps/gps.h:140-145 over libacq_b200.so) inside the receiver harness the tests use
-(integration/harness_gpu.cpp).  The library is compiled against the reference's own headers where the reference tree
-exists (integration/Makefile); the prebuilt file travels to the GPU box."""
+(integration/harness_gpu.cpp).  The library is compiled against integration/ref_api, the declarations of the
+reference's types.h, gps/gps.h and its gps/sats.cpp table restated in this repository (integration/Makefile)."""
 import ctypes as C
 import os
 import subprocess
@@ -11,7 +11,7 @@ import numpy as np
 HERE = os.path.dirname(os.path.abspath(__file__))
 INTEGRATION = os.path.join(os.path.dirname(HERE), "integration")
 LIB = os.path.join(INTEGRATION, "_build", "libsearch_gpu.so")
-REF = "/root/reference"
+REF = os.path.join(INTEGRATION, "ref_api")
 
 EVENT_DTYPE = np.dtype([("kind", "<i4"), ("a", "<i4"), ("b", "<i4"), ("c", "<i4"), ("d", "<i4"),
                         ("e", "<i4"), ("x", "<f8"), ("y", "<f8")])
@@ -24,20 +24,18 @@ REFERENCE_SYMBOLS = {
 
 
 def build():
-    """Build the adapter where the reference tree is present (a no-op otherwise); returns the library path or None."""
+    """Build the adapter (make keeps a fresh library); returns the library path."""
     from . import _build
-    if not os.path.exists(os.path.join(REF, "gps", "gps.h")):
-        return LIB if os.path.exists(LIB) else None
     if _build.needs_build():
         _build.build()
-    subprocess.run(["make", "-C", INTEGRATION, "--no-print-directory", "REF=" + REF], check=True, stdout=subprocess.DEVNULL)
+    subprocess.run(["make", "-C", INTEGRATION, "--no-print-directory"], check=True, stdout=subprocess.DEVNULL)
     return LIB
 
 
 class Adapter:
     def __init__(self):
-        if not os.path.exists(LIB) and build() is None:
-            raise RuntimeError("integration/_build/libsearch_gpu.so is missing and the reference tree is not here to build it")
+        if not os.path.exists(LIB):
+            build()
         L = C.CDLL(LIB)
         L.adp_init.argtypes = [C.c_int, C.POINTER(C.c_char_p)]
         L.adp_search_task.argtypes = [C.c_void_p] + [C.c_int] * 8
