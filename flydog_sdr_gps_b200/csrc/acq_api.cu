@@ -140,6 +140,11 @@ struct acq_engine {
     acq_fine *d_fine = nullptr;
     size_t cap_ref_rec = 0, cap_fine = 0;
     int last_captures = 0;  // 0: no search whose spectra are still on the device
+    // aided host search (acq_search_aided): Doppler centres staged in pinned memory, copied to the device with the capture
+    int32_t *h_center = nullptr;
+    size_t cap_h_center = 0;
+    int *d_center = nullptr;
+    size_t cap_center = 0;
 };
 
 namespace {
@@ -207,6 +212,8 @@ int free_engine(acq_engine *e)
     cudaFree(e->d_sat_type);
     cudaFree(e->d_ref_rec);
     cudaFree(e->d_fine);
+    cudaFree(e->d_center);
+    if (e->h_center) cudaFreeHost(e->h_center);
     if (e->h_packed) cudaFreeHost(e->h_packed);
     if (e->h_records) cudaFreeHost(e->h_records);
     if (e->h_flag) cudaFreeHost(e->h_flag);
@@ -246,7 +253,8 @@ int grow(acq_engine *e, T *&ptr, size_t &cap, size_t need_elems, bool zero = fal
     return ACQ_OK;
 }
 
-int ensure_scratch(acq_engine *e, int n_captures, int n_slots, bool host_path)
+// n_dop: Doppler cells per row of this search (the engine's range, or the window of an aided search)
+int ensure_scratch(acq_engine *e, int n_captures, int n_slots, bool host_path, int n_dop)
 {
     const size_t blocks = (size_t)n_captures * e->prm.k_noncoh;
     if (blocks > e->cap_blocks || !e->d_x2) {
@@ -262,7 +270,7 @@ int ensure_scratch(acq_engine *e, int n_captures, int n_slots, bool host_path)
     }
     const size_t rows = (size_t)n_captures * n_slots;
     int rc;
-    if ((rc = grow(e, e->d_cells, e->cap_cells, rows * e->n_dop))) return rc;
+    if ((rc = grow(e, e->d_cells, e->cap_cells, rows * n_dop))) return rc;
     if (!host_path) return ACQ_OK;
     const size_t bytes = blocks * e->block_bytes;
     if ((rc = grow(e, e->d_packed, e->cap_packed, bytes))) return rc;
@@ -366,13 +374,19 @@ int set_selection(acq_engine *e, const int32_t *sel, int n_sel)
     return ACQ_OK;
 }
 
+// Doppler cells per row: the engine's whole range, or the window of an aided search (center != NULL)
+int row_dops(const acq_engine *e, const void *center, int half_width) { return center ? 2 * half_width + 1 : e->n_dop; }
+
 // Enqueue front end + forward FFT + search (which ends in the best-Doppler pick) on `st` for captures already on the
 // device.  records_dev: where the kernels write the records (device memory, or the device alias of mapped host memory);
-// flag_dev: mapped completion word, or NULL.
+// flag_dev: mapped completion word, or NULL.  center_dev: the rows' Doppler centres on the device (an aided search), or
+// NULL for the whole range.
 int enqueue_search(acq_engine *e, const uint8_t *packed_dev, int n_captures, acq_record *records_dev, unsigned *flag_dev,
-                   cudaStream_t st, const uint8_t *packed_host_arg = nullptr)
+                   cudaStream_t st, const uint8_t *packed_host_arg = nullptr, const int *center_dev = nullptr,
+                   int half_width = 0)
 {
     const int K = e->prm.k_noncoh;
+    const int n_dop = row_dops(e, center_dev, half_width);
     const int blocks = n_captures * K;
     const bool prof = e->profiling;
     if (e->dev_pending) CU(cudaStreamWaitEvent(st, e->dev_done, 0));  // a no-op on the stream that recorded it
@@ -401,8 +415,11 @@ int enqueue_search(acq_engine *e, const uint8_t *packed_dev, int n_captures, acq
     a.tables = e->d_tables;
     a.cells = e->d_cells;
     a.n_slots = e->n_slots;
-    a.n_dop = e->n_dop;
+    a.n_dop = n_dop;
     a.dop_lo = e->prm.dop_lo;
+    a.dop_center = center_dev;
+    a.half_width = half_width;
+    a.dop_hi = e->prm.dop_hi;
     a.half_bin = e->prm.half_bin;
     a.K = K;
     a.nvar = e->nvar;
@@ -413,7 +430,7 @@ int enqueue_search(acq_engine *e, const uint8_t *packed_dev, int n_captures, acq
     a.cd_div = e->cd_div;
     const int n_rows = n_captures * e->n_slots;
     const bool fold = n_rows <= kFoldPickRowsMax;
-    const long long tiles_l1 = (long long)n_captures * e->n_l1 * e->n_dop, tiles_e1b = (long long)n_captures * e->n_e1b * e->n_dop;
+    const long long tiles_l1 = (long long)n_captures * e->n_l1 * n_dop, tiles_e1b = (long long)n_captures * e->n_e1b * n_dop;
     // Cluster/DSMEM form of the E1B search when every tile can have a cluster of its own (one wave: 9 us per tile
     // against 12.5 us for the one-CTA form, measured) or when forced (variant builds).  With more tiles than that the
     // one-CTA-per-tile forms (k_search_e1b, k_search_e1b_multi for non-coherent sums) have ~2.9x the throughput.
@@ -444,12 +461,12 @@ int enqueue_search(acq_engine *e, const uint8_t *packed_dev, int n_captures, acq
         else e->launches += launch_search(a, true, e->sm_count, st, pdl);
     }
     if (prof) CU(cudaEventRecord(e->prof[3], st));
+    const PickDop pd{e->prm.dop_lo, center_dev, half_width, e->prm.dop_hi};
     if (fold)
         e->launches += launch_pick_small(e->d_cells, e->cur_slot_sat, records_dev, e->d_ctas_done, a.ctas_total, flag_dev,
-                                         e->epoch, n_rows, e->n_slots, e->n_dop, e->prm.dop_lo, st, pdl);
+                                         e->epoch, n_rows, e->n_slots, n_dop, pd, st, pdl);
     else
-        e->launches += launch_best_dop(e->d_cells, e->cur_slot_sat, records_dev, n_captures, e->n_slots, e->n_dop,
-                                       e->prm.dop_lo, st, pdl);
+        e->launches += launch_best_dop(e->d_cells, e->cur_slot_sat, records_dev, n_captures, e->n_slots, n_dop, pd, st, pdl);
     if (prof) {
         CU(cudaEventRecord(e->prof[4], st));
         e->prof_valid = true;
@@ -469,10 +486,37 @@ int check_search_args(acq_engine *e, const void *packed, int n_captures, const v
 }
 
 // after set_selection: a search kernel launch indexes its tiles with 32 bits (and four units per tile with 64)
-int check_tile_count(acq_engine *e, int n_captures)
+int check_tile_count(acq_engine *e, int n_captures, int n_dop)
 {
-    if ((double)n_captures * (double)e->n_slots * (double)e->n_dop > (double)acq::kMaxTilesPerLaunch)
+    if ((double)n_captures * (double)e->n_slots * (double)n_dop > (double)acq::kMaxTilesPerLaunch)
         return fail(ACQ_ERR_UNSUPPORTED, "search too large for one call (more than 2^31 - 1 tiles): split the captures");
+    return ACQ_OK;
+}
+
+// Largest Doppler range an engine can have: |index| <= 4094 half-bins (acq_create: at most 2048 bins either side).
+constexpr int kMaxHalfWidth = 4094;
+
+// Arguments of an aided search that need no engine come first, so that they are reported whatever the engine.
+int check_aided_args(acq_engine *e, const int32_t *dop_center, int half_width)
+{
+    if (!dop_center) return fail(ACQ_ERR_ARG, "dop_center is NULL");
+    if (half_width < 0) return fail(ACQ_ERR_ARG, "half_width must be >= 0 (got %d)", half_width);
+    if (half_width > kMaxHalfWidth)
+        return fail(ACQ_ERR_ARG, "Doppler window W = 2*half_width+1 with half_width %d exceeds n_dop of any engine", half_width);
+    if (!e) return fail(ACQ_ERR_ARG, "engine is NULL");
+    if (2 * half_width + 1 > e->n_dop)
+        return fail(ACQ_ERR_ARG, "Doppler window W = 2*half_width+1 = %d exceeds n_dop = %d", 2 * half_width + 1, e->n_dop);
+    return ACQ_OK;
+}
+
+// after set_selection: the aided search kernels are instantiations of the product's; the experiment kernels of the variant
+// libraries (k_search_l1_dr and its team forms, which step the Doppler index themselves, and the other A/B forms) know
+// nothing of windows, so an aided search that would run on them is refused rather than computed wrong
+int check_aided_kernels(acq_engine *e, int n_captures, int n_dop)
+{
+    if (!search_aided_supported(e->prm.k_noncoh, e->prm.half_bin, (long long)n_captures * e->n_l1 * n_dop,
+                                (long long)n_captures * e->n_e1b * n_dop, e->sm_count))
+        return fail(ACQ_ERR_UNSUPPORTED, "aided search: this library runs the search of that shape on a kernel without Doppler windows");
     return ACQ_OK;
 }
 
@@ -511,20 +555,34 @@ int poll_records(acq_engine *e, acq_record *out, size_t rows)
     return ACQ_OK;
 }
 
+// center (HOST, one per row) and half_width: an aided search (acq_search_aided), or NULL for the whole range
 int search_host(acq_engine *e, const uint8_t *packed, int n_captures, const int32_t *sel, int n_sel, acq_record *out,
-                acq_cell *grid, bool sync)
+                acq_cell *grid, bool sync, const int32_t *center = nullptr, int half_width = 0)
 {
     int rc = check_search_args(e, packed, n_captures, out);
     if (rc) return rc;
     DeviceGuard g(e->device);
     e->last_captures = 0;  // until this search is enqueued, there are no spectra acq_refine could use
+    const int n_dop = row_dops(e, center, half_width);
     if ((rc = set_selection(e, sel, n_sel))) return rc;
-    if ((rc = check_tile_count(e, n_captures))) return rc;
-    if ((rc = ensure_scratch(e, n_captures, e->n_slots, true))) return rc;
+    if ((rc = check_tile_count(e, n_captures, n_dop))) return rc;
+    if (center && (rc = check_aided_kernels(e, n_captures, n_dop))) return rc;
+    if ((rc = ensure_scratch(e, n_captures, e->n_slots, true, n_dop))) return rc;
     const size_t bytes = (size_t)n_captures * e->prm.k_noncoh * e->block_bytes;
     const size_t rows = (size_t)n_captures * e->n_slots;
+    if (center) {
+        if ((rc = grow(e, e->d_center, e->cap_center, rows))) return rc;
+        if (rows > e->cap_h_center) {
+            if ((rc = drain(e))) return rc;
+            if (e->h_center) CU(cudaFreeHost(e->h_center));
+            e->h_center = nullptr;
+            e->cap_h_center = 0;
+            CU(cudaHostAlloc(&e->h_center, rows * sizeof(int32_t), cudaHostAllocDefault));
+            e->cap_h_center = rows;
+        }
+    }
     const bool host_records = ACQ_HOST_RECORDS && rows <= (size_t)kHostRecordRowsMax;
-    const long long tiles_total = (long long)rows * e->n_dop * e->prm.k_noncoh;
+    const long long tiles_total = (long long)rows * n_dop * e->prm.k_noncoh;
     const bool poll = host_records && sync && !grid && !e->profiling && tiles_total <= 64LL * e->sm_count;
     // The reference's own search -- one 1-bit block (gps/search.cpp:389-411) -- hands its 8 KiB to the front end as a
     // kernel argument: the launch carries the bytes, nothing is staged or copied ahead of the first kernel.
@@ -540,13 +598,18 @@ int search_host(acq_engine *e, const uint8_t *packed, int n_captures, const int3
         if (ACQ_ZC_INPUT && src == e->h_packed && bytes <= kZeroCopyMax) packed_dev = e->dh_packed;
         else CU(cudaMemcpyAsync(e->d_packed, src, bytes, cudaMemcpyHostToDevice, e->stream));
     }
+    if (center) {   // from pinned memory: an asynchronous copy node ahead of the front end, even when the capture rides as an argument
+        memcpy(e->h_center, center, rows * sizeof(int32_t));
+        CU(cudaMemcpyAsync(e->d_center, e->h_center, rows * sizeof(int32_t), cudaMemcpyHostToDevice, e->stream));
+    }
     if ((rc = enqueue_search(e, packed_dev, n_captures, host_records ? e->dh_records : e->d_records,
-                             poll ? e->dh_flag : nullptr, e->stream, as_arg ? packed : nullptr)))
+                             poll ? e->dh_flag : nullptr, e->stream, as_arg ? packed : nullptr, center ? e->d_center : nullptr,
+                             half_width)))
         return rc;
     e->last_captures = n_captures;
     if (!host_records) CU(cudaMemcpyAsync(out, e->d_records, rows * sizeof(acq_record), cudaMemcpyDeviceToHost, e->stream));
     if (grid)
-        CU(cudaMemcpyAsync(grid, e->d_cells, rows * e->n_dop * sizeof(acq_cell), cudaMemcpyDeviceToHost, e->stream));
+        CU(cudaMemcpyAsync(grid, e->d_cells, rows * n_dop * sizeof(acq_cell), cudaMemcpyDeviceToHost, e->stream));
     if (!sync) {
         CU(cudaEventRecord(e->done, e->stream));
         e->pending = true;
@@ -572,6 +635,30 @@ void finish_pending(acq_engine *e)
     e->pending = false;
     e->pending_rows = 0;
     e->pending_out = nullptr;
+}
+
+// acq_search_device and acq_search_aided_device (center_dev != NULL)
+int search_device(acq_engine *e, const uint8_t *packed_dev, int n_captures, const int32_t *sel, int n_sel,
+                  acq_record *out_dev, void *stream, const int *center_dev = nullptr, int half_width = 0)
+{
+    int rc = check_search_args(e, packed_dev, n_captures, out_dev);
+    if (rc) return rc;
+    if (((uintptr_t)packed_dev & 15) != 0)
+        return fail(ACQ_ERR_ARG, "packed_dev must be 16-byte aligned (the front end stages it with bulk async copies)");
+    DeviceGuard g(e->device);
+    e->last_captures = 0;  // spectra now belong to a search on the caller's stream: acq_refine does not apply
+    const int n_dop = row_dops(e, center_dev, half_width);
+    if ((rc = set_selection(e, sel, n_sel))) return rc;
+    if ((rc = check_tile_count(e, n_captures, n_dop))) return rc;
+    if (center_dev && (rc = check_aided_kernels(e, n_captures, n_dop))) return rc;
+    if ((rc = ensure_scratch(e, n_captures, e->n_slots, false, n_dop))) return rc;
+    cudaStream_t st = stream ? (cudaStream_t)stream : e->stream;
+    if ((rc = enqueue_search(e, packed_dev, n_captures, out_dev, nullptr, st, nullptr, center_dev, half_width))) return rc;
+    if (st != e->stream) {  // whatever uses the engine's scratch next (any stream, or the host) waits for this search
+        CU(cudaEventRecord(e->dev_done, st));
+        e->dev_pending = true;
+    }
+    return ACQ_OK;
 }
 
 }  // namespace
@@ -832,25 +919,26 @@ int acq_search_grid(acq_engine *e, const uint8_t *packed, int n_captures, const 
     return search_host(e, packed, n_captures, sel, n_sel, out, grid, true);
 }
 
+int acq_search_aided(acq_engine *e, const uint8_t *packed, int n_captures, const int32_t *sel, int n_sel,
+                     const int32_t *dop_center, int half_width, acq_record *out, acq_cell *grid)
+{
+    const int rc = check_aided_args(e, dop_center, half_width);
+    if (rc) return rc;
+    return search_host(e, packed, n_captures, sel, n_sel, out, grid, true, dop_center, half_width);
+}
+
 int acq_search_device(acq_engine *e, const uint8_t *packed_dev, int n_captures, const int32_t *sel, int n_sel,
                       acq_record *out_dev, void *stream)
 {
-    int rc = check_search_args(e, packed_dev, n_captures, out_dev);
+    return search_device(e, packed_dev, n_captures, sel, n_sel, out_dev, stream);
+}
+
+int acq_search_aided_device(acq_engine *e, const uint8_t *packed_dev, int n_captures, const int32_t *sel, int n_sel,
+                            const int32_t *dop_center_dev, int half_width, acq_record *out_dev, void *stream)
+{
+    const int rc = check_aided_args(e, dop_center_dev, half_width);
     if (rc) return rc;
-    if (((uintptr_t)packed_dev & 15) != 0)
-        return fail(ACQ_ERR_ARG, "packed_dev must be 16-byte aligned (the front end stages it with bulk async copies)");
-    DeviceGuard g(e->device);
-    e->last_captures = 0;  // spectra now belong to a search on the caller's stream: acq_refine does not apply
-    if ((rc = set_selection(e, sel, n_sel))) return rc;
-    if ((rc = check_tile_count(e, n_captures))) return rc;
-    if ((rc = ensure_scratch(e, n_captures, e->n_slots, false))) return rc;
-    cudaStream_t st = stream ? (cudaStream_t)stream : e->stream;
-    if ((rc = enqueue_search(e, packed_dev, n_captures, out_dev, nullptr, st))) return rc;
-    if (st != e->stream) {  // whatever uses the engine's scratch next (any stream, or the host) waits for this search
-        CU(cudaEventRecord(e->dev_done, st));
-        e->dev_pending = true;
-    }
-    return ACQ_OK;
+    return search_device(e, packed_dev, n_captures, sel, n_sel, out_dev, stream, dop_center_dev, half_width);
 }
 
 int acq_submit(acq_engine *e, const uint8_t *packed, int n_captures, const int32_t *sel, int n_sel, acq_record *out)

@@ -545,7 +545,8 @@ struct TileIdx {
     __device__ __forceinline__ TileIdx() {}
     // The host keeps a launch below 2^31 tiles (launch_search), so the decomposition runs on 32-bit unsigned
     // divisions: every warp pays it once per tile, and a K = 1 tile is only four sub-FFTs long.
-    __device__ __forceinline__ TileIdx(const SearchArgs &p, long long tile)
+    template <class PA>
+    __device__ __forceinline__ TileIdx(const PA &p, long long tile)
     {
         const unsigned tl = (unsigned)tile, nd = (unsigned)p.n_dop, nw = (unsigned)p.n_work;
         const unsigned cw = tl / nd;
@@ -558,7 +559,8 @@ struct TileIdx {
         set_dop(p);
     }
     // the tile `stride` further on, stride given as mixed-radix digits (sd, sw, sc) over (n_dop, n_work): no division
-    __device__ __forceinline__ void step(const SearchArgs &p, int sd, int sw, int sc)
+    template <class PA>
+    __device__ __forceinline__ void step(const PA &p, int sd, int sw, int sc)
     {
         d += sd;
         int carry = d >= p.n_dop;
@@ -572,9 +574,14 @@ struct TileIdx {
         slot = wk.y;
         set_dop(p);
     }
-    __device__ __forceinline__ void set_dop(const SearchArgs &p)
+    // Doppler index h of the tile: dop_lo + d, or in an aided search (AidedSearchArgs) d steps into its row's window.  The
+    // claiming kernels form a tile's indices in the one thread that publishes them, so the centre's load stays there.
+    template <class PA>
+    __device__ __forceinline__ void set_dop(const PA &p)
     {
-        const int h = p.dop_lo + d;
+        int h;
+        if constexpr (PA::kAided) h = window_lo(__ldg(p.dop_center + cap * p.n_slots + slot), p.half_width, p.dop_lo, p.dop_hi) + d;
+        else h = p.dop_lo + d;
         v = p.half_bin ? (h & 1) : 0;
         dop = p.half_bin ? ((h - v) >> 1) : h;
     }
@@ -609,7 +616,8 @@ __device__ __forceinline__ void claims_done(const SearchArgs &p, int t)
         *(volatile unsigned *)(p.tile_ctr + 2) = 0u;
     }
 }
-__device__ __forceinline__ void publish_tile(int *feed, const SearchArgs &p, unsigned nxt)   // one thread
+template <class PA>
+__device__ __forceinline__ void publish_tile(int *feed, const PA &p, unsigned nxt)   // one thread
 {
     if (nxt < (unsigned)p.n_tiles) {
         const TileIdx tn(p, nxt);
@@ -628,11 +636,16 @@ __device__ __forceinline__ bool next_tile(const int *feed, TileIdx &ti)
 
 // Row of the capture-spectrum array for (capture, block b, variant) at this tile's Doppler index: with code-Doppler
 // compensation the copy delayed by s(b, h) more samples (SearchArgs::n_shift), otherwise the only one.
-__device__ __forceinline__ size_t d_row(const SearchArgs &p, const TileIdx &ti, int b)
+template <class PA>
+__device__ __forceinline__ size_t d_row(const PA &p, const TileIdx &ti, int b)
 {
     const size_t bv = (size_t)((size_t)ti.cap * p.K + b) * p.nvar + ti.v;
     if (p.n_shift == 1) return bv;
-    return bv * p.n_shift + (size_t)(p.smax + code_shift(b, p.dop_lo + ti.d, p.cd_div));
+    // the tile's Doppler index h; in an aided search rebuilt from (dop, v), which set_dop formed from the window base
+    int h;
+    if constexpr (PA::kAided) h = ti.dop * (1 + p.half_bin) + ti.v;
+    else h = p.dop_lo + ti.d;
+    return bv * p.n_shift + (size_t)(p.smax + code_shift(b, h, p.cd_div));
 }
 
 // The cell of a finished tile (one thread): ave_pwr = tot_pwr / L, snr = max_pwr / ave_pwr with IEEE division
@@ -657,7 +670,7 @@ __device__ __forceinline__ void store_cell(const SearchArgs &p, int cap, int slo
 // three per row (measured with the trace variant: 1.4 us per row before, 82 rows of the all-constellation search).
 template <int ROWS>
 __device__ __forceinline__ void pick_rows(const acq_cell *cells, const int *__restrict__ slot_sat, acq_record *out, int row0,
-                                          int row_step, int n_rows, int n_slots, int n_dop, int dop_lo, int lane)
+                                          int row_step, int n_rows, int n_slots, int n_dop, const PickDop &pd, int lane)
 {
     for (int rb = row0; rb < n_rows; rb += ROWS * row_step) {
         float4 c[ROWS][2];
@@ -703,7 +716,7 @@ __device__ __forceinline__ void pick_rows(const acq_cell *cells, const int *__re
                 r.snr = 0.0f;
                 if (best.z > 0.0f) {
                     r.lag = __float_as_int(best.w);
-                    r.dop = dop_lo + best_d;
+                    r.dop = (pd.dop_center ? window_lo(__ldg(pd.dop_center + row), pd.half_width, pd.dop_lo, pd.dop_hi) : pd.dop_lo) + best_d;
                     r.peak = best.x;
                     r.noise = best.y;
                     r.snr = best.z;
@@ -730,7 +743,8 @@ __device__ __forceinline__ void search_cta_epilogue(const SearchArgs &p, int t)
 
 // x[a] = conj(data[k]) * code[k - dop], k = 1024 a + 4 t + k2   (search.cpp:471, support/simd.cpp:12-40).
 // The Doppler shift is a pointer offset (r, q) into the margin-extended polyphase code rows.
-__device__ __forceinline__ void load_products(float2 (&x)[16], const SearchArgs &p, const TileIdx &ti, int b, int k2,
+template <class PA>
+__device__ __forceinline__ void load_products(float2 (&x)[16], const PA &p, const TileIdx &ti, int b, int k2,
                                               int t)
 {
     const int r = (k2 - ti.dop) & 3;
@@ -852,8 +866,8 @@ __device__ __forceinline__ Peak thread_peak_l1(const float (&pw)[16], int t)
 #ifndef ACQ_L1_LEAN
 #define ACQ_L1_LEAN 1   // K = 1: tile indices advance without divisions, max / first index by REDUX (+0.3..1 % cfg5, -1.3 us cfg1; 0 = round-1 form)
 #endif
-template <bool MULTI>
-__global__ void __launch_bounds__(256, 2) k_search_l1(const SearchArgs p)
+template <bool MULTI, class PA>
+__global__ void __launch_bounds__(256, 2) k_search_l1(const PA p)
 {
     extern __shared__ __align__(1024) unsigned char smem[];
     const L1Smem m = l1_smem_carve(smem);
@@ -1259,7 +1273,8 @@ __host__ __device__ constexpr size_t l1_multi_smem_bytes()
 #ifndef ACQ_MULTI_UNROLL
 #define ACQ_MULTI_UNROLL 4
 #endif
-__global__ void __launch_bounds__(256, 2) k_search_l1_multi(const SearchArgs p)
+template <class PA>
+__global__ void __launch_bounds__(256, 2) k_search_l1_multi(const PA p)
 {
     extern __shared__ __align__(1024) unsigned char smem[];
     L1MultiSmem s;
@@ -1319,7 +1334,8 @@ __global__ void __launch_bounds__(256, 2) k_search_l1_multi(const SearchArgs p)
         float2 acc[16];
         for (int b = 0; b < p.K; b++) {
             float2 x[16];
-            constexpr int kMultiUnroll = ACQ_MULTI_UNROLL;
+            // aided: by two, which does not spill (at four the window code takes the spill from 24 to 56 bytes)
+            constexpr int kMultiUnroll = PA::kAided ? 2 : ACQ_MULTI_UNROLL;
 #pragma unroll kMultiUnroll
             for (int k2 = 0; k2 < 4; k2++) {
                 float2 *S1b = s.S1 + (it & 1) * kSub;
@@ -1418,7 +1434,8 @@ __device__ __forceinline__ bool chunk_of(const SearchArgs &p, unsigned c, unsign
 #ifndef ACQ_CR_UNROLL
 #define ACQ_CR_UNROLL 4
 #endif
-__global__ void __launch_bounds__(256, 2) k_search_l1_cr(const SearchArgs p)
+template <class PA>
+__global__ void __launch_bounds__(256, 2) k_search_l1_cr(const PA p)
 {
     extern __shared__ __align__(1024) unsigned char smem[];
     L1MultiSmem s;
@@ -1483,7 +1500,8 @@ __global__ void __launch_bounds__(256, 2) k_search_l1_cr(const SearchArgs p)
         float P[16];
         float2 acc[16];
         float2 x[16];
-        constexpr int kCrUnroll = ACQ_CR_UNROLL;
+        // aided: by two (at four the window base in thread 0's publish_tile costs the loop a 28-byte spill)
+        constexpr int kCrUnroll = PA::kAided ? 2 : ACQ_CR_UNROLL;
 #pragma unroll kCrUnroll
         for (int k2 = 0; k2 < 4; k2++) {
             float2 *S1b = s.S1 + (it & 1) * kSub;
@@ -1606,7 +1624,8 @@ __device__ __forceinline__ E1bSmem e1b_smem_carve(unsigned char *base)
     return s;
 }
 
-__global__ void __launch_bounds__(256, 2) k_search_e1b(const SearchArgs p)
+template <class PA>
+__global__ void __launch_bounds__(256, 2) k_search_e1b(const PA p)
 {
     extern __shared__ __align__(1024) unsigned char smem[];
     const E1bSmem s = e1b_smem_carve(smem);
@@ -1801,7 +1820,8 @@ constexpr int kE1bPowCol = 96;  // TMEM columns [96, 128): block powers of the l
 #ifndef ACQ_E1B_MULTI_UNROLL
 #define ACQ_E1B_MULTI_UNROLL 4
 #endif
-__global__ void __launch_bounds__(256, 2) k_search_e1b_multi(const SearchArgs p)
+template <class PA>
+__global__ void __launch_bounds__(256, 2) k_search_e1b_multi(const PA p)
 {
     extern __shared__ __align__(1024) unsigned char smem[];
     E1bMultiSmem s;
@@ -1989,8 +2009,8 @@ __global__ void __launch_bounds__(256, 2) k_search_e1b_multi(const SearchArgs p)
 // in registers exactly as in k_search_l1 (front-end block delay, see k_hb2).  Y is double
 // buffered: one cluster barrier per block (a buffer is rewritten two blocks later, after the barrier every
 // CTA reached only when it had finished reading it).
-template <bool MULTI>
-__global__ void __cluster_dims__(4, 1, 1) __launch_bounds__(256, 1) k_search_e1b_cluster(const SearchArgs p)
+template <bool MULTI, class PA>
+__global__ void __cluster_dims__(4, 1, 1) __launch_bounds__(256, 1) k_search_e1b_cluster(const PA p)
 {
     namespace cg = cooperative_groups;
     cg::cluster_group cluster = cg::this_cluster();
@@ -2086,7 +2106,7 @@ __global__ void __cluster_dims__(4, 1, 1) __launch_bounds__(256, 1) k_search_e1b
 // the completion word is raised behind the records.
 __global__ void __launch_bounds__(1024) k_pick_small(const acq_cell *cells, const int *__restrict__ slot_sat, acq_record *out,
                                                     unsigned *ctas_done, unsigned ctas_total, unsigned *host_flag, unsigned epoch,
-                                                    int n_rows, int n_slots, int n_dop, int dop_lo)
+                                                    int n_rows, int n_slots, int n_dop, PickDop pd)
 {
     // Records are staged in shared memory and leave in 16-byte pieces: written one 4-byte member at a time straight into
     // mapped host memory they cost 0.17 us per record (every store its own PCIe write: 6.8 us of a 74 us cold-start
@@ -2119,7 +2139,7 @@ __global__ void __launch_bounds__(1024) k_pick_small(const acq_cell *cells, cons
     }
     __syncthreads();
     ACQ_TRACE_STAMP(kTrPick, 1);
-    pick_rows<4>(cells, slot_sat, s_rec, t >> 5, 32, n_rows, n_slots, n_dop, dop_lo, t & 31);
+    pick_rows<4>(cells, slot_sat, s_rec, t >> 5, 32, n_rows, n_slots, n_dop, pd, t & 31);
     __syncthreads();
     ACQ_TRACE_STAMP(kTrPick, 3);
     if (host_flag) {
@@ -2156,11 +2176,11 @@ __global__ void __launch_bounds__(1024) k_pick_small(const acq_cell *cells, cons
 // K5b for large searches: one warp per (capture, sat) row, after the search grids have completed.
 __global__ void __launch_bounds__(128) k_best_dop(const acq_cell *__restrict__ cells, const int *__restrict__ slot_sat,
                                                   acq_record *__restrict__ out, int n_rows, int n_slots, int n_dop,
-                                                  int dop_lo)
+                                                  PickDop pd)
 {
     pdl_wait();  // before the early exit: completion of this grid must imply completion of its predecessors
     ACQ_TRACE_STAMP(kTrPick, 1);
-    pick_rows<1>(cells, slot_sat, out, blockIdx.x * 4 + (threadIdx.x >> 5), n_rows, n_rows, n_slots, n_dop, dop_lo,
+    pick_rows<1>(cells, slot_sat, out, blockIdx.x * 4 + (threadIdx.x >> 5), n_rows, n_rows, n_slots, n_dop, pd,
                  threadIdx.x & 31);
 }
 
@@ -2318,11 +2338,36 @@ static size_t search_e1b_smem_bytes() { return e1b_smem_bytes(); }
 static size_t search_e1b_cluster_smem_bytes() { return fft_smem3_bytes() + 2 * sizeof(float2) * kSub + 64 * sizeof(float); }
 static size_t fwd_smem_bytes() { return fft_smem3_bytes() + kZBytes; }
 
+#ifndef ACQ_CARVEOUT_MAX
+#define ACQ_CARVEOUT_MAX 1   // 0 (variant carve0): the driver's choice per kernel
+#endif
+
+// The search kernels of an aided search (AidedSearchArgs): the product forms only, with the shared-memory size and carveout
+// of their full-range instantiations.
+static cudaError_t aided_kernels_configure()
+{
+    using A = AidedSearchArgs;
+    const void *k[] = {(const void *)k_search_l1<false, A>, (const void *)k_search_l1_multi<A>, (const void *)k_search_l1_cr<A>,
+                       (const void *)k_search_e1b<A>, (const void *)k_search_e1b_multi<A>, (const void *)k_search_e1b_cluster<false, A>,
+                       (const void *)k_search_e1b_cluster<true, A>};
+    const int smem[] = {(int)search_l1_smem_bytes(), (int)l1_multi_smem_bytes(), (int)l1_multi_smem_bytes(), (int)search_e1b_smem_bytes(),
+                        (int)e1b_multi_smem_bytes(), (int)search_e1b_cluster_smem_bytes(), (int)search_e1b_cluster_smem_bytes()};
+    cudaError_t e;
+    for (int i = 0; i < 7; i++) {
+        if ((e = cudaFuncSetAttribute(k[i], cudaFuncAttributeMaxDynamicSharedMemorySize, smem[i]))) return e;
+#if ACQ_CARVEOUT_MAX
+        if ((e = cudaFuncSetAttribute(k[i], cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared))) return e;
+#endif
+    }
+    return cudaSuccess;
+}
+
 cudaError_t search_kernels_configure()
 {
+    using S = SearchArgs;
     cudaError_t e;
     const int l1 = (int)search_l1_smem_bytes(), e1 = (int)search_e1b_smem_bytes(), fw = (int)fwd_smem_bytes();
-    if ((e = cudaFuncSetAttribute(k_search_l1<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, l1))) return e;
+    if ((e = cudaFuncSetAttribute(k_search_l1<false, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, l1))) return e;
 #if ACQ_DR_MIN_TILES_PER_SM >= 0
     if ((e = cudaFuncSetAttribute(k_search_l1_dr, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dr_smem_bytes()))) return e;
 #endif
@@ -2336,12 +2381,12 @@ cudaError_t search_kernels_configure()
     if ((e = cudaFuncSetAttribute(k_search_l1_st, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)st_smem_bytes()))) return e;
 #endif
 #ifdef ACQ_VARIANT_L1_MULTI_TW
-    if ((e = cudaFuncSetAttribute(k_search_l1<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, l1))) return e;
+    if ((e = cudaFuncSetAttribute(k_search_l1<true, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, l1))) return e;
 #endif
-    if ((e = cudaFuncSetAttribute(k_search_l1_multi, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)l1_multi_smem_bytes()))) return e;
-    if ((e = cudaFuncSetAttribute(k_search_l1_cr, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)l1_multi_smem_bytes()))) return e;
-    if ((e = cudaFuncSetAttribute(k_search_e1b, cudaFuncAttributeMaxDynamicSharedMemorySize, e1))) return e;
-    if ((e = cudaFuncSetAttribute(k_search_e1b_multi, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)e1b_multi_smem_bytes()))) return e;
+    if ((e = cudaFuncSetAttribute(k_search_l1_multi<S>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)l1_multi_smem_bytes()))) return e;
+    if ((e = cudaFuncSetAttribute(k_search_l1_cr<S>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)l1_multi_smem_bytes()))) return e;
+    if ((e = cudaFuncSetAttribute(k_search_e1b<S>, cudaFuncAttributeMaxDynamicSharedMemorySize, e1))) return e;
+    if ((e = cudaFuncSetAttribute(k_search_e1b_multi<S>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)e1b_multi_smem_bytes()))) return e;
 #ifdef ACQ_VARIANT_L1_X3
     const int l1x = (int)search_l1_x3_smem();
     if ((e = cudaFuncSetAttribute(k_search_l1_x3<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, l1x))) return e;
@@ -2357,8 +2402,8 @@ cudaError_t search_kernels_configure()
     if ((e = cudaFuncSetAttribute(k_search_e1b_ldg, cudaFuncAttributeMaxDynamicSharedMemorySize, e1g))) return e;
 #endif
     const int ec = (int)search_e1b_cluster_smem_bytes();
-    if ((e = cudaFuncSetAttribute(k_search_e1b_cluster<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, ec))) return e;
-    if ((e = cudaFuncSetAttribute(k_search_e1b_cluster<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, ec))) return e;
+    if ((e = cudaFuncSetAttribute(k_search_e1b_cluster<false, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, ec))) return e;
+    if ((e = cudaFuncSetAttribute(k_search_e1b_cluster<true, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, ec))) return e;
     const int fc = (int)(fft_smem3_bytes() + 2 * sizeof(float2) * kSub);
     if ((e = cudaFuncSetAttribute(k_fwd_fft_cluster<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, fc))) return e;
     if ((e = cudaFuncSetAttribute(k_fwd_fft_cluster<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, fc))) return e;
@@ -2368,26 +2413,23 @@ cudaError_t search_kernels_configure()
     // its SMs at the 196 KiB split and the E1B kernel (2 x 103.8 KiB) at 228 KiB, and an SM changes its split only when
     // it is empty: in a GPS + Galileo search the E1B CTAs -- launched to move in as the C/A CTAs retire -- entered no SM
     // before BOTH its C/A CTAs had gone (trace: first E1B CTA at 54.8 us although half the C/A CTAs leave by 50 us).
-#ifndef ACQ_CARVEOUT_MAX
-#define ACQ_CARVEOUT_MAX 1   // 0 (variant carve0): the driver's choice per kernel
-#endif
 #if ACQ_CARVEOUT_MAX
     const void *chain[] = {(const void *)k_front_end<false>, (const void *)k_front_end<true>, (const void *)k_front_end_arg,
                            (const void *)k_fwd_fft<true>, (const void *)k_fwd_fft<false>, (const void *)k_fwd_fft_cluster<true>,
-                           (const void *)k_fwd_fft_cluster<false>, (const void *)k_search_l1<false>,
+                           (const void *)k_fwd_fft_cluster<false>, (const void *)k_search_l1<false, S>,
 #ifdef ACQ_VARIANT_L1_MULTI_TW
-                           (const void *)k_search_l1<true>,
+                           (const void *)k_search_l1<true, S>,
 #endif
 #if ACQ_DR_MIN_TILES_PER_SM >= 0
                            (const void *)k_search_l1_dr,
 #endif
-                           (const void *)k_search_l1_cr, (const void *)k_search_l1_multi, (const void *)k_search_e1b,
-                           (const void *)k_search_e1b_multi, (const void *)k_search_e1b_cluster<false>,
-                           (const void *)k_search_e1b_cluster<true>, (const void *)k_pick_small, (const void *)k_best_dop};
+                           (const void *)k_search_l1_cr<S>, (const void *)k_search_l1_multi<S>, (const void *)k_search_e1b<S>,
+                           (const void *)k_search_e1b_multi<S>, (const void *)k_search_e1b_cluster<false, S>,
+                           (const void *)k_search_e1b_cluster<true, S>, (const void *)k_pick_small, (const void *)k_best_dop};
     for (const void *f : chain)
         if ((e = cudaFuncSetAttribute(f, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared))) return e;
 #endif
-    return cudaSuccess;
+    return aided_kernels_configure();
 }
 
 int launch_front_end(const uint8_t *packed, float2 *x2, const float2 *rot, int n_blocks, int nvar, int K, int sample_bits,
@@ -2556,6 +2598,40 @@ int search_grid_ctas(long long n_tiles, int kind, int sm_count)
     return (int)(n_tiles < cap ? n_tiles : cap);
 }
 
+// Which searches have an aided form: those that run on the product's search kernels (search_aided_supported).
+bool search_aided_supported(int K, int half_bin, long long tiles_l1, long long tiles_e1b, int sm_count)
+{
+#if defined(ACQ_VARIANT_L1_X3) || defined(ACQ_VARIANT_L1_LDG) || defined(ACQ_VARIANT_L1_MULTI_TW)
+    if (tiles_l1 > 0) return false;
+#endif
+#ifdef ACQ_VARIANT_E1B_LDG
+    if (tiles_e1b > 0) return false;
+#endif
+    (void)tiles_e1b;
+    if (tiles_l1 <= 0) return true;
+    const int kind = search_kind_l1(K, half_bin, tiles_l1, sm_count);
+    return kind == kSearchL1 || kind == kSearchL1Multi || kind == kSearchL1Cr;
+}
+
+// The aided instantiations of the product search kernels (launch_search with SearchArgs::dop_center set).
+static int launch_search_aided(const AidedSearchArgs &a, int kind, int grid, bool e1b, int sm_count, cudaStream_t st, bool pdl)
+{
+    using A = AidedSearchArgs;
+    if (e1b) {
+        if (a.K > 1) launch_k(k_search_e1b_multi<A>, grid, 256, e1b_multi_smem_bytes(), st, pdl, a);
+        else launch_k(k_search_e1b<A>, grid, 256, search_e1b_smem_bytes(), st, pdl, a);
+    } else if (a.K > 1) {
+        launch_k(k_search_l1_multi<A>, grid, 256, l1_multi_smem_bytes(), st, pdl, a);
+    } else if (kind == kSearchL1Cr) {
+        AidedSearchArgs c = a;
+        search_chunks(c.n_tiles, 2 * sm_count, &c.ck_n16, &c.ck_n4);
+        launch_k(k_search_l1_cr<A>, grid, 256, l1_multi_smem_bytes(), st, pdl, c);
+    } else {
+        launch_k(k_search_l1<false, A>, grid, 256, search_l1_smem_bytes(), st, pdl, a);
+    }
+    return 1;
+}
+
 int launch_search(const SearchArgs &a_in, bool e1b, int sm_count, cudaStream_t st, bool pdl)
 {
     const int kind = e1b ? kSearchE1b : search_kind_l1(a_in.K, a_in.half_bin, a_in.n_tiles, sm_count);
@@ -2563,12 +2639,14 @@ int launch_search(const SearchArgs &a_in, bool e1b, int sm_count, cudaStream_t s
     if (grid <= 0) return 0;
     SearchArgs a = a_in;
     if (!search_claims_tiles(a.n_tiles, grid)) a.tile_ctr = nullptr;   // few rounds: static stride
+    if (a.dop_center) return launch_search_aided(AidedSearchArgs(a), kind, grid, e1b, sm_count, st, pdl);
+    using S = SearchArgs;
     if (e1b) {
 #ifdef ACQ_VARIANT_E1B_LDG
         launch_k(k_search_e1b_ldg, grid, 256, fft_smem3_bytes() + 64 * sizeof(float), st, pdl, a);
 #else
-        if (a.K > 1) launch_k(k_search_e1b_multi, grid, 256, e1b_multi_smem_bytes(), st, pdl, a);
-        else launch_k(k_search_e1b, grid, 256, search_e1b_smem_bytes(), st, pdl, a);
+        if (a.K > 1) launch_k(k_search_e1b_multi<S>, grid, 256, e1b_multi_smem_bytes(), st, pdl, a);
+        else launch_k(k_search_e1b<S>, grid, 256, search_e1b_smem_bytes(), st, pdl, a);
 #endif
         return 1;
     }
@@ -2578,16 +2656,16 @@ int launch_search(const SearchArgs &a_in, bool e1b, int sm_count, cudaStream_t s
     launch_k(a.K > 1 ? k_search_l1_ldg<true> : k_search_l1_ldg<false>, grid, 256, fft_smem3t_bytes() + 64 * sizeof(float), st,
              pdl, a);
 #elif defined(ACQ_VARIANT_L1_MULTI_TW)   // the K > 1 form that keeps the stage-B twiddles (not the code run) in tensor memory
-    launch_k(a.K > 1 ? k_search_l1<true> : k_search_l1<false>, grid, 256, search_l1_smem_bytes(), st, pdl, a);
+    launch_k(a.K > 1 ? k_search_l1<true, S> : k_search_l1<false, S>, grid, 256, search_l1_smem_bytes(), st, pdl, a);
 #else
 #ifdef ACQ_VARIANT_L1_MST
     if (kind == kSearchL1Mst) launch_k(k_search_l1_mst, grid, kStThreads, dr_smem_bytes(), st, pdl, a);
     else
 #endif
-    if (a.K > 1) launch_k(k_search_l1_multi, grid, 256, l1_multi_smem_bytes(), st, pdl, a);
+    if (a.K > 1) launch_k(k_search_l1_multi<S>, grid, 256, l1_multi_smem_bytes(), st, pdl, a);
     else if (kind == kSearchL1Cr) {
         search_chunks(a.n_tiles, 2 * sm_count, &a.ck_n16, &a.ck_n4);
-        launch_k(k_search_l1_cr, grid, 256, l1_multi_smem_bytes(), st, pdl, a);
+        launch_k(k_search_l1_cr<S>, grid, 256, l1_multi_smem_bytes(), st, pdl, a);
     }
 #if defined(ACQ_VARIANT_L1_SP)
     else if (kind == kSearchL1Dr) launch_k(k_search_l1_sp, grid, kSpThreads, sp_smem_bytes(), st, pdl, a);
@@ -2597,7 +2675,7 @@ int launch_search(const SearchArgs &a_in, bool e1b, int sm_count, cudaStream_t s
 #if ACQ_DR_MIN_TILES_PER_SM >= 0
     else if (kind == kSearchL1Dr) launch_k(k_search_l1_dr, grid, kStThreads, dr_smem_bytes(), st, pdl, a);
 #endif
-    else launch_k(k_search_l1<false>, grid, 256, search_l1_smem_bytes(), st, pdl, a);
+    else launch_k(k_search_l1<false, S>, grid, 256, search_l1_smem_bytes(), st, pdl, a);
 #endif
     return 1;
 }
@@ -2606,8 +2684,12 @@ int launch_search_e1b_cluster(const SearchArgs &a, int sm_count, cudaStream_t st
 {
     const int n_clusters = search_grid_ctas(a.n_tiles, kSearchE1bCluster, sm_count);
     if (n_clusters <= 0) return 0;
-    launch_k(a.K > 1 ? k_search_e1b_cluster<true> : k_search_e1b_cluster<false>, 4 * n_clusters, 256,
-             search_e1b_cluster_smem_bytes(), st, pdl, a);
+    if (a.dop_center)
+        launch_k(a.K > 1 ? k_search_e1b_cluster<true, AidedSearchArgs> : k_search_e1b_cluster<false, AidedSearchArgs>, 4 * n_clusters,
+                 256, search_e1b_cluster_smem_bytes(), st, pdl, AidedSearchArgs(a));
+    else
+        launch_k(a.K > 1 ? k_search_e1b_cluster<true, SearchArgs> : k_search_e1b_cluster<false, SearchArgs>, 4 * n_clusters, 256,
+                 search_e1b_cluster_smem_bytes(), st, pdl, a);
     return 1;
 }
 
@@ -2637,19 +2719,19 @@ namespace acq {
 #endif
 
 int launch_best_dop(const acq_cell *cells, const int *slot_sat, acq_record *out, int n_cap, int n_slots, int n_dop,
-                    int dop_lo, cudaStream_t st, bool pdl)
+                    PickDop pd, cudaStream_t st, bool pdl)
 {
     const int n_rows = n_cap * n_slots;
-    launch_k(k_best_dop, (n_rows + 3) / 4, 128, 0, st, pdl, cells, slot_sat, out, n_rows, n_slots, n_dop, dop_lo);
+    launch_k(k_best_dop, (n_rows + 3) / 4, 128, 0, st, pdl, cells, slot_sat, out, n_rows, n_slots, n_dop, pd);
     return 1;
 }
 
 int launch_pick_small(const acq_cell *cells, const int *slot_sat, acq_record *out, unsigned *ctas_done, unsigned ctas_total,
-                      unsigned *host_flag, unsigned epoch, int n_rows, int n_slots, int n_dop, int dop_lo, cudaStream_t st,
+                      unsigned *host_flag, unsigned epoch, int n_rows, int n_slots, int n_dop, PickDop pd, cudaStream_t st,
                       bool pdl)
 {
     launch_k(k_pick_small, 1, 1024, 0, st, pdl, cells, slot_sat, out, ctas_done, ctas_total, host_flag, epoch, n_rows, n_slots,
-             n_dop, dop_lo);
+             n_dop, pd);
     return 1;
 }
 

@@ -37,6 +37,21 @@ struct SearchArgs {
     // 1: wait for the preceding grids of the stream (griddepcontrol.wait).  0: this launch directly follows another
     // search launch of the same search, which has already waited (see launch_search).
     int wait_prior;
+    // Aided search (acq_search_aided): dop_center[cap * n_slots + slot] is the raw Doppler centre of that row, which
+    // then searches only n_dop = 2 half_width + 1 indices from window_lo(); d of a tile is the index inside the window.
+    // NULL: every row searches the engine's whole range dop_lo..dop_hi (n_dop indices).
+    const int *dop_center;
+    int half_width, dop_hi;
+    static constexpr bool kAided = false;
+};
+// The arguments of an aided search, a type of their own: the search kernels are templates over the argument type and
+// read the window only in this instantiation, so the full-range kernels compile to the code they had without the
+// feature (k_search_l1_cr sits at 126 registers with its residue loop unrolled: a runtime branch on dop_center moved
+// it to 128 and a spill).
+struct AidedSearchArgs : SearchArgs {
+    static constexpr bool kAided = true;
+    AidedSearchArgs() = default;
+    explicit AidedSearchArgs(const SearchArgs &a) : SearchArgs(a) {}
 };
 
 // s(b, h) of acq_params.code_doppler (same integer arithmetic as the oracle's orc_code_shift)
@@ -45,6 +60,15 @@ __host__ __device__ inline int code_shift(int b, int h, int cd_div)
     const int a = b * h, m = a < 0 ? -a : a;
     const int s = (2 * m + cd_div) / (2 * cd_div);
     return a < 0 ? -s : s;
+}
+
+// First Doppler index of an aided row's window: clamp(center - half_width, dop_lo, dop_hi - 2 half_width), formed
+// without overflow for any int32 centre (2 half_width + 1 <= dop_hi - dop_lo + 1, checked by the host).
+__host__ __device__ inline int window_lo(int center, int half_width, int dop_lo, int dop_hi)
+{
+    const int c_lo = dop_lo + half_width, c_hi = dop_hi - half_width;
+    const int c = center < c_lo ? c_lo : (center > c_hi ? c_hi : center);
+    return c - half_width;
 }
 
 // A search launch decomposes its tile index with 32-bit arithmetic; acq_api.cu refuses larger searches.
@@ -67,17 +91,26 @@ int launch_fwd_fft(const float2 *x2, float2 *out, const float2 *tables, int n_ro
 int launch_build_ext(const float2 *C, float2 *Ep, int n_sats, int Q, int ext_len, int wrap_mode, cudaStream_t st);
 int launch_search(const SearchArgs &a, bool e1b, int sm_count, cudaStream_t st, bool pdl = false);
 int launch_search_e1b_cluster(const SearchArgs &a, int sm_count, cudaStream_t st, bool pdl = false);
+// Doppler indices of the cell rows a best-Doppler pick reads: cell d of row r is index dop_lo + d, or, with
+// dop_center (an aided search), window_lo(dop_center[r], half_width, dop_lo, dop_hi) + d.
+struct PickDop {
+    int dop_lo;
+    const int *dop_center;
+    int half_width, dop_hi;
+};
 int launch_best_dop(const acq_cell *cells, const int *slot_sat, acq_record *out, int n_cap, int n_slots, int n_dop,
-                    int dop_lo, cudaStream_t st, bool pdl = false);
+                    PickDop pd, cudaStream_t st, bool pdl = false);
 // best-Doppler pick of a small search: one CTA that polls the search CTAs' counter (see k_pick_small).  host_flag
 // (mapped pinned memory, or NULL) selects the polled-host form: `out` is then an acq_record_tagged array in mapped
 // memory (tags = epoch), and *host_flag is written only to report a failure (0xffffffff)
 int launch_pick_small(const acq_cell *cells, const int *slot_sat, acq_record *out, unsigned *ctas_done, unsigned ctas_total,
-                      unsigned *host_flag, unsigned epoch, int n_rows, int n_slots, int n_dop, int dop_lo, cudaStream_t st,
+                      unsigned *host_flag, unsigned epoch, int n_rows, int n_slots, int n_dop, PickDop pd, cudaStream_t st,
                       bool pdl = false);
 // CTAs of a search launch that store cells (what SearchArgs::ctas_total sums over the launches of one search)
 enum { kSearchL1 = 0, kSearchE1b = 1, kSearchE1bCluster = 2, kSearchL1Multi = 3, kSearchL1Dr = 4, kSearchL1Mst = 5, kSearchL1Cr = 6 };
 int search_kind_l1(int K, int half_bin, long long n_tiles, int sm_count);   // which C/A search kernel (and so which grid) a search uses
+// an aided search runs only on the product's search kernels: false where this library would pick another form
+bool search_aided_supported(int K, int half_bin, long long tiles_l1, long long tiles_e1b, int sm_count);
 constexpr int kPickSmallRowsMax = 256;  // rows k_pick_small stages in shared memory
 // A record as k_pick_small hands it to a POLLING host (mapped pinned memory): two 16-byte halves, each carrying the
 // search's epoch in its last word.  Each half arrives by one 16-byte store, so a host that sees the epoch in a half has

@@ -181,6 +181,29 @@ class AcqEngine:
         sp, n_sel, keep = self._sel(sel)
         _check(self._L.acq_search_device(self._h, packed_dev, n_cap, sp, n_sel, out_dev, stream_ptr), self._L)
 
+    # ---- aided search: each (capture, satellite) row over its own Doppler window of W = 2 * half_width + 1 indices
+    def search_aided(self, packed, dop_center, half_width, sel=None, want_grid=False):
+        """acq_search_aided.  dop_center: int [n_cap, n_sel] (or anything of that size), Doppler indices in the engine's
+        units; row r searches [lo_r, lo_r + W - 1], lo_r = clamp(center - half_width, dop_lo, dop_hi - 2 half_width).
+        Returns records [n_cap, n_sel] (dop absolute) and, if asked, the window cells [n_cap, n_sel, W]."""
+        a, n_cap = self._packed(packed)
+        sp, n_sel, keep = self._sel(sel)
+        c = np.ascontiguousarray(dop_center, np.int32).reshape(-1)
+        if c.size != n_cap * n_sel:
+            raise ValueError("dop_center must hold n_captures * n_sel = %d centres (got %d)" % (n_cap * n_sel, c.size))
+        out = np.zeros((n_cap, n_sel), RECORD_DTYPE)
+        grid = np.zeros((n_cap, n_sel, 2 * max(int(half_width), 0) + 1), CELL_DTYPE) if want_grid else None
+        _check(self._L.acq_search_aided(self._h, a.ctypes.data, n_cap, sp, n_sel, c.ctypes.data, int(half_width),
+                                        out.ctypes.data, grid.ctypes.data if want_grid else None), self._L)
+        return (out, grid) if want_grid else out
+
+    def search_aided_device(self, packed_dev, dop_center_dev, half_width, out_dev, n_cap, sel=None, stream_ptr=None):
+        """acq_search_aided_device: packed_dev / dop_center_dev (int32, n_cap * n_sel) / out_dev are device pointers
+        (ints).  Enqueues on stream_ptr (None = engine stream); the centres are read by the kernels."""
+        sp, n_sel, keep = self._sel(sel)
+        _check(self._L.acq_search_aided_device(self._h, packed_dev, n_cap, sp, n_sel, dop_center_dev, int(half_width), out_dev,
+                                               stream_ptr), self._L)
+
     def refine(self, records):
         """acq_refine: hand-off refinement of the records of the most recent search()/wait() -- FINE_DTYPE array of
         the same shape (Doppler in Hz from a three-bin interpolation, code phase in FS samples from early/late)."""

@@ -59,31 +59,50 @@ class _Farm:
 
 class CaptureFarm(_Farm):
     """n_captures independent captures (each `capture_bytes` long) sharded over the ranks; the whole table is searched on
-    each.  Records come back as [n_captures, n_sel] on every rank."""
+    each.  Records come back as [n_captures, n_sel] on every rank.
 
-    def __init__(self, engine, n_captures, capture_bytes, n_sel, dist=None, device=None):
+    half_width (optional): an aided farm -- every (capture, satellite) row searches only the 2 * half_width + 1 Doppler
+    indices around its own centre (acq_search_aided_device); load() then takes the centres with the captures."""
+
+    def __init__(self, engine, n_captures, capture_bytes, n_sel, dist=None, device=None, half_width=None):
         super().__init__(engine, n_captures, dist, device)
         self.capture_bytes, self.n_sel = capture_bytes, n_sel
+        self.half_width = half_width
         self.h_in = self._empty(self.n_local * capture_bytes, device="cpu", pin=self.pin)
         self.d_in = self._empty(self.n_local * capture_bytes)
+        if half_width is not None:   # this rank's Doppler centres, int32 [n_local, n_sel], kept in HBM with the captures
+            self.d_center = self.torch.zeros(max(self.n_local * n_sel, 1), dtype=self.torch.int32, device=self.device)
         self.d_rec = self._empty(self.max_local * n_sel * REC)           # local records, padded to the largest shard
         self.d_all = self._empty(self.world * self.max_local * n_sel * REC) if self.world > 1 else self.d_rec
         self.h_all = self._empty(self.d_all.numel(), device="cpu", pin=self.pin)
 
-    def load(self, captures):
+    def load(self, captures, dop_center=None):
         """captures: uint8 numpy [n_captures, capture_bytes] (every rank may pass the whole set) or just this rank's
-        [n_local, capture_bytes] slice.  Stages the local slice in pinned memory and in HBM."""
+        [n_local, capture_bytes] slice.  Stages the local slice in pinned memory and in HBM.  dop_center (aided farm
+        only, required there): int [n_captures, n_sel] or this rank's [n_local, n_sel], sharded like the captures."""
         a = np.ascontiguousarray(captures, np.uint8).reshape(-1, self.capture_bytes)
         if a.shape[0] == self.n_units:
             a = a[self.lo:self.hi]
         assert a.shape[0] == self.n_local, (a.shape, self.n_local)
+        if (dop_center is None) != (self.half_width is None):
+            raise ValueError("dop_center is given exactly when the farm was created with half_width")
+        if dop_center is not None:
+            c = np.ascontiguousarray(dop_center, np.int32).reshape(-1, self.n_sel)
+            if c.shape[0] == self.n_units:
+                c = c[self.lo:self.hi]
+            assert c.shape[0] == self.n_local, (c.shape, self.n_local)
+            if self.n_local:
+                self.d_center[:c.size].copy_(self.torch.from_numpy(c.reshape(-1)))
         if self.n_local:
             self.h_in[:a.size].copy_(self.torch.from_numpy(a.reshape(-1)))
             self.d_in.copy_(self.h_in)
 
     def search_resident(self):
-        """Captures already in HBM (load()); leaves the gathered records in self.d_all.  Asynchronous."""
-        if self.n_local:
+        """Captures (and, aided, centres) already in HBM (load()); leaves the gathered records in self.d_all.  Asynchronous."""
+        if self.n_local and self.half_width is not None:
+            self.eng.search_aided_device(self.d_in.data_ptr(), self.d_center.data_ptr(), self.half_width, self.d_rec.data_ptr(),
+                                         self.n_local, stream_ptr=self._stream_ptr())
+        elif self.n_local:
             self.eng.search_device(self.d_in.data_ptr(), self.d_rec.data_ptr(), self.n_local, stream_ptr=self._stream_ptr())
         self._gather()
         return self.d_all

@@ -187,6 +187,21 @@ int acq_search_grid(acq_engine *e, const uint8_t *packed, int n_captures, const 
 int acq_search_device(acq_engine *e, const uint8_t *packed_dev, int n_captures, const int32_t *sel, int n_sel,
                       acq_record *out_dev, void *stream);
 
+/* Aided search: row r = c*n_sel + s (capture c, selected satellite s) searches only the W = 2*half_width+1 Doppler
+ * indices [lo_r, lo_r + W - 1], where lo_r = clamp(dop_center[r] - half_width, dop_lo, dop_hi - 2*half_width).
+ * Indices are in the engine's units (half-bins when half_bin = 1).  A centre outside the range is clamped, so every
+ * row searches a full-width window.  W must not exceed n_dop.  The record is Correlate()'s rule over the window
+ * (largest snr, lowest Doppler index on ties, snr > 0), and its dop is the absolute index.
+ *   dop_center : HOST, n_captures * n_sel int32 (n_sel = table size when sel is NULL)
+ *   grid       : HOST or NULL; n_captures * n_sel * W cells, cell j of row r = Doppler index lo_r + j
+ * Synchronous, like acq_search.  acq_refine accepts its records afterwards. */
+int acq_search_aided(acq_engine *e, const uint8_t *packed, int n_captures, const int32_t *sel, int n_sel,
+                     const int32_t *dop_center, int half_width, acq_record *out, acq_cell *grid);
+/* The device-resident form.  Ordering and validity rules are those of acq_search_device; dop_center_dev is a
+ * DEVICE array read by the kernels, so it must stay valid until `stream` has passed the search. */
+int acq_search_aided_device(acq_engine *e, const uint8_t *packed_dev, int n_captures, const int32_t *sel, int n_sel,
+                            const int32_t *dop_center_dev, int half_width, acq_record *out_dev, void *stream);
+
 /* Asynchronous pair over host buffers (the reference yields to other tasks while it computes,
  * gps/search.cpp:479-491): submit enqueues copy-in, search and copy-out on the engine's stream;
  * acq_wait blocks until done, acq_poll returns 1 when done, 0 while running.  The host buffers
@@ -197,7 +212,7 @@ int acq_poll(acq_engine *e);
 int acq_wait(acq_engine *e);
 
 /* Acquisition refinement for the hand-off to tracking.  `rec` (HOST) are the n_captures * n_sel records of the MOST
- * RECENT host-path search on this engine (acq_search, acq_search_grid, or acq_submit after acq_wait), in the same
+ * RECENT host-path search on this engine (acq_search, acq_search_grid, acq_search_aided, or acq_submit after acq_wait), in the same
  * order; the capture spectra that search left on the device are reused, so no capture is passed again.  For each
  * record the correlation is evaluated at the five points (dop-1..dop+1 at lag; lag-1..lag+1 at dop), a three-bin
  * Doppler interpolation and an early/late code-phase interpolation are formed, and `out` (HOST, same count) is
