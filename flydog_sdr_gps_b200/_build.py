@@ -51,32 +51,18 @@ def build(force=False, verbose=False, defines=(), out=None):
     return lib
 
 
-# Experiment variants (A/B forms of the kernels and launch policy).  They are separate libraries: the product
-# library contains none of this code and reads no environment variable.
+# Experiment variants: the reference sides of the kernel-equivalence tests, and instrumentation.  They are separate
+# libraries: the product library contains none of this code and reads no environment variable.
 VARIANTS = {
     "l1_multi_tw": ["ACQ_VARIANT_L1_MULTI_TW"],  # K > 1 C/A search with the twiddles (not the code run) in tensor memory
-    "l1_mst": ["ACQ_VARIANT_L1_MST"],        # K > 1 C/A search in the two-team form with staging warps (measured: no gain)
     "l1_cta": ["ACQ_FORCE_L1_CTA=1"],        # K = 1 C/A search always by k_search_l1<false> (two CTAs per SM, thread 0 stages)
-    "l1_dr_all": ["ACQ_DR_MIN_TILES_PER_SM=0"],  # K = 1 full-bin C/A search by k_search_l1_dr at every size (the product: never)
-    "l1_dr12": ["ACQ_DR_MIN_TILES_PER_SM=12"],   # ... from 12 tiles per SM (the product for most of round 2)
-    "l1_nocr": ["ACQ_L1_CR=0"],              # full-bin K = 1 searches on k_search_l1<false> at every size (the product: k_search_l1_cr where tiles are claimed)
-    "l1_sp": ["ACQ_VARIANT_L1_SP"],          # K = 1 C/A search software-pipelined across sub-FFTs, one CTA per SM (measured: -3.7 %)
-    "l1_st": ["ACQ_VARIANT_L1_ST"],          # staging warps only (capture residue still staged per sub-FFT): +1.9 %
-    "l1_ldg": ["ACQ_VARIANT_L1_LDG"],        # C/A search, operands straight from L2
-    "l1_x3": ["ACQ_VARIANT_L1_X3"],
-    "l1_x3t": ["ACQ_VARIANT_L1_X3", "ACQ_X3_TMA_D"],  # ... with the capture residue TMA-staged, the code run from L2 issued early          # C/A search at three CTAs per SM (accumulators in tensor memory)
     "e1b_ldg": ["ACQ_VARIANT_E1B_LDG", "ACQ_FORCE_E1B_KERNEL=1"],  # one-CTA E1B search, operands straight from L2
     "e1b_cta": ["ACQ_FORCE_E1B_KERNEL=1"],   # always the one-CTA E1B form
     "e1b_cluster": ["ACQ_FORCE_E1B_KERNEL=2"],  # always the cluster/DSMEM E1B form
     "trace": ["ACQ_TRACE"],                  # %globaltimer stamps per CTA (tools/trace_timeline.py)
-    "pdl0": ["ACQ_FORCE_PDL=0"],
-    "pdl1": ["ACQ_FORCE_PDL=1"],
-    "zcin": ["ACQ_ZC_INPUT=1"],              # front end reads small captures from mapped pinned memory (no H2D copy node)
     "static_tiles": ["ACQ_DYN_MIN_ROUNDS=1000000000"],  # strided search kernels always on the static stride (the product: tiles claimed from a counter from 6 rounds up)
     "dyn_tiles": ["ACQ_DYN_MIN_ROUNDS=0"],    # ... always claiming
-    "carve0": ["ACQ_CARVEOUT_MAX=0"],        # shared-memory carveout left to the driver per kernel (the product: max shared for the whole chain)
     "argin0": ["ACQ_ARG_INPUT=0"],           # single-block captures through the staging buffer + copy node (the product: kernel argument)
-    "devrec": ["ACQ_HOST_RECORDS=0"],        # records through device memory + copy, stream wait (no mapped memory, no polling)
 }
 
 
@@ -86,7 +72,7 @@ def variant_path(name):
 
 def build_variant(name, force=False):
     path = variant_path(name)
-    deps = [os.path.join(CSRC, f) for f in CU_SOURCES + CPP_SOURCES + HEADERS + ["acq_variants.cuh"]]
+    deps = [os.path.join(CSRC, f) for f in CU_SOURCES + CPP_SOURCES + HEADERS]
     fresh = os.path.exists(path) and all(os.path.getmtime(d) <= os.path.getmtime(path) for d in deps if os.path.exists(d))
     if fresh and not force:
         return path

@@ -119,7 +119,7 @@ struct acq_engine {
     unsigned epoch = 0;                // search counter: value of the completion word
     // host path: pinned staging of small captures; records and the completion word in mapped pinned memory,
     // written by the search kernels themselves
-    uint8_t *h_packed = nullptr, *dh_packed = nullptr;  // host / device address of the (mapped) staging buffer
+    uint8_t *h_packed = nullptr;
     size_t cap_h_packed = 0;
     acq_record *h_records = nullptr, *dh_records = nullptr;  // host / device address of the same mapped buffer
     size_t cap_h_records = 0;
@@ -153,22 +153,9 @@ using namespace acq;
 
 // Build-time switches of the experiment variants (tools/build_variants.py); the product library defines none of
 // them and reads no environment variable.
-//   ACQ_FORCE_PDL=0|1        programmatic dependent launch off / on (default: on for every search)
 //   ACQ_FORCE_E1B_KERNEL=1|2 one-CTA / cluster form of the E1B search regardless of the tile count
-//   ACQ_HOST_RECORDS=0       records through device memory + copy even for small searches
-#ifndef ACQ_FORCE_PDL
-#define ACQ_FORCE_PDL -1
-#endif
 #ifndef ACQ_FORCE_E1B_KERNEL
 #define ACQ_FORCE_E1B_KERNEL 0
-#endif
-#ifndef ACQ_HOST_RECORDS
-#define ACQ_HOST_RECORDS 1
-#endif
-//   ACQ_ZC_INPUT=0|1         small captures: host->device copy node (0) or read by the front end straight from the
-//                            mapped pinned staging buffer (1: its bulk copies then cross PCIe, no copy node)
-#ifndef ACQ_ZC_INPUT
-#define ACQ_ZC_INPUT 0
 #endif
 //   ACQ_ARG_INPUT=1|0        a search of ONE 1-bit block: the capture travels as the front end's kernel argument (1) or by
 //                            the staging buffer and a copy node like every other search (0, variant "argin0")
@@ -179,7 +166,6 @@ using namespace acq;
 // make cudaMemcpyAsync synchronous), the kernels write the records straight into mapped pinned memory, and the host
 // polls a completion word there instead of waiting for the stream.  Above these sizes: plain copies and a stream wait.
 constexpr size_t kStagePackedMax = 256u << 10;  // bytes
-constexpr size_t kZeroCopyMax = 64u << 10;      // bytes the front end may fetch over PCIe itself (ACQ_ZC_INPUT)
 constexpr int kHostRecordRowsMax = 256;          // records (24 B each: single PCIe writes from the SMs)
 // Up to this many (capture, sat) rows the best-Doppler pick is one CTA that polls the search CTAs' completion counter
 // (k_pick_small: no wait for the grids to drain; a few microseconds at most); above, k_best_dop follows the search the
@@ -277,13 +263,12 @@ int ensure_scratch(acq_engine *e, int n_captures, int n_slots, bool host_path, i
     if (bytes <= kStagePackedMax && bytes > e->cap_h_packed) {
         if ((rc = drain(e))) return rc;
         if (e->h_packed) CU(cudaFreeHost(e->h_packed));
-        e->h_packed = e->dh_packed = nullptr;
+        e->h_packed = nullptr;
         e->cap_h_packed = 0;
-        CU(cudaHostAlloc(&e->h_packed, bytes, cudaHostAllocMapped));
-        CU(cudaHostGetDevicePointer(&e->dh_packed, e->h_packed, 0));
+        CU(cudaHostAlloc(&e->h_packed, bytes, cudaHostAllocDefault));
         e->cap_h_packed = bytes;
     }
-    if (ACQ_HOST_RECORDS && rows <= (size_t)kHostRecordRowsMax) {
+    if (rows <= (size_t)kHostRecordRowsMax) {
         if (rows > e->cap_h_records) {
             if ((rc = drain(e))) return rc;
             if (e->h_records) CU(cudaFreeHost(e->h_records));
@@ -396,7 +381,7 @@ int enqueue_search(acq_engine *e, const uint8_t *packed_dev, int n_captures, acq
     // 3.437 ms, E1B with K = 4: 0.709 -> 0.702 ms, a 128-capture farm 5.97 -> 5.95 ms).  Before that it cost long searches
     // 3 %: an SM had to empty before it could change its split, so the search CTAs of the early-launched grid were placed
     // unevenly.  Event records between the kernels (profiling) would serialise them anyway.
-    const bool pdl = !prof && ACQ_FORCE_PDL != 0;
+    const bool pdl = !prof;
     if (++e->epoch >= 0xfffffffeu) e->epoch = 1;
     if (prof) CU(cudaEventRecord(e->prof[0], st));
     if (packed_host_arg) {   // one 1-bit block still in host memory: it rides in the front end's launch
@@ -436,7 +421,7 @@ int enqueue_search(acq_engine *e, const uint8_t *packed_dev, int n_captures, acq
     // one-CTA-per-tile forms (k_search_e1b, k_search_e1b_multi for non-coherent sums) have ~2.9x the throughput.
     const bool e1b_cluster = ACQ_FORCE_E1B_KERNEL == 2 || (ACQ_FORCE_E1B_KERNEL == 0 && tiles_e1b <= e->sm_count / 4);
     a.ctas_done = e->d_ctas_done;
-    a.ctas_total = fold ? (unsigned)(search_grid_ctas(tiles_l1, search_kind_l1(K, e->prm.half_bin, tiles_l1, e->sm_count), e->sm_count) +
+    a.ctas_total = fold ? (unsigned)(search_grid_ctas(tiles_l1, search_kind_l1(K, e->prm.half_bin), e->sm_count) +
                                      search_grid_ctas(tiles_e1b, e1b_cluster ? kSearchE1bCluster : kSearchE1b, e->sm_count))
                         : 0u;
     a.wait_prior = 1;
@@ -509,17 +494,6 @@ int check_aided_args(acq_engine *e, const int32_t *dop_center, int half_width)
     return ACQ_OK;
 }
 
-// after set_selection: the aided search kernels are instantiations of the product's; the experiment kernels of the variant
-// libraries (k_search_l1_dr and its team forms, which step the Doppler index themselves, and the other A/B forms) know
-// nothing of windows, so an aided search that would run on them is refused rather than computed wrong
-int check_aided_kernels(acq_engine *e, int n_captures, int n_dop)
-{
-    if (!search_aided_supported(e->prm.k_noncoh, e->prm.half_bin, (long long)n_captures * e->n_l1 * n_dop,
-                                (long long)n_captures * e->n_e1b * n_dop, e->sm_count))
-        return fail(ACQ_ERR_UNSUPPORTED, "aided search: this library runs the search of that shape on a kernel without Doppler windows");
-    return ACQ_OK;
-}
-
 // Wait for a host-polled search and collect its records: k_pick_small writes every record into mapped memory as two
 // 16-byte halves that each end in the search's epoch (acq_record_tagged), so a half whose tag matches has arrived whole.
 // The stream is queried now and then so that a failed launch cannot hang the caller; the mapped word *h_flag is only
@@ -566,7 +540,6 @@ int search_host(acq_engine *e, const uint8_t *packed, int n_captures, const int3
     const int n_dop = row_dops(e, center, half_width);
     if ((rc = set_selection(e, sel, n_sel))) return rc;
     if ((rc = check_tile_count(e, n_captures, n_dop))) return rc;
-    if (center && (rc = check_aided_kernels(e, n_captures, n_dop))) return rc;
     if ((rc = ensure_scratch(e, n_captures, e->n_slots, true, n_dop))) return rc;
     const size_t bytes = (size_t)n_captures * e->prm.k_noncoh * e->block_bytes;
     const size_t rows = (size_t)n_captures * e->n_slots;
@@ -581,7 +554,7 @@ int search_host(acq_engine *e, const uint8_t *packed, int n_captures, const int3
             e->cap_h_center = rows;
         }
     }
-    const bool host_records = ACQ_HOST_RECORDS && rows <= (size_t)kHostRecordRowsMax;
+    const bool host_records = rows <= (size_t)kHostRecordRowsMax;
     const long long tiles_total = (long long)rows * n_dop * e->prm.k_noncoh;
     const bool poll = host_records && sync && !grid && !e->profiling && tiles_total <= 64LL * e->sm_count;
     // The reference's own search -- one 1-bit block (gps/search.cpp:389-411) -- hands its 8 KiB to the front end as a
@@ -589,20 +562,18 @@ int search_host(acq_engine *e, const uint8_t *packed, int n_captures, const int3
     const bool as_arg = ACQ_ARG_INPUT && n_captures == 1 && e->prm.k_noncoh == 1 && e->sample_bits == 1 &&
                         bytes == (size_t)ACQ_BLOCK_BYTES;
     const uint8_t *src = packed;
-    const uint8_t *packed_dev = e->d_packed;
     if (!as_arg) {
         if (bytes <= kStagePackedMax) {
             memcpy(e->h_packed, packed, bytes);
             src = e->h_packed;
         }
-        if (ACQ_ZC_INPUT && src == e->h_packed && bytes <= kZeroCopyMax) packed_dev = e->dh_packed;
-        else CU(cudaMemcpyAsync(e->d_packed, src, bytes, cudaMemcpyHostToDevice, e->stream));
+        CU(cudaMemcpyAsync(e->d_packed, src, bytes, cudaMemcpyHostToDevice, e->stream));
     }
     if (center) {   // from pinned memory: an asynchronous copy node ahead of the front end, even when the capture rides as an argument
         memcpy(e->h_center, center, rows * sizeof(int32_t));
         CU(cudaMemcpyAsync(e->d_center, e->h_center, rows * sizeof(int32_t), cudaMemcpyHostToDevice, e->stream));
     }
-    if ((rc = enqueue_search(e, packed_dev, n_captures, host_records ? e->dh_records : e->d_records,
+    if ((rc = enqueue_search(e, e->d_packed, n_captures, host_records ? e->dh_records : e->d_records,
                              poll ? e->dh_flag : nullptr, e->stream, as_arg ? packed : nullptr, center ? e->d_center : nullptr,
                              half_width)))
         return rc;
@@ -650,7 +621,6 @@ int search_device(acq_engine *e, const uint8_t *packed_dev, int n_captures, cons
     const int n_dop = row_dops(e, center_dev, half_width);
     if ((rc = set_selection(e, sel, n_sel))) return rc;
     if ((rc = check_tile_count(e, n_captures, n_dop))) return rc;
-    if (center_dev && (rc = check_aided_kernels(e, n_captures, n_dop))) return rc;
     if ((rc = ensure_scratch(e, n_captures, e->n_slots, false, n_dop))) return rc;
     cudaStream_t st = stream ? (cudaStream_t)stream : e->stream;
     if ((rc = enqueue_search(e, packed_dev, n_captures, out_dev, nullptr, st, nullptr, center_dev, half_width))) return rc;
@@ -1086,10 +1056,10 @@ int acq_plan_launch(int k_noncoh, int half_bin, int e1b, int64_t n_tiles, int sm
     memset(out, 0, sizeof *out);
     int kind;
     if (e1b) kind = (ACQ_FORCE_E1B_KERNEL == 2 || (ACQ_FORCE_E1B_KERNEL == 0 && n_tiles <= sm_count / 4)) ? acq::kSearchE1bCluster : acq::kSearchE1b;
-    else kind = acq::search_kind_l1(k_noncoh, half_bin, n_tiles, sm_count);
+    else kind = acq::search_kind_l1(k_noncoh, half_bin);
     out->kernel = kind;
     out->grid = acq::search_grid_ctas(n_tiles, kind, sm_count);
-    out->claims = kind != acq::kSearchE1bCluster && kind != acq::kSearchL1Dr && acq::search_claims_tiles(n_tiles, out->grid);
+    out->claims = kind != acq::kSearchE1bCluster && acq::search_claims_tiles(n_tiles, out->grid);
     out->n_chunks = n_tiles;
     acq::search_chunk_lengths(&out->chunk_big, &out->chunk_mid);
     if (kind == acq::kSearchL1Cr) {

@@ -87,9 +87,6 @@ __device__ __forceinline__ void radix4_inv(float2 &a, float2 &b, float2 &c, floa
 // Input x[a] in natural order.  Output X[n] is left at register index  r16(n) = (n >> 2) | ((n & 3) << 2).
 __host__ __device__ constexpr int r16(int n) { return (n >> 2) | ((n & 3) << 2); }
 
-#ifndef ACQ_R16_FUSED
-#define ACQ_R16_FUSED 1
-#endif
 __device__ __forceinline__ void radix16_inv(float2 (&x)[16])
 {
     constexpr float C1 = 0.92387953251128675613f;  // cos(pi/8)
@@ -98,7 +95,6 @@ __device__ __forceinline__ void radix16_inv(float2 (&x)[16])
     // layer 1: for each a0, radix-4 over a = a0 + 4*a1  ->  u[a0][nl] at index a0 + 4*nl
 #pragma unroll
     for (int a0 = 0; a0 < 4; a0++) radix4_inv(x[a0], x[a0 + 4], x[a0 + 8], x[a0 + 12]);
-#if ACQ_R16_FUSED
     // Twiddles u[a0][nl] *= W16^{a0*nl} folded into layer 2 where they are (+-1 +- j)/sqrt2: the 1/sqrt2 rides
     // on the fused multiply-add of the following butterfly (4 packed instructions fewer than twiddle-then-add).
     // nl = 0: no twiddles
@@ -132,21 +128,6 @@ __device__ __forceinline__ void radix16_inv(float2 (&x)[16])
         x[14] = csub(apc, bpd);
         x[15] = csub_jb(amc, bmd);
     }
-#else
-    // twiddle u[a0][nl] *= W16^{a0*nl}
-    x[5] = cmul(x[5], make_float2(C1, S1));                           // W16^1
-    x[9] = __fmul2_rn(cadd(x[9], jmul(x[9])), bc(R2));               // W16^2 = (1+j)/sqrt2
-    x[13] = cmul(x[13], make_float2(S1, C1));                         // W16^3
-    x[6] = __fmul2_rn(cadd(x[6], jmul(x[6])), bc(R2));               // W16^2
-    x[10] = jmul(x[10]);                                              // W16^4 = j
-    x[14] = __fmul2_rn(csub(jmul(x[14]), x[14]), bc(R2));            // W16^6 = (-1+j)/sqrt2
-    x[7] = cmul(x[7], make_float2(S1, C1));                           // W16^3
-    x[11] = __fmul2_rn(csub(jmul(x[11]), x[11]), bc(R2));            // W16^6
-    x[15] = cmul(x[15], make_float2(-C1, -S1));                       // W16^9
-    // layer 2: for each nl, radix-4 over a0  ->  X[nl + 4*nh] at index nh + 4*nl
-#pragma unroll
-    for (int nl = 0; nl < 4; nl++) radix4_inv(x[4 * nl], x[4 * nl + 1], x[4 * nl + 2], x[4 * nl + 3]);
-#endif
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -338,76 +319,7 @@ __device__ __forceinline__ void subfft4096_inv3(float2 (&x)[16], const int k2, c
     radix16_inv(x);
 }
 
-// Same sub-FFT with the stage-B twiddles W1024^{(4c+k2)*n1} held in tensor memory instead of shared memory:
-// each thread keeps its own 4 x 15 values (c = t & 15) in 4 x 32 columns at `tw_taddr` (filled once per
-// kernel by subfft3_park_twiddles).  Takes 30 of the 240 L1/shared wavefronts per warp and sub-FFT off the
-// busiest pipe of the search kernel at no arithmetic cost.
-struct FftSmem3T {
-    float2 *S1;  // [2][4096]
-    float2 *S2;  // [16 half-warps][16*17]
-};
-__host__ __device__ constexpr size_t fft_smem3t_bytes() { return sizeof(float2) * (size_t)(2 * kS1Elems + 16 * kS2TileElems); }
-__device__ __forceinline__ FftSmem3T fft_smem3t_carve(unsigned char *base)
-{
-    FftSmem3T s;
-    s.S1 = reinterpret_cast<float2 *>(base);
-    s.S2 = s.S1 + 2 * kS1Elems;
-    return s;
-}
-constexpr int kTwCols = 4 * 32;  // TMEM columns of one thread's stage-B twiddles
-
-// tables: global T2 [4][15][16]; writes this thread's values to TMEM columns [32*k2 + 2*(n1-1), +2)
-__device__ __forceinline__ void subfft3_park_twiddles(const float2 *__restrict__ tables, uint32_t tw_taddr, int t)
-{
-#pragma unroll
-    for (int k2 = 0; k2 < 4; k2++) {
-        float2 v[8];
-#pragma unroll
-        for (int h = 0; h < 2; h++) {
-#pragma unroll
-            for (int i = 0; i < 8; i++) {
-                const int n1 = 8 * h + i + 1;
-                v[i] = (n1 < 16) ? __ldg(tables + (k2 * 15 + (n1 - 1)) * 16 + (t & 15)) : make_float2(0.0f, 0.0f);
-            }
-            tmem_st8(tw_taddr + 32 * k2 + 16 * h, v);
-        }
-    }
-    tmem_wait_st();
-}
-
-__device__ __forceinline__ void subfft4096_inv3t(float2 (&x)[16], const int k2, const float2 b, const int buf,
-                                                 const FftSmem3T &s, const int t, const uint32_t tw_taddr)
-{
-    radix16_inv(x);
-    stage_a_store<256>(x, b, s.S1 + buf * kS1Elems + t);
-    float2 tw[8], tw2[8];
-    tmem_ld8(tw_taddr + 32 * k2, tw);        // n1 = 1..8, in flight across the barrier
-    tmem_ld8(tw_taddr + 32 * k2 + 16, tw2);  // n1 = 9..15 (+ one unused)
-    __syncthreads();
-    {
-        const float2 *src = s.S1 + buf * kS1Elems + (t & ~15) * 16 + (t & 15);
-#pragma unroll
-        for (int bb = 0; bb < 16; bb++) x[bb] = src[16 * bb];
-    }
-    radix16_inv(x);
-    tmem_wait_ld();
-    float2 *tile = s.S2 + (t >> 4) * kS2TileElems;
-    {
-        float2 *dst = tile + (t & 15);  // element (n1, c) at n1*17 + c
-        dst[0] = x[r16(0)];
-#pragma unroll
-        for (int i = 0; i < 8; i++) dst[(i + 1) * 17] = cmul(x[r16(i + 1)], tw[i]);
-#pragma unroll
-        for (int i = 0; i < 7; i++) dst[(i + 9) * 17] = cmul(x[r16(i + 9)], tw2[i]);
-    }
-    __syncwarp();
-    {
-        const float2 *src = tile + 17 * (t & 15);
-#pragma unroll
-        for (int c = 0; c < 16; c++) x[c] = src[c];
-    }
-    radix16_inv(x);
-}
+constexpr int kTwCols = 4 * 32;  // TMEM columns of one thread's stage-B twiddles (subfft4_park_twiddles)
 
 // ---------------------------------------------------------------------------------------------
 // Operand-prefetching form of the sub-FFT (used by k_search_l1).
@@ -426,9 +338,6 @@ __device__ __forceinline__ void subfft4096_inv3t(float2 (&x)[16], const int k2, 
 // Shared memory per CTA: 2 x 34 KiB (S1) + 32 KiB + 16 B (E) + one mbarrier.
 // ---------------------------------------------------------------------------------------------
 constexpr int kEBufElems = kSub + 2;
-#ifndef ACQ_SWZ128
-#define ACQ_SWZ128 1   // E1B kernel (subfft4096_inv4s); the C/A kernel takes it as a template parameter
-#endif
 constexpr int kRowElems = 256;                // exchange row; the B->C tile of a half-warp lives in it, XOR-swizzled
 constexpr int kS1pElems = 16 * kRowElems;     // one half of the exchange buffer
 struct FftSmem4 {
@@ -453,17 +362,6 @@ __device__ __forceinline__ FftSmem4 fft_smem4_carve(unsigned char *base)
 // every thread of every kernel in the chain calls it before touching search data, so completion is transitive.
 // Both are no-ops for a kernel launched without the attribute.
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-// experiment switches (tools/build_variants.py): drop the trigger of one kernel class
-#ifdef ACQ_PDL_NO_TRIGGER_SEARCH
-__device__ __forceinline__ void pdl_trigger_search() {}
-#else
-__device__ __forceinline__ void pdl_trigger_search() { pdl_launch_dependents(); }
-#endif
-#ifdef ACQ_PDL_NO_TRIGGER_FFT
-__device__ __forceinline__ void pdl_trigger_fft() {}
-#else
-__device__ __forceinline__ void pdl_trigger_fft() { pdl_launch_dependents(); }
-#endif
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 
 // Timeline instrumentation of the experiment variant "trace" (tools/trace_timeline.py): thread 0 of every CTA stamps
@@ -519,8 +417,9 @@ __device__ __forceinline__ void tma_load_1d(uint32_t dst, const void *src, uint3
 }
 __device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 
-// Twiddle parking for subfft4096_inv4: as subfft3_park_twiddles, plus the next residue's stage-A base in the
-// sixteenth slot.  tables: T2 [4][15][16], then bases [4][256].
+// Twiddle parking for subfft4096_inv4: this thread's stage-B twiddles (c = t & 15) to TMEM columns
+// [32*k2 + 2*(n1-1), +2), plus the next residue's stage-A base in the sixteenth slot.  tables: T2 [4][15][16], then
+// bases [4][256].
 __device__ __forceinline__ void subfft4_park_twiddles(const float2 *__restrict__ tables, uint32_t tw_taddr, int t)
 {
 #pragma unroll
@@ -544,14 +443,12 @@ __device__ __forceinline__ void subfft4_park_twiddles(const float2 *__restrict__
 //        next residue's base);  S1b = this sub-FFT's half of S1
 //   post_barrier(): called by every thread right after the CTA barrier (warp 0 issues the next TMA there)
 //   out: x[r16(n2)] = stage-C output for lag lag_of3(t, n2), before the W64^{k2*n2} factor
-// SWZ128: B->C tile swizzled in 16-byte chunks and read with 128-bit loads (below).  Measured (variants A/B, same
-// box): +1.2 % on the K > 1 kernel (cfg2), +0.9 % on E1B (cfg3); on the K = 1 kernel -0.8 % with the rolled residue
-// loop, +1.5 % (cfg5) once that loop is unrolled by two -- every product kernel uses it now, the 8-byte swizzle
-// stays as the template's other branch.
-//   team_barrier(): the barrier of the 256 threads of this sub-FFT (the CTA barrier, or a named barrier of a team)
-template <bool SWZ128, class TeamBarrier, class PostBarrier>
+// The B->C tile is swizzled in 16-byte chunks and read with 128-bit loads (below).  Measured against an 8-byte
+// swizzle read with 64-bit loads (same box): +1.2 % on the K > 1 kernel (cfg2), +0.9 % on E1B (cfg3); on the K = 1
+// kernel -0.8 % with the rolled residue loop, +1.5 % (cfg5) once that loop is unrolled by two.
+template <class PostBarrier>
 __device__ __forceinline__ void subfft4096_inv4(float2 (&x)[16], const int k2, float2 &b, float2 *S1b, const int t,
-                                                const uint32_t tw_taddr, TeamBarrier &&team_barrier, PostBarrier &&post_barrier)
+                                                const uint32_t tw_taddr, PostBarrier &&post_barrier)
 {
     radix16_inv(x);
     stage_a_store<kRowElems>(x, b, S1b + t);
@@ -559,7 +456,7 @@ __device__ __forceinline__ void subfft4096_inv4(float2 (&x)[16], const int k2, f
     tmem_ld8(tw_taddr + 32 * k2, tw);        // n1 = 1..8, in flight across the barrier
     tmem_ld8(tw_taddr + 32 * k2 + 16, tw2);  // n1 = 9..15, then the next residue's stage-A base
 #define TW_AT(i) ((i) < 8 ? tw[(i)] : tw2[(i) - 8])
-    team_barrier();
+    __syncthreads();
     post_barrier();
     float2 *row = S1b + (t >> 4) * kRowElems;  // row n0 = t >> 4
     const int c = t & 15;
@@ -572,59 +469,31 @@ __device__ __forceinline__ void subfft4096_inv4(float2 (&x)[16], const int k2, f
     tmem_wait_ld();
     b = TW_AT(15);
     __syncwarp();  // the half-warp has consumed its row: reuse it as the B->C tile, element (n1, c) at 17 n1 + c
-    if constexpr (SWZ128) {
-        {   // unpadded row, swizzled in 16-byte chunks: element (n1, c) in chunk (c >> 1) ^ (n1 & 7), slot c & 1 of tile row
-            // n1, so that stage C reads two adjacent elements with one 128-bit load (half the loads and address XORs):
-            // address = ((row + 8 c) ^ (16 (n1 & 7))) + 128 n1
-            const uint32_t wb = smem_u32(row + c);
-            asm volatile("st.shared.v2.f32 [%0], {%1, %2};" ::"r"(wb), "f"(x[r16(0)].x), "f"(x[r16(0)].y) : "memory");
+    {   // unpadded row, swizzled in 16-byte chunks: element (n1, c) in chunk (c >> 1) ^ (n1 & 7), slot c & 1 of tile row
+        // n1, so that stage C reads two adjacent elements with one 128-bit load (half the loads and address XORs):
+        // address = ((row + 8 c) ^ (16 (n1 & 7))) + 128 n1
+        const uint32_t wb = smem_u32(row + c);
+        asm volatile("st.shared.v2.f32 [%0], {%1, %2};" ::"r"(wb), "f"(x[r16(0)].x), "f"(x[r16(0)].y) : "memory");
 #pragma unroll
-            for (int i = 0; i < 15; i++) {
-                const int n1 = i + 1;
-                const float2 v = cmul(x[r16(n1)], TW_AT(i));
-                asm volatile("st.shared.v2.f32 [%0], {%1, %2};" ::"r"((wb ^ (16u * (n1 & 7))) + 128u * n1), "f"(v.x), "f"(v.y) : "memory");
-            }
+        for (int i = 0; i < 15; i++) {
+            const int n1 = i + 1;
+            const float2 v = cmul(x[r16(n1)], TW_AT(i));
+            asm volatile("st.shared.v2.f32 [%0], {%1, %2};" ::"r"((wb ^ (16u * (n1 & 7))) + 128u * n1), "f"(v.x), "f"(v.y) : "memory");
         }
-        __syncwarp();
-        {   // this thread is now (n0, n1 = c): elements (c, 2 j), (c, 2 j + 1) in chunk j ^ (c & 7) of tile row c
-            const uint32_t rb = smem_u32(row + 16 * c + 2 * (c & 7));
+    }
+    __syncwarp();
+    {   // this thread is now (n0, n1 = c): elements (c, 2 j), (c, 2 j + 1) in chunk j ^ (c & 7) of tile row c
+        const uint32_t rb = smem_u32(row + 16 * c + 2 * (c & 7));
 #pragma unroll
-            for (int j = 0; j < 8; j++)
-                asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];"
-                             : "=f"(x[2 * j].x), "=f"(x[2 * j].y), "=f"(x[2 * j + 1].x), "=f"(x[2 * j + 1].y)
-                             : "r"(rb ^ (16u * j))
-                             : "memory");
-        }
-    } else {
-        {   // unpadded row: element (n1, c) at 16 n1 + (c ^ n1); on byte addresses (row is 128-byte aligned) the XOR
-            // touches bits 3..6 only: address = ((row + 8 c) ^ (8 n1)) + 128 n1
-            const uint32_t wb = smem_u32(row + c);
-            asm volatile("st.shared.v2.f32 [%0], {%1, %2};" ::"r"(wb), "f"(x[r16(0)].x), "f"(x[r16(0)].y) : "memory");
-#pragma unroll
-            for (int i = 0; i < 15; i++) {
-                const int n1 = i + 1;
-                const float2 v = cmul(x[r16(n1)], TW_AT(i));
-                asm volatile("st.shared.v2.f32 [%0], {%1, %2};" ::"r"((wb ^ (8u * n1)) + 128u * n1), "f"(v.x), "f"(v.y) : "memory");
-            }
-        }
-        __syncwarp();
-        {   // this thread is now (n0, n1 = c): element (c, cc) at 16 c + (cc ^ c) -> ((row + 136 c) ^ (8 cc))
-            const uint32_t rb = smem_u32(row + 17 * c);
-#pragma unroll
-            for (int cc = 0; cc < 16; cc++)
-                asm volatile("ld.shared.v2.f32 {%0, %1}, [%2];" : "=f"(x[cc].x), "=f"(x[cc].y) : "r"(rb ^ (8u * cc)) : "memory");
-        }
+        for (int j = 0; j < 8; j++)
+            asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];"
+                         : "=f"(x[2 * j].x), "=f"(x[2 * j].y), "=f"(x[2 * j + 1].x), "=f"(x[2 * j + 1].y)
+                         : "r"(rb ^ (16u * j))
+                         : "memory");
     }
     radix16_inv(x);
 }
 #undef TW_AT
-
-template <bool SWZ128, class PostBarrier>
-__device__ __forceinline__ void subfft4096_inv4(float2 (&x)[16], const int k2, float2 &b, float2 *S1b, const int t,
-                                                const uint32_t tw_taddr, PostBarrier &&post_barrier)
-{
-    subfft4096_inv4<SWZ128>(x, k2, b, S1b, t, tw_taddr, [] { __syncthreads(); }, post_barrier);
-}
 
 // Form of subfft4096_inv4 for kernels whose tensor memory is taken by parked data (k_search_e1b: 96 of a thread's
 // 128 columns hold three residues): the stage-B twiddles W1024^{(4c+k2)*n1} come from a 7.5 KiB shared-memory
@@ -639,10 +508,6 @@ __device__ __forceinline__ void tmem_st1(uint32_t taddr, const float2 v)
 {
     asm volatile("tcgen05.st.sync.aligned.32x32b.x2.b32 [%0], {%1,%2};" ::"r"(taddr), "f"(v.x), "f"(v.y) : "memory");
 }
-
-// B->C swizzle unit of the unpadded rows: 8-byte elements XORed with n1, or 16-byte chunks XORed with n1 & 7 (ACQ_SWZ128)
-constexpr uint32_t kSwz = ACQ_SWZ128 ? 16u : 8u;
-constexpr int kSwzMask = ACQ_SWZ128 ? 7 : 15;
 
 // Where the stage-A base W16384^{4t + k2'} of the NEXT residue k2' = (k2 + 1) & 3 comes from: two TMEM columns per
 // residue (kernels with columns to spare), or the 8 KiB table in global memory (L1/L2-resident; kernels whose tensor
@@ -664,24 +529,20 @@ struct BaseFromGlobal {
     __device__ __forceinline__ float2 get() { return v; }
 };
 
-template <class BaseSrc, class TeamBarrier, class PostBarrier>
+template <class BaseSrc, class PostBarrier>
 __device__ __forceinline__ void subfft4096_inv4s(float2 (&x)[16], const int k2, float2 &b, float2 *S1b, const int t,
-                                                 const float2 *T2s, BaseSrc base_src, TeamBarrier &&team_barrier,
-                                                 PostBarrier &&post_barrier)
+                                                 const float2 *T2s, BaseSrc base_src, PostBarrier &&post_barrier)
 {
     radix16_inv(x);
     stage_a_store<256>(x, b, S1b + t);
-    // all 15 stage-B twiddles before the barrier (1), or eight before it and seven during stage B (0).  With the
-    // residue loop of k_search_e1b unrolled: 20.7 M tiles/s against 20.35 M on cfg3, and no spill.
-#ifndef ACQ_E1B_TW15
-#define ACQ_E1B_TW15 1
-#endif
-    float2 tw[ACQ_E1B_TW15 ? 15 : 8];
+    // all 15 stage-B twiddles before the barrier: with the residue loop of k_search_e1b unrolled 20.7 M tiles/s on
+    // cfg3, against 20.35 M with eight before it and seven during stage B, and no spill
+    float2 tw[15];
     const float2 *twp = T2s + k2 * (15 * 16) + (t & 15);
 #pragma unroll
-    for (int i = 0; i < (ACQ_E1B_TW15 ? 15 : 8); i++) tw[i] = twp[i * 16];  // n1 = 1..8 (or all 15)
+    for (int i = 0; i < 15; i++) tw[i] = twp[i * 16];  // n1 = 1..15
     base_src.issue(k2);
-    team_barrier();
+    __syncthreads();
     post_barrier();
     float2 *row = S1b + (t >> 4) * 256;  // row n0 = t >> 4
     const int c = t & 15;
@@ -692,7 +553,7 @@ __device__ __forceinline__ void subfft4096_inv4s(float2 (&x)[16], const int k2, 
     }
     radix16_inv(x);
     b = base_src.get();
-    __syncwarp();  // the half-warp has consumed its row: reuse it as the B->C tile, element (n1, c) at 16 n1 + (c ^ n1)
+    __syncwarp();  // the half-warp has consumed its row: reuse it as the B->C tile, swizzled as in subfft4096_inv4
     {
         const uint32_t wb = smem_u32(row + c);
         asm volatile("st.shared.v2.f32 [%0], {%1, %2};" ::"r"(wb), "f"(x[r16(0)].x), "f"(x[r16(0)].y) : "memory");
@@ -700,21 +561,16 @@ __device__ __forceinline__ void subfft4096_inv4s(float2 (&x)[16], const int k2, 
         for (int i = 0; i < 8; i++) {
             const int n1 = i + 1;
             const float2 v = cmul(x[r16(n1)], tw[i]);
-            asm volatile("st.shared.v2.f32 [%0], {%1, %2};" ::"r"((wb ^ (kSwz * (n1 & kSwzMask))) + 128u * n1), "f"(v.x), "f"(v.y) : "memory");
+            asm volatile("st.shared.v2.f32 [%0], {%1, %2};" ::"r"((wb ^ (16u * (n1 & 7))) + 128u * n1), "f"(v.x), "f"(v.y) : "memory");
         }
-#if !ACQ_E1B_TW15
-#pragma unroll
-        for (int i = 0; i < 7; i++) tw[i] = twp[(i + 8) * 16];  // n1 = 9..15
-#endif
 #pragma unroll
         for (int i = 0; i < 7; i++) {
             const int n1 = i + 9;
-            const float2 v = cmul(x[r16(n1)], tw[ACQ_E1B_TW15 ? i + 8 : i]);
-            asm volatile("st.shared.v2.f32 [%0], {%1, %2};" ::"r"((wb ^ (kSwz * (n1 & kSwzMask))) + 128u * n1), "f"(v.x), "f"(v.y) : "memory");
+            const float2 v = cmul(x[r16(n1)], tw[i + 8]);
+            asm volatile("st.shared.v2.f32 [%0], {%1, %2};" ::"r"((wb ^ (16u * (n1 & 7))) + 128u * n1), "f"(v.x), "f"(v.y) : "memory");
         }
     }
     __syncwarp();
-#if ACQ_SWZ128
     {
         const uint32_t rb = smem_u32(row + 16 * c + 2 * (c & 7));
 #pragma unroll
@@ -724,21 +580,7 @@ __device__ __forceinline__ void subfft4096_inv4s(float2 (&x)[16], const int k2, 
                          : "r"(rb ^ (16u * j))
                          : "memory");
     }
-#else
-    {
-        const uint32_t rb = smem_u32(row + 17 * c);
-#pragma unroll
-        for (int cc = 0; cc < 16; cc++)
-            asm volatile("ld.shared.v2.f32 {%0, %1}, [%2];" : "=f"(x[cc].x), "=f"(x[cc].y) : "r"(rb ^ (8u * cc)) : "memory");
-    }
-#endif
     radix16_inv(x);
-}
-template <class BaseSrc, class PostBarrier>
-__device__ __forceinline__ void subfft4096_inv4s(float2 (&x)[16], const int k2, float2 &b, float2 *S1b, const int t,
-                                                 const float2 *T2s, BaseSrc base_src, PostBarrier &&post_barrier)
-{
-    subfft4096_inv4s(x, k2, b, S1b, t, T2s, base_src, [] { __syncthreads(); }, post_barrier);
 }
 
 }  // namespace acq

@@ -331,7 +331,7 @@ __global__ void __launch_bounds__(256, 1) k_fwd_fft(const float2 *__restrict__ x
     float2 *Z = reinterpret_cast<float2 *>(smem + fft_smem3_bytes());
     const int t = threadIdx.x;
     ACQ_TRACE_STAMP(kTrFwdFft, 0);
-    pdl_trigger_fft();
+    pdl_launch_dependents();
     load_t2(s, tables, t);
     const float2 *base = tables + kT2Elems + t;
     int buf = 0;
@@ -394,7 +394,7 @@ __global__ void __cluster_dims__(4, 1, 1) __launch_bounds__(256, 1)
     const int t = threadIdx.x;
     const int rank = (int)cluster.block_rank();
     ACQ_TRACE_STAMP(kTrFwdFft, 0);
-    pdl_trigger_fft();
+    pdl_launch_dependents();
     load_t2(s, tables, t);
     const float2 bw = __ldg(tables + kT2Elems + rank * 256 + t);
     const float2 *Yr[4];
@@ -553,22 +553,6 @@ struct TileIdx {
         d = (int)(tl - cw * nd);
         cap = (int)(cw / nw);
         wi = (int)(cw - (unsigned)cap * nw);
-        const int2 wk = p.work[wi];
-        sat = wk.x;
-        slot = wk.y;
-        set_dop(p);
-    }
-    // the tile `stride` further on, stride given as mixed-radix digits (sd, sw, sc) over (n_dop, n_work): no division
-    template <class PA>
-    __device__ __forceinline__ void step(const PA &p, int sd, int sw, int sc)
-    {
-        d += sd;
-        int carry = d >= p.n_dop;
-        if (carry) d -= p.n_dop;
-        wi += sw + carry;
-        carry = wi >= p.n_work;
-        if (carry) wi -= p.n_work;
-        cap += sc + carry;
         const int2 wk = p.work[wi];
         sat = wk.x;
         slot = wk.y;
@@ -811,8 +795,8 @@ __device__ __forceinline__ Peak merge_warp_peaks(const float *slot_f, const int 
 
 // The C/A search kernels.  Both operands of a sub-FFT are staged in shared memory by TMA bulk copies issued one
 // sub-FFT ahead (see subfft4096_inv4): D into the idle half of the exchange buffer, E into its own 32 KiB buffer; the
-// B->C tiles live inside the exchange rows.  The L2 round trip is off every warp's dependent chain (the load-from-L2
-// A/B form, acq_variants.cuh, is 7 % slower); 98.6 KiB of shared memory per CTA, two CTAs per SM.
+// B->C tiles live inside the exchange rows.  The L2 round trip is off every warp's dependent chain (a form that loaded
+// both operands straight from L2 was measured 7 % slower on cfg2); 98.6 KiB of shared memory per CTA, two CTAs per SM.
 //
 // Unroll factor of the loop over the four residues of a transform.  Rolled, the compiler moves the 16 accumulators
 // between two register sets once per sub-FFT (about 40 MOVs per warp and sub-FFT in the ncu source view); unrolled
@@ -863,9 +847,6 @@ __device__ __forceinline__ Peak thread_peak_l1(const float (&pw)[16], int t)
 // CTA and hands the partial accumulators of a split tile over through L2 -- "stream-K" -- so that 1312 tiles do not
 // run as five rounds on 296 CTAs.  Bitwise-equal cells, but 78.6 -> 81.4 us per cold-start search and no change on
 // the receiver farm: the last round already runs one CTA per SM, which is 1.6x faster per tile than two.)
-#ifndef ACQ_L1_LEAN
-#define ACQ_L1_LEAN 1   // K = 1: tile indices advance without divisions, max / first index by REDUX (+0.3..1 % cfg5, -1.3 us cfg1; 0 = round-1 form)
-#endif
 template <bool MULTI, class PA>
 __global__ void __launch_bounds__(256, 2) k_search_l1(const PA p)
 {
@@ -886,26 +867,16 @@ __global__ void __launch_bounds__(256, 2) k_search_l1(const PA p)
     __syncthreads();
     if (p.wait_prior) pdl_wait();
     ACQ_TRACE_STAMP(kTrSearchL1, 1);
-    pdl_trigger_search();
+    pdl_launch_dependents();
     // thread 0: stage the operands of sub-FFT (tn, bn, k2n) -- D into S1 half `half`, E into the E buffer
     auto issue = [&](const TileIdx &tn, int bn, int k2n, int half) {
         const int r = (k2n - tn.dop) & 3;
         const int q = (k2n - tn.dop - r) >> 2;
-#ifdef ACQ_KO_SAME_OPERANDS  // knock-out experiment (wrong results): every tile reads the same 64 KiB of operands
-        const float2 *Dk = p.Dp + k2n * kSub;
-        const float2 *Ek = p.Ep + (size_t)r * p.ext_len + ((p.Q + q) & ~1);
-#else
         const float2 *Dk = p.Dp + d_row(p, tn, bn) * kN + k2n * kSub;
         const float2 *Ek = p.Ep + (size_t)(tn.sat * 4 + r) * p.ext_len + ((p.Q + q) & ~1);
-#endif
         fence_proxy_async();  // generic-proxy reads of these buffers (ordered by the CTA barrier) before the async writes
-#ifdef ACQ_K1_E_LDG   // experiment: the code run straight from L2 (issued before the wait for D), only D staged
-        (void)Ek;
-        mbar_expect_tx(bar, (uint32_t)(sizeof(float2) * kSub));
-#else
         mbar_expect_tx(bar, (uint32_t)(sizeof(float2) * (kSub + kEBufElems)));
         tma_load_1d(smem_u32(s.E), Ek, (uint32_t)(sizeof(float2) * kEBufElems), bar);
-#endif
         tma_load_1d(smem_u32(s.S1 + half * kS1pElems), Dk, (uint32_t)(sizeof(float2) * kSub), bar);
     };
     TileIdx ti(p, blockIdx.x);   // the grid never exceeds the tile count: every CTA has a first tile
@@ -934,21 +905,12 @@ __global__ void __launch_bounds__(256, 2) k_search_l1(const PA p)
                     const int r = (k2 - ti.dop) & 3;
                     const int q = (k2 - ti.dop - r) >> 2;
                     const float2 *Dk = S1b + t;
-#ifdef ACQ_K1_E_LDG
-                    const float2 *Eg = p.Ep + (size_t)(ti.sat * 4 + r) * p.ext_len + p.Q + q + t;
-#pragma unroll
-                    for (int a = 0; a < 16; a++) x[a] = __ldg(Eg + 256 * a);
-                    mbar_wait(bar, (uint32_t)(it & 1));
-#pragma unroll
-                    for (int a = 0; a < 16; a++) x[a] = cmul_conj_a(Dk[kRowElems * a], x[a]);
-#else
                     const float2 *Ek = s.E + ((p.Q + q) & 1) + t;
                     mbar_wait(bar, (uint32_t)(it & 1));
 #pragma unroll
                     for (int a = 0; a < 16; a++) x[a] = cmul_conj_a(Dk[kRowElems * a], Ek[256 * a]);
-#endif
                 }
-                subfft4096_inv4<true>(x, k2, bw, S1b, t, tw_taddr, [&]() {
+                subfft4096_inv4(x, k2, bw, S1b, t, tw_taddr, [&]() {
                     if (t == 0) {  // every warp is past its operand reads of this sub-FFT and past stage C of the previous one
                         if (b == 0 && k2 == 0) nxt = claim_tile(p, nxt);
                         if (b == p.K - 1 && k2 == 2) publish_tile(feed, p, nxt);
@@ -974,11 +936,7 @@ __global__ void __launch_bounds__(256, 2) k_search_l1(const PA p)
 #pragma unroll
             for (int n2 = 0; n2 < 16; n2++) P[n2] = (!MULTI || b == 0) ? cpower(acc[n2]) : (P[n2] + cpower(acc[n2]));
         }
-#if ACQ_L1_LEAN
         warp_reduce_peak_redux(thread_peak_l1(P, t), red_f + 16 * par, red_i + 8 * par, t);
-#else
-        warp_reduce_peak(thread_peak_l1(P, t), red_f + 16 * par, red_i + 8 * par, t);
-#endif
         pend_cap = ti.cap;
         pend_slot = ti.slot;
         pend_d = ti.d;
@@ -992,257 +950,6 @@ __global__ void __launch_bounds__(256, 2) k_search_l1(const PA p)
     ACQ_TRACE_STAMP(kTrSearchL1, 2);
     tmem_free_cta<2 * kTwCols>(tmem_base, t);
 }
-
-// Staging warps (k_search_l1_dr below; measured first in the experiment form k_search_l1_st, acq_variants.cuh).  In
-// k_search_l1 thread 0 of a CTA issues the next sub-FFT's bulk copies right after the CTA barrier (address arithmetic, proxy
-// fence, expect_tx, the copies) and once per tile merges the warp partials and stores the cell: ncu's warp samples put a
-// third of a sub-FFT period of warp 0 on that path, and the other seven warps wait for it at the next barrier (10 % of all
-// warp samples were barrier stalls).  Here one CTA per SM holds TWO teams of eight FFT warps -- each team is what a CTA
-// of k_search_l1 is, with its own exchange and code-run buffers, mbarrier, tensor-memory columns and named barrier -- plus
-// one staging warp per team that takes part in the team's barrier and does all of the above, so no FFT warp ever leaves
-// the common instruction stream.  Five warpgroups: the launch allocates 96 registers per thread, the staging warpgroup
-// drops to 32 (setmaxnreg.dec) and the four FFT warpgroups rise to 112 with exactly what it released.
-[[maybe_unused]] constexpr int kStThreads = 640, kStHandOver = 288;   // 2 x 256 FFT threads + a warpgroup of staging warps; hand-over = 8 + 1 warps
-// Named barriers of a team (ids 1..3 for team 0, 4..6 for team 1):
-//   A (256 threads): the FFT warps' own barrier, one per sub-FFT;
-//   B (288): hand-over to the staging warp.  Every FFT warp ARRIVES (no wait) just before it waits on A, and the staging
-//      warp SYNCs: it runs on once all eight have reached this sub-FFT's barrier, i.e. are past their operand reads of this
-//      sub-FFT and past stage C of the one before, and stages the next sub-FFT's operands.  An FFT warp cannot reach the
-//      next sub-FFT's barrier before the staging warp has passed (that sub-FFT's operands are staged only after it), so
-//      the phases of B cannot mix;
-//   C (288): the same hand-over once more after a team's last sub-FFT (the last tile's warp partials are in place).
-// All waiting participants of a barrier execute the same instruction: compute-sanitizer's synccheck rejects a bar.sync
-// reached from two code locations (tools/exp/mb_namedbar.cu), which rules out the simplest form -- the staging warp inside
-// barrier A, one barrier instruction per FFT warp: 5.84 ms on cfg5 with 128 captures, against 5.97 ms for this form,
-// 6.02 ms with the arrive moved up behind the products, 6.18 ms with one warp arriving after A, 6.29 ms with the staging
-// warp polling a shared-memory mbarrier, and 6.30 ms for k_search_l1<false>.
-__device__ __forceinline__ void st_fft_sync(int team)         // barrier A
-{
-    if (team == 0) asm volatile("bar.sync 1, 256;" ::: "memory");
-    else asm volatile("bar.sync 4, 256;" ::: "memory");
-}
-__device__ __forceinline__ void st_fft_arrive(int team)       // barrier B, FFT warps
-{
-    if (team == 0) asm volatile("bar.arrive 2, %0;" ::"n"(kStHandOver) : "memory");
-    else asm volatile("bar.arrive 5, %0;" ::"n"(kStHandOver) : "memory");
-}
-__device__ __forceinline__ void st_fft_done(int team)         // barrier C, FFT warps
-{
-    if (team == 0) asm volatile("bar.arrive 3, %0;" ::"n"(kStHandOver) : "memory");
-    else asm volatile("bar.arrive 6, %0;" ::"n"(kStHandOver) : "memory");
-}
-__device__ __forceinline__ void st_stage_wait(int team)       // barrier B, staging warp
-{
-    if (team == 0) asm volatile("bar.sync 2, %0;" ::"n"(kStHandOver) : "memory");
-    else asm volatile("bar.sync 5, %0;" ::"n"(kStHandOver) : "memory");
-}
-__device__ __forceinline__ void st_stage_wait_done(int team)  // barrier C, staging warp
-{
-    if (team == 0) asm volatile("bar.sync 3, %0;" ::"n"(kStHandOver) : "memory");
-    else asm volatile("bar.sync 6, %0;" ::"n"(kStHandOver) : "memory");
-}
-
-// k_search_l1_dr -- the staging-warp form with the CAPTURE operand resident in tensor memory.  The capture residue D of a
-// sub-FFT depends on (capture, residue k2) only, and a thread always reads the same 16 values of it (D[256 a + t]):
-// 4 residues x 16 complex = the 128 TMEM columns a thread owns.  A team takes a CONTIGUOUS range of tiles (capture-major
-// order: all (satellite, Doppler) tiles of a capture are neighbours), so D is staged by TMA and parked only in the first
-// tile of a capture and comes back by one tcgen05.ld per sub-FFT in every other tile: neither its 32 KiB bulk copy nor its 16
-// shared-memory loads per thread touch the L1/shared data pipe.  The stage-B twiddles move to a 7.5 KiB shared table per
-// team, the stage-A bases to the global table (as in k_search_l1_multi).  Same arithmetic in the same order as
-// k_search_l1<false>: bitwise-equal cells (tested).
-struct DrSmem {
-    float2 *S1;  // [2][4096]
-    float2 *E;   // [4098]
-    unsigned long long *bar;
-    float2 *T2;  // [4][15][16]
-    float *red_f;
-    int *red_i;
-};
-__host__ __device__ constexpr size_t dr_team_smem_bytes()
-{
-    return (sizeof(float2) * (size_t)(2 * kSub + kEBufElems) + 16 + sizeof(float2) * kT2Elems + 64 * sizeof(float) + 1023) / 1024 * 1024;
-}
-__host__ __device__ constexpr size_t dr_smem_bytes() { return 2 * dr_team_smem_bytes(); }
-__device__ __forceinline__ DrSmem dr_smem_carve(unsigned char *smem)
-{
-    DrSmem s;
-    s.S1 = reinterpret_cast<float2 *>(smem);
-    s.E = s.S1 + 2 * kSub;
-    s.bar = reinterpret_cast<unsigned long long *>(s.E + kEBufElems);
-    s.T2 = reinterpret_cast<float2 *>(s.bar + 2);
-    s.red_f = reinterpret_cast<float *>(s.T2 + kT2Elems);
-    s.red_i = reinterpret_cast<int *>(s.red_f + 32);
-    return s;
-}
-
-// Compiled only into the variant libraries that route searches to it (l1_dr_all, l1_dr12): the product library holds no
-// A/B kernel.
-#ifndef ACQ_DR_MIN_TILES_PER_SM
-#define ACQ_DR_MIN_TILES_PER_SM -1   // product: never (see search_kind_l1)
-#endif
-#if ACQ_DR_MIN_TILES_PER_SM >= 0
-__global__ void __launch_bounds__(kStThreads, 1) k_search_l1_dr(const SearchArgs p)
-{
-    extern __shared__ __align__(1024) unsigned char smem[];
-    const int t = threadIdx.x;
-    ACQ_TRACE_STAMP(kTrSearchL1, 0);
-    constexpr int L = ACQ_LAGS_L1;
-    __shared__ uint32_t tmem_slot;
-    const uint32_t tmem_base = tmem_alloc_cta<4 * kTwCols>(&tmem_slot, t);
-    if (t < 2) mbar_init(smem_u32(dr_smem_carve(smem + t * dr_team_smem_bytes()).bar), 1);
-    __syncthreads();
-    if (p.wait_prior) pdl_wait();
-    ACQ_TRACE_STAMP(kTrSearchL1, 1);
-    pdl_trigger_search();
-    // Team T of 2 gridDim.x takes the T-th of as many balanced contiguous tile ranges (team 1 of a CTA comes after every
-    // team 0: a search of no more tiles than SMs runs one team per SM).
-    const int team = (t < 512) ? (t >> 8) : ((t >> 5) & 1);
-    const unsigned T = (unsigned)team * gridDim.x + blockIdx.x, n_teams = 2u * gridDim.x;
-    const unsigned n_tiles = (unsigned)p.n_tiles, base = n_tiles / n_teams, extra = n_tiles % n_teams;
-    const unsigned tile0 = T * base + (T < extra ? T : extra), my_tiles = base + (T < extra ? 1u : 0u);
-    const unsigned per_cap = (unsigned)p.n_work * (unsigned)p.n_dop;   // tiles of one capture
-    const DrSmem s = dr_smem_carve(smem + team * dr_team_smem_bytes());
-    const uint32_t bar = smem_u32(s.bar);
-    if (t >= 512) {
-        asm volatile("setmaxnreg.dec.sync.aligned.u32 32;");
-        if (t < 576 && my_tiles > 0) {
-            // ---- staging warp of `team` (lane 0 works)
-            const bool lead = (t & 31) == 0;
-            float *red_f = s.red_f;
-            int *red_i = s.red_i;
-            auto issue = [&](const TileIdx &tn, bool fresh, int k2n, int half) {   // E always, D in the first tile of a capture
-                const int r = (k2n - tn.dop) & 3;
-                const int q = (k2n - tn.dop - r) >> 2;
-                const float2 *Ek = p.Ep + (size_t)(tn.sat * 4 + r) * p.ext_len + ((p.Q + q) & ~1);
-                fence_proxy_async();  // generic-proxy accesses of these buffers (ordered by the team barrier) before the async writes
-                mbar_expect_tx(bar, (uint32_t)(sizeof(float2) * (kEBufElems + (fresh ? kSub : 0))));
-                tma_load_1d(smem_u32(s.E), Ek, (uint32_t)(sizeof(float2) * kEBufElems), bar);
-                if (fresh) {
-                    const float2 *Dk = p.Dp + d_row(p, tn, 0) * kN + k2n * kSub;
-                    tma_load_1d(smem_u32(s.S1 + half * kSub), Dk, (uint32_t)(sizeof(float2) * kSub), bar);
-                }
-            };
-            TileIdx ti(p, tile0);
-            bool fresh = true;
-            if (lead) issue(ti, true, 0, 0);
-            int it = 0, par = 0, pend_cap = -1, pend_slot = 0, pend_d = 0;
-            for (unsigned i = 0; i < my_tiles; i++) {
-                TileIdx tn = ti;
-                const bool more = i + 1 < my_tiles;
-                if (more) tn.step(p, 1, 0, 0);
-                const bool fresh_n = tn.cap != ti.cap;
-#pragma unroll 1
-                for (int k2 = 0; k2 < 4; k2++) {
-                    __syncwarp();
-                    st_stage_wait(team);   // every FFT warp is past its operand reads of this sub-FFT and past stage C of the previous one
-                    if (lead) {
-                        if (k2 < 3) issue(ti, fresh, k2 + 1, (it + 1) & 1);
-                        else if (more) issue(tn, fresh_n, 0, (it + 1) & 1);
-                        if (k2 == 0 && pend_cap >= 0)   // the previous tile's peak: its warp partials precede this barrier
-                            store_cell(p, pend_cap, pend_slot, pend_d, merge_warp_peaks(red_f + 16 * (par ^ 1), red_i + 8 * (par ^ 1)), L);
-                    }
-                    it++;
-                }
-                pend_cap = ti.cap;
-                pend_slot = ti.slot;
-                pend_d = ti.d;
-                par ^= 1;
-                ti = tn;
-                fresh = fresh_n;
-            }
-            __syncwarp();
-            st_stage_wait_done(team);   // the last tile's warp partials are in place
-            if (lead) {
-                store_cell(p, pend_cap, pend_slot, pend_d, merge_warp_peaks(red_f + 16 * (par ^ 1), red_i + 8 * (par ^ 1)), L);
-                __threadfence();  // this team's cells (all stored by this thread) before the CTA's count
-#ifdef ACQ_TRACE
-                if (blockIdx.x < kTraceCtas) {   // slot 3: team 0 done; team 1 done goes to the second half of the CTA axis
-                    unsigned long long tm;
-                    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(tm));
-                    g_trace[kTrSearchL1][blockIdx.x + (team ? 512 : 0)][3] = tm;
-                }
-#endif
-            }
-        }
-    } else {
-        asm volatile("setmaxnreg.inc.sync.aligned.u32 112;");
-        if (my_tiles > 0) {
-            // ---- the eight FFT warps of `team`
-            const int tt = t & 255;
-            float *red_f = s.red_f;
-            int *red_i = s.red_i;
-            const uint32_t d_taddr = tmem_base + (uint32_t)(team * 2 * kTwCols) + tmem_lane_base(tt) + (uint32_t)((tt >> 7) * kTwCols);  // [k2][16 complex]
-            {   // stage-B twiddle table into this team's shared memory
-                const float4 *src = reinterpret_cast<const float4 *>(p.tables);
-                float4 *dst = reinterpret_cast<float4 *>(s.T2);
-                for (int i = tt; i < kT2Elems / 2; i += 256) dst[i] = __ldg(src + i);
-            }
-            const float2 *bases = p.tables + kT2Elems + tt;  // [k2][256]: W16384^{4t+k2}
-            float2 bw = __ldg(bases);
-            int it = 0, par = 0;
-            const TileIdx t0(p, tile0);
-            int d = t0.d, dop = t0.dop;
-            unsigned left = per_cap - tile0 % per_cap;   // tiles of this team's range before the next capture begins
-            bool fresh = true;
-            st_fft_sync(team);   // the twiddle table is in place
-            for (unsigned i = 0; i < my_tiles; i++) {
-                float P[16];
-                float2 acc[16];
-                float2 x[16];
-                // rolled: at 112 registers the loop unrolled by two spills (28.75 M against 27.7 M tiles/s on cfg5, measured)
-#pragma unroll 1
-                for (int k2 = 0; k2 < 4; k2++) {
-                    float2 *S1b = s.S1 + (it & 1) * kSub;
-                    const int r = (k2 - dop) & 3;
-                    const int q = (k2 - dop - r) >> 2;
-                    const float2 *Ek = s.E + ((p.Q + q) & 1) + tt;
-                    if (fresh) {   // D from the staged residue; park this thread's 16 values for the capture's other tiles
-                        const float2 *Dk = S1b + tt;
-                        mbar_wait(bar, (uint32_t)(it & 1));
-#pragma unroll
-                        for (int a = 0; a < 16; a++) x[a] = Dk[256 * a];
-                        tmem_st16(d_taddr + 32 * k2, x);
-                        tmem_wait_st();
-                    } else {
-                        tmem_ld16(d_taddr + 32 * k2, x);
-                        mbar_wait(bar, (uint32_t)(it & 1));
-                        tmem_wait_ld();
-                    }
-                    // x[a] = conj(data[k]) * code[k - dop], k = 1024 a + 4 t + k2   (search.cpp:471)
-#pragma unroll
-                    for (int a = 0; a < 16; a++) x[a] = cmul_conj_a(x[a], Ek[256 * a]);
-                    subfft4096_inv4s(x, k2, bw, S1b, tt, s.T2, BaseFromGlobal{bases}, [&] { st_fft_arrive(team); st_fft_sync(team); }, [] {});
-                    it++;
-                    if (k2 == 0) {
-#pragma unroll
-                        for (int n2 = 0; n2 < 16; n2++) acc[n2] = x[r16(n2)];
-                    } else {
-#pragma unroll
-                        for (int n2 = 0; n2 < 16; n2++) acc[n2] = cfma(x[r16(n2)], c_cC[k2][n2], acc[n2]);
-                    }
-                }
-#pragma unroll
-                for (int n2 = 0; n2 < 16; n2++) P[n2] = cpower(acc[n2]);
-                warp_reduce_peak_redux(thread_peak_l1(P, tt), red_f + 16 * par, red_i + 8 * par, tt);
-                par ^= 1;
-                {   // next tile of the range: the Doppler index (the only tile coordinate an FFT warp needs) and the capture boundary
-                    if (++d >= p.n_dop) d = 0;
-                    const int h = p.dop_lo + d;
-                    const int v = p.half_bin ? (h & 1) : 0;
-                    dop = p.half_bin ? ((h - v) >> 1) : h;
-                    fresh = (--left == 0);
-                    if (fresh) left = per_cap;
-                }
-            }
-            st_fft_done(team);   // the last tile's warp partials are in place
-        }
-    }
-    __syncthreads();
-    if (t == 0 && p.ctas_total) atomicAdd(p.ctas_done, 1u);   // both teams' cells are stored and fenced (staging warps, above)
-    ACQ_TRACE_STAMP(kTrSearchL1, 2);
-    tmem_free_cta<4 * kTwCols>(tmem_base, t);
-}
-#endif  // ACQ_DR_MIN_TILES_PER_SM >= 0
 
 
 // k_search_l1_multi -- k_noncoh > 1 with the CODE operand resident in tensor memory.  The code run E of a tile depends on
@@ -1303,7 +1010,7 @@ __global__ void __launch_bounds__(256, 2) k_search_l1_multi(const PA p)
     __syncthreads();
     if (p.wait_prior) pdl_wait();
     ACQ_TRACE_STAMP(kTrSearchL1, 1);
-    pdl_trigger_search();
+    pdl_launch_dependents();
     // thread 0: stage the operands of sub-FFT (tn, bn, k2n) -- D into S1 half `half`; E only for block 0
     auto issue = [&](const TileIdx &tn, int bn, int k2n, int half) {
         const int r = (k2n - tn.dop) & 3;
@@ -1399,11 +1106,11 @@ __global__ void __launch_bounds__(256, 2) k_search_l1_multi(const PA p)
 }
 
 // k_search_l1_cr -- K = 1 on full bins with the CAPTURE operand resident in tensor memory and tiles claimed in CHUNKS.
-// The idea of k_search_l1_dr (a thread always reads the same 16 values of a capture residue: 4 residues x 16 complex = its
-// 128 TMEM columns, so D is staged and parked once and comes back by one tcgen05.ld per sub-FFT) in the two-CTAs-per-SM
-// form that claims its work: a CTA draws runs of consecutive tiles (same capture, bar the boundaries), 16 tiles long while
-// the launch is young, 4 and then single tiles towards its end (SearchArgs::ck_n16 / ck_n4, search_chunks()), so the
-// greedy tail stays one tile long while D is re-staged for ~1 tile in 14.  Stage-B twiddles: the 7.5 KiB shared table;
+// A thread always reads the same 16 values of a capture residue: 4 residues x 16 complex = its 128 TMEM columns, so D is
+// staged and parked once per capture and comes back by one tcgen05.ld per sub-FFT.  Two CTAs per SM; a CTA draws runs
+// of consecutive tiles (same capture, bar the boundaries), 16 tiles long while the launch is young, 4 and then single
+// tiles towards its end (SearchArgs::ck_n16 / ck_n4, search_chunks()), so the greedy tail stays one tile long while D is
+// re-staged for ~1 tile in 14.  Stage-B twiddles: the 7.5 KiB shared table;
 // stage-A bases: the global table (as k_search_l1_multi, whose shared-memory layout this kernel uses).  Same arithmetic in
 // the same order as k_search_l1<false>: bitwise-equal cells (tested).
 #ifndef ACQ_CK_BIG
@@ -1430,7 +1137,8 @@ __device__ __forceinline__ bool chunk_of(const SearchArgs &p, unsigned c, unsign
 }
 
 // Residue loop fully unrolled (126 registers, no spill): on a 128-capture farm 5.98 ms rolled, 5.49 ms by two, 5.24 ms by
-// four (28.1 / 30.6 / 32.1 M tiles/s; k_search_l1<false> with claimed tiles: 5.78 ms, k_search_l1_dr: 5.96 ms).
+// four (28.1 / 30.6 / 32.1 M tiles/s; k_search_l1<false> with claimed tiles: 5.78 ms, the two-team staging-warp kernel of
+// round 2: 5.96 ms).
 #ifndef ACQ_CR_UNROLL
 #define ACQ_CR_UNROLL 4
 #endif
@@ -1464,7 +1172,7 @@ __global__ void __launch_bounds__(256, 2) k_search_l1_cr(const PA p)
     __syncthreads();
     if (p.wait_prior) pdl_wait();
     ACQ_TRACE_STAMP(kTrSearchL1, 1);
-    pdl_trigger_search();
+    pdl_launch_dependents();
     // thread 0: stage the operands of sub-FFT (tn, k2n) -- E always, D (into S1 half `half`) only while the capture is new
     auto issue = [&](const TileIdx &tn, bool fresh_n, int k2n, int half) {
         const int r = (k2n - tn.dop) & 3;
@@ -1590,9 +1298,6 @@ constexpr int kE1bTmemCols = 256;  // 2 warp sets x 96 columns, rounded up to a 
 // next tile (no reduction barrier).  A thread's 128 TMEM columns hold the three parked residues (96) and the four
 // stage-A bases (8), so the stage-B twiddles stay in a 7.5 KiB shared-memory table.  106 KiB of shared memory per
 // CTA, two CTAs per SM.
-#ifndef ACQ_E1B_BEST4
-#define ACQ_E1B_BEST4 1
-#endif
 constexpr int kE1bBaseCol = 96;  // TMEM columns [96, 104): W16384^{4t+k2}, k2 = 0..3
 // Unroll factor of the residue loop (see ACQ_K2_UNROLL): measured on cfg3 19.6 M tiles/s rolled, 19.9 M by two,
 // 20.4 M fully unrolled (the park/no-park branch and the residue-dependent constants fold away; 24 bytes of spill).
@@ -1652,7 +1357,7 @@ __global__ void __launch_bounds__(256, 2) k_search_e1b(const PA p)
     __syncthreads();
     if (p.wait_prior) pdl_wait();
     ACQ_TRACE_STAMP(kTrSearchE1b, 1);
-    pdl_trigger_search();
+    pdl_launch_dependents();
     auto issue = [&](const TileIdx &tn, int k2n, int half) {  // thread 0: stage the operands of sub-FFT (tn, k2n)
         const int r = (k2n - tn.dop) & 3;
         const int q = (k2n - tn.dop - r) >> 2;
@@ -1708,12 +1413,9 @@ __global__ void __launch_bounds__(256, 2) k_search_e1b(const PA p)
                 tmem_wait_st();
             }
         }
-        // radix-4 combine over k2, lags n = lag_of3(t, n2) + 4096 m < 16368.  Lags are not visited in
-        // increasing order here, so ties compare the index explicitly (first index wins, search.cpp:488).
-#if ACQ_E1B_BEST4
-        // A thread's lags grow with n2 inside a quarter m and with m across quarters: one running (max, n2) per
-        // quarter with a strict >, merged in the order m = 0..3 with a strict >, keeps the first maximum
-        // (search.cpp:488) without comparing indices.
+        // radix-4 combine over k2, lags n = lag_of3(t, n2) + 4096 m < 16368.  A thread's lags grow with n2 inside a
+        // quarter m and with m across quarters: one running (max, n2) per quarter with a strict >, merged in the order
+        // m = 0..3 with a strict >, keeps the first maximum (search.cpp:488) without comparing indices.
         float bp[4] = {0.0f, 0.0f, 0.0f, 0.0f}, bsum = 0.0f;
         int bn2[4] = {0, 0, 0, 0};
         const int lag0 = lag_of3(t, 0);
@@ -1749,34 +1451,6 @@ __global__ void __launch_bounds__(256, 2) k_search_e1b(const PA p)
 #pragma unroll
         for (int m = 0; m < 4; m++)
             if (bp[m] > best.p) best.p = bp[m], best.n = lag0 + 256 * bn2[m] + 4096 * m;
-#else
-        Peak best;
-        best.p = 0.0f;
-        best.n = 0x7fffffff;
-        best.sum = 0.0f;
-#pragma unroll
-        for (int c4 = 0; c4 < 4; c4++) {
-            float2 za[4], zb[4], zc[4];
-            tmem_ld4(zaddr + 0 * 32 + 8 * c4, za);
-            tmem_ld4(zaddr + 1 * 32 + 8 * c4, zb);
-            tmem_ld4(zaddr + 2 * 32 + 8 * c4, zc);
-            tmem_wait_ld();
-#pragma unroll
-            for (int i = 0; i < 4; i++) {
-                const int n2 = 4 * c4 + i;
-                float2 z0 = za[i], z1 = zb[i], z2 = zc[i];
-                float2 z3 = cmul(x[r16(n2)], c_cC[3][n2]);
-                radix4_inv(z0, z1, z2, z3);  // z_m = sum_k2 z_k2 * j^{k2*m}
-                const float2 zz[4] = {z0, z1, z2, z3};
-#pragma unroll
-                for (int m = 0; m < 4; m++) {
-                    const int n = lag_of3(t, n2) + 4096 * m;
-                    const float pw = cpower(zz[m]);
-                    if (n < L) peak_merge(best, pw, n, pw);
-                }
-            }
-        }
-#endif
         // parity slot `par` was last read (flush) during the previous tile, before >= 3 CTA barriers
         warp_reduce_peak(best, red_f + 16 * par, red_i + 8 * par, t);
         pend_cap = ti.cap;
@@ -1851,7 +1525,7 @@ __global__ void __launch_bounds__(256, 2) k_search_e1b_multi(const PA p)
     __syncthreads();
     if (p.wait_prior) pdl_wait();
     ACQ_TRACE_STAMP(kTrSearchE1b, 1);
-    pdl_trigger_search();
+    pdl_launch_dependents();
     auto issue = [&](const TileIdx &tn, int bn, int k2n, int half) {  // thread 0: stage the capture residue of sub-FFT (tn, bn, k2n)
         const float2 *Dk = p.Dp + d_row(p, tn, bn) * kN + k2n * kSub;
         fence_proxy_async();
@@ -2004,7 +1678,7 @@ __global__ void __launch_bounds__(256, 2) k_search_e1b_multi(const PA p)
 // remote reads per CTA and tile.  (Splitting by m instead would make every CTA read all of every Y: 96 KiB.)
 // Peaks are reduced per CTA, sent to rank 0 through DSMEM and merged there; only the 16-byte cell leaves the
 // cluster.  No thread-private scratch, four SMs per tile: shorter latency per tile and a 4x finer scheduling
-// grain than k_search_e1b.  The host picks the form in acq_api.cu (ACQ_E1B_KERNEL=cta|cluster forces one).
+// grain than k_search_e1b.  The host picks the form in acq_api.cu (variants e1b_cta / e1b_cluster force one).
 // MULTI (k_noncoh > 1): each thread owns 16 lags (4 values of n2 x 4 quarters), so the block powers are summed
 // in registers exactly as in k_search_l1 (front-end block delay, see k_hb2).  Y is double
 // buffered: one cluster barrier per block (a buffer is rewritten two blocks later, after the barrier every
@@ -2035,7 +1709,7 @@ __global__ void __cluster_dims__(4, 1, 1) __launch_bounds__(256, 1) k_search_e1b
     int buf = 0, yb = 0;
     if (p.wait_prior) pdl_wait();
     ACQ_TRACE_STAMP(kTrE1bCluster, 1);
-    pdl_trigger_search();
+    pdl_launch_dependents();
 
     for (long long tile = blockIdx.x >> 2; tile < p.n_tiles; tile += n_clusters) {
         const TileIdx ti(p, tile);
@@ -2184,10 +1858,79 @@ __global__ void __launch_bounds__(128) k_best_dop(const acq_cell *__restrict__ c
                  threadIdx.x & 31);
 }
 
-#if defined(ACQ_VARIANT_L1_LDG) || defined(ACQ_VARIANT_L1_X3) || defined(ACQ_VARIANT_E1B_LDG) || defined(ACQ_VARIANT_L1_SP) || \
-    defined(ACQ_VARIANT_L1_ST) || defined(ACQ_VARIANT_L1_MST)
-#include "acq_variants.cuh"  // A/B forms: experiment builds only (tools/build_variants.py)
-#endif
+#ifdef ACQ_VARIANT_E1B_LDG
+// k_search_e1b_ldg: the one-CTA E1B search with operands read straight from L2 and a reduction barrier per tile -- the
+// reference k_search_e1b is tested against (variant library e1b_ldg; the product library does not contain it).
+__global__ void __launch_bounds__(256, 2) k_search_e1b_ldg(const SearchArgs p)
+{
+    extern __shared__ __align__(1024) unsigned char smem[];
+    const FftSmem3 s = fft_smem3_carve(smem);
+    float *red_f = reinterpret_cast<float *>(smem + fft_smem3_bytes());
+    int *red_i = reinterpret_cast<int *>(red_f + 16);
+    const int t = threadIdx.x;
+    constexpr int L = ACQ_LAGS_E1B;
+    const uint32_t tmem_base = tmem_alloc_cta<kE1bTmemCols>(reinterpret_cast<uint32_t *>(red_f + 32), t);
+    load_t2(s, p.tables, t);
+    // this thread's scratch: lane 32*(warp%4) + (t%32), columns [96*(warp/4), +96): [k2][n2] complex
+    const uint32_t zaddr = tmem_base + tmem_lane_base(t) + (uint32_t)((t >> 7) * 96);
+    const float2 *base = p.tables + kT2Elems + t;
+    int buf = 0;
+    if (p.wait_prior) pdl_wait();
+    pdl_launch_dependents();  // after the wait (see k_search_l1)
+
+    for (long long tile = blockIdx.x; tile < p.n_tiles; tile += gridDim.x) {
+        const TileIdx ti(p, tile);
+        float2 x[16];
+#pragma unroll 1
+        for (int k2 = 0; k2 < 4; k2++) {
+            load_products(x, p, ti, 0, k2, t);
+            subfft4096_inv3(x, k2, __ldg(base + k2 * 256), buf, s, t);
+            buf ^= 1;
+            if (k2 < 3) {
+                float2 z[16];
+#pragma unroll
+                for (int n2 = 0; n2 < 16; n2++) z[n2] = (k2 == 0) ? x[r16(n2)] : cmul(x[r16(n2)], c_cC[k2][n2]);
+                tmem_st16(zaddr + 32 * k2, z);
+                tmem_wait_st();
+            }
+        }
+        // radix-4 combine over k2, lags n = lag_of3(t, n2) + 4096 m < 16368.  Lags are not visited in
+        // increasing order here, so ties compare the index explicitly (first index wins, search.cpp:488).
+        Peak best;
+        best.p = 0.0f;
+        best.n = 0x7fffffff;
+        best.sum = 0.0f;
+#pragma unroll
+        for (int c4 = 0; c4 < 4; c4++) {
+            float2 za[4], zb[4], zc[4];
+            tmem_ld4(zaddr + 0 * 32 + 8 * c4, za);
+            tmem_ld4(zaddr + 1 * 32 + 8 * c4, zb);
+            tmem_ld4(zaddr + 2 * 32 + 8 * c4, zc);
+            tmem_wait_ld();
+#pragma unroll
+            for (int i = 0; i < 4; i++) {
+                const int n2 = 4 * c4 + i;
+                float2 z0 = za[i], z1 = zb[i], z2 = zc[i];
+                float2 z3 = cmul(x[r16(n2)], c_cC[3][n2]);
+                radix4_inv(z0, z1, z2, z3);  // z_m = sum_k2 z_k2 * j^{k2*m}
+                const float2 zz[4] = {z0, z1, z2, z3};
+#pragma unroll
+                for (int m = 0; m < 4; m++) {
+                    const int n = lag_of3(t, n2) + 4096 * m;
+                    const float pw = cpower(zz[m]);
+                    if (n < L) peak_merge(best, pw, n, pw);
+                }
+            }
+        }
+        const Peak tot = block_reduce_peak(best, red_f, red_i, t);
+        if (t == 0) store_cell(p, ti.cap, ti.slot, ti.d, tot, L);
+    }
+    __syncthreads();
+    search_cta_epilogue(p, t);
+    tmem_free_cta<kE1bTmemCols>(tmem_base, t);
+}
+
+#endif  // ACQ_VARIANT_E1B_LDG
 
 // ---------------------------------------------------------------------------------------------
 // K6.  Acquisition refinement for the hand-off to tracking (SURVEY 8(f) rank 4).  The search reports the code phase
@@ -2338,10 +2081,6 @@ static size_t search_e1b_smem_bytes() { return e1b_smem_bytes(); }
 static size_t search_e1b_cluster_smem_bytes() { return fft_smem3_bytes() + 2 * sizeof(float2) * kSub + 64 * sizeof(float); }
 static size_t fwd_smem_bytes() { return fft_smem3_bytes() + kZBytes; }
 
-#ifndef ACQ_CARVEOUT_MAX
-#define ACQ_CARVEOUT_MAX 1   // 0 (variant carve0): the driver's choice per kernel
-#endif
-
 // The search kernels of an aided search (AidedSearchArgs): the product forms only, with the shared-memory size and carveout
 // of their full-range instantiations.
 static cudaError_t aided_kernels_configure()
@@ -2355,9 +2094,7 @@ static cudaError_t aided_kernels_configure()
     cudaError_t e;
     for (int i = 0; i < 7; i++) {
         if ((e = cudaFuncSetAttribute(k[i], cudaFuncAttributeMaxDynamicSharedMemorySize, smem[i]))) return e;
-#if ACQ_CARVEOUT_MAX
         if ((e = cudaFuncSetAttribute(k[i], cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared))) return e;
-#endif
     }
     return cudaSuccess;
 }
@@ -2368,18 +2105,6 @@ cudaError_t search_kernels_configure()
     cudaError_t e;
     const int l1 = (int)search_l1_smem_bytes(), e1 = (int)search_e1b_smem_bytes(), fw = (int)fwd_smem_bytes();
     if ((e = cudaFuncSetAttribute(k_search_l1<false, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, l1))) return e;
-#if ACQ_DR_MIN_TILES_PER_SM >= 0
-    if ((e = cudaFuncSetAttribute(k_search_l1_dr, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dr_smem_bytes()))) return e;
-#endif
-#ifdef ACQ_VARIANT_L1_MST
-    if ((e = cudaFuncSetAttribute(k_search_l1_mst, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dr_smem_bytes()))) return e;
-#endif
-#ifdef ACQ_VARIANT_L1_SP
-    if ((e = cudaFuncSetAttribute(k_search_l1_sp, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sp_smem_bytes()))) return e;
-#endif
-#ifdef ACQ_VARIANT_L1_ST
-    if ((e = cudaFuncSetAttribute(k_search_l1_st, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)st_smem_bytes()))) return e;
-#endif
 #ifdef ACQ_VARIANT_L1_MULTI_TW
     if ((e = cudaFuncSetAttribute(k_search_l1<true, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, l1))) return e;
 #endif
@@ -2387,16 +2112,6 @@ cudaError_t search_kernels_configure()
     if ((e = cudaFuncSetAttribute(k_search_l1_cr<S>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)l1_multi_smem_bytes()))) return e;
     if ((e = cudaFuncSetAttribute(k_search_e1b<S>, cudaFuncAttributeMaxDynamicSharedMemorySize, e1))) return e;
     if ((e = cudaFuncSetAttribute(k_search_e1b_multi<S>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)e1b_multi_smem_bytes()))) return e;
-#ifdef ACQ_VARIANT_L1_X3
-    const int l1x = (int)search_l1_x3_smem();
-    if ((e = cudaFuncSetAttribute(k_search_l1_x3<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, l1x))) return e;
-    if ((e = cudaFuncSetAttribute(k_search_l1_x3<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, l1x))) return e;
-#endif
-#ifdef ACQ_VARIANT_L1_LDG
-    const int l1g = (int)(fft_smem3t_bytes() + 64 * sizeof(float));
-    if ((e = cudaFuncSetAttribute(k_search_l1_ldg<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, l1g))) return e;
-    if ((e = cudaFuncSetAttribute(k_search_l1_ldg<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, l1g))) return e;
-#endif
 #ifdef ACQ_VARIANT_E1B_LDG
     const int e1g = (int)(fft_smem3_bytes() + 64 * sizeof(float));
     if ((e = cudaFuncSetAttribute(k_search_e1b_ldg, cudaFuncAttributeMaxDynamicSharedMemorySize, e1g))) return e;
@@ -2413,22 +2128,17 @@ cudaError_t search_kernels_configure()
     // its SMs at the 196 KiB split and the E1B kernel (2 x 103.8 KiB) at 228 KiB, and an SM changes its split only when
     // it is empty: in a GPS + Galileo search the E1B CTAs -- launched to move in as the C/A CTAs retire -- entered no SM
     // before BOTH its C/A CTAs had gone (trace: first E1B CTA at 54.8 us although half the C/A CTAs leave by 50 us).
-#if ACQ_CARVEOUT_MAX
     const void *chain[] = {(const void *)k_front_end<false>, (const void *)k_front_end<true>, (const void *)k_front_end_arg,
                            (const void *)k_fwd_fft<true>, (const void *)k_fwd_fft<false>, (const void *)k_fwd_fft_cluster<true>,
                            (const void *)k_fwd_fft_cluster<false>, (const void *)k_search_l1<false, S>,
 #ifdef ACQ_VARIANT_L1_MULTI_TW
                            (const void *)k_search_l1<true, S>,
 #endif
-#if ACQ_DR_MIN_TILES_PER_SM >= 0
-                           (const void *)k_search_l1_dr,
-#endif
                            (const void *)k_search_l1_cr<S>, (const void *)k_search_l1_multi<S>, (const void *)k_search_e1b<S>,
                            (const void *)k_search_e1b_multi<S>, (const void *)k_search_e1b_cluster<false, S>,
                            (const void *)k_search_e1b_cluster<true, S>, (const void *)k_pick_small, (const void *)k_best_dop};
     for (const void *f : chain)
         if ((e = cudaFuncSetAttribute(f, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared))) return e;
-#endif
     return aided_kernels_configure();
 }
 
@@ -2505,39 +2215,26 @@ int launch_build_ext(const float2 *C, float2 *Ep, int n_sats, int Q, int ext_len
 // Which C/A search kernel a search runs: non-coherent sums -> k_search_l1_multi (code run resident in tensor memory);
 // K = 1 on full bins -> k_search_l1_cr (capture residue resident in tensor memory, chunks of tiles claimed); K = 1 on
 // half-bins -> k_search_l1<false> (odd and even half-bins read different capture spectra: nothing could stay resident).
-// k_search_l1_dr (one CTA per SM, two teams with staging warps, capture residue resident, contiguous team ranges) was the
-// K = 1 full-bin kernel for most of round 2: +4.7 % over k_search_l1<false> ON THE STATIC STRIDE (6.30 -> 6.02 ms,
-// 128-capture farm).  Most of that turned out to be the static stride's own loss -- the two CTAs of an SM run at
-// different rates (see claim_tile) -- which the two-team CTA happened not to have: with claimed tiles k_search_l1<false>
-// does the same farm in 5.78 ms, k_search_l1_dr in 5.96 ms, and k_search_l1_cr -- the resident capture residue in the
-// two-CTA form, residue loop fully unrolled at 126 registers -- in 5.24 ms (32.1 M tiles/s).  On the reference's
-// one-capture search: 70.9 us through acq_search against 75.4 us (k_search_l1<false>) and 77.5 us (k_search_l1_dr).
-// k_search_l1_dr is compiled only into variant libraries, for the equivalence tests and A/B runs: ACQ_DR_MIN_TILES_PER_SM
-// >= 0 (l1_dr_all = 0, l1_dr12 = 12) sends full-bin K = 1 searches of at least that many tiles per SM to it.
+// The K = 1 full-bin kernel for most of round 2 (one CTA per SM, two teams with staging warps, capture residue resident,
+// contiguous team ranges; since removed, DESIGN.md section 4) was +4.7 % over k_search_l1<false> ON THE STATIC STRIDE
+// (6.30 -> 6.02 ms, 128-capture farm).  Most of that turned out to be the static stride's own loss -- the two CTAs of an
+// SM run at different rates (see claim_tile) -- which the two-team CTA happened not to have: with claimed tiles
+// k_search_l1<false> does the same farm in 5.78 ms, the two-team kernel in 5.96 ms, and k_search_l1_cr -- the resident
+// capture residue in the two-CTA form, residue loop fully unrolled at 126 registers -- in 5.24 ms (32.1 M tiles/s).  On
+// the reference's one-capture search: 70.9 us through acq_search against 75.4 us (k_search_l1<false>) and 77.5 us (the
+// two-team kernel).
 #ifndef ACQ_FORCE_L1_CTA
 #define ACQ_FORCE_L1_CTA 0   // variant l1_cta: always k_search_l1<false> for K = 1 (the kernel-equivalence tests)
 #endif
-#ifndef ACQ_DR_MIN_TILES_PER_SM
-#define ACQ_DR_MIN_TILES_PER_SM -1   // product: never
-#endif
-constexpr int kDrMinTilesPerSm = ACQ_DR_MIN_TILES_PER_SM;
-#ifndef ACQ_L1_CR
-#define ACQ_L1_CR 1   // 0 (variant l1_nocr): full-bin K = 1 searches on k_search_l1<false>
-#endif
-bool search_claims_tiles(long long n_tiles, int grid);
-int search_kind_l1(int K, int half_bin, long long n_tiles, int sm_count)
+int search_kind_l1(int K, int half_bin)
 {
-#if defined(ACQ_VARIANT_L1_X3) || defined(ACQ_VARIANT_L1_LDG) || defined(ACQ_VARIANT_L1_MULTI_TW)
-    return kSearchL1;   // these experiment builds run every C/A search on their own 256-thread kernels
-#endif
-#ifdef ACQ_VARIANT_L1_MST
-    if (K > 1) return kSearchL1Mst;
+#ifdef ACQ_VARIANT_L1_MULTI_TW
+    return kSearchL1;   // this experiment build runs every C/A search on k_search_l1<MULTI>
 #endif
     if (K > 1) return kSearchL1Multi;
     if (half_bin || ACQ_FORCE_L1_CTA) return kSearchL1;
-    if (kDrMinTilesPerSm >= 0) return n_tiles < (long long)kDrMinTilesPerSm * sm_count ? kSearchL1 : kSearchL1Dr;
     // full bins: the capture-resident kernel (chunks claimed from six rounds of tiles per CTA up, static stride below)
-    return ACQ_L1_CR ? kSearchL1Cr : kSearchL1;
+    return kSearchL1Cr;
 }
 
 // Claimed tiles or the static stride?  Claiming evens out the two CTAs of an SM and the SMs among themselves, at the price
@@ -2591,26 +2288,7 @@ int search_grid_ctas(long long n_tiles, int kind, int sm_count)
     }
     long long cap = (long long)sm_count * 2;  // two persistent CTAs per SM
     if (kind == kSearchE1bCluster) cap = sm_count / 4;
-    if (kind == kSearchL1Dr || kind == kSearchL1Mst) cap = sm_count;   // one CTA per SM, two teams in it
-#ifdef ACQ_VARIANT_L1_X3
-    if (kind == kSearchL1) cap = (long long)sm_count * 3;
-#endif
     return (int)(n_tiles < cap ? n_tiles : cap);
-}
-
-// Which searches have an aided form: those that run on the product's search kernels (search_aided_supported).
-bool search_aided_supported(int K, int half_bin, long long tiles_l1, long long tiles_e1b, int sm_count)
-{
-#if defined(ACQ_VARIANT_L1_X3) || defined(ACQ_VARIANT_L1_LDG) || defined(ACQ_VARIANT_L1_MULTI_TW)
-    if (tiles_l1 > 0) return false;
-#endif
-#ifdef ACQ_VARIANT_E1B_LDG
-    if (tiles_e1b > 0) return false;
-#endif
-    (void)tiles_e1b;
-    if (tiles_l1 <= 0) return true;
-    const int kind = search_kind_l1(K, half_bin, tiles_l1, sm_count);
-    return kind == kSearchL1 || kind == kSearchL1Multi || kind == kSearchL1Cr;
 }
 
 // The aided instantiations of the product search kernels (launch_search with SearchArgs::dop_center set).
@@ -2634,7 +2312,7 @@ static int launch_search_aided(const AidedSearchArgs &a, int kind, int grid, boo
 
 int launch_search(const SearchArgs &a_in, bool e1b, int sm_count, cudaStream_t st, bool pdl)
 {
-    const int kind = e1b ? kSearchE1b : search_kind_l1(a_in.K, a_in.half_bin, a_in.n_tiles, sm_count);
+    const int kind = e1b ? kSearchE1b : search_kind_l1(a_in.K, a_in.half_bin);
     const int grid = search_grid_ctas(a_in.n_tiles, kind, sm_count);
     if (grid <= 0) return 0;
     SearchArgs a = a_in;
@@ -2650,31 +2328,14 @@ int launch_search(const SearchArgs &a_in, bool e1b, int sm_count, cudaStream_t s
 #endif
         return 1;
     }
-#if defined(ACQ_VARIANT_L1_X3)
-    launch_k(a.K > 1 ? k_search_l1_x3<true> : k_search_l1_x3<false>, grid, 256, search_l1_x3_smem(), st, pdl, a);
-#elif defined(ACQ_VARIANT_L1_LDG)
-    launch_k(a.K > 1 ? k_search_l1_ldg<true> : k_search_l1_ldg<false>, grid, 256, fft_smem3t_bytes() + 64 * sizeof(float), st,
-             pdl, a);
-#elif defined(ACQ_VARIANT_L1_MULTI_TW)   // the K > 1 form that keeps the stage-B twiddles (not the code run) in tensor memory
+#ifdef ACQ_VARIANT_L1_MULTI_TW   // the K > 1 form that keeps the stage-B twiddles (not the code run) in tensor memory
     launch_k(a.K > 1 ? k_search_l1<true, S> : k_search_l1<false, S>, grid, 256, search_l1_smem_bytes(), st, pdl, a);
 #else
-#ifdef ACQ_VARIANT_L1_MST
-    if (kind == kSearchL1Mst) launch_k(k_search_l1_mst, grid, kStThreads, dr_smem_bytes(), st, pdl, a);
-    else
-#endif
     if (a.K > 1) launch_k(k_search_l1_multi<S>, grid, 256, l1_multi_smem_bytes(), st, pdl, a);
     else if (kind == kSearchL1Cr) {
         search_chunks(a.n_tiles, 2 * sm_count, &a.ck_n16, &a.ck_n4);
         launch_k(k_search_l1_cr<S>, grid, 256, l1_multi_smem_bytes(), st, pdl, a);
     }
-#if defined(ACQ_VARIANT_L1_SP)
-    else if (kind == kSearchL1Dr) launch_k(k_search_l1_sp, grid, kSpThreads, sp_smem_bytes(), st, pdl, a);
-#elif defined(ACQ_VARIANT_L1_ST)
-    else if (kind == kSearchL1Dr) launch_k(k_search_l1_st, grid, kStThreads, st_smem_bytes(), st, pdl, a);
-#endif
-#if ACQ_DR_MIN_TILES_PER_SM >= 0
-    else if (kind == kSearchL1Dr) launch_k(k_search_l1_dr, grid, kStThreads, dr_smem_bytes(), st, pdl, a);
-#endif
     else launch_k(k_search_l1<false, S>, grid, 256, search_l1_smem_bytes(), st, pdl, a);
 #endif
     return 1;

@@ -107,10 +107,9 @@ int launch_pick_small(const acq_cell *cells, const int *slot_sat, acq_record *ou
                       unsigned *host_flag, unsigned epoch, int n_rows, int n_slots, int n_dop, PickDop pd, cudaStream_t st,
                       bool pdl = false);
 // CTAs of a search launch that store cells (what SearchArgs::ctas_total sums over the launches of one search)
-enum { kSearchL1 = 0, kSearchE1b = 1, kSearchE1bCluster = 2, kSearchL1Multi = 3, kSearchL1Dr = 4, kSearchL1Mst = 5, kSearchL1Cr = 6 };
-int search_kind_l1(int K, int half_bin, long long n_tiles, int sm_count);   // which C/A search kernel (and so which grid) a search uses
-// an aided search runs only on the product's search kernels: false where this library would pick another form
-bool search_aided_supported(int K, int half_bin, long long tiles_l1, long long tiles_e1b, int sm_count);
+// Search kernel kinds, reported as acq_launch_plan.kernel: the values are ABI (4 and 5 named kernels since removed)
+enum { kSearchL1 = 0, kSearchE1b = 1, kSearchE1bCluster = 2, kSearchL1Multi = 3, kSearchL1Cr = 6 };
+int search_kind_l1(int K, int half_bin);   // which C/A search kernel (and so which grid) a search uses
 constexpr int kPickSmallRowsMax = 256;  // rows k_pick_small stages in shared memory
 // A record as k_pick_small hands it to a POLLING host (mapped pinned memory): two 16-byte halves, each carrying the
 // search's epoch in its last word.  Each half arrives by one 16-byte store, so a host that sees the epoch in a half has

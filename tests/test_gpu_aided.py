@@ -191,31 +191,46 @@ def test_every_kernel_path(gpu_required):
     assert plan.kernel == 6 and plan.claims == 1 and plan.n_big > 0   # k_search_l1_cr, chunks claimed
 
 
+def aided_and_full(table, params, variant, caps, centers, hw, sel=None):
+    """Aided search of `caps` on a library variant; with `variant` set its window cells are asserted to be the variant's
+    own full grid, to the byte (a forced kernel choice)."""
+    with F.AcqEngine(table, params, variant=variant) as eng:
+        p = eng.params
+        _, full_g = eng.search(caps, sel=sel, want_grid=True)
+        rec, grid = eng.search_aided(caps, centers, hw, sel=sel, want_grid=True)
+    if variant is not None:
+        for c in range(grid.shape[0]):
+            for s in range(grid.shape[1]):
+                lo = window_lo(centers[c, s], hw, p.dop_lo, p.dop_hi) - p.dop_lo
+                assert grid[c, s].tobytes() == full_g[c, s, lo: lo + 2 * hw + 1].tobytes(), (variant, c, s)
+    return rec, grid
+
+
 def test_variant_libraries_agree(gpu_required):
     """The library variants run the aided search on their own kernel choices: each equals its own full search in the
-    window bytewise, and the C/A rows equal the product's bytes."""
+    window bytewise, and the C/A rows equal the product's bytes.  With K = 3, l1_multi_tw runs its full search on
+    k_search_l1<true> and its aided search on the product's k_search_l1_multi: the windows still agree."""
     table = scenarios.table("cfg4")
     caps = np.concatenate([synth.make_capture(70 + i, 1, table, scenarios.signals("cfg4", 70 + i)) for i in range(3)])
     sel = np.array([0, 3, 17, 31, 32, 40, 60, 81], np.int32)
     rng = np.random.default_rng(4)
     centers = rng.integers(-24, 25, (3, len(sel))).astype(np.int32)
     out = {}
-    for variant in (None, "l1_cta", "static_tiles", "dyn_tiles", "e1b_cta", "e1b_cluster"):
-        with F.AcqEngine(table, variant=variant) as eng:
-            _, full_g = eng.search(caps, sel=sel, want_grid=True)
-            rec, grid = eng.search_aided(caps, centers, 3, sel=sel, want_grid=True)
-            if variant is not None:   # a forced kernel choice: the window is the full grid's, to the byte
-                for c in range(3):
-                    for s in range(len(sel)):
-                        lo = window_lo(centers[c, s], 3, -20, 20)
-                        assert grid[c, s].tobytes() == full_g[c, s, lo + 20: lo + 27].tobytes(), (variant, c, s)
-            out[variant] = (rec, grid)
+    for variant in (None, "l1_cta", "l1_multi_tw", "static_tiles", "dyn_tiles", "e1b_cta", "e1b_cluster", "e1b_ldg"):
+        out[variant] = aided_and_full(table, F.default_params(), variant, caps, centers, 3, sel)
     ca = np.array([table[s][3] != S.E1B for s in sel])
-    for variant in ("l1_cta", "static_tiles", "dyn_tiles", "e1b_cta", "e1b_cluster"):
+    for variant in ("l1_cta", "l1_multi_tw", "static_tiles", "dyn_tiles", "e1b_cta", "e1b_cluster", "e1b_ldg"):
         assert out[variant][1][:, ca].tobytes() == out[None][1][:, ca].tobytes(), variant
         assert out[variant][0][:, ca].tobytes() == out[None][0][:, ca].tobytes(), variant
-    for variant in ("l1_cta", "static_tiles", "dyn_tiles"):
+    for variant in ("l1_cta", "l1_multi_tw", "static_tiles", "dyn_tiles"):
         assert out[variant][0].tobytes() == out[None][0].tobytes(), variant
+    nav = S.navstar()
+    kw = dict(k_noncoh=3, thr_l1=8.0)
+    caps3 = np.concatenate([synth.make_capture(80 + i, 3, nav, scenarios.signals("cfg1", 80 + i)) for i in range(2)])
+    centers3 = rng.integers(-24, 25, (2, len(nav))).astype(np.int32)
+    prod = aided_and_full(nav, F.default_params(**kw), None, caps3, centers3, 3)
+    tw = aided_and_full(nav, F.default_params(**kw), "l1_multi_tw", caps3, centers3, 3)
+    assert tw[0].tobytes() == prod[0].tobytes() and tw[1].tobytes() == prod[1].tobytes()
 
 
 def test_device_form_on_a_torch_stream(gpu_required):
@@ -294,10 +309,6 @@ def test_alternating_aided_and_full_searches(gpu_required):
         assert "pending" in str(ei.value)
         eng.wait()
         assert eng.search_aided(caps, centers, 4).tobytes() == a0.tobytes()
-    with F.AcqEngine(table, variant="l1_dr_all") as eng:   # k_search_l1_dr steps its own Doppler index: refused
-        with pytest.raises(F.AcqError) as ei:
-            eng.search_aided(caps[:8192], centers[:1], 1)
-        assert ei.value.code == -4
 
 
 def test_capture_farm_aided_equals_search_aided(gpu_required):

@@ -806,57 +806,37 @@ def test_code_doppler_compensation(gpu_required, oracle):
     assert rec[0]["dop"][1] == -39 and rec[0]["snr"][1] >= 5.0
 
 
-def test_three_cta_kernel_equals_two_cta_kernel(gpu_required, oracle):
-    """k_search_l1_x3 (three CTAs per SM: accumulators and block powers in tensor memory, operands from L2) against
-    k_search_l1 (two CTAs per SM, TMA-staged operands): the same arithmetic in the same order, so cells are bitwise
-    equal -- K = 1 with more tiles than resident CTAs, and K = 5 half-bin sums with code-Doppler copies."""
-    table = S.navstar()
-    cases = [({}, synth.make_capture(3, 1, table, scenarios.signals("cfg1", 3)), 40),
-             (dict(dop_lo=-60, dop_hi=60, half_bin=1, k_noncoh=5, thr_l1=5.0, code_doppler=1),
-              synth.make_capture(4, 5, table, scenarios.signals("cfg2", 2), code_doppler=True), 1)]
-    for kw, cap, reps in cases:
-        out = {}
-        for kind, variant in (("tma", None), ("x3", "l1_x3")):   # the product kernels against the variant library
-            with F.AcqEngine(table, F.default_params(**kw), variant=variant) as eng:
-                out[kind] = eng.search(np.concatenate([cap] * reps), want_grid=True)
-        (ra, ga), (rb, gb) = out["tma"], out["x3"]
-        for f in ("peak", "lag", "noise", "snr"):
-            assert np.array_equal(ga[f], gb[f]), f
-        assert ra.tobytes() == rb.tobytes()
-        assert (ga[0] == ga[-1]).all()
-
-
 def test_capture_resident_kernel_equals_cta_kernel(gpu_required, oracle):
     """k_search_l1_cr (the K = 1 full-bin product kernel: two CTAs per SM, the capture residue parked in tensor memory,
     chunks of 16 / 4 / 1 consecutive tiles claimed from a counter once a launch has six rounds of tiles, the static stride
-    below) and k_search_l1_dr (one CTA per SM, two teams of FFT warps with a staging warp each,
-    contiguous tile ranges, the capture residue parked in tensor memory for all tiles of a capture) against
-    k_search_l1<false> (two CTAs per SM striding over the tiles, both operands staged per sub-FFT; variant library l1_cta):
-    the same arithmetic in the same order, so the whole per-Doppler table is bitwise equal.  Shapes: one capture (every team
-    starts inside the capture), 40 captures (capture boundaries inside team ranges), 600 two-tile captures (several
-    boundaries per range, alternating captures so that a residue left over from the neighbour would show), fewer tiles than
-    SMs (one team per SM), a single tile."""
+    below) against k_search_l1<false> (two CTAs per SM striding over the tiles, both operands staged per sub-FFT; variant
+    library l1_cta): the same arithmetic in the same order, so the whole per-Doppler table is bitwise equal.  Shapes: one
+    capture, 40 captures (capture boundaries inside chunks), one capture 40 times (more tiles than resident CTAs; every
+    copy's table equals the first's), 600 two-tile captures (several boundaries per chunk, alternating captures so that a
+    residue left over from the neighbour would show), fewer tiles than SMs, a single tile."""
     table = S.navstar()
     cap = synth.make_capture(3, 1, table, scenarios.signals("cfg1", 3))
     cap2 = synth.make_capture(5, 1, table, scenarios.signals("cfg1", 5))
-    cases = [({}, [cap], None), ({}, [cap, cap2] * 20, None),
+    cases = [({}, [cap], None), ({}, [cap, cap2] * 20, None), ({}, [cap] * 40, None),
              (dict(dop_lo=3, dop_hi=4), [cap, cap2] * 300, np.array([2], np.int32)),
              (dict(dop_lo=-3, dop_hi=1), [cap2], np.array([2], np.int32)),
              (dict(dop_lo=0, dop_hi=0), [cap], np.array([6], np.int32)),
              (dict(dop_lo=-20, dop_hi=20), [cap2, cap], np.array([2, 6, 10, 13, 18], np.int32))]
     for kw, caps, sel in cases:
         out = {}
-        # product: k_search_l1_cr (claiming from six rounds of tiles); l1_dr_all: k_search_l1_dr at every size
+        # product: k_search_l1_cr (claiming from six rounds of tiles)
         # cr: k_search_l1_cr (capture resident, chunks of tiles claimed) at every size -- the variant that always claims
-        for kind, variant in (("product", None), ("dr", "l1_dr_all"), ("cr", "dyn_tiles"), ("cta", "l1_cta")):
+        for kind, variant in (("product", None), ("cr", "dyn_tiles"), ("cta", "l1_cta")):
             with F.AcqEngine(table, F.default_params(**kw), variant=variant) as eng:
                 out[kind] = eng.search(np.concatenate(caps), sel=sel, want_grid=True)
         rb, gb = out["cta"]
-        for kind in ("product", "dr", "cr"):
+        for kind in ("product", "cr"):
             ra, ga = out[kind]
             for f in ("peak", "lag", "noise", "snr"):
                 assert np.array_equal(ga[f], gb[f]), (kind, kw, len(caps), f)
             assert ra.tobytes() == rb.tobytes(), kind
+        if all(c is caps[0] for c in caps):   # one capture repeated: every copy's table is the first's
+            assert (out["product"][1][0] == out["product"][1][-1]).all()
     # half-bin K = 1 searches stay on k_search_l1<false> (odd and even half-bins read different capture spectra)
     with F.AcqEngine(table, F.default_params(half_bin=1, dop_lo=-9, dop_hi=9)) as eng:
         rec, grid = eng.search(cap, want_grid=True)
@@ -868,23 +848,23 @@ def test_code_resident_multi_kernel_equals_twiddle_resident_kernel(gpu_required,
     """k_search_l1_multi (K > 1: the tile's code run parked in tensor memory after block 0, stage-B twiddles from a
     shared-memory table) against k_search_l1<true> (twiddles in tensor memory, code run staged for every block; variant
     library l1_multi_tw): the same arithmetic in the same order, so the whole per-Doppler table is bitwise equal --
-    K = 20 half-bins (cfg2), and K = 3 full bins over three captures with an asymmetric Doppler range."""
+    K = 20 half-bins (cfg2), K = 3 full bins over three captures with an asymmetric Doppler range, and K = 5 half-bins
+    with code-Doppler copies."""
     table = S.navstar()
     cases = [(scenarios.params_kw("cfg2"), synth.make_capture(26, 20, table, scenarios.signals("cfg2", 6)), 1),
-             (dict(dop_lo=-7, dop_hi=30, k_noncoh=3, thr_l1=8.0), synth.make_capture(27, 3, table, scenarios.signals("cfg1", 7)), 3)]
+             (dict(dop_lo=-7, dop_hi=30, k_noncoh=3, thr_l1=8.0), synth.make_capture(27, 3, table, scenarios.signals("cfg1", 7)), 3),
+             (dict(dop_lo=-60, dop_hi=60, half_bin=1, k_noncoh=5, thr_l1=5.0, code_doppler=1),
+              synth.make_capture(4, 5, table, scenarios.signals("cfg2", 2), code_doppler=True), 1)]
     for kw, cap, reps in cases:
         out = {}
-        # product: k_search_l1_multi; l1_mst: its two-team form with staging warps (experiment, no gain); l1_multi_tw:
-        # k_search_l1<true>
-        for kind, variant in (("code", None), ("cta", "l1_mst"), ("tw", "l1_multi_tw")):
+        # product: k_search_l1_multi; l1_multi_tw: k_search_l1<true>
+        for kind, variant in (("code", None), ("tw", "l1_multi_tw")):
             with F.AcqEngine(table, F.default_params(**kw), variant=variant) as eng:
                 out[kind] = eng.search(np.concatenate([cap] * reps), want_grid=True)
-        (ra, ga) = out["code"]
-        for other in ("cta", "tw"):
-            rb, gb = out[other]
-            for f in ("peak", "lag", "noise", "snr"):
-                assert np.array_equal(ga[f], gb[f]), (other, f)
-            assert ra.tobytes() == rb.tobytes(), other
+        (ra, ga), (rb, gb) = out["code"], out["tw"]
+        for f in ("peak", "lag", "noise", "snr"):
+            assert np.array_equal(ga[f], gb[f]), (kw, f)
+        assert ra.tobytes() == rb.tobytes(), kw
         assert (ga[0] == ga[-1]).all()
 
 

@@ -1,6 +1,6 @@
 #!/usr/bin/env python3
 """Bitwise A/B of a variant library against the product on K = 1 C/A searches of several shapes (GPU).
-    python tools/ab_equal.py l1_sp"""
+    python tools/ab_equal.py l1_cta"""
 import os
 import sys
 

@@ -2,7 +2,7 @@
 """Build experiment variants of libacq_b200.so next to the product library (flydog_sdr_gps_b200/csrc/variants/).
 
     python tools/build_variants.py                 every named variant of flydog_sdr_gps_b200/_build.py VARIANTS
-    python tools/build_variants.py l1_x3 e1b_cta   the named ones
+    python tools/build_variants.py l1_cta e1b_cta  the named ones
     python tools/build_variants.py name=DEF1,DEF2  an ad-hoc variant with the given -D defines (name= alone: none)
 """
 import concurrent.futures as cf

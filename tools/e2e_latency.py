@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Host-side latency of acq_search() (C ABI, host buffers) for single-capture searches, per library variant.
     python tools/e2e_latency.py [variant|product ...]     (configs cfg1 cfg4 cfg3, and one satellite = the literal SearchTask step)
-    E2E_CAPS=2,4: additionally cfg1 searches of that many captures per call (where k_search_l1_dr takes over)"""
+    E2E_CAPS=2,4: additionally cfg1 searches of that many captures per call (where k_search_l1_cr starts claiming chunks of tiles)"""
 import os
 import sys
 import time

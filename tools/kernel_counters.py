@@ -42,7 +42,7 @@ def main():
             "issue_active_pct": val(d, "smsp__issue_active.avg.pct_of_peak_sustained_active"),
             "registers": int(val(d, "launch__registers_per_thread")),
         }
-    out["cfg4"] = {"note": "cfg4 runs k_search_l1_dr (cfg1's) and k_search_e1b (cfg3's) back to back"}
+    out["cfg4"] = {"note": "cfg4 runs k_search_l1_cr (cfg1's) and k_search_e1b (cfg3's) back to back"}
     json.dump(out, open(os.path.join(ROOT, "profiles", "r2_kernel_counters.json"), "w"), indent=1, sort_keys=True)
     for k, v in out.items():
         if isinstance(v, dict) and "tiles" in v:

@@ -55,12 +55,6 @@ for cfg in sys.argv[1:] or ["cfg1"]:
             print("  %s exit deciles:" % name, " ".join("%.1f" % v for v in np.percentile(xs, range(0, 101, 10))))
             ex_all = (tr[k][used][:, 2] - start) / 1e3
             print("  %s exit by CTA index (every 8th):" % name, " ".join("%.0f" % v for v in ex_all[::8]))
-            if (tr[k][512:, 3] > 0).any():   # k_search_l1_dr: team 0 done at [cta][3], team 1 done at [512 + cta][3]
-                t0 = (tr[k][:512, 3][tr[k][:512, 3] > 0] - start) / 1e3
-                t1 = (tr[k][512:, 3][tr[k][512:, 3] > 0] - start) / 1e3
-                print("  %s team 0 done deciles:" % name, " ".join("%.0f" % v for v in np.percentile(t0, range(0, 101, 10))))
-                print("  %s team 1 done deciles:" % name, " ".join("%.0f" % v for v in np.percentile(t1, range(0, 101, 10))))
-                print("  %s team1 - team0 per CTA (every 8th):" % name, " ".join("%.0f" % v for v in (t1 - t0)[::8]))
             m3 = (tr[k][used][:, 3] - start) / 1e3
             if (tr[k][used][:, 3] > 0).any():
                 print("  %s mark3 by CTA index (every 8th):" % name, " ".join("%.0f" % v for v in m3[::8]))
