@@ -140,6 +140,10 @@ struct acq_engine {
     acq_fine *d_fine = nullptr;
     size_t cap_ref_rec = 0, cap_fine = 0;
     int last_captures = 0;  // 0: no search whose spectra are still on the device
+    // shape of the most recent search of either path (acq_refine_device): captures (0: none whose spectra are still on
+    // the device), slots, and its slot -> satellite map on the device
+    int ref_captures = 0, ref_slots = 0;
+    const int *ref_slot_sat = nullptr;
     // aided host search (acq_search_aided): Doppler centres staged in pinned memory, copied to the device with the capture
     int32_t *h_center = nullptr;
     size_t cap_h_center = 0;
@@ -529,6 +533,25 @@ int poll_records(acq_engine *e, acq_record *out, size_t rows)
     return ACQ_OK;
 }
 
+// After a search of either path is enqueued: the shape acq_refine_device checks its call and its records against.
+void set_refine_shape(acq_engine *e, int n_captures)
+{
+    e->ref_captures = n_captures;
+    e->ref_slots = e->n_slots;
+    e->ref_slot_sat = e->cur_slot_sat;
+}
+
+int enqueue_refine(acq_engine *e, const acq_record *rec_dev, int n_records, int flags, acq_fine *out_dev,
+                   const int *slot_sat, int n_slots, cudaStream_t st)
+{
+    e->launches += launch_refine(e->d_Dp, e->d_Ep, rec_dev, e->d_sat_type, slot_sat, out_dev, n_records, n_slots,
+                                 e->prm.k_noncoh, e->nvar, e->prm.half_bin, e->ext_len, e->Q, e->n_shift, e->smax,
+                                 e->cd_div, (int)e->sats.size(), e->prm.dop_lo, e->prm.dop_hi, e->prm.thr_l1,
+                                 e->prm.thr_e1b, flags, st);
+    CU(cudaGetLastError());
+    return ACQ_OK;
+}
+
 // center (HOST, one per row) and half_width: an aided search (acq_search_aided), or NULL for the whole range
 int search_host(acq_engine *e, const uint8_t *packed, int n_captures, const int32_t *sel, int n_sel, acq_record *out,
                 acq_cell *grid, bool sync, const int32_t *center = nullptr, int half_width = 0)
@@ -537,6 +560,7 @@ int search_host(acq_engine *e, const uint8_t *packed, int n_captures, const int3
     if (rc) return rc;
     DeviceGuard g(e->device);
     e->last_captures = 0;  // until this search is enqueued, there are no spectra acq_refine could use
+    e->ref_captures = 0;
     const int n_dop = row_dops(e, center, half_width);
     if ((rc = set_selection(e, sel, n_sel))) return rc;
     if ((rc = check_tile_count(e, n_captures, n_dop))) return rc;
@@ -578,6 +602,7 @@ int search_host(acq_engine *e, const uint8_t *packed, int n_captures, const int3
                              half_width)))
         return rc;
     e->last_captures = n_captures;
+    set_refine_shape(e, n_captures);
     if (!host_records) CU(cudaMemcpyAsync(out, e->d_records, rows * sizeof(acq_record), cudaMemcpyDeviceToHost, e->stream));
     if (grid)
         CU(cudaMemcpyAsync(grid, e->d_cells, rows * n_dop * sizeof(acq_cell), cudaMemcpyDeviceToHost, e->stream));
@@ -618,12 +643,14 @@ int search_device(acq_engine *e, const uint8_t *packed_dev, int n_captures, cons
         return fail(ACQ_ERR_ARG, "packed_dev must be 16-byte aligned (the front end stages it with bulk async copies)");
     DeviceGuard g(e->device);
     e->last_captures = 0;  // spectra now belong to a search on the caller's stream: acq_refine does not apply
+    e->ref_captures = 0;   // ... and acq_refine_device applies once this search is enqueued
     const int n_dop = row_dops(e, center_dev, half_width);
     if ((rc = set_selection(e, sel, n_sel))) return rc;
     if ((rc = check_tile_count(e, n_captures, n_dop))) return rc;
     if ((rc = ensure_scratch(e, n_captures, e->n_slots, false, n_dop))) return rc;
     cudaStream_t st = stream ? (cudaStream_t)stream : e->stream;
     if ((rc = enqueue_search(e, packed_dev, n_captures, out_dev, nullptr, st, nullptr, center_dev, half_width))) return rc;
+    set_refine_shape(e, n_captures);
     if (st != e->stream) {  // whatever uses the engine's scratch next (any stream, or the host) waits for this search
         CU(cudaEventRecord(e->dev_done, st));
         e->dev_pending = true;
@@ -969,12 +996,40 @@ int acq_refine(acq_engine *e, const acq_record *rec, int n_records, acq_fine *ou
     if (rc) return rc;
     if ((rc = grow(e, e->d_fine, e->cap_fine, (size_t)n_records))) return rc;
     CU(cudaMemcpyAsync(e->d_ref_rec, rec, (size_t)n_records * sizeof(acq_record), cudaMemcpyHostToDevice, e->stream));
-    e->launches += launch_refine(e->d_Dp, e->d_Ep, e->d_ref_rec, e->d_sat_type, e->d_fine, n_records, e->n_slots,
-                                 e->prm.k_noncoh, e->nvar, e->prm.half_bin, e->ext_len, e->Q, e->n_shift, e->smax,
-                                 e->cd_div, e->stream);
-    CU(cudaGetLastError());
+    // the records are checked above, so the kernel's own checks pass every row
+    if ((rc = enqueue_refine(e, e->d_ref_rec, n_records, 0, e->d_fine, e->cur_slot_sat, e->n_slots, e->stream))) return rc;
     CU(cudaMemcpyAsync(out, e->d_fine, (size_t)n_records * sizeof(acq_fine), cudaMemcpyDeviceToHost, e->stream));
     CU(cudaStreamSynchronize(e->stream));
+    return ACQ_OK;
+}
+
+int acq_refine_device(acq_engine *e, const acq_record *rec_dev, int n_records, int flags, acq_fine *out_dev, void *stream)
+{
+    if (!e) return fail(ACQ_ERR_ARG, "engine is NULL");
+    if (!rec_dev || !out_dev) return fail(ACQ_ERR_ARG, "rec_dev/out_dev must not be NULL");
+    if (flags & ~ACQ_REFINE_DETECTED) return fail(ACQ_ERR_ARG, "unknown flag bits 0x%x", (unsigned)(flags & ~ACQ_REFINE_DETECTED));
+    if (e->ref_captures <= 0) return fail(ACQ_ERR_ARG, "no search whose spectra are still on the device to refine");
+    if (e->pending) return fail(ACQ_ERR_ARG, "a submitted search is still pending: call acq_wait first");
+    const long long rows = (long long)e->ref_captures * e->ref_slots;
+    if (n_records != rows)
+        return fail(ACQ_ERR_ARG, "n_records=%d but the last search produced %lld records", n_records, rows);
+    if (((uintptr_t)out_dev & 15) != 0) return fail(ACQ_ERR_ARG, "out_dev must be 16-byte aligned (one 16-byte store per row)");
+    if (((uintptr_t)rec_dev & 3) != 0) return fail(ACQ_ERR_ARG, "rec_dev must be 4-byte aligned");
+    DeviceGuard g(e->device);
+    cudaStream_t st = stream ? (cudaStream_t)stream : e->stream;
+    // after the search that left the spectra: a device-path search on another stream is behind dev_done, anything
+    // else on the engine stream
+    if (e->dev_pending) CU(cudaStreamWaitEvent(st, e->dev_done, 0));
+    if (st != e->stream) {
+        CU(cudaEventRecord(e->dev_done, e->stream));
+        CU(cudaStreamWaitEvent(st, e->dev_done, 0));
+    }
+    int rc = enqueue_refine(e, rec_dev, n_records, flags, out_dev, e->ref_slot_sat, e->ref_slots, st);
+    if (rc) return rc;
+    if (st != e->stream) {  // the next search overwrites the spectra: whatever touches the scratch next waits for this
+        CU(cudaEventRecord(e->dev_done, st));
+        e->dev_pending = true;
+    }
     return ACQ_OK;
 }
 

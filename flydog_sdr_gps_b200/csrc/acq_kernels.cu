@@ -1944,14 +1944,21 @@ __global__ void __launch_bounds__(256, 2) k_search_e1b_ldg(const SearchArgs p)
 //   code   : eps = slope (l - e) / (l + e),  e/l = Re(r[n-+1] conj(r[n]))       (early-minus-late over the
 //            correlation triangle: 4 samples per chip -> slope 3; BOC(1,1) main peak -> slope 1/3),
 // each summed over the K blocks.  One CTA per record; thread t owns k1 = t + 256 i for all four residues.
+// The records may come from device memory the host never saw (acq_refine_device), so each CTA checks its own record
+// first -- the checks of acq_refine, in the same order, the satellite's range before sat_type is indexed with it -- and
+// a CTA whose record fails one, or that ACQ_REFINE_DETECTED skips, writes a marker row and exits before any load of
+// the spectra (a uniform branch: every thread reads the same record).
 // ---------------------------------------------------------------------------------------------
 struct RefineArgs {
     const float2 *Dp;
     const float2 *Ep;
     const acq_record *rec;   // [n_rows], row = cap * n_slots + slot
     const int *sat_type;     // [n_sats]
+    const int *slot_sat;     // [n_slots] satellite searched in each slot
     acq_fine *out;
     int n_slots, K, nvar, half_bin, ext_len, Q, n_shift, smax, cd_div;
+    int n_sats, dop_lo, dop_hi, flags;
+    float thr_l1, thr_e1b;
 };
 
 __global__ void __launch_bounds__(256) k_refine(const RefineArgs p)
@@ -1960,7 +1967,28 @@ __global__ void __launch_bounds__(256) k_refine(const RefineArgs p)
     const int row = blockIdx.x, t = threadIdx.x;
     const acq_record rc = p.rec[row];
     const int cap = row / p.n_slots;
-    const bool e1b = p.sat_type[rc.sat] == ACQ_E1B;
+    int marker = 0;   // -2: the record fails a check, -1: skipped below the detection threshold
+    bool e1b = false;
+    if (rc.sat < 0 || rc.sat >= p.n_sats || rc.sat != p.slot_sat[row % p.n_slots]) {
+        marker = -2;
+    } else {
+        e1b = p.sat_type[rc.sat] == ACQ_E1B;
+        const int L = e1b ? ACQ_LAGS_E1B : ACQ_LAGS_L1;
+        if (rc.lag < 0 || rc.lag >= L) marker = -2;
+        // a row that never exceeded snr 0 carries dop 0 (k_best_dop), which may lie outside an asymmetric range
+        else if ((rc.dop < p.dop_lo || rc.dop > p.dop_hi) && !(rc.dop == 0 && rc.snr == 0.0f)) marker = -2;
+        else if ((p.flags & ACQ_REFINE_DETECTED) && !(rc.snr >= (e1b ? p.thr_e1b : p.thr_l1))) marker = -1;
+    }
+    if (marker != 0) {
+        if (t == 0) {
+            acq_fine o;
+            o.dop_hz = o.code_fs = __int_as_float(0x7fc00000);   // quiet NaN
+            o.peak = 0.0f;
+            o.ca_shift = marker;
+            p.out[row] = o;
+        }
+        return;
+    }
     const int v = p.half_bin ? (rc.dop & 1) : 0;
     const int dop = p.half_bin ? ((rc.dop - v) >> 1) : rc.dop;
     const int n = rc.lag;
@@ -2354,12 +2382,14 @@ int launch_search_e1b_cluster(const SearchArgs &a, int sm_count, cudaStream_t st
     return 1;
 }
 
-int launch_refine(const float2 *Dp, const float2 *Ep, const acq_record *rec, const int *sat_type, acq_fine *out, int n_rows,
-                  int n_slots, int K, int nvar, int half_bin, int ext_len, int Q, int n_shift, int smax, int cd_div,
+int launch_refine(const float2 *Dp, const float2 *Ep, const acq_record *rec, const int *sat_type, const int *slot_sat,
+                  acq_fine *out, int n_rows, int n_slots, int K, int nvar, int half_bin, int ext_len, int Q, int n_shift,
+                  int smax, int cd_div, int n_sats, int dop_lo, int dop_hi, float thr_l1, float thr_e1b, int flags,
                   cudaStream_t st)
 {
     if (n_rows <= 0) return 0;
-    RefineArgs a{Dp, Ep, rec, sat_type, out, n_slots, K, nvar, half_bin, ext_len, Q, n_shift, smax, cd_div};
+    RefineArgs a{Dp, Ep, rec, sat_type, slot_sat, out, n_slots, K, nvar, half_bin, ext_len, Q, n_shift, smax, cd_div,
+                 n_sats, dop_lo, dop_hi, flags, thr_l1, thr_e1b};
     k_refine<<<n_rows, 256, 0, st>>>(a);
     return 1;
 }

@@ -127,9 +127,12 @@ bool search_claims_tiles(long long n_tiles, int grid);   // tiles claimed from a
 void search_chunks(long long n_tiles, int grid, unsigned *n_big, unsigned *n_mid);
 long long search_chunk_count(long long n_tiles, int grid);
 void search_chunk_lengths(int *big, int *mid);
-// refinement of the records of the most recent search (one CTA per record)
-int launch_refine(const float2 *Dp, const float2 *Ep, const acq_record *rec, const int *sat_type, acq_fine *out, int n_rows,
-                  int n_slots, int K, int nvar, int half_bin, int ext_len, int Q, int n_shift, int smax, int cd_div,
+// refinement of the records of the most recent search (one CTA per record).  Each CTA checks its record against the
+// search's shape (slot_sat, n_sats, dop_lo..dop_hi) and writes a marker row for one that fails (ca_shift -2) or, with
+// ACQ_REFINE_DETECTED in flags, for one below its satellite type's threshold (ca_shift -1)
+int launch_refine(const float2 *Dp, const float2 *Ep, const acq_record *rec, const int *sat_type, const int *slot_sat,
+                  acq_fine *out, int n_rows, int n_slots, int K, int nvar, int half_bin, int ext_len, int Q, int n_shift,
+                  int smax, int cd_div, int n_sats, int dop_lo, int dop_hi, float thr_l1, float thr_e1b, int flags,
                   cudaStream_t st);
 cudaError_t search_kernels_configure();
 

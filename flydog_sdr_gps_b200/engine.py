@@ -15,6 +15,7 @@ BIN_HZ = 249.755859375
 LAGS_L1 = 4092
 LAGS_E1B = 16368
 WRAP_REFERENCE, WRAP_CIRCULAR = 0, 1
+REFINE_DETECTED = 1   # ACQ_REFINE_DETECTED
 
 RECORD_DTYPE = np.dtype([("sat", "<i4"), ("lag", "<i4"), ("dop", "<i4"),
                          ("peak", "<f4"), ("noise", "<f4"), ("snr", "<f4")])
@@ -211,6 +212,13 @@ class AcqEngine:
         out = np.zeros(r.shape, FINE_DTYPE)
         _check(self._L.acq_refine(self._h, r.ctypes.data, r.size, out.ctypes.data), self._L)
         return out
+
+    def refine_device(self, rec_dev, out_dev, n_records, detected_only=False, stream_ptr=None):
+        """acq_refine_device: rec_dev (acq_record) / out_dev (acq_fine, 16-byte aligned) are device pointers (ints) of
+        n_records rows of the most recent search of either path.  Enqueues one kernel on stream_ptr (None = engine
+        stream).  detected_only: rows below their detection threshold are marked (ca_shift -1), not refined."""
+        flags = REFINE_DETECTED if detected_only else 0
+        _check(self._L.acq_refine_device(self._h, rec_dev, int(n_records), flags, out_dev, stream_ptr), self._L)
 
     def detected(self, records):
         """Detection rule of SearchTask (search.cpp:549,591) applied to a record array."""

@@ -9,18 +9,21 @@ Doppler) tiles share nothing but read-only inputs, and the only cross-tile step 
 Both keep their buffers for the life of the object (pinned host staging, device captures, device records, the gathered
 record array), so a search is: host->device copy of the local captures, acq_search_device on the current torch stream,
 all_gather_into_tensor of the 24-byte records over NCCL, device->host copy of the gathered array.  `search_resident`
-is the same without the two copies (captures already in HBM, records left there).
+is the same without the two copies (captures already in HBM, records left there).  `refine` / `refine_resident` do the
+same for the hand-off refinement of those records (acq_refine_device on each rank, then the 16-byte fine records gathered
+the same way).
 
 `engine` is an AcqEngine.  The CPU suite exercises the same classes under gloo with a stand-in whose
-`search_device(...)` runs the oracle on CPU tensors; nothing in this module computes a search itself.
+`search_device(...)` and `refine_device(...)` run the oracle on CPU tensors; nothing in this module computes a search itself.
 The function forms below (`search_sharded_by_*`) are the numpy/host-gather variant of the same plumbing.
 """
 import numpy as np
 
-from .engine import RECORD_DTYPE
+from .engine import FINE_DTYPE, RECORD_DTYPE
 from .scenarios import shard
 
 REC = RECORD_DTYPE.itemsize
+FINE = FINE_DTYPE.itemsize
 
 
 class _Farm:
@@ -37,6 +40,7 @@ class _Farm:
         self.counts = [shard(n_units, r, self.world)[1] - shard(n_units, r, self.world)[0] for r in range(self.world)]
         self.max_local = max(self.counts)
         self.pin = self.device.type == "cuda"
+        self.d_fine = None
 
     def _empty(self, n, device=None, pin=False):
         t = self.torch.zeros(max(n, 1), dtype=self.torch.uint8, device=device or self.device)
@@ -45,16 +49,41 @@ class _Farm:
     def _stream_ptr(self):
         return self.torch.cuda.current_stream().cuda_stream if self.device.type == "cuda" else None
 
-    def _gather(self):
-        """Padded all_gather of the local record bytes; afterwards self.d_all holds every rank's slot."""
+    def _gather(self, out, local):
+        """Padded all_gather of local bytes (records or fine records); afterwards `out` holds every rank's slot."""
         if self.world > 1:
-            self.dist.all_gather_into_tensor(self.d_all, self.d_rec)
+            self.dist.all_gather_into_tensor(out, local)
 
-    def _unpad(self, host_bytes, per_unit):
-        """host_bytes: uint8 numpy [world * max_local * per_unit * REC] -> records in unit order."""
-        slot = self.max_local * per_unit * REC
-        parts = [host_bytes[r * slot: r * slot + self.counts[r] * per_unit * REC] for r in range(self.world)]
-        return np.concatenate(parts).view(RECORD_DTYPE)
+    def _unpad(self, host_bytes, per_unit, dtype=RECORD_DTYPE):
+        """host_bytes: uint8 numpy [world * max_local * per_unit * dtype.itemsize] -> items in unit order."""
+        size = dtype.itemsize
+        slot = self.max_local * per_unit * size
+        parts = [host_bytes[r * slot: r * slot + self.counts[r] * per_unit * size] for r in range(self.world)]
+        return np.concatenate(parts).view(dtype)
+
+    def refine_resident(self, detected_only=True):
+        """Hand-off refinement of the local records of the last search_resident() (acq_refine_device on the current torch
+        stream) into a local fine buffer padded like d_rec, then the same padded gather; returns the gathered 16-byte
+        fine records.  detected_only: undetected rows carry the marker ca_shift = -1 instead of values.  Asynchronous."""
+        if self.d_fine is None:   # allocated on first use: a farm that never refines keeps no fine buffers
+            n = self.max_local * self.per_unit * FINE
+            self.d_fine = self._empty(n)
+            self.d_fine_all = self._empty(self.world * n) if self.world > 1 else self.d_fine
+            self.h_fine_all = self._empty(self.d_fine_all.numel(), device="cpu", pin=self.pin)
+        if self.n_local:
+            self.eng.refine_device(self.d_rec.data_ptr(), self.d_fine.data_ptr(), self.n_local * self.per_unit,
+                                   detected_only=detected_only, stream_ptr=self._stream_ptr())
+        self._gather(self.d_fine_all, self.d_fine)
+        return self.d_fine_all
+
+    def refine(self, detected_only=True):
+        """refine_resident, copy out, wait.  Returns a FINE_DTYPE array shaped like search()'s records (numpy view of the
+        pinned result buffer: valid until the next refine)."""
+        self.refine_resident(detected_only)
+        self.h_fine_all.copy_(self.d_fine_all, non_blocking=True)
+        if self.device.type == "cuda":
+            self.torch.cuda.current_stream().synchronize()
+        return self._unpad(self.h_fine_all.numpy(), self.per_unit, FINE_DTYPE).reshape(self.records_shape)
 
 
 class CaptureFarm(_Farm):
@@ -67,6 +96,7 @@ class CaptureFarm(_Farm):
     def __init__(self, engine, n_captures, capture_bytes, n_sel, dist=None, device=None, half_width=None):
         super().__init__(engine, n_captures, dist, device)
         self.capture_bytes, self.n_sel = capture_bytes, n_sel
+        self.per_unit, self.records_shape = n_sel, (n_captures, n_sel)
         self.half_width = half_width
         self.h_in = self._empty(self.n_local * capture_bytes, device="cpu", pin=self.pin)
         self.d_in = self._empty(self.n_local * capture_bytes)
@@ -104,7 +134,7 @@ class CaptureFarm(_Farm):
                                          self.n_local, stream_ptr=self._stream_ptr())
         elif self.n_local:
             self.eng.search_device(self.d_in.data_ptr(), self.d_rec.data_ptr(), self.n_local, stream_ptr=self._stream_ptr())
-        self._gather()
+        self._gather(self.d_all, self.d_rec)
         return self.d_all
 
     def search(self):
@@ -135,6 +165,7 @@ class SatFarm(_Farm):
     def __init__(self, engine, n_sats, capture_bytes, dist=None, device=None):
         super().__init__(engine, n_sats, dist, device)
         self.capture_bytes = capture_bytes
+        self.per_unit, self.records_shape = 1, (n_sats,)
         self.sel = np.arange(self.lo, self.hi, dtype=np.int32)
         self.h_in = self._empty(capture_bytes, device="cpu", pin=self.pin)
         self.d_in = self._empty(capture_bytes)
@@ -151,7 +182,7 @@ class SatFarm(_Farm):
     def search_resident(self):
         if self.n_local:
             self.eng.search_device(self.d_in.data_ptr(), self.d_rec.data_ptr(), 1, sel=self.sel, stream_ptr=self._stream_ptr())
-        self._gather()
+        self._gather(self.d_all, self.d_rec)
         return self.d_all
 
     def search(self):

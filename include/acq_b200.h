@@ -221,6 +221,31 @@ int acq_wait(acq_engine *e);
  * table / Doppler range. */
 int acq_refine(acq_engine *e, const acq_record *rec, int n_records, acq_fine *out);
 
+/* Device-resident refinement: the same values as acq_refine, for the records of the MOST RECENT search of EITHER path
+ * (acq_search, acq_search_grid, acq_search_aided, acq_submit after acq_wait, acq_search_device,
+ * acq_search_aided_device).  rec_dev and out_dev are DEVICE arrays of n_records entries on the engine's GPU, row
+ * i = capture i / n_sel, slot i % n_sel (the layout of the search's output); rec_dev must be 4-byte and out_dev 16-byte
+ * aligned.  One kernel launch is enqueued on `stream` (NULL = the engine's stream) and the call returns without
+ * synchronising.
+ *   flags : 0, or ACQ_REFINE_DETECTED to refine only the rows acq_detected would accept (snr >= the threshold of the
+ *           satellite's type); the others are skipped and marked.
+ * Ordering: the rules of acq_search_device.  The refinement waits for the search that left the spectra (on the engine's
+ * stream or on another one), and whatever touches the engine's scratch next waits for the refinement, since the next
+ * search overwrites those spectra.  It consumes nothing: repeating it gives the same bytes.  The caller keeps rec_dev
+ * and out_dev valid until `stream` has passed it.
+ * The host cannot see the records, so the kernel checks each one, in this order: 0 <= sat < table size, sat is the
+ * satellite of its slot, 0 <= lag < L of its type, dop inside dop_lo..dop_hi (dop 0 with snr 0 is also accepted, the
+ * record of a row without any positive snr).  A row that is not refined carries a marker instead of values:
+ *   skipped by ACQ_REFINE_DETECTED : dop_hz = code_fs = NaN, peak = 0, ca_shift = -1
+ *   record failed a check          : dop_hz = code_fs = NaN, peak = 0, ca_shift = -2
+ * A refined row always has ca_shift >= 0, and its bytes equal acq_refine's for the same record.
+ * ACQ_ERR_ARG, before any device work: a NULL engine, rec_dev or out_dev; unknown flag bits; no search whose spectra
+ * are still on the device; an acq_submit not yet waited for; n_records different from that search's record count;
+ * a misaligned rec_dev or out_dev. */
+#define ACQ_REFINE_DETECTED 1
+int acq_refine_device(acq_engine *e, const acq_record *rec_dev, int n_records, int flags, acq_fine *out_dev,
+                      void *stream);
+
 /* Detection rule of SearchTask (gps/search.cpp:549,591): snr >= threshold of the sat's type. */
 int acq_detected(const acq_engine *e, const acq_record *r);
 

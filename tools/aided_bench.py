@@ -63,15 +63,22 @@ def cfg1(F, S, synth, scenarios, calls, warmup):
     return res
 
 
-def cfg5(F, S, torch, bench, steps):
-    table = S.navstar()
-    n_cap, n_sel, hw = 1024, 32, 2
-    caps = bench.farm_captures_numpy(range(n_cap))
+def farm_centers(F, bench, n_cap, n_sel):
+    """Doppler centres of the farm's aided search: the true Doppler of each injected signal + a seeded offset in +-2, a
+    seeded random index for satellites without a signal."""
     rng = np.random.default_rng(5)
     centers = rng.integers(-20, 21, (n_cap, n_sel)).astype(np.int32)
     for c in range(n_cap):
         for sat, _, f, _, _ in bench.farm_signals(c):
             centers[c, sat] = int(np.round(f / F.BIN_HZ)) + int(rng.integers(-2, 3))
+    return centers
+
+
+def cfg5(F, S, torch, bench, steps):
+    table = S.navstar()
+    n_cap, n_sel, hw = 1024, 32, 2
+    caps = bench.farm_captures_numpy(range(n_cap))
+    centers = farm_centers(F, bench, n_cap, n_sel)
     res = {}
     with F.AcqEngine(table) as eng:
         d_in = torch.from_numpy(caps.reshape(-1)).cuda()
