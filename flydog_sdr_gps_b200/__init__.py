@@ -2,4 +2,4 @@
 hand-written sm_100a CUDA kernels behind a C ABI (include/acq_b200.h)."""
 from . import sats  # noqa: F401
 from .engine import (AcqEngine, AcqError, BIN_HZ, BLOCK_BYTES, CELL_DTYPE, FINE_DTYPE, LAGS_E1B, LAGS_L1, N,  # noqa: F401
-                     RECORD_DTYPE, WRAP_CIRCULAR, WRAP_REFERENCE, default_params, microbench)
+                     PEAK2_DTYPE, RECORD_DTYPE, WRAP_CIRCULAR, WRAP_REFERENCE, default_params, microbench)

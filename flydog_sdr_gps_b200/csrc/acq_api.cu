@@ -144,6 +144,10 @@ struct acq_engine {
     // the device), slots, and its slot -> satellite map on the device
     int ref_captures = 0, ref_slots = 0;
     const int *ref_slot_sat = nullptr;
+    int ref_n_l1 = 0, ref_n_e1b = 0;   // ... and its C/A and E1B slot counts (acq_profile_device)
+    // peak-quality profile (acq_profile): row output scratch of the host form (its lag profiles get a buffer per call)
+    acq_peak2 *d_peak2 = nullptr;
+    size_t cap_peak2 = 0;
     // aided host search (acq_search_aided): Doppler centres staged in pinned memory, copied to the device with the capture
     int32_t *h_center = nullptr;
     size_t cap_h_center = 0;
@@ -202,6 +206,7 @@ int free_engine(acq_engine *e)
     cudaFree(e->d_sat_type);
     cudaFree(e->d_ref_rec);
     cudaFree(e->d_fine);
+    cudaFree(e->d_peak2);
     cudaFree(e->d_center);
     if (e->h_center) cudaFreeHost(e->h_center);
     if (e->h_packed) cudaFreeHost(e->h_packed);
@@ -533,12 +538,15 @@ int poll_records(acq_engine *e, acq_record *out, size_t rows)
     return ACQ_OK;
 }
 
-// After a search of either path is enqueued: the shape acq_refine_device checks its call and its records against.
+// After a search of either path is enqueued: the shape acq_refine_device and acq_profile_device check their call and
+// their records against.
 void set_refine_shape(acq_engine *e, int n_captures)
 {
     e->ref_captures = n_captures;
     e->ref_slots = e->n_slots;
     e->ref_slot_sat = e->cur_slot_sat;
+    e->ref_n_l1 = e->n_l1;
+    e->ref_n_e1b = e->n_e1b;
 }
 
 int enqueue_refine(acq_engine *e, const acq_record *rec_dev, int n_records, int flags, acq_fine *out_dev,
@@ -548,6 +556,29 @@ int enqueue_refine(acq_engine *e, const acq_record *rec_dev, int n_records, int 
                                  e->prm.k_noncoh, e->nvar, e->prm.half_bin, e->ext_len, e->Q, e->n_shift, e->smax,
                                  e->cd_div, (int)e->sats.size(), e->prm.dop_lo, e->prm.dop_hi, e->prm.thr_l1,
                                  e->prm.thr_e1b, flags, st);
+    CU(cudaGetLastError());
+    return ACQ_OK;
+}
+
+// excl of acq_profile against the search it follows: 0 <= excl < L_min / 2, L_min the smallest L of its satellites
+int check_excl(int excl, int n_l1)
+{
+    const int l_min = n_l1 > 0 ? ACQ_LAGS_L1 : ACQ_LAGS_E1B;
+    if (excl < 0 || 2 * excl >= l_min)
+        return fail(ACQ_ERR_ARG, "excl=%d outside 0..%d (L_min / 2 - 1 of the searched satellites)", excl, (l_min - 1) / 2);
+    return ACQ_OK;
+}
+
+// Lag-vector floats of one capture's rows (acq_b200.h: L per slot)
+size_t profile_capture_len(int n_l1, int n_e1b) { return (size_t)n_l1 * ACQ_LAGS_L1 + (size_t)n_e1b * ACQ_LAGS_E1B; }
+
+int enqueue_profile(acq_engine *e, const acq_record *rec_dev, int n_records, int flags, int excl, acq_peak2 *out_dev,
+                    float *profile_dev, const int *slot_sat, int n_slots, int n_l1, int n_e1b, cudaStream_t st)
+{
+    e->launches += launch_profile(e->d_Dp, e->d_Ep, e->d_tables, rec_dev, e->d_sat_type, slot_sat, out_dev, profile_dev,
+                                  n_records, n_slots, n_l1, n_e1b, e->prm.k_noncoh, e->nvar, e->prm.half_bin, e->ext_len, e->Q,
+                                  e->n_shift, e->smax, e->cd_div, (int)e->sats.size(), e->prm.dop_lo, e->prm.dop_hi,
+                                  e->prm.thr_l1, e->prm.thr_e1b, flags, excl, st);
     CU(cudaGetLastError());
     return ACQ_OK;
 }
@@ -1027,6 +1058,91 @@ int acq_refine_device(acq_engine *e, const acq_record *rec_dev, int n_records, i
     int rc = enqueue_refine(e, rec_dev, n_records, flags, out_dev, e->ref_slot_sat, e->ref_slots, st);
     if (rc) return rc;
     if (st != e->stream) {  // the next search overwrites the spectra: whatever touches the scratch next waits for this
+        CU(cudaEventRecord(e->dev_done, st));
+        e->dev_pending = true;
+    }
+    return ACQ_OK;
+}
+
+int acq_profile(acq_engine *e, const acq_record *rec, int n_records, int excl, acq_peak2 *out, float *profile)
+{
+    if (!e) return fail(ACQ_ERR_ARG, "engine is NULL");
+    if (!rec || !out) return fail(ACQ_ERR_ARG, "rec/out must not be NULL");
+    if (excl < 0) return fail(ACQ_ERR_ARG, "excl must be >= 0 (got %d)", excl);
+    if (e->pending) return fail(ACQ_ERR_ARG, "a submitted search is still pending: call acq_wait first");
+    if (e->last_captures <= 0) return fail(ACQ_ERR_ARG, "no completed host-path search to profile");
+    const long long rows = (long long)e->last_captures * e->n_slots;
+    if (n_records != rows)
+        return fail(ACQ_ERR_ARG, "n_records=%d but the last search produced %lld records", n_records, rows);
+    int rc = check_excl(excl, e->n_l1);
+    if (rc) return rc;
+    for (int i = 0; i < n_records; i++) {   // acq_refine's checks
+        const acq_record &r = rec[i];
+        if (r.sat != e->sel_cache[i % e->n_slots])
+            return fail(ACQ_ERR_ARG, "record %d: sat %d is not the satellite searched in that slot", i, r.sat);
+        const int L = (e->sats[r.sat].type == ACQ_E1B) ? ACQ_LAGS_E1B : ACQ_LAGS_L1;
+        if (r.lag < 0 || r.lag >= L) return fail(ACQ_ERR_ARG, "record %d: lag %d outside 0..%d", i, r.lag, L - 1);
+        if ((r.dop < e->prm.dop_lo || r.dop > e->prm.dop_hi) && !(r.dop == 0 && r.snr == 0.0f))
+            return fail(ACQ_ERR_ARG, "record %d: Doppler index %d outside %d..%d", i, r.dop, e->prm.dop_lo, e->prm.dop_hi);
+    }
+    DeviceGuard g(e->device);
+    const size_t n_prof = (size_t)e->last_captures * profile_capture_len(e->n_l1, e->n_e1b);
+    if ((rc = grow(e, e->d_ref_rec, e->cap_ref_rec, (size_t)n_records))) return rc;
+    if ((rc = grow(e, e->d_peak2, e->cap_peak2, (size_t)n_records))) return rc;
+    // The lag profiles (512 MiB for a 1024-capture C/A search) live only for this call: the engine keeps no buffer of
+    // that size.  The buffer is freed after the engine stream has passed every use of it, on the error paths too.
+    struct CallBuffer {
+        cudaStream_t st;
+        float *p = nullptr;
+        ~CallBuffer()
+        {
+            if (p) {
+                cudaStreamSynchronize(st);
+                cudaFree(p);
+            }
+        }
+    } d_prof{e->stream};
+    if (profile) CU(cudaMalloc(&d_prof.p, n_prof * sizeof(float)));
+    CU(cudaMemcpyAsync(e->d_ref_rec, rec, (size_t)n_records * sizeof(acq_record), cudaMemcpyHostToDevice, e->stream));
+    // the records are checked above, so the kernel's own checks pass every row
+    if ((rc = enqueue_profile(e, e->d_ref_rec, n_records, 0, excl, e->d_peak2, d_prof.p,
+                              e->cur_slot_sat, e->n_slots, e->n_l1, e->n_e1b, e->stream)))
+        return rc;
+    CU(cudaMemcpyAsync(out, e->d_peak2, (size_t)n_records * sizeof(acq_peak2), cudaMemcpyDeviceToHost, e->stream));
+    if (profile) CU(cudaMemcpyAsync(profile, d_prof.p, n_prof * sizeof(float), cudaMemcpyDeviceToHost, e->stream));
+    CU(cudaStreamSynchronize(e->stream));
+    return ACQ_OK;
+}
+
+int acq_profile_device(acq_engine *e, const acq_record *rec_dev, int n_records, int flags, int excl, acq_peak2 *out_dev,
+                       float *profile_dev, void *stream)
+{
+    if (!e) return fail(ACQ_ERR_ARG, "engine is NULL");
+    if (!rec_dev || !out_dev) return fail(ACQ_ERR_ARG, "rec_dev/out_dev must not be NULL");
+    if (flags & ~ACQ_PROFILE_DETECTED) return fail(ACQ_ERR_ARG, "unknown flag bits 0x%x", (unsigned)(flags & ~ACQ_PROFILE_DETECTED));
+    if (excl < 0) return fail(ACQ_ERR_ARG, "excl must be >= 0 (got %d)", excl);
+    if (e->ref_captures <= 0) return fail(ACQ_ERR_ARG, "no search whose spectra are still on the device to profile");
+    if (e->pending) return fail(ACQ_ERR_ARG, "a submitted search is still pending: call acq_wait first");
+    const long long rows = (long long)e->ref_captures * e->ref_slots;
+    if (n_records != rows)
+        return fail(ACQ_ERR_ARG, "n_records=%d but the last search produced %lld records", n_records, rows);
+    int rc = check_excl(excl, e->ref_n_l1);
+    if (rc) return rc;
+    if (((uintptr_t)out_dev & 15) != 0) return fail(ACQ_ERR_ARG, "out_dev must be 16-byte aligned (one 16-byte store per row)");
+    if (((uintptr_t)rec_dev & 3) != 0) return fail(ACQ_ERR_ARG, "rec_dev must be 4-byte aligned");
+    if (((uintptr_t)profile_dev & 3) != 0) return fail(ACQ_ERR_ARG, "profile_dev must be 4-byte aligned");
+    DeviceGuard g(e->device);
+    cudaStream_t st = stream ? (cudaStream_t)stream : e->stream;
+    // ordered as acq_refine_device: after the search that left the spectra, before the next one
+    if (e->dev_pending) CU(cudaStreamWaitEvent(st, e->dev_done, 0));
+    if (st != e->stream) {
+        CU(cudaEventRecord(e->dev_done, e->stream));
+        CU(cudaStreamWaitEvent(st, e->dev_done, 0));
+    }
+    if ((rc = enqueue_profile(e, rec_dev, n_records, flags, excl, out_dev, profile_dev, e->ref_slot_sat, e->ref_slots,
+                              e->ref_n_l1, e->ref_n_e1b, st)))
+        return rc;
+    if (st != e->stream) {
         CU(cudaEventRecord(e->dev_done, st));
         e->dev_pending = true;
     }

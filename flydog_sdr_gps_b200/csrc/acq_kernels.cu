@@ -1967,6 +1967,8 @@ __global__ void __launch_bounds__(256) k_refine(const RefineArgs p)
     const int row = blockIdx.x, t = threadIdx.x;
     const acq_record rc = p.rec[row];
     const int cap = row / p.n_slots;
+    // the record checks of acq_refine, made here on a record the host may never have seen; record_marker (k_profile)
+    // restates them and must stay in step with this copy and with the host forms
     int marker = 0;   // -2: the record fails a check, -1: skipped below the detection threshold
     bool e1b = false;
     if (rc.sat < 0 || rc.sat >= p.n_sats || rc.sat != p.slot_sat[row % p.n_slots]) {
@@ -2084,6 +2086,213 @@ __global__ void __launch_bounds__(256) k_refine(const RefineArgs p)
 }
 
 // ---------------------------------------------------------------------------------------------
+// K7.  Peak-quality profile of searched rows (acq_profile / acq_profile_device).  For each record the row is evaluated at
+// the record's Doppler index, exactly as the search evaluated it: the product of the capture spectrum the search left
+// in HBM (the same half-bin spectrum and code-Doppler copy, d_row's rule) with the extended code row (the same wrap),
+// four sub-FFTs of 4096 points per block, the search's radix-4 combine -- the running accumulation of the C/A kernels,
+// the parked-residue butterfly of the E1B kernels -- and the block powers summed in block order.  Every step is the
+// search kernels' own arithmetic in their order (subfft4096_inv3 computes what subfft4096_inv4 / inv4s compute), so
+// the power at every lag is bitwise the one the search reduced: the profile at the record's lag is acq_record.peak and
+// the first maximum of the profile is the record's lag.  Then one pass over the lags forms the largest power outside
+// the main lobe (circular distance > excl, the lowest lag on ties), the mean power there, and the profile row.
+// One CTA per row; E1B parks three residues in tensor memory as k_search_e1b does and, for K > 1, keeps the 64 running
+// block sums of a thread in a thread-private 64 KiB shared-memory array (the C/A sums stay in registers).  The two
+// types are two instantiations launched over the same rows: a CTA whose slot is of the other type exits at once.
+// Records are checked in the kernel with k_refine's checks and markers (lag2 = -2 / -1).
+// ---------------------------------------------------------------------------------------------
+// k_refine's checks of a record the host never saw, in the same order (k_refine keeps its own copy of them, so that its
+// code does not change; the host forms make the same checks in acq_refine / acq_profile): 0 if the record passes, -2 if
+// it fails one (the satellite's range is checked before sat_type is indexed with it), -1 if `detected_only` and it is
+// below its type's threshold.
+__device__ __forceinline__ int record_marker(const acq_record &rc, const int *slot_sat, int slot, const int *sat_type, int n_sats,
+                                             int dop_lo, int dop_hi, bool detected_only, float thr_l1, float thr_e1b)
+{
+    int marker = 0;
+    if (rc.sat < 0 || rc.sat >= n_sats || rc.sat != slot_sat[slot]) {
+        marker = -2;
+    } else {
+        const bool e1b = sat_type[rc.sat] == ACQ_E1B;
+        const int L = e1b ? ACQ_LAGS_E1B : ACQ_LAGS_L1;
+        if (rc.lag < 0 || rc.lag >= L) marker = -2;
+        // a row that never exceeded snr 0 carries dop 0 (k_best_dop), which may lie outside an asymmetric range
+        else if ((rc.dop < dop_lo || rc.dop > dop_hi) && !(rc.dop == 0 && rc.snr == 0.0f)) marker = -2;
+        else if (detected_only && !(rc.snr >= (e1b ? thr_e1b : thr_l1))) marker = -1;
+    }
+    return marker;
+}
+
+struct ProfileArgs {
+    const float2 *Dp;
+    const float2 *Ep;
+    const float2 *tables;
+    const acq_record *rec;   // [n_rows], row = cap * n_slots + slot
+    const int *sat_type;     // [n_sats]
+    const int *slot_sat;     // [n_slots] satellite searched in each slot
+    acq_peak2 *out;
+    float *profile;          // NULL, or the packed lag vectors (acq_b200.h)
+    int n_slots, n_e1b_slots, K, nvar, half_bin, ext_len, Q, n_shift, smax, cd_div;
+    int n_sats, dop_lo, dop_hi, flags, excl;
+    float thr_l1, thr_e1b;
+};
+
+constexpr size_t kProfileRedBytes = 64 * sizeof(float);                 // reduction slots, the record's power, TMEM slot
+constexpr size_t kProfilePsBytes = sizeof(float) * 64 * 256;            // E1B, K > 1: running block sums [64][256]
+__host__ __device__ constexpr size_t profile_smem_bytes(bool e1b, int K)
+{
+    return fft_smem3_bytes() + kProfileRedBytes + (e1b && K > 1 ? kProfilePsBytes : 0);
+}
+
+// One lag of the final powers: the record's power, the running maximum / sum outside the main lobe, the profile.
+__device__ __forceinline__ void profile_visit(int n, float pw, int lag, int excl, int L, Peak &best, float *pk, float *prof)
+{
+    if (n == lag) *pk = pw;
+    int d = n - lag;
+    d = d < 0 ? -d : d;
+    d = min(d, L - d);
+    if (d > excl) peak_merge(best, pw, n, pw);   // strict > or the lower lag on equal power
+    if (prof) prof[n] = pw;
+}
+
+template <bool E1B>
+__global__ void __launch_bounds__(256, E1B ? 1 : 2) k_profile(const ProfileArgs p)
+{
+    extern __shared__ __align__(1024) unsigned char smem[];
+    constexpr int L = E1B ? ACQ_LAGS_E1B : ACQ_LAGS_L1;
+    const int row = blockIdx.x, t = threadIdx.x;
+    const int slot = row % p.n_slots, cap = row / p.n_slots;
+    if ((p.sat_type[p.slot_sat[slot]] == ACQ_E1B) != E1B) return;   // a row of the other launch
+    const acq_record rc = p.rec[row];
+    const int marker = record_marker(rc, p.slot_sat, slot, p.sat_type, p.n_sats, p.dop_lo, p.dop_hi,
+                                     (p.flags & ACQ_PROFILE_DETECTED) != 0, p.thr_l1, p.thr_e1b);
+    float *prof = nullptr;
+    if (p.profile) {   // row offset: the L of every earlier slot of this capture (uniform loop: every thread counts)
+        int e1b_before = 0;
+        for (int s0 = 0; s0 < slot; s0 += 256) {
+            const int s = s0 + t;
+            e1b_before += __syncthreads_count(s < slot && p.sat_type[p.slot_sat[s]] == ACQ_E1B);
+        }
+        const size_t cap_len = (size_t)p.n_slots * ACQ_LAGS_L1 + (size_t)p.n_e1b_slots * (ACQ_LAGS_E1B - ACQ_LAGS_L1);
+        prof = p.profile + (size_t)cap * cap_len + (size_t)slot * ACQ_LAGS_L1 + (size_t)e1b_before * (ACQ_LAGS_E1B - ACQ_LAGS_L1);
+    }
+    if (marker != 0) {   // uniform: every thread read the same record
+        const float nan = __int_as_float(0x7fc00000);   // quiet NaN
+        if (t == 0) {
+            acq_peak2 o;
+            o.peak2 = o.ratio = o.noise_ex = nan;
+            o.lag2 = marker;
+            p.out[row] = o;
+        }
+        if (prof)
+            for (int n = t; n < L; n += 256) prof[n] = nan;
+        return;
+    }
+    const FftSmem3 s = fft_smem3_carve(smem);
+    float *red_f = reinterpret_cast<float *>(smem + fft_smem3_bytes());   // [16] warp partials, [16] record's power, [48] TMEM slot
+    int *red_i = reinterpret_cast<int *>(red_f + 32);                     // [8]
+    float *pk = red_f + 16;
+    float *Pt = reinterpret_cast<float *>(smem + fft_smem3_bytes() + kProfileRedBytes) + t;   // E1B, K > 1: [64][256]
+    load_t2(s, p.tables, t);
+    uint32_t tmem_base = 0, zaddr = 0;
+    if constexpr (E1B) {   // this thread's TMEM: lane 32*(warp%4) + (t%32), columns [96*(warp/4), +96): [k2][n2] parked
+        tmem_base = tmem_alloc_cta<kE1bTmemCols>(reinterpret_cast<uint32_t *>(red_f + 48), t);
+        zaddr = tmem_base + tmem_lane_base(t) + (uint32_t)((t >> 7) * 96);
+    }
+    const float2 *base = p.tables + kT2Elems + t;
+    const int v = p.half_bin ? (rc.dop & 1) : 0;
+    const int dop = p.half_bin ? ((rc.dop - v) >> 1) : rc.dop;
+    Peak best;
+    best.p = -1.0f;   // every power (>= 0) wins over it
+    best.n = 0x7fffffff;
+    best.sum = 0.0f;
+    int buf = 0;
+    float P[16];   // C/A: block sums of this thread's lags lag_of3(t, n2)
+    for (int b = 0; b < p.K; b++) {
+        // the copy of block b the search read at this Doppler index (d_row): delayed by 16 b (+ the code-Doppler shift)
+        // samples in the front end, so lag n lines up across blocks
+        const int cshift = p.n_shift > 1 ? code_shift(b, rc.dop, p.cd_div) : 0;
+        const float2 *D = p.Dp + (((size_t)((size_t)cap * p.K + b) * p.nvar + v) * p.n_shift + (p.smax + cshift)) * kN;
+        float2 x[16], acc[16];
+#pragma unroll 1
+        for (int k2 = 0; k2 < 4; k2++) {
+            {   // x[a] = conj(data[k]) * code[k - dop], k = 1024 a + 4 t + k2   (search.cpp:471; load_products)
+                const int r = (k2 - dop) & 3;
+                const int q = (k2 - dop - r) >> 2;
+                const float2 *Dk = D + k2 * kSub + t;
+                const float2 *Ek = p.Ep + (size_t)(rc.sat * 4 + r) * p.ext_len + p.Q + q + t;
+#pragma unroll
+                for (int a = 0; a < 16; a++) x[a] = cmul_conj_a(__ldg(Dk + 256 * a), __ldg(Ek + 256 * a));
+            }
+            subfft4096_inv3(x, k2, __ldg(base + k2 * 256), buf, s, t);
+            buf ^= 1;
+            if constexpr (E1B) {
+                if (k2 < 3) {
+                    float2 z[16];
+#pragma unroll
+                    for (int n2 = 0; n2 < 16; n2++) z[n2] = (k2 == 0) ? x[r16(n2)] : cmul(x[r16(n2)], c_cC[k2][n2]);
+                    tmem_st16(zaddr + 32 * k2, z);
+                    tmem_wait_st();
+                }
+            } else {   // lags 0..4095 only: m = 0 of the radix-4 combine, accumulated as in k_search_l1
+                if (k2 == 0) {
+#pragma unroll
+                    for (int n2 = 0; n2 < 16; n2++) acc[n2] = x[r16(n2)];
+                } else {
+#pragma unroll
+                    for (int n2 = 0; n2 < 16; n2++) acc[n2] = cfma(x[r16(n2)], c_cC[k2][n2], acc[n2]);
+                }
+            }
+        }
+        const bool last = b + 1 == p.K;
+        if constexpr (E1B) {   // radix-4 combine over k2 (k_search_e1b / k_search_e1b_multi), lags lag_of3(t, n2) + 4096 m
+#pragma unroll
+            for (int c4 = 0; c4 < 4; c4++) {
+                float2 za[4], zb[4], zc[4];
+                tmem_ld4(zaddr + 0 * 32 + 8 * c4, za);
+                tmem_ld4(zaddr + 1 * 32 + 8 * c4, zb);
+                tmem_ld4(zaddr + 2 * 32 + 8 * c4, zc);
+                tmem_wait_ld();
+#pragma unroll
+                for (int i = 0; i < 4; i++) {
+                    const int n2 = 4 * c4 + i;
+                    float2 z0 = za[i], z1 = zb[i], z2 = zc[i];
+                    float2 z3 = cmul(x[r16(n2)], c_cC[3][n2]);
+                    radix4_inv(z0, z1, z2, z3);  // z_m = sum_k2 z_k2 * j^{k2*m}
+                    const float2 zz[4] = {z0, z1, z2, z3};
+#pragma unroll
+                    for (int m = 0; m < 4; m++) {
+                        float pw = cpower(zz[m]);
+                        if (b > 0) pw = Pt[(4 * n2 + m) * 256] + pw;
+                        if (!last) Pt[(4 * n2 + m) * 256] = pw;
+                        const int n = lag_of3(t, n2) + 4096 * m;
+                        if (last && n < L) profile_visit(n, pw, rc.lag, p.excl, L, best, pk, prof);
+                    }
+                }
+            }
+        } else {
+#pragma unroll
+            for (int n2 = 0; n2 < 16; n2++) P[n2] = (b == 0) ? cpower(acc[n2]) : (P[n2] + cpower(acc[n2]));
+        }
+    }
+    if constexpr (!E1B) {
+#pragma unroll
+        for (int n2 = 0; n2 < 16; n2++) {
+            const int n = lag_of3(t, n2);
+            if (n < L) profile_visit(n, P[n2], rc.lag, p.excl, L, best, pk, prof);
+        }
+    }
+    const Peak tot = block_reduce_peak(best, red_f, red_i, t);   // its barrier also publishes *pk
+    if (t == 0) {
+        acq_peak2 o;
+        o.peak2 = tot.p;
+        o.lag2 = tot.n;
+        o.ratio = __fdiv_rn(*pk, tot.p);
+        o.noise_ex = __fdiv_rn(tot.sum, (float)(L - 2 * p.excl - 1));
+        p.out[row] = o;
+    }
+    if constexpr (E1B) tmem_free_cta<kE1bTmemCols>(tmem_base, t);
+}
+
+// ---------------------------------------------------------------------------------------------
 // launchers
 // ---------------------------------------------------------------------------------------------
 // Launch with (pdl) or without programmatic stream serialization: with it the grid may become resident while the
@@ -2152,6 +2361,8 @@ cudaError_t search_kernels_configure()
     if ((e = cudaFuncSetAttribute(k_fwd_fft_cluster<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, fc))) return e;
     if ((e = cudaFuncSetAttribute(k_fwd_fft<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, fw))) return e;
     if ((e = cudaFuncSetAttribute(k_fwd_fft<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, fw))) return e;
+    if ((e = cudaFuncSetAttribute(k_profile<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)profile_smem_bytes(false, 1)))) return e;
+    if ((e = cudaFuncSetAttribute(k_profile<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)profile_smem_bytes(true, 2)))) return e;
     // One shared-memory carveout for every kernel of a search.  Left to the driver, the C/A kernel (2 x 96.3 KiB) runs
     // its SMs at the 196 KiB split and the E1B kernel (2 x 103.8 KiB) at 228 KiB, and an SM changes its split only when
     // it is empty: in a GPS + Galileo search the E1B CTAs -- launched to move in as the C/A CTAs retire -- entered no SM
@@ -2392,6 +2603,26 @@ int launch_refine(const float2 *Dp, const float2 *Ep, const acq_record *rec, con
                  n_sats, dop_lo, dop_hi, flags, thr_l1, thr_e1b};
     k_refine<<<n_rows, 256, 0, st>>>(a);
     return 1;
+}
+
+int launch_profile(const float2 *Dp, const float2 *Ep, const float2 *tables, const acq_record *rec, const int *sat_type,
+                   const int *slot_sat, acq_peak2 *out, float *profile, int n_rows, int n_slots, int n_l1_slots,
+                   int n_e1b_slots, int K, int nvar, int half_bin, int ext_len, int Q, int n_shift, int smax, int cd_div,
+                   int n_sats, int dop_lo, int dop_hi, float thr_l1, float thr_e1b, int flags, int excl, cudaStream_t st)
+{
+    if (n_rows <= 0) return 0;
+    ProfileArgs a{Dp, Ep, tables, rec, sat_type, slot_sat, out, profile, n_slots, n_e1b_slots, K, nvar, half_bin, ext_len, Q,
+                  n_shift, smax, cd_div, n_sats, dop_lo, dop_hi, flags, excl, thr_l1, thr_e1b};
+    int n = 0;
+    if (n_l1_slots > 0) {
+        k_profile<false><<<n_rows, 256, profile_smem_bytes(false, K), st>>>(a);
+        n++;
+    }
+    if (n_e1b_slots > 0) {
+        k_profile<true><<<n_rows, 256, profile_smem_bytes(true, K), st>>>(a);
+        n++;
+    }
+    return n;
 }
 
 #ifdef ACQ_TRACE

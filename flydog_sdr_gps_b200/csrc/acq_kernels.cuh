@@ -134,6 +134,13 @@ int launch_refine(const float2 *Dp, const float2 *Ep, const acq_record *rec, con
                   acq_fine *out, int n_rows, int n_slots, int K, int nvar, int half_bin, int ext_len, int Q, int n_shift,
                   int smax, int cd_div, int n_sats, int dop_lo, int dop_hi, float thr_l1, float thr_e1b, int flags,
                   cudaStream_t st);
+// peak-quality profile of the records of the most recent search (acq_profile): one CTA per record in each of two
+// launches, the C/A rows (n_l1_slots > 0) and the E1B rows (n_e1b_slots > 0).  Record checks and markers (lag2 -2 / -1
+// with ACQ_PROFILE_DETECTED in flags) as launch_refine; profile NULL or the packed lag vectors of acq_b200.h
+int launch_profile(const float2 *Dp, const float2 *Ep, const float2 *tables, const acq_record *rec, const int *sat_type,
+                   const int *slot_sat, acq_peak2 *out, float *profile, int n_rows, int n_slots, int n_l1_slots,
+                   int n_e1b_slots, int K, int nvar, int half_bin, int ext_len, int Q, int n_shift, int smax, int cd_div,
+                   int n_sats, int dop_lo, int dop_hi, float thr_l1, float thr_e1b, int flags, int excl, cudaStream_t st);
 cudaError_t search_kernels_configure();
 
 }  // namespace acq

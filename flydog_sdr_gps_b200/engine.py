@@ -16,12 +16,14 @@ LAGS_L1 = 4092
 LAGS_E1B = 16368
 WRAP_REFERENCE, WRAP_CIRCULAR = 0, 1
 REFINE_DETECTED = 1   # ACQ_REFINE_DETECTED
+PROFILE_DETECTED = 1  # ACQ_PROFILE_DETECTED
 
 RECORD_DTYPE = np.dtype([("sat", "<i4"), ("lag", "<i4"), ("dop", "<i4"),
                          ("peak", "<f4"), ("noise", "<f4"), ("snr", "<f4")])
 CELL_DTYPE = np.dtype([("peak", "<f4"), ("noise", "<f4"), ("snr", "<f4"), ("lag", "<i4")])
 FINE_DTYPE = np.dtype([("dop_hz", "<f4"), ("code_fs", "<f4"), ("peak", "<f4"), ("ca_shift", "<i4")])
-assert RECORD_DTYPE.itemsize == 24 and CELL_DTYPE.itemsize == 16 and FINE_DTYPE.itemsize == 16
+PEAK2_DTYPE = np.dtype([("peak2", "<f4"), ("lag2", "<i4"), ("ratio", "<f4"), ("noise_ex", "<f4")])
+assert RECORD_DTYPE.itemsize == 24 and CELL_DTYPE.itemsize == 16 and FINE_DTYPE.itemsize == 16 and PEAK2_DTYPE.itemsize == 16
 
 
 class AcqError(RuntimeError):
@@ -219,6 +221,42 @@ class AcqEngine:
         stream).  detected_only: rows below their detection threshold are marked (ca_shift -1), not refined."""
         flags = REFINE_DETECTED if detected_only else 0
         _check(self._L.acq_refine_device(self._h, rec_dev, int(n_records), flags, out_dev, stream_ptr), self._L)
+
+    # ---- peak quality: second peak outside the main lobe, peak-to-second-peak ratio, lag profile
+    def lags_of(self, sats):
+        """L of each satellite index (4092 C/A, QZSS, SBAS; 16368 E1B): the length of its profile row."""
+        return np.array([LAGS_E1B if self.sats[int(i)][3] == E1B else LAGS_L1 for i in np.asarray(sats).reshape(-1)],
+                        np.int64)
+
+    def profile_offsets(self, n_captures=1, sel=None):
+        """Offsets of the profile rows of a search of n_captures over `sel` (None = the whole table) in the packed
+        layout of acq_profile: int64 [n_captures * n_sel + 1], row i is profile[off[i]:off[i + 1]]."""
+        ls = self.lags_of(range(len(self.sats)) if sel is None else sel)
+        return np.concatenate([[0], np.cumsum(np.tile(ls, int(n_captures)))]).astype(np.int64)
+
+    def profile(self, records, excl=4, want_profile=False):
+        """acq_profile: peak quality of the records of the most recent search()/wait() -- PEAK2_DTYPE array of the same
+        shape.  excl: half-width of the main lobe in /DECIM lags (4 = one chip).  want_profile: also return the packed
+        |r|^2 lag vectors (float32, rows at profile_offsets())."""
+        r = np.ascontiguousarray(records, RECORD_DTYPE)
+        out = np.zeros(r.shape, PEAK2_DTYPE)
+        prof = None
+        if want_profile:
+            sats = r["sat"].reshape(-1)
+            ok = (sats >= 0) & (sats < len(self.sats))   # a bad record is refused before anything is written
+            prof = np.zeros(int(self.lags_of(sats[ok]).sum()) if ok.all() else 0, np.float32)
+        _check(self._L.acq_profile(self._h, r.ctypes.data, r.size, int(excl), out.ctypes.data,
+                                   prof.ctypes.data if want_profile and prof.size else None), self._L)
+        return (out, prof) if want_profile else out
+
+    def profile_device(self, rec_dev, out_dev, n, excl=4, detected_only=False, profile_dev=None, stream_ptr=None):
+        """acq_profile_device: rec_dev (acq_record) / out_dev (acq_peak2, 16-byte aligned) / profile_dev (float32 in the
+        packed layout, or None) are device pointers (ints) of the n rows of the most recent search of either path.
+        Enqueues on stream_ptr (None = engine stream).  detected_only: rows below their detection threshold are marked
+        (lag2 -1), not evaluated."""
+        flags = PROFILE_DETECTED if detected_only else 0
+        _check(self._L.acq_profile_device(self._h, rec_dev, int(n), flags, int(excl), out_dev, profile_dev, stream_ptr),
+               self._L)
 
     def detected(self, records):
         """Detection rule of SearchTask (search.cpp:549,591) applied to a record array."""

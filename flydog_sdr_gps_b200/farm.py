@@ -11,19 +11,21 @@ record array), so a search is: host->device copy of the local captures, acq_sear
 all_gather_into_tensor of the 24-byte records over NCCL, device->host copy of the gathered array.  `search_resident`
 is the same without the two copies (captures already in HBM, records left there).  `refine` / `refine_resident` do the
 same for the hand-off refinement of those records (acq_refine_device on each rank, then the 16-byte fine records gathered
-the same way).
+the same way), and `profile` / `profile_resident` for their peak quality (acq_profile_device, 16-byte acq_peak2 rows; the
+lag profiles themselves stay on each rank).
 
 `engine` is an AcqEngine.  The CPU suite exercises the same classes under gloo with a stand-in whose
-`search_device(...)` and `refine_device(...)` run the oracle on CPU tensors; nothing in this module computes a search itself.
+`search_device(...)`, `refine_device(...)` and `profile_device(...)` run the oracle on CPU tensors; nothing in this module computes a search itself.
 The function forms below (`search_sharded_by_*`) are the numpy/host-gather variant of the same plumbing.
 """
 import numpy as np
 
-from .engine import FINE_DTYPE, RECORD_DTYPE
+from .engine import FINE_DTYPE, PEAK2_DTYPE, RECORD_DTYPE
 from .scenarios import shard
 
 REC = RECORD_DTYPE.itemsize
 FINE = FINE_DTYPE.itemsize
+PEAK2 = PEAK2_DTYPE.itemsize
 
 
 class _Farm:
@@ -41,6 +43,7 @@ class _Farm:
         self.max_local = max(self.counts)
         self.pin = self.device.type == "cuda"
         self.d_fine = None
+        self.d_pk = None
 
     def _empty(self, n, device=None, pin=False):
         t = self.torch.zeros(max(n, 1), dtype=self.torch.uint8, device=device or self.device)
@@ -84,6 +87,30 @@ class _Farm:
         if self.device.type == "cuda":
             self.torch.cuda.current_stream().synchronize()
         return self._unpad(self.h_fine_all.numpy(), self.per_unit, FINE_DTYPE).reshape(self.records_shape)
+
+    def profile_resident(self, excl=4, detected_only=True):
+        """Peak quality of the local records of the last search_resident() (acq_profile_device on the current torch
+        stream, no lag profiles) into a local buffer padded like d_rec, then the same padded gather; returns the gathered
+        16-byte acq_peak2 rows.  detected_only: undetected rows carry the marker lag2 = -1.  Asynchronous."""
+        if self.d_pk is None:   # allocated on first use, as the fine buffers
+            n = self.max_local * self.per_unit * PEAK2
+            self.d_pk = self._empty(n)
+            self.d_pk_all = self._empty(self.world * n) if self.world > 1 else self.d_pk
+            self.h_pk_all = self._empty(self.d_pk_all.numel(), device="cpu", pin=self.pin)
+        if self.n_local:
+            self.eng.profile_device(self.d_rec.data_ptr(), self.d_pk.data_ptr(), self.n_local * self.per_unit, excl=excl,
+                                    detected_only=detected_only, stream_ptr=self._stream_ptr())
+        self._gather(self.d_pk_all, self.d_pk)
+        return self.d_pk_all
+
+    def profile(self, excl=4, detected_only=True):
+        """profile_resident, copy out, wait.  Returns a PEAK2_DTYPE array shaped like search()'s records (numpy view of
+        the pinned result buffer: valid until the next profile)."""
+        self.profile_resident(excl, detected_only)
+        self.h_pk_all.copy_(self.d_pk_all, non_blocking=True)
+        if self.device.type == "cuda":
+            self.torch.cuda.current_stream().synchronize()
+        return self._unpad(self.h_pk_all.numpy(), self.per_unit, PEAK2_DTYPE).reshape(self.records_shape)
 
 
 class CaptureFarm(_Farm):

@@ -246,6 +246,52 @@ int acq_refine(acq_engine *e, const acq_record *rec, int n_records, acq_fine *ou
 int acq_refine_device(acq_engine *e, const acq_record *rec_dev, int n_records, int flags, acq_fine *out_dev,
                       void *stream);
 
+/* Peak quality of one searched row (acq_profile / acq_profile_device): the second test of FFT acquisition, the main
+ * peak against the highest peak outside its main lobe.  Correlate()'s snr = peak / (mean over ALL lags, the peak
+ * included) cannot tell a clean peak from a cross-correlation or multipath shoulder, a second copy of the same code
+ * (a reflection or a spoofer) or the largest of many similar noise maxima; ratio can.  16 bytes. */
+typedef struct acq_peak2 {
+    float peak2;    /* largest |r|^2 (summed over the K blocks like the search) at the record's Doppler over the lags
+                       outside the main lobe: circular distance min(|n - lag|, L - |n - lag|) > excl */
+    int32_t lag2;   /* its lag (the lowest on ties); -1 / -2 mark a row that was not evaluated (below) */
+    float ratio;    /* the record's peak as recomputed here (the profile at the record's lag) / peak2 */
+    float noise_ex; /* mean |r|^2 over the L - (2 excl + 1) lags outside the main lobe */
+} acq_peak2;
+
+/* Peak-quality profile of the records of the MOST RECENT host-path search (acq_search, acq_search_grid,
+ * acq_search_aided, or acq_submit after acq_wait): `rec` (HOST) holds its n_captures * n_sel records in the same order,
+ * and their checks and errors are acq_refine's.  For each record the row is evaluated at the record's Doppler index
+ * from the spectra that search left on the device: the product with the code row (same wrap rule, same half-bin
+ * spectrum), the 16384-point inverse FFT, and |r|^2 summed over the K blocks with the search's lag shifts (16 b per
+ * block, plus the code-Doppler shift).  These are the search's own operations in the search's own order, so the
+ * profile at the record's lag equals acq_record.peak to the bit and the profile's first maximum is the record's lag.
+ * out (HOST, n_records) receives the acq_peak2 rows.
+ *   excl    : half-width of the main lobe in /DECIM lags, 0 <= excl < L_min / 2 (L_min: the smallest L of the
+ *             searched satellites' types); 4 is one chip.  For E1B one chip also covers the BOC(1,1) side lobes at
+ *             +-0.5 chip (+-2 lags) around the main peak.
+ *   profile : NULL, or (HOST) the whole |r|^2 lag vector of every row at its record's Doppler: L floats per row (4092
+ *             for C/A, QZSS and SBAS, 16368 for E1B), rows packed in record order.  Row i = capture c, slot s starts at
+ *             c * (sum over slots of L) + (sum of L over slots 0..s-1).  The device buffer the host form fills for this
+ *             is allocated for the call and freed before it returns.
+ * ACQ_ERR_ARG as acq_refine, and for a NULL out or an excl outside its range. */
+int acq_profile(acq_engine *e, const acq_record *rec, int n_records, int excl, acq_peak2 *out, float *profile);
+
+/* Device-resident form: the records of the MOST RECENT search of EITHER path (acq_refine_device's rule, aided searches
+ * included), DEVICE arrays, one or two kernel launches (C/A rows and E1B rows) enqueued on `stream` (NULL = the
+ * engine's stream) and no synchronise.  Ordering and the per-record checks in the kernel are acq_refine_device's.
+ * rec_dev must be 4-byte and out_dev 16-byte aligned; profile_dev (NULL allowed) 4-byte aligned, laid out as above.
+ *   flags : 0, or ACQ_PROFILE_DETECTED to evaluate only the rows acq_detected would accept.
+ * A row that is not evaluated carries a marker, and its profile row (when asked for) is all NaN:
+ *   skipped by ACQ_PROFILE_DETECTED : lag2 = -1, peak2 = ratio = noise_ex = NaN
+ *   record failed a check           : lag2 = -2, peak2 = ratio = noise_ex = NaN
+ * An evaluated row always has lag2 >= 0, and its bytes (and profile) equal acq_profile's for the same record.
+ * ACQ_ERR_ARG, before any device work: a NULL engine, rec_dev or out_dev; unknown flag bits; excl outside its range;
+ * no search whose spectra are still on the device; an acq_submit not yet waited for; n_records different from that
+ * search's record count; a misaligned rec_dev, out_dev or profile_dev. */
+#define ACQ_PROFILE_DETECTED 1
+int acq_profile_device(acq_engine *e, const acq_record *rec_dev, int n_records, int flags, int excl, acq_peak2 *out_dev,
+                       float *profile_dev, void *stream);
+
 /* Detection rule of SearchTask (gps/search.cpp:549,591): snr >= threshold of the sat's type. */
 int acq_detected(const acq_engine *e, const acq_record *r);
 
