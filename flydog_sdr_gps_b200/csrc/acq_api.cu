@@ -10,6 +10,7 @@
 
 #include <algorithm>
 #include <cstdarg>
+#include <numeric>
 
 #include "acq_geom.h"
 #include "acq_kernels.cuh"
@@ -109,7 +110,7 @@ struct acq_engine {
     // persistent device data
     float2 *d_tables = nullptr, *d_rot = nullptr, *d_C = nullptr, *d_Ep = nullptr;
     // per-call scratch (grown on demand)
-    size_t cap_blocks = 0, cap_cells = 0, cap_rows = 0, cap_packed = 0;
+    size_t cap_blocks = 0 /* spectrum rows */, cap_cells = 0, cap_rows = 0, cap_packed = 0;
     uint8_t *d_packed = nullptr;
     float2 *d_x2 = nullptr, *d_Dp = nullptr;
     acq_cell *d_cells = nullptr;
@@ -153,6 +154,8 @@ struct acq_engine {
     size_t cap_h_center = 0;
     int *d_center = nullptr;
     size_t cap_center = 0;
+    // coherent search (acq_search_coherent): sub-bin rotation table [F][16384] of each m_coh, built on first use
+    float2 *d_rot_coh[ACQ_COH_MAX + 1] = {};
 };
 
 namespace {
@@ -208,6 +211,7 @@ int free_engine(acq_engine *e)
     cudaFree(e->d_fine);
     cudaFree(e->d_peak2);
     cudaFree(e->d_center);
+    for (float2 *r : e->d_rot_coh) cudaFree(r);
     if (e->h_center) cudaFreeHost(e->h_center);
     if (e->h_packed) cudaFreeHost(e->h_packed);
     if (e->h_records) cudaFreeHost(e->h_records);
@@ -248,20 +252,22 @@ int grow(acq_engine *e, T *&ptr, size_t &cap, size_t need_elems, bool zero = fal
     return ACQ_OK;
 }
 
-// n_dop: Doppler cells per row of this search (the engine's range, or the window of an aided search)
-int ensure_scratch(acq_engine *e, int n_captures, int n_slots, bool host_path, int n_dop)
+// n_dop: Doppler cells per row of this search (the engine's range, the window of an aided search, or the 1/M-bin grid of
+// a coherent one); nvar: spectrum variants per block (e->nvar, or F of a coherent search)
+int ensure_scratch(acq_engine *e, int n_captures, int n_slots, bool host_path, int n_dop, int nvar)
 {
     const size_t blocks = (size_t)n_captures * e->prm.k_noncoh;
-    if (blocks > e->cap_blocks || !e->d_x2) {
+    const size_t spectra = blocks * nvar * e->n_shift;   // rows of x2 and of the capture spectra
+    if (spectra > e->cap_blocks || !e->d_x2) {
         int rc = drain(e);  // changing scratch under an in-flight search is not allowed
         if (rc) return rc;
         if (e->d_x2) CU(cudaFree(e->d_x2));
         if (e->d_Dp) CU(cudaFree(e->d_Dp));
         e->d_x2 = e->d_Dp = nullptr;
         e->cap_blocks = 0;
-        CU(cudaMalloc(&e->d_x2, blocks * e->nvar * e->n_shift * kN * sizeof(float2)));
-        CU(cudaMalloc(&e->d_Dp, blocks * e->nvar * e->n_shift * kN * sizeof(float2)));
-        e->cap_blocks = blocks;
+        CU(cudaMalloc(&e->d_x2, spectra * kN * sizeof(float2)));
+        CU(cudaMalloc(&e->d_Dp, spectra * kN * sizeof(float2)));
+        e->cap_blocks = spectra;
     }
     const size_t rows = (size_t)n_captures * n_slots;
     int rc;
@@ -371,16 +377,83 @@ int set_selection(acq_engine *e, const int32_t *sel, int n_sel)
 // Doppler cells per row: the engine's whole range, or the window of an aided search (center != NULL)
 int row_dops(const acq_engine *e, const void *center, int half_width) { return center ? 2 * half_width + 1 : e->n_dop; }
 
+// Coherent search of M = m_coh blocks per group: n_dop_c = M (n_dop - 1) + 1 cells per row (1/M of the engine's Doppler
+// step), F = M (1 + half_bin) spectrum variants per block
+int coh_dops(const acq_engine *e, int m_coh) { return m_coh * (e->n_dop - 1) + 1; }
+int coh_variants(const acq_engine *e, int m_coh) { return m_coh * (1 + e->prm.half_bin); }
+
+// Rotation table of the sub-bin variants, [F][16384]: row v = exp(-2 pi i (v / F) n / N), double precision rounded once.
+// The angle is pi (a n) / (b N) with a / b = 2 v / F in lowest terms, so that the row v = F / 2 of an even F is formed by
+// the same operations as the half-bin table of acq_create (pi n / N) and rounds to the same floats.
+int ensure_coh_rot(acq_engine *e, int m_coh)
+{
+    if (e->d_rot_coh[m_coh]) return ACQ_OK;
+    const int F = coh_variants(e, m_coh);
+    const double pi = 3.14159265358979323846264338327950288;
+    std::vector<float2> rot((size_t)F * kN);
+    for (int v = 0; v < F; v++) {
+        const int g = std::gcd(2 * v, F), a = 2 * v / g, b = F / g;
+        for (int n = 0; n < kN; n++) {
+            const double ang = pi * (double)((long long)a * n) / (double)((long long)b * kN);
+            rot[(size_t)v * kN + n] = make_float2((float)cos(ang), (float)(-sin(ang)));
+        }
+    }
+    float2 *d = nullptr;
+    CU(cudaMalloc(&d, rot.size() * sizeof(float2)));
+    const cudaError_t ce = cudaMemcpy(d, rot.data(), rot.size() * sizeof(float2), cudaMemcpyHostToDevice);
+    if (ce != cudaSuccess) {
+        cudaFree(d);
+        return fail(ACQ_ERR_CUDA, "coherent rotation table: %s", cudaGetErrorString(ce));
+    }
+    e->d_rot_coh[m_coh] = d;
+    return ACQ_OK;
+}
+
+int check_search_args(acq_engine *e, const void *packed, int n_captures, const void *out);
+
+// The arguments of a coherent search, checked before anything touches the device: ACQ_ERR_ARG for the argument errors,
+// ACQ_ERR_UNSUPPORTED for what the coherent search does not cover (E1B rows, code-Doppler engines, searches above the
+// tile and spectrum-row bounds).
+int check_coherent(acq_engine *e, const void *packed, int n_captures, const int32_t *sel, int n_sel, int m_coh,
+                   const void *out)
+{
+    if (!e) return fail(ACQ_ERR_ARG, "engine is NULL");
+    if (m_coh < 1 || m_coh > ACQ_COH_MAX) return fail(ACQ_ERR_ARG, "m_coh=%d outside 1..%d", m_coh, ACQ_COH_MAX);
+    int rc = check_search_args(e, packed, n_captures, out);
+    if (rc) return rc;
+    if (e->prm.k_noncoh % m_coh)
+        return fail(ACQ_ERR_ARG, "k_noncoh=%d is not a multiple of m_coh=%d", e->prm.k_noncoh, m_coh);
+    const int n_sats = (int)e->sats.size();
+    if (sel && n_sel <= 0) return fail(ACQ_ERR_ARG, "n_sel must be > 0 when sel is given");
+    const int n_slots = sel ? n_sel : n_sats;
+    for (int i = 0; i < n_slots; i++) {
+        const int s = sel ? sel[i] : i;
+        if (s < 0 || s >= n_sats) return fail(ACQ_ERR_ARG, "satellite index %d outside the table (0..%d)", s, n_sats - 1);
+    }
+    if (e->prm.code_doppler)
+        return fail(ACQ_ERR_UNSUPPORTED, "coherent search of a code_doppler engine is not implemented");
+    for (int i = 0; i < n_slots; i++)
+        if (e->sats[sel ? sel[i] : i].type == ACQ_E1B)
+            return fail(ACQ_ERR_UNSUPPORTED, "coherent search of E1B rows is not implemented (satellite %d): E1B symbols "
+                        "drift against the block edges", sel ? sel[i] : i);
+    if ((long long)n_captures * e->prm.k_noncoh * coh_variants(e, m_coh) > (1 << 24))
+        return fail(ACQ_ERR_UNSUPPORTED, "coherent search too large for one call (more than 2^24 capture spectra): split the captures");
+    if ((double)n_captures * (double)n_slots * (double)coh_dops(e, m_coh) > (double)acq::kMaxTilesPerLaunch)
+        return fail(ACQ_ERR_UNSUPPORTED, "coherent search too large for one call (more than 2^31 - 1 tiles): split the captures");
+    return ACQ_OK;
+}
+
 // Enqueue front end + forward FFT + search (which ends in the best-Doppler pick) on `st` for captures already on the
 // device.  records_dev: where the kernels write the records (device memory, or the device alias of mapped host memory);
 // flag_dev: mapped completion word, or NULL.  center_dev: the rows' Doppler centres on the device (an aided search), or
-// NULL for the whole range.
+// NULL for the whole range.  m_coh > 0: a coherent search (acq_search_coherent) of M = m_coh blocks per group.
 int enqueue_search(acq_engine *e, const uint8_t *packed_dev, int n_captures, acq_record *records_dev, unsigned *flag_dev,
                    cudaStream_t st, const uint8_t *packed_host_arg = nullptr, const int *center_dev = nullptr,
-                   int half_width = 0)
+                   int half_width = 0, int m_coh = 0)
 {
     const int K = e->prm.k_noncoh;
-    const int n_dop = row_dops(e, center_dev, half_width);
+    const int n_dop = m_coh ? coh_dops(e, m_coh) : row_dops(e, center_dev, half_width);
+    const int nvar = m_coh ? coh_variants(e, m_coh) : e->nvar;
     const int blocks = n_captures * K;
     const bool prof = e->profiling;
     if (e->dev_pending) CU(cudaStreamWaitEvent(st, e->dev_done, 0));  // a no-op on the stream that recorded it
@@ -398,10 +471,14 @@ int enqueue_search(acq_engine *e, const uint8_t *packed_dev, int n_captures, acq
             return fail(ACQ_ERR_CUDA, "front-end launch failed: %s", cudaGetErrorString(cudaGetLastError()));
         e->launches++;
     } else {
-        e->launches += launch_front_end(packed_dev, e->d_x2, e->d_rot, blocks, e->nvar, K, e->sample_bits, e->n_shift, e->smax, st);
+        // a coherent search: k_front_end writes variant 0 (and with F = 2 variant 1, from row 1 of the table, which equals
+        // the half-bin table), k_coh_variants the others
+        const float2 *rot = m_coh ? e->d_rot_coh[m_coh] + kN : e->d_rot;
+        e->launches += launch_front_end(packed_dev, e->d_x2, rot, blocks, nvar, K, e->sample_bits, e->n_shift, e->smax, st);
+        if (nvar > 2) e->launches += launch_coh_variants(e->d_x2, e->d_rot_coh[m_coh], blocks, nvar, K, st);
     }
     if (prof) CU(cudaEventRecord(e->prof[1], st));
-    e->launches += launch_fwd_fft(e->d_x2, e->d_Dp, e->d_tables, blocks * e->nvar * e->n_shift, true, e->sm_count, st, pdl);
+    e->launches += launch_fwd_fft(e->d_x2, e->d_Dp, e->d_tables, blocks * nvar * e->n_shift, true, e->sm_count, st, pdl);
     if (prof) CU(cudaEventRecord(e->prof[2], st));
     SearchArgs a{};
     a.Dp = e->d_Dp;
@@ -410,13 +487,13 @@ int enqueue_search(acq_engine *e, const uint8_t *packed_dev, int n_captures, acq
     a.cells = e->d_cells;
     a.n_slots = e->n_slots;
     a.n_dop = n_dop;
-    a.dop_lo = e->prm.dop_lo;
+    a.dop_lo = e->prm.dop_lo * (m_coh ? m_coh : 1);
     a.dop_center = center_dev;
     a.half_width = half_width;
-    a.dop_hi = e->prm.dop_hi;
+    a.dop_hi = e->prm.dop_hi * (m_coh ? m_coh : 1);
     a.half_bin = e->prm.half_bin;
     a.K = K;
-    a.nvar = e->nvar;
+    a.nvar = nvar;
     a.ext_len = e->ext_len;
     a.Q = e->Q;
     a.n_shift = e->n_shift;
@@ -430,11 +507,18 @@ int enqueue_search(acq_engine *e, const uint8_t *packed_dev, int n_captures, acq
     // one-CTA-per-tile forms (k_search_e1b, k_search_e1b_multi for non-coherent sums) have ~2.9x the throughput.
     const bool e1b_cluster = ACQ_FORCE_E1B_KERNEL == 2 || (ACQ_FORCE_E1B_KERNEL == 0 && tiles_e1b <= e->sm_count / 4);
     a.ctas_done = e->d_ctas_done;
-    a.ctas_total = fold ? (unsigned)(search_grid_ctas(tiles_l1, search_kind_l1(K, e->prm.half_bin), e->sm_count) +
+    a.ctas_total = fold ? (unsigned)((m_coh ? coh_grid_ctas(tiles_l1, e->sm_count)
+                                            : search_grid_ctas(tiles_l1, search_kind_l1(K, e->prm.half_bin), e->sm_count)) +
                                      search_grid_ctas(tiles_e1b, e1b_cluster ? kSearchE1bCluster : kSearchE1b, e->sm_count))
                         : 0u;
     a.wait_prior = 1;
-    if (e->n_l1 > 0) {
+    if (m_coh && e->n_l1 > 0) {   // the selection holds no E1B row (check_coherent)
+        a.work = e->cur_work;
+        a.n_work = e->n_l1;
+        a.n_tiles = tiles_l1;
+        a.tile_ctr = e->d_tile_ctr;
+        e->launches += launch_search_coh(CohSearchArgs(a, m_coh), e->sm_count, st, pdl);
+    } else if (e->n_l1 > 0) {
         a.work = e->cur_work;
         a.n_work = e->n_l1;
         a.n_tiles = tiles_l1;
@@ -455,7 +539,7 @@ int enqueue_search(acq_engine *e, const uint8_t *packed_dev, int n_captures, acq
         else e->launches += launch_search(a, true, e->sm_count, st, pdl);
     }
     if (prof) CU(cudaEventRecord(e->prof[3], st));
-    const PickDop pd{e->prm.dop_lo, center_dev, half_width, e->prm.dop_hi};
+    const PickDop pd{a.dop_lo, center_dev, half_width, a.dop_hi};
     if (fold)
         e->launches += launch_pick_small(e->d_cells, e->cur_slot_sat, records_dev, e->d_ctas_done, a.ctas_total, flag_dev,
                                          e->epoch, n_rows, e->n_slots, n_dop, pd, st, pdl);
@@ -584,18 +668,20 @@ int enqueue_profile(acq_engine *e, const acq_record *rec_dev, int n_records, int
 }
 
 // center (HOST, one per row) and half_width: an aided search (acq_search_aided), or NULL for the whole range
+// m_coh > 0: a coherent search (acq_search_coherent), its arguments already checked by check_coherent
 int search_host(acq_engine *e, const uint8_t *packed, int n_captures, const int32_t *sel, int n_sel, acq_record *out,
-                acq_cell *grid, bool sync, const int32_t *center = nullptr, int half_width = 0)
+                acq_cell *grid, bool sync, const int32_t *center = nullptr, int half_width = 0, int m_coh = 0)
 {
     int rc = check_search_args(e, packed, n_captures, out);
     if (rc) return rc;
     DeviceGuard g(e->device);
     e->last_captures = 0;  // until this search is enqueued, there are no spectra acq_refine could use
     e->ref_captures = 0;
-    const int n_dop = row_dops(e, center, half_width);
+    const int n_dop = m_coh ? coh_dops(e, m_coh) : row_dops(e, center, half_width);
     if ((rc = set_selection(e, sel, n_sel))) return rc;
     if ((rc = check_tile_count(e, n_captures, n_dop))) return rc;
-    if ((rc = ensure_scratch(e, n_captures, e->n_slots, true, n_dop))) return rc;
+    if ((rc = ensure_scratch(e, n_captures, e->n_slots, true, n_dop, m_coh ? coh_variants(e, m_coh) : e->nvar))) return rc;
+    if (m_coh && (rc = ensure_coh_rot(e, m_coh))) return rc;
     const size_t bytes = (size_t)n_captures * e->prm.k_noncoh * e->block_bytes;
     const size_t rows = (size_t)n_captures * e->n_slots;
     if (center) {
@@ -614,7 +700,7 @@ int search_host(acq_engine *e, const uint8_t *packed, int n_captures, const int3
     const bool poll = host_records && sync && !grid && !e->profiling && tiles_total <= 64LL * e->sm_count;
     // The reference's own search -- one 1-bit block (gps/search.cpp:389-411) -- hands its 8 KiB to the front end as a
     // kernel argument: the launch carries the bytes, nothing is staged or copied ahead of the first kernel.
-    const bool as_arg = ACQ_ARG_INPUT && n_captures == 1 && e->prm.k_noncoh == 1 && e->sample_bits == 1 &&
+    const bool as_arg = ACQ_ARG_INPUT && !m_coh && n_captures == 1 && e->prm.k_noncoh == 1 && e->sample_bits == 1 &&
                         bytes == (size_t)ACQ_BLOCK_BYTES;
     const uint8_t *src = packed;
     if (!as_arg) {
@@ -630,10 +716,12 @@ int search_host(acq_engine *e, const uint8_t *packed, int n_captures, const int3
     }
     if ((rc = enqueue_search(e, e->d_packed, n_captures, host_records ? e->dh_records : e->d_records,
                              poll ? e->dh_flag : nullptr, e->stream, as_arg ? packed : nullptr, center ? e->d_center : nullptr,
-                             half_width)))
+                             half_width, m_coh)))
         return rc;
-    e->last_captures = n_captures;
-    set_refine_shape(e, n_captures);
+    if (!m_coh) {   // a coherent search leaves spectra that refinement and profile cannot read
+        e->last_captures = n_captures;
+        set_refine_shape(e, n_captures);
+    }
     if (!host_records) CU(cudaMemcpyAsync(out, e->d_records, rows * sizeof(acq_record), cudaMemcpyDeviceToHost, e->stream));
     if (grid)
         CU(cudaMemcpyAsync(grid, e->d_cells, rows * n_dop * sizeof(acq_cell), cudaMemcpyDeviceToHost, e->stream));
@@ -666,7 +754,7 @@ void finish_pending(acq_engine *e)
 
 // acq_search_device and acq_search_aided_device (center_dev != NULL)
 int search_device(acq_engine *e, const uint8_t *packed_dev, int n_captures, const int32_t *sel, int n_sel,
-                  acq_record *out_dev, void *stream, const int *center_dev = nullptr, int half_width = 0)
+                  acq_record *out_dev, void *stream, const int *center_dev = nullptr, int half_width = 0, int m_coh = 0)
 {
     int rc = check_search_args(e, packed_dev, n_captures, out_dev);
     if (rc) return rc;
@@ -675,13 +763,14 @@ int search_device(acq_engine *e, const uint8_t *packed_dev, int n_captures, cons
     DeviceGuard g(e->device);
     e->last_captures = 0;  // spectra now belong to a search on the caller's stream: acq_refine does not apply
     e->ref_captures = 0;   // ... and acq_refine_device applies once this search is enqueued
-    const int n_dop = row_dops(e, center_dev, half_width);
+    const int n_dop = m_coh ? coh_dops(e, m_coh) : row_dops(e, center_dev, half_width);
     if ((rc = set_selection(e, sel, n_sel))) return rc;
     if ((rc = check_tile_count(e, n_captures, n_dop))) return rc;
-    if ((rc = ensure_scratch(e, n_captures, e->n_slots, false, n_dop))) return rc;
+    if ((rc = ensure_scratch(e, n_captures, e->n_slots, false, n_dop, m_coh ? coh_variants(e, m_coh) : e->nvar))) return rc;
+    if (m_coh && (rc = ensure_coh_rot(e, m_coh))) return rc;
     cudaStream_t st = stream ? (cudaStream_t)stream : e->stream;
-    if ((rc = enqueue_search(e, packed_dev, n_captures, out_dev, nullptr, st, nullptr, center_dev, half_width))) return rc;
-    set_refine_shape(e, n_captures);
+    if ((rc = enqueue_search(e, packed_dev, n_captures, out_dev, nullptr, st, nullptr, center_dev, half_width, m_coh))) return rc;
+    if (!m_coh) set_refine_shape(e, n_captures);
     if (st != e->stream) {  // whatever uses the engine's scratch next (any stream, or the host) waits for this search
         CU(cudaEventRecord(e->dev_done, st));
         e->dev_pending = true;
@@ -967,6 +1056,22 @@ int acq_search_aided_device(acq_engine *e, const uint8_t *packed_dev, int n_capt
     const int rc = check_aided_args(e, dop_center_dev, half_width);
     if (rc) return rc;
     return search_device(e, packed_dev, n_captures, sel, n_sel, out_dev, stream, dop_center_dev, half_width);
+}
+
+int acq_search_coherent(acq_engine *e, const uint8_t *packed, int n_captures, const int32_t *sel, int n_sel, int m_coh,
+                        acq_record *out, acq_cell *grid)
+{
+    const int rc = check_coherent(e, packed, n_captures, sel, n_sel, m_coh, out);
+    if (rc) return rc;
+    return search_host(e, packed, n_captures, sel, n_sel, out, grid, true, nullptr, 0, m_coh);
+}
+
+int acq_search_coherent_device(acq_engine *e, const uint8_t *packed_dev, int n_captures, const int32_t *sel, int n_sel,
+                               int m_coh, acq_record *out_dev, void *stream)
+{
+    const int rc = check_coherent(e, packed_dev, n_captures, sel, n_sel, m_coh, out_dev);
+    if (rc) return rc;
+    return search_device(e, packed_dev, n_captures, sel, n_sel, out_dev, stream, nullptr, 0, m_coh);
 }
 
 int acq_submit(acq_engine *e, const uint8_t *packed, int n_captures, const int32_t *sel, int n_sel, acq_record *out)

@@ -564,6 +564,13 @@ struct TileIdx {
     __device__ __forceinline__ void set_dop(const PA &p)
     {
         int h;
+        if constexpr (PA::kCoh) {   // 1/F-bin steps: integer bin (floored) and sub-bin variant
+            h = p.dop_lo + d;
+            const int F = p.nvar;
+            dop = (h >= 0 ? h : h - F + 1) / F;
+            v = h - F * dop;
+            return;
+        }
         if constexpr (PA::kAided) h = window_lo(__ldg(p.dop_center + cap * p.n_slots + slot), p.half_width, p.dop_lo, p.dop_hi) + d;
         else h = p.dop_lo + d;
         v = p.half_bin ? (h & 1) : 0;
@@ -1103,6 +1110,197 @@ __global__ void __launch_bounds__(256, 2) k_search_l1_multi(const PA p)
     search_cta_epilogue(p, t);
     ACQ_TRACE_STAMP(kTrSearchL1, 2);
     tmem_free_cta<2 * kTwCols>(tmem_base, t);
+}
+
+// k_search_l1_coh -- coherent search (acq_search_coherent): k_search_l1_multi's tile (code run E resident in tensor memory
+// across the K blocks, D staged per block by TMA, same sub-FFTs and combine), but the K blocks form G = K / M groups of M
+// and the lag vectors of a group are added as complex numbers before any power is taken.
+//   Block j of a group is rotated by exp(i theta_j), theta_j = 2 pi j (v / F - 16 d / N): the carrier phase that block's
+//   processing removed.  A carrier exp(2 pi i (d + v / F) n / N) (the signal Doppler index h = F d + v selects; see the
+//   front end's conventions) advances by d + v / F cycles per 16384-sample block; the sub-bin rotation restarts every block
+//   and so leaves v / F cycles per block, the integer d cycles vanish, and the 16 b-sample circular delay that lines the
+//   code up (k_front_end) moves the block's carrier back by 16 b d / N cycles.  The correlation conj(D) C carries the
+//   conjugate phase, so r'_b ~ exp(-2 pi i b (v / F - 16 d / N)) and theta_j undoes it.  theta_0 = 0: block 0 of a group
+//   is used as computed.
+//   Data-bit hypotheses: T = sum of the group's rotated blocks u_j, prefixes S_s = sum_{j<s} u_j (s = 1..M-1); a bit
+//   edge before block s gives |S_s - (T - S_s)|^2 = |2 S_s - T|^2, no edge |T|^2; the group adds max over the M
+//   hypotheses into P.  The prefixes live in tensor memory: the thread's 128 columns next to the code run (512 columns
+//   per CTA, so one CTA per SM; 255 registers for T, P, the accumulators and the sub-FFT operands).
+//   M = 1: one hypothesis, P[n] = sum_b |r'_b[n]|^2 with k_search_l1_multi's operations in its order: the same cells.
+#ifndef ACQ_COH_UNROLL
+#define ACQ_COH_UNROLL 4
+#endif
+template <class PA>
+__global__ void __launch_bounds__(256, 1) k_search_l1_coh(const PA p)
+{
+    extern __shared__ __align__(1024) unsigned char smem[];
+    L1MultiSmem s;
+    s.S1 = reinterpret_cast<float2 *>(smem);
+    s.E = s.S1 + 2 * kSub;
+    s.bar = reinterpret_cast<unsigned long long *>(s.E + kEBufElems);
+    s.T2 = reinterpret_cast<float2 *>(s.bar + 2);
+    s.red_f = reinterpret_cast<float *>(s.T2 + kT2Elems);  // [2 parities][16], then the TMEM slot at [48]
+    s.red_i = reinterpret_cast<int *>(s.red_f + 32);        // [2 parities][8]
+    float *red_f = s.red_f;
+    int *red_i = s.red_i;
+    const int t = threadIdx.x;
+    constexpr int L = ACQ_LAGS_L1;
+    const int M = p.m_coh;
+    const int FN = p.nvar * kN;   // phase unit: 1 / (F N) cycle
+    const uint32_t tmem_base = tmem_alloc_cta<4 * kTwCols>(reinterpret_cast<uint32_t *>(red_f + 48), t);
+    const uint32_t e_taddr = tmem_base + tmem_lane_base(t) + (uint32_t)((t >> 7) * 2 * kTwCols);  // [k2][16 complex]
+    const uint32_t s_taddr = e_taddr + kTwCols;                                                   // [s - 1][16 complex]
+    {   // stage-B twiddle table into shared memory
+        const float4 *src = reinterpret_cast<const float4 *>(p.tables);
+        float4 *dst = reinterpret_cast<float4 *>(s.T2);
+        for (int i = t; i < kT2Elems / 2; i += 256) dst[i] = __ldg(src + i);
+    }
+    const float2 *bases = p.tables + kT2Elems + t;  // [k2][256]: W16384^{4t+k2}
+    float2 bw = __ldg(bases);
+    const uint32_t bar = smem_u32(s.bar);
+    if (t == 0) mbar_init(bar, 1);
+    __syncthreads();
+    if (p.wait_prior) pdl_wait();
+    pdl_launch_dependents();
+    auto issue = [&](const TileIdx &tn, int bn, int k2n, int half) {
+        const int r = (k2n - tn.dop) & 3;
+        const int q = (k2n - tn.dop - r) >> 2;
+        const float2 *Dk = p.Dp + d_row(p, tn, bn) * kN + k2n * kSub;
+        fence_proxy_async();
+        if (bn == 0) {
+            const float2 *Ek = p.Ep + (size_t)(tn.sat * 4 + r) * p.ext_len + ((p.Q + q) & ~1);
+            mbar_expect_tx(bar, (uint32_t)(sizeof(float2) * (kSub + kEBufElems)));
+            tma_load_1d(smem_u32(s.E), Ek, (uint32_t)(sizeof(float2) * kEBufElems), bar);
+        } else {
+            mbar_expect_tx(bar, (uint32_t)(sizeof(float2) * kSub));
+        }
+        tma_load_1d(smem_u32(s.S1 + half * kSub), Dk, (uint32_t)(sizeof(float2) * kSub), bar);
+    };
+    TileIdx ti(p, blockIdx.x);
+    if (t == 0) issue(ti, 0, 0, 0);
+    int *feed = red_i + 20;
+    unsigned nxt = blockIdx.x;
+    int it = 0;
+    int par = 0, pend_cap = -1, pend_slot = 0, pend_d = 0;
+    auto flush = [&]() {
+        store_cell(p, pend_cap, pend_slot, pend_d, merge_warp_peaks(red_f + 16 * (par ^ 1), red_i + 8 * (par ^ 1)), L);
+    };
+
+    for (;;) {
+        float P[16];
+        float2 acc[16], T[16];
+        // theta_j of this tile in units of 1 / (F N) cycle: j * (v N - 16 d F) mod F N
+        int step = (ti.v * kN - 16 * ti.dop * p.nvar) % FN;
+        if (step < 0) step += FN;
+        int j = 0, ph = 0;
+        for (int b = 0; b < p.K; b++) {
+            float2 x[16];
+            constexpr int kCohUnroll = ACQ_COH_UNROLL;
+#pragma unroll kCohUnroll
+            for (int k2 = 0; k2 < 4; k2++) {
+                float2 *S1b = s.S1 + (it & 1) * kSub;
+                const float2 *Dk = S1b + t;
+                if (b == 0) {
+                    const int r = (k2 - ti.dop) & 3;
+                    const int q = (k2 - ti.dop - r) >> 2;
+                    const float2 *Ek = s.E + ((p.Q + q) & 1) + t;
+                    mbar_wait(bar, (uint32_t)(it & 1));
+#pragma unroll
+                    for (int a = 0; a < 16; a++) x[a] = Ek[256 * a];
+                    tmem_st16(e_taddr + 32 * k2, x);
+                    tmem_wait_st();
+                } else {
+                    tmem_ld16(e_taddr + 32 * k2, x);
+                    mbar_wait(bar, (uint32_t)(it & 1));
+                    tmem_wait_ld();
+                }
+#pragma unroll
+                for (int a = 0; a < 16; a++) x[a] = cmul_conj_a(Dk[256 * a], x[a]);
+                subfft4096_inv4s(x, k2, bw, S1b, t, s.T2, BaseFromGlobal{bases}, [&]() {
+                    if (t == 0) {
+                        if (b == 0 && k2 == 0) nxt = claim_tile(p, nxt);
+                        if (b == p.K - 1 && k2 == 2) publish_tile(feed, p, nxt);
+                        if (k2 < 3) issue(ti, b, k2 + 1, (it + 1) & 1);
+                        else if (b + 1 < p.K) issue(ti, b + 1, 0, (it + 1) & 1);
+                        else {
+                            TileIdx tn;
+                            if (next_tile(feed, tn)) issue(tn, 0, 0, (it + 1) & 1);
+                        }
+                    }
+                });
+                it++;
+                if (t == 0 && b == 0 && k2 == 0 && pend_cap >= 0) flush();
+                if (k2 == 0) {
+#pragma unroll
+                    for (int n2 = 0; n2 < 16; n2++) acc[n2] = x[r16(n2)];
+                } else {
+#pragma unroll
+                    for (int n2 = 0; n2 < 16; n2++) acc[n2] = cfma(x[r16(n2)], c_cC[k2][n2], acc[n2]);
+                }
+            }
+            if (j == 0) {
+#pragma unroll
+                for (int n2 = 0; n2 < 16; n2++) T[n2] = acc[n2];
+            } else {   // S_j = T, then T += exp(i theta_j) r'_b
+                tmem_st16(s_taddr + 32 * (j - 1), T);
+                tmem_wait_st();
+                float sn, cs;
+                sincospif(__fdiv_rn((float)(2 * ph), (float)FN), &sn, &cs);
+                const float2 w = make_float2(cs, sn);
+#pragma unroll
+                for (int n2 = 0; n2 < 16; n2++) T[n2] = cfma(acc[n2], w, T[n2]);
+            }
+            if (j == M - 1) {   // end of the group: best data-bit hypothesis per lag
+                float pg[16];
+#pragma unroll
+                for (int n2 = 0; n2 < 16; n2++) pg[n2] = cpower(T[n2]);
+                for (int e = 1; e < M; e++) {
+                    float2 S[16];
+                    tmem_ld16(s_taddr + 32 * (e - 1), S);
+                    tmem_wait_ld();
+#pragma unroll
+                    for (int n2 = 0; n2 < 16; n2++)
+                        pg[n2] = fmaxf(pg[n2], cpower(make_float2(2.0f * S[n2].x - T[n2].x, 2.0f * S[n2].y - T[n2].y)));
+                }
+#pragma unroll
+                for (int n2 = 0; n2 < 16; n2++) P[n2] = (b == M - 1) ? pg[n2] : (P[n2] + pg[n2]);
+                j = 0;
+                ph = 0;
+            } else {
+                j++;
+                ph += step;
+                if (ph >= FN) ph -= FN;
+            }
+        }
+        warp_reduce_peak(thread_peak_l1(P, t), red_f + 16 * par, red_i + 8 * par, t);
+        pend_cap = ti.cap;
+        pend_slot = ti.slot;
+        pend_d = ti.d;
+        par ^= 1;
+        if (!next_tile(feed, ti)) break;
+    }
+    __syncthreads();
+    if (t == 0 && pend_cap >= 0) flush();
+    claims_done(p, t);
+    search_cta_epilogue(p, t);
+    tmem_free_cta<4 * kTwCols>(tmem_base, t);
+}
+
+// Sub-bin variants of a coherent search: variant v (1..F-1) of block row r = variant 0 (k_front_end's output, delayed by
+// 16 (r mod K) samples) times rot[v][o] at the sample's undelayed index o, with the half-bin variant's arithmetic, so
+// variant F/2 of an even F is bit-identical to the half-bin variant of k_front_end.
+__global__ void __launch_bounds__(256) k_coh_variants(float2 *__restrict__ x2, const float2 *__restrict__ rot, int F, int K,
+                                                      int row0)
+{
+    const int m = blockIdx.x * 256 + threadIdx.x;
+    float2 *row = x2 + (size_t)blockIdx.y * F * kN;
+    const int o = (m - 16 * ((row0 + (int)blockIdx.y) % K)) & (kN - 1);
+    const float2 y = row[m];
+    for (int v = 1; v < F; v++) {
+        const float2 w = __ldg(rot + (size_t)v * kN + o);
+        row[(size_t)v * kN + m] = make_float2(__fsub_rn(__fmul_rn(y.x, w.x), __fmul_rn(y.y, w.y)),
+                                              __fadd_rn(__fmul_rn(y.x, w.y), __fmul_rn(y.y, w.x)));
+    }
 }
 
 // k_search_l1_cr -- K = 1 on full bins with the CAPTURE operand resident in tensor memory and tiles claimed in CHUNKS.
@@ -2378,7 +2576,13 @@ cudaError_t search_kernels_configure()
                            (const void *)k_search_e1b_cluster<true, S>, (const void *)k_pick_small, (const void *)k_best_dop};
     for (const void *f : chain)
         if ((e = cudaFuncSetAttribute(f, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared))) return e;
-    return aided_kernels_configure();
+    if ((e = aided_kernels_configure())) return e;
+    using CA = CohSearchArgs;
+    if ((e = cudaFuncSetAttribute(k_search_l1_coh<CA>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)l1_multi_smem_bytes()))) return e;
+    const void *coh[] = {(const void *)k_search_l1_coh<CA>, (const void *)k_coh_variants};
+    for (const void *f : coh)
+        if ((e = cudaFuncSetAttribute(f, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared))) return e;
+    return cudaSuccess;
 }
 
 int launch_front_end(const uint8_t *packed, float2 *x2, const float2 *rot, int n_blocks, int nvar, int K, int sample_bits,
@@ -2577,6 +2781,34 @@ int launch_search(const SearchArgs &a_in, bool e1b, int sm_count, cudaStream_t s
     }
     else launch_k(k_search_l1<false, S>, grid, 256, search_l1_smem_bytes(), st, pdl, a);
 #endif
+    return 1;
+}
+
+int launch_coh_variants(float2 *x2, const float2 *rot, int n_rows, int F, int K, cudaStream_t st)
+{
+    int launched = 0;
+    for (int r0 = 0; r0 < n_rows; r0 += 32768) {  // gridDim.y <= 65535
+        const int nr = (n_rows - r0 < 32768) ? (n_rows - r0) : 32768;
+        k_coh_variants<<<dim3(kN / 256, nr), 256, 0, st>>>(x2 + (size_t)r0 * F * kN, rot, F, K, r0);
+        launched++;
+    }
+    return launched;
+}
+
+// one persistent CTA per SM (512 tensor-memory columns each); tiles claimed from a counter from ACQ_DYN_MIN_ROUNDS rounds
+int coh_grid_ctas(long long n_tiles, int sm_count)
+{
+    if (n_tiles <= 0 || n_tiles > kMaxTilesPerLaunch) return 0;
+    return (int)(n_tiles < sm_count ? n_tiles : sm_count);
+}
+
+int launch_search_coh(const CohSearchArgs &a_in, int sm_count, cudaStream_t st, bool pdl)
+{
+    const int grid = coh_grid_ctas(a_in.n_tiles, sm_count);
+    if (grid <= 0) return 0;
+    CohSearchArgs a = a_in;
+    if (!search_claims_tiles(a.n_tiles, grid)) a.tile_ctr = nullptr;
+    launch_k(k_search_l1_coh<CohSearchArgs>, grid, 256, l1_multi_smem_bytes(), st, pdl, a);
     return 1;
 }
 

@@ -43,6 +43,7 @@ struct SearchArgs {
     const int *dop_center;
     int half_width, dop_hi;
     static constexpr bool kAided = false;
+    static constexpr bool kCoh = false;
 };
 // The arguments of an aided search, a type of their own: the search kernels are templates over the argument type and
 // read the window only in this instantiation, so the full-range kernels compile to the code they had without the
@@ -52,6 +53,16 @@ struct AidedSearchArgs : SearchArgs {
     static constexpr bool kAided = true;
     AidedSearchArgs() = default;
     explicit AidedSearchArgs(const SearchArgs &a) : SearchArgs(a) {}
+};
+// The arguments of a coherent search (acq_search_coherent), read only by k_search_l1_coh.  Doppler index h runs over
+// dop_lo..dop_hi in steps of 1/F bin (F = nvar = m_coh * (1 + half_bin) spectrum variants per block): the code row is
+// shifted by d = floor(h / F) bins and block b reads variant v = h - F d, which the front end rotated by
+// exp(-2 pi i (v / F) n / N).  m_coh consecutive blocks form a group whose lag vectors are added coherently.
+struct CohSearchArgs : SearchArgs {
+    static constexpr bool kCoh = true;
+    int m_coh;
+    CohSearchArgs() = default;
+    explicit CohSearchArgs(const SearchArgs &a, int m) : SearchArgs(a), m_coh(m) {}
 };
 
 // s(b, h) of acq_params.code_doppler (same integer arithmetic as the oracle's orc_code_shift)
@@ -91,6 +102,12 @@ int launch_fwd_fft(const float2 *x2, float2 *out, const float2 *tables, int n_ro
 int launch_build_ext(const float2 *C, float2 *Ep, int n_sats, int Q, int ext_len, int wrap_mode, cudaStream_t st);
 int launch_search(const SearchArgs &a, bool e1b, int sm_count, cudaStream_t st, bool pdl = false);
 int launch_search_e1b_cluster(const SearchArgs &a, int sm_count, cudaStream_t st, bool pdl = false);
+// Coherent search (acq_search_coherent): the sub-bin variants 1..F-1 of every block row of x2 (layout [row][F][16384]),
+// formed from variant 0 with the host-built table rot ([F][16384]); then the C/A search kernel k_search_l1_coh, one CTA
+// per SM, with grid coh_grid_ctas() (what SearchArgs::ctas_total counts).
+int launch_coh_variants(float2 *x2, const float2 *rot, int n_rows, int F, int K, cudaStream_t st);
+int coh_grid_ctas(long long n_tiles, int sm_count);
+int launch_search_coh(const CohSearchArgs &a, int sm_count, cudaStream_t st, bool pdl = false);
 // Doppler indices of the cell rows a best-Doppler pick reads: cell d of row r is index dop_lo + d, or, with
 // dop_center (an aided search), window_lo(dop_center[r], half_width, dop_lo, dop_hi) + d.
 struct PickDop {

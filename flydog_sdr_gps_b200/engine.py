@@ -207,6 +207,33 @@ class AcqEngine:
         _check(self._L.acq_search_aided_device(self._h, packed_dev, n_cap, sp, n_sel, dop_center_dev, int(half_width), out_dev,
                                                stream_ptr), self._L)
 
+    # ---- coherent search: M = m_coh blocks added as complex lag vectors (with a data-bit hypothesis), then powers
+    def coherent_dops(self, m_coh):
+        """n_dop_c = M (n_dop - 1) + 1: cells per row of a coherent search (1/M of the engine's Doppler step)."""
+        return int(m_coh) * (self.n_dop - 1) + 1
+
+    def coherent_dop_hz(self, dop, m_coh):
+        """Doppler in Hz of a coherent record's (or cell's) index: dop * BIN_HZ / F, F = M (1 + half_bin)."""
+        return np.asarray(dop, np.float64) * BIN_HZ / (int(m_coh) * (1 + self.params.half_bin))
+
+    def search_coherent(self, packed, m_coh, sel=None, want_grid=False):
+        """acq_search_coherent: records [n_cap, n_sel] (dop in 1/F-bin steps, see coherent_dop_hz) and, if asked, the
+        cells [n_cap, n_sel, n_dop_c]; cell j of a row is Doppler index M * dop_lo + j."""
+        a, n_cap = self._packed(packed)
+        sp, n_sel, keep = self._sel(sel)
+        out = np.zeros((n_cap, n_sel), RECORD_DTYPE)
+        grid = np.zeros((n_cap, n_sel, self.coherent_dops(m_coh)), CELL_DTYPE) if want_grid else None
+        _check(self._L.acq_search_coherent(self._h, a.ctypes.data, n_cap, sp, n_sel, int(m_coh), out.ctypes.data,
+                                           grid.ctypes.data if want_grid else None), self._L)
+        return (out, grid) if want_grid else out
+
+    def search_coherent_device(self, packed_dev, m_coh, out_dev, n_cap, sel=None, stream_ptr=None):
+        """acq_search_coherent_device: packed_dev / out_dev are device pointers (ints).  Enqueues on stream_ptr (None =
+        engine stream)."""
+        sp, n_sel, keep = self._sel(sel)
+        _check(self._L.acq_search_coherent_device(self._h, packed_dev, n_cap, sp, n_sel, int(m_coh), out_dev, stream_ptr),
+               self._L)
+
     def refine(self, records):
         """acq_refine: hand-off refinement of the records of the most recent search()/wait() -- FINE_DTYPE array of
         the same shape (Doppler in Hz from a three-bin interpolation, code phase in FS samples from early/late)."""

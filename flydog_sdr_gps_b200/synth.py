@@ -71,15 +71,20 @@ def _planes(s, sample_bits, mag_thr):
 
 
 F_L1 = 1575.42e6
+BIT_SAMPLES = 327360   # one 20 ms GPS/QZSS L1 C/A data bit at FS
 
 
-def make_capture(seed, n_blocks, sats, signals, sample_bits=1, mag_thr=0.98, code_doppler=False, chip_source=None):
+def make_capture(seed, n_blocks, sats, signals, sample_bits=1, mag_thr=0.98, code_doppler=False, chip_source=None,
+                 data_bits=None, bit_edge=0):
     """numpy generator.  signals: iterable of (sat, tau, doppler_hz, cn0_dbhz, phase).  Returns uint8[n_blocks*8192]
     (sample_bits=2: uint8[n_blocks*16384], 2-bit sign/magnitude with the same sign bits; mag_thr in noise sigmas --
     0.98 is the optimum of a 4-level quantiser with levels +-1, +-3, a magnitude duty cycle of about 1/3).
     code_doppler=True also applies each signal's Doppler to its code rate (0.52 chip of drift over 80 ms at 10 kHz).
     chip_source: optional callable(row) -> (chips, boc) replacing this module's code tables (the golden generator passes
-    the reference's own code classes, so that those fixtures do not depend on the product's tables)."""
+    the reference's own code classes, so that those fixtures do not depend on the product's tables).
+    data_bits: optional GPS data-bit modulation of every non-E1B signal: a sequence of signs (+1 / -1), bit k covering
+    samples [bit_edge + k BIT_SAMPLES, bit_edge + (k + 1) BIT_SAMPLES) (20 ms bits; k < 0 before bit_edge), taken
+    cyclically.  None (the default) leaves the samples, and so the bytes, as without it."""
     rng = np.random.Generator(np.random.Philox(int(seed)))
     n = n_blocks * BLOCK_SAMPLES
     i = np.arange(n, dtype=np.int64)
@@ -93,6 +98,9 @@ def make_capture(seed, n_blocks, sats, signals, sample_bits=1, mag_thr=0.98, cod
             c = c ^ ((idx & 15) >= 8)
         amp = np.sqrt(4.0 * 10.0 ** (cn0 / 10.0) / FS)
         cyc = (dop / FS * i) % 1.0 + 0.25 * (i & 3)
+        if data_bits is not None and not boc:
+            bits = np.asarray(data_bits, np.float64)
+            amp = amp * bits[np.floor_divide(i - int(bit_edge), BIT_SAMPLES) % bits.size]
         s += amp * (1.0 - 2.0 * c) * np.cos(2.0 * np.pi * cyc + phase)
     return _planes(s, sample_bits, mag_thr)
 

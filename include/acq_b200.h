@@ -202,6 +202,34 @@ int acq_search_aided(acq_engine *e, const uint8_t *packed, int n_captures, const
 int acq_search_aided_device(acq_engine *e, const uint8_t *packed_dev, int n_captures, const int32_t *sel, int n_sel,
                             const int32_t *dop_center_dev, int half_width, acq_record *out_dev, void *stream);
 
+/* Coherent integration across capture blocks (extension).  The k_noncoh blocks of a capture form G = k_noncoh / m_coh
+ * groups of M = m_coh consecutive blocks (1 <= M <= ACQ_COH_MAX, k_noncoh % M == 0).  Inside a group the blocks' complex
+ * lag vectors are added after each block is rotated back to the carrier phase of the group's first block, and only then
+ * squared; the G group powers are added like the non-coherent sum.  A GPS/QZSS data bit lasts 20 ms, so a group
+ * (M x 4.004 ms <= 20.02 ms) holds at most one sign change: for each lag the largest of the M hypotheses "no change" and
+ * "change before block s" (s = 1..M-1) is taken.  A bit edge inside a block partly cancels that block; no block-aligned
+ * hypothesis can undo that.
+ *   Doppler: the grid is M times finer than the engine's.  Record and cell index h runs over M*dop_lo .. M*dop_hi, so a
+ *   row has n_dop_c = M*(n_dop - 1) + 1 cells, and h stands for h * ACQ_BIN_HZ / F Hz with F = M * (1 + half_bin).
+ *   M = 1 is acq_search / acq_search_grid of the same engine and bytes, bit for bit.
+ *   Records and cells follow Correlate()'s rules (peak = max, noise = mean over the 4092 lags, snr = peak / noise; the
+ *   record is the best cell, lowest index on ties).  Under noise alone snr is distributed differently for each (M, G):
+ *   choose the detection threshold again for a coherent search (acq_detected applies thr_l1 as is).
+ *   packed, sel and out as acq_search; grid NULL or HOST n_captures * n_sel * n_dop_c cells.  Synchronous.
+ * ACQ_ERR_ARG: m_coh outside 1..ACQ_COH_MAX, k_noncoh % m_coh != 0, and acq_search's argument errors.
+ * ACQ_ERR_UNSUPPORTED, before any device work and leaving the engine usable: an E1B row in the selection (its symbols
+ * last one 4 ms code period and drift 16 samples per block against the block edges), an engine with code_doppler = 1, a
+ * search of more than 2^31 - 1 (capture, satellite, cell) tiles or 2^24 capture spectra (F per block).  SBAS rows give
+ * the records of acq_search.  A coherent search leaves no spectra acq_refine, acq_refine_device, acq_profile or
+ * acq_profile_device could use: they return ACQ_ERR_ARG until the next acq_search. */
+#define ACQ_COH_MAX 5
+int acq_search_coherent(acq_engine *e, const uint8_t *packed, int n_captures, const int32_t *sel, int n_sel, int m_coh,
+                        acq_record *out, acq_cell *grid);
+/* The device-resident form: packed_dev and out_dev are DEVICE pointers; ordering and validity rules are those of
+ * acq_search_device (packed_dev 16-byte aligned, sel consumed before return, no synchronise). */
+int acq_search_coherent_device(acq_engine *e, const uint8_t *packed_dev, int n_captures, const int32_t *sel, int n_sel,
+                               int m_coh, acq_record *out_dev, void *stream);
+
 /* Asynchronous pair over host buffers (the reference yields to other tasks while it computes,
  * gps/search.cpp:479-491): submit enqueues copy-in, search and copy-out on the engine's stream;
  * acq_wait blocks until done, acq_poll returns 1 when done, 0 while running.  The host buffers
