@@ -45,6 +45,16 @@ class CoherentRef:
         self._D = {}
         self.n = np.arange(N)
 
+    def for_sat(self, sat):
+        """The reference of another satellite on the same capture, sharing its block basebands and spectra."""
+        other = object.__new__(CoherentRef)
+        other.__dict__.update(self.__dict__)
+        other.sat = sat
+        other.C = self.O.code_spectrum(self.sats[sat]).astype(np.complex128)
+        other.nxt = (self.O.code_spectrum(self.sats[sat + 1]).astype(np.complex128) if sat + 1 < len(self.sats)
+                     else np.zeros(N, np.complex128))
+        return other
+
     def spectrum(self, b, v, F):
         key = (b, v, F)
         if key not in self._D:

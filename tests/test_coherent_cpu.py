@@ -45,6 +45,11 @@ M1_CASES = {
     "half_bins_k4": (dict(half_bin=1, k_noncoh=4, dop_lo=-9, dop_hi=7), 4, 1),
     "circular_wrap_k4": (dict(wrap_mode=1, k_noncoh=4, dop_lo=-12, dop_hi=3), 4, 1),
     "two_bit_half_bins": (dict(sample_bits=2, half_bin=1, dop_lo=-8, dop_hi=8), 1, 2),
+    # the shapes of the GPU limit tests: K = 255, the circular wrap on 2-bit samples, both ends of the +-2048-bin span
+    "k255_narrow": (dict(k_noncoh=255, dop_lo=-1, dop_hi=1), 255, 1),
+    "circular_wrap_two_bit_k3": (dict(wrap_mode=1, sample_bits=2, k_noncoh=3, dop_lo=-6, dop_hi=4), 3, 2),
+    "span_top_full_bins": (dict(dop_lo=2042, dop_hi=2048), 1, 1),
+    "span_bottom_half_bins": (dict(half_bin=1, dop_lo=-4094, dop_hi=-4087), 1, 1),
 }
 
 
@@ -59,8 +64,9 @@ def test_reference_m1_is_the_oracle_search(oracle, case):
     cap = synth.make_capture(31, K, table, sig, sample_bits=bits)
     sel = [4, 11, 20, 0]   # 0: wraps into row 1 at negative Doppler in the reference wrap
     _, grid = oracle.search(cap, table, sel=sel, params=params, want_grid=True)
+    base = CoherentRef(oracle, params, cap, table, sel[0])
     for s, sat in enumerate(sel):
-        hs, peak, noise, snr, lag, P = CoherentRef(oracle, params, cap, table, sat).cells(1)
+        hs, peak, noise, snr, lag, P = base.for_sat(sat).cells(1)
         assert np.array_equal(hs, grid_h(params, 1))
         g = grid[s]
         np.testing.assert_allclose(peak, g["peak"], rtol=2e-5)

@@ -53,7 +53,7 @@ def test_m1_is_acq_search_grid(gpu_required, name):
 RTOL = 1e-4
 
 
-@pytest.mark.parametrize("m_coh,groups,half_bin", [(m, g, hb) for m in (2, 3, 5) for g in (1, 2) for hb in (0, 1)])
+@pytest.mark.parametrize("m_coh,groups,half_bin", [(m, g, hb) for m in (2, 3, 4, 5) for g in (1, 2) for hb in (0, 1)])
 def test_against_reference(gpu_required, oracle, m_coh, groups, half_bin):
     """Cells of two satellites (one with a signal, one without) against the float64 reference: peak, noise, snr within
     RTOL; lag where the reference's power at the search's lag is not within RTOL of its peak; the record's dop where the
