@@ -1,8 +1,10 @@
 """Reference side of the coherent-search tests (acq_search_coherent): the power vectors and cells of a coherent search,
-rebuilt in numpy from the oracle's exported stages -- capture baseband, code spectrum, the row addressing of its
-Correlate restatement (tests/profile_ref.py::orc_profile) -- with the sub-bin rotation, the block phases theta_j and the
+rebuilt in numpy from the oracle's exported stages -- capture baseband, code baseband, the row addressing of its
+Correlate restatement (tests/profile_ref.py) -- with every FFT, the sub-bin rotation, the block phases theta_j and the
 data-bit hypotheses in float64.  The oracle itself knows nothing of coherent sums."""
 import numpy as np
+
+from profile_ref import block_lags, code_row, code_spectra64
 
 N = 16384
 LAGS_L1 = 4092
@@ -39,9 +41,7 @@ class CoherentRef:
         cap = np.ascontiguousarray(capture, np.uint8).reshape(-1)
         self.x = [O.capture_baseband(cap[b * bb:(b + 1) * bb], half_rot=0, sample_bits=bits).astype(np.complex128)
                   for b in range(self.K)]
-        self.C = O.code_spectrum(sats[sat]).astype(np.complex128)
-        self.nxt = (O.code_spectrum(sats[sat + 1]).astype(np.complex128) if sat + 1 < len(sats)
-                    else np.zeros(N, np.complex128))
+        self.C, self.nxt = code_spectra64(O, sats, sat)
         self._D = {}
         self.n = np.arange(N)
 
@@ -50,9 +50,7 @@ class CoherentRef:
         other = object.__new__(CoherentRef)
         other.__dict__.update(self.__dict__)
         other.sat = sat
-        other.C = self.O.code_spectrum(self.sats[sat]).astype(np.complex128)
-        other.nxt = (self.O.code_spectrum(self.sats[sat + 1]).astype(np.complex128) if sat + 1 < len(self.sats)
-                     else np.zeros(N, np.complex128))
+        other.C, other.nxt = code_spectra64(self.O, self.sats, sat)
         return other
 
     def spectrum(self, b, v, F):
@@ -62,20 +60,11 @@ class CoherentRef:
             self._D[key] = np.fft.fft(self.x[b] * rot)
         return self._D[key]
 
-    def code_row(self, d):
-        """code[(k - d) mod N] with correlate_one's wrap rule for d < 0 (orc_profile)."""
-        j = self.n - d
-        code = self.C[j % N].copy()
-        past = j >= N
-        if self.p.wrap_mode == self.O.WRAP_REFERENCE:
-            code[past] = self.nxt[j[past] - N]
-        return code
-
     def lags(self, b, d, v, F):
         """r'_b over the 4092 lags: r_b[(n + 16 b) mod N] (no shift for K = 1, as the search)."""
-        r = np.fft.ifft(np.conj(self.spectrum(b, v, F)) * self.code_row(d)) * N
-        m = (np.arange(LAGS_L1) + (16 * b if self.K > 1 else 0)) % N
-        return r[m]
+        code = code_row(self.C, self.nxt, d, self.p.wrap_mode == self.O.WRAP_REFERENCE)
+        r = np.fft.ifft(np.conj(self.spectrum(b, v, F)) * code) * N
+        return r[block_lags(LAGS_L1, b, 0, self.K, 0, False)]
 
     def power(self, h, m_coh, mode="coherent", sign16=-1):
         M = int(m_coh)

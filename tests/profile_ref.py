@@ -1,7 +1,8 @@
 """Reference side of the peak-quality tests (acq_profile): the power vector that the oracle's Correlate restatement
 (oracle/acq_oracle.c, correlate_one) forms at one Doppler index, summed over the K blocks, rebuilt from the oracle's own
 exported stages -- capture baseband, code spectrum, 16384-point FFT -- with nothing new but the indexing; and the
-second-peak reduction over such a vector."""
+second-peak reduction over such a vector.  The indexing helpers (code_row, block_lags) are the one statement of
+correlate_one's addressing that the float64 references (search_ref, coherent_ref) use too."""
 import numpy as np
 
 N = 16384
@@ -17,33 +18,63 @@ def code_shift(b, h, half_bin):
     return -s if a < 0 else s
 
 
-def orc_profile(O, params, capture, sats, sat, dop):
-    """float64 [L]: sum over the K blocks of |r_b[(n + 16 b + s(b, dop)) mod N]|^2 (s = 0 without code_doppler; for K = 1
-    just |r[n]|^2), r_b = IFFT(conj(D_b) * code[(k - d) mod N]) with correlate_one's row addressing: for a negative
-    Doppler the bins past the end of the doubled row come from the next table row (reference wrap, zeros after the last
-    row) or from the same row (circular wrap).  dop is the Doppler index (half-bins when half_bin)."""
-    K, half_bin = int(params.k_noncoh), int(params.half_bin)
-    bits = int(params.sample_bits) or 1
-    bb = O.block_bytes(bits)
+def lags_of(sat):
+    """L of a table row (prn, t1, t2, type): 16368 lags for E1B, 4092 otherwise."""
+    return LAGS_E1B if sat[3] == E1B else LAGS_L1
+
+
+def code_spectra64(O, sats, sat):
+    """complex128 spectra of row sat and of the next row (zeros after the last row): float64 FFTs of the oracle's code
+    baseband (the decimated +-1 chips; zeros for an SBAS row)."""
+    def fft(s):
+        return np.fft.fft(O.code_baseband(sats[s]).astype(np.complex128)) if s < len(sats) else np.zeros(N, np.complex128)
+    return fft(sat), fft(sat + 1)
+
+
+def split_dop(dop, half_bin):
+    """(d, v) of Doppler index dop: the integer bin d and the half-bin variant v (0 on full bins)."""
     v = (dop & 1) if half_bin else 0
-    d = (dop - v) // 2 if half_bin else dop
-    C = O.code_spectrum(sats[sat])
-    nxt = O.code_spectrum(sats[sat + 1]) if sat + 1 < len(sats) else np.zeros(N, np.complex64)
+    return ((dop - v) // 2 if half_bin else dop), v
+
+
+def code_row(C, nxt, d, reference_wrap):
+    """correlate_one's code row for bin d, code[(k - d) mod N], in C's dtype: for a negative d the bins past the end of
+    the doubled row come from the next table row's spectrum nxt (reference wrap; zeros after the last row) or from the
+    same row (circular wrap)."""
     j = np.arange(N) - d
     code = C[j % N].copy()
     past = j >= N   # only for d < 0
-    if params.wrap_mode == O.WRAP_REFERENCE:
+    if reference_wrap:
         code[past] = nxt[j[past] - N]
-    L = LAGS_E1B if sats[sat][3] == E1B else LAGS_L1
+    return code
+
+
+def block_lags(L, b, dop, K, half_bin, code_doppler):
+    """Where lag n of the search sits in block b's IFFT: (n + 16 b + s(b, dop)) mod N for K > 1 (s = 0 without
+    code_doppler), n for K = 1."""
+    n = np.arange(L)
+    if K == 1:
+        return n
+    return (n + 16 * b + (code_shift(b, dop, half_bin) if code_doppler else 0)) % N
+
+
+def orc_profile(O, params, capture, sats, sat, dop):
+    """float64 [L]: sum over the K blocks of |r_b[block_lags]|^2, r_b = IFFT(conj(D_b) * code_row(d)), from the oracle's
+    fp32 spectra and fp32 FFTs.  dop is the Doppler index (half-bins when half_bin)."""
+    K, half_bin = int(params.k_noncoh), int(params.half_bin)
+    bits = int(params.sample_bits) or 1
+    bb = O.block_bytes(bits)
+    d, v = split_dop(dop, half_bin)
+    C = O.code_spectrum(sats[sat])
+    nxt = O.code_spectrum(sats[sat + 1]) if sat + 1 < len(sats) else np.zeros(N, np.complex64)
+    code = code_row(C, nxt, d, params.wrap_mode == O.WRAP_REFERENCE)
+    L = lags_of(sats[sat])
     cap = np.ascontiguousarray(capture, np.uint8).reshape(-1)
     P = np.zeros(L, np.float64)
-    n = np.arange(L)
     for b in range(K):
         D = O.fft16384(O.capture_baseband(cap[b * bb:(b + 1) * bb], half_rot=v, sample_bits=bits), -1)
         r = O.fft16384(np.conj(D) * code, +1).astype(np.complex128)
-        cs = code_shift(b, dop, half_bin) if params.code_doppler else 0
-        m = (n + (16 * b + cs if K > 1 else 0)) % N
-        P += np.abs(r[m]) ** 2
+        P += np.abs(r[block_lags(L, b, dop, K, half_bin, params.code_doppler)]) ** 2
     return P
 
 
