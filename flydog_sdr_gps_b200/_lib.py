@@ -34,6 +34,8 @@ _SIGNATURES = [
     ("acq_search_aided_device", C.c_int, [_P, _P, C.c_int, _P, C.c_int, _P, C.c_int, _P, _P]),
     ("acq_search_coherent", C.c_int, [_P, _P, C.c_int, _P, C.c_int, C.c_int, _P, _P]),
     ("acq_search_coherent_device", C.c_int, [_P, _P, C.c_int, _P, C.c_int, C.c_int, _P, _P]),
+    ("acq_search_coherent_aided", C.c_int, [_P, _P, C.c_int, _P, C.c_int, C.c_int, _P, C.c_int, _P, _P]),
+    ("acq_search_coherent_aided_device", C.c_int, [_P, _P, C.c_int, _P, C.c_int, C.c_int, _P, C.c_int, _P, _P]),
     ("acq_submit", C.c_int, [_P, _P, C.c_int, _P, C.c_int, _P]),
     ("acq_poll", C.c_int, [_P]),
     ("acq_wait", C.c_int, [_P]),

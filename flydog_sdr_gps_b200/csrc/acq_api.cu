@@ -381,6 +381,11 @@ int row_dops(const acq_engine *e, const void *center, int half_width) { return c
 // step), F = M (1 + half_bin) spectrum variants per block
 int coh_dops(const acq_engine *e, int m_coh) { return m_coh * (e->n_dop - 1) + 1; }
 int coh_variants(const acq_engine *e, int m_coh) { return m_coh * (1 + e->prm.half_bin); }
+// Doppler cells per row of any search: a window (center != NULL) of either grid, else the coherent or the engine's range
+int search_dops(const acq_engine *e, const void *center, int half_width, int m_coh)
+{
+    return (m_coh && !center) ? coh_dops(e, m_coh) : row_dops(e, center, half_width);
+}
 
 // Rotation table of the sub-bin variants, [F][16384]: row v = exp(-2 pi i (v / F) n / N), double precision rounded once.
 // The angle is pi (a n) / (b N) with a / b = 2 v / F in lowest terms, so that the row v = F / 2 of an even F is formed by
@@ -413,9 +418,10 @@ int check_search_args(acq_engine *e, const void *packed, int n_captures, const v
 
 // The arguments of a coherent search, checked before anything touches the device: ACQ_ERR_ARG for the argument errors,
 // ACQ_ERR_UNSUPPORTED for what the coherent search does not cover (E1B rows, code-Doppler engines, searches above the
-// tile and spectrum-row bounds).
+// tile and spectrum-row bounds).  center != NULL: an aided coherent search, whose rows hold W = 2 half_width + 1 cells
+// (W <= n_dop_c) rather than n_dop_c; check_coherent_aided_args has checked what needs no engine.
 int check_coherent(acq_engine *e, const void *packed, int n_captures, const int32_t *sel, int n_sel, int m_coh,
-                   const void *out)
+                   const void *out, const int32_t *center = nullptr, int half_width = 0)
 {
     if (!e) return fail(ACQ_ERR_ARG, "engine is NULL");
     if (m_coh < 1 || m_coh > ACQ_COH_MAX) return fail(ACQ_ERR_ARG, "m_coh=%d outside 1..%d", m_coh, ACQ_COH_MAX);
@@ -423,6 +429,9 @@ int check_coherent(acq_engine *e, const void *packed, int n_captures, const int3
     if (rc) return rc;
     if (e->prm.k_noncoh % m_coh)
         return fail(ACQ_ERR_ARG, "k_noncoh=%d is not a multiple of m_coh=%d", e->prm.k_noncoh, m_coh);
+    if (center && half_width > (coh_dops(e, m_coh) - 1) / 2)
+        return fail(ACQ_ERR_ARG, "Doppler window W = 2*half_width+1 with half_width %d exceeds n_dop_c = %d", half_width,
+                    coh_dops(e, m_coh));
     const int n_sats = (int)e->sats.size();
     if (sel && n_sel <= 0) return fail(ACQ_ERR_ARG, "n_sel must be > 0 when sel is given");
     const int n_slots = sel ? n_sel : n_sats;
@@ -438,7 +447,8 @@ int check_coherent(acq_engine *e, const void *packed, int n_captures, const int3
                         "drift against the block edges", sel ? sel[i] : i);
     if ((long long)n_captures * e->prm.k_noncoh * coh_variants(e, m_coh) > (1 << 24))
         return fail(ACQ_ERR_UNSUPPORTED, "coherent search too large for one call (more than 2^24 capture spectra): split the captures");
-    if ((double)n_captures * (double)n_slots * (double)coh_dops(e, m_coh) > (double)acq::kMaxTilesPerLaunch)
+    const int n_dop = center ? 2 * half_width + 1 : coh_dops(e, m_coh);
+    if ((double)n_captures * (double)n_slots * (double)n_dop > (double)acq::kMaxTilesPerLaunch)
         return fail(ACQ_ERR_UNSUPPORTED, "coherent search too large for one call (more than 2^31 - 1 tiles): split the captures");
     return ACQ_OK;
 }
@@ -446,13 +456,14 @@ int check_coherent(acq_engine *e, const void *packed, int n_captures, const int3
 // Enqueue front end + forward FFT + search (which ends in the best-Doppler pick) on `st` for captures already on the
 // device.  records_dev: where the kernels write the records (device memory, or the device alias of mapped host memory);
 // flag_dev: mapped completion word, or NULL.  center_dev: the rows' Doppler centres on the device (an aided search), or
-// NULL for the whole range.  m_coh > 0: a coherent search (acq_search_coherent) of M = m_coh blocks per group.
+// NULL for the whole range.  m_coh > 0: a coherent search (acq_search_coherent) of M = m_coh blocks per group, with
+// center_dev its aided form (acq_search_coherent_aided: centres and half_width in the coherent grid's units).
 int enqueue_search(acq_engine *e, const uint8_t *packed_dev, int n_captures, acq_record *records_dev, unsigned *flag_dev,
                    cudaStream_t st, const uint8_t *packed_host_arg = nullptr, const int *center_dev = nullptr,
                    int half_width = 0, int m_coh = 0)
 {
     const int K = e->prm.k_noncoh;
-    const int n_dop = m_coh ? coh_dops(e, m_coh) : row_dops(e, center_dev, half_width);
+    const int n_dop = search_dops(e, center_dev, half_width, m_coh);
     const int nvar = m_coh ? coh_variants(e, m_coh) : e->nvar;
     const int blocks = n_captures * K;
     const bool prof = e->profiling;
@@ -587,6 +598,18 @@ int check_aided_args(acq_engine *e, const int32_t *dop_center, int half_width)
     return ACQ_OK;
 }
 
+// Arguments of an aided coherent search that need no engine come first, as in check_aided_args.
+int check_coherent_aided_args(acq_engine *e, const int32_t *dop_center, int half_width, int m_coh)
+{
+    if (!dop_center) return fail(ACQ_ERR_ARG, "dop_center is NULL");
+    if (half_width < 0) return fail(ACQ_ERR_ARG, "half_width must be >= 0 (got %d)", half_width);
+    if (m_coh < 1 || m_coh > ACQ_COH_MAX) return fail(ACQ_ERR_ARG, "m_coh=%d outside 1..%d", m_coh, ACQ_COH_MAX);
+    if (half_width > ACQ_COH_MAX * kMaxHalfWidth)
+        return fail(ACQ_ERR_ARG, "Doppler window W = 2*half_width+1 with half_width %d exceeds n_dop_c of any engine", half_width);
+    if (!e) return fail(ACQ_ERR_ARG, "engine is NULL");
+    return ACQ_OK;
+}
+
 // Wait for a host-polled search and collect its records: k_pick_small writes every record into mapped memory as two
 // 16-byte halves that each end in the search's epoch (acq_record_tagged), so a half whose tag matches has arrived whole.
 // The stream is queried now and then so that a failed launch cannot hang the caller; the mapped word *h_flag is only
@@ -668,7 +691,8 @@ int enqueue_profile(acq_engine *e, const acq_record *rec_dev, int n_records, int
 }
 
 // center (HOST, one per row) and half_width: an aided search (acq_search_aided), or NULL for the whole range
-// m_coh > 0: a coherent search (acq_search_coherent), its arguments already checked by check_coherent
+// m_coh > 0: a coherent search (acq_search_coherent, or with center acq_search_coherent_aided), its arguments already
+// checked by check_coherent
 int search_host(acq_engine *e, const uint8_t *packed, int n_captures, const int32_t *sel, int n_sel, acq_record *out,
                 acq_cell *grid, bool sync, const int32_t *center = nullptr, int half_width = 0, int m_coh = 0)
 {
@@ -677,7 +701,7 @@ int search_host(acq_engine *e, const uint8_t *packed, int n_captures, const int3
     DeviceGuard g(e->device);
     e->last_captures = 0;  // until this search is enqueued, there are no spectra acq_refine could use
     e->ref_captures = 0;
-    const int n_dop = m_coh ? coh_dops(e, m_coh) : row_dops(e, center, half_width);
+    const int n_dop = search_dops(e, center, half_width, m_coh);
     if ((rc = set_selection(e, sel, n_sel))) return rc;
     if ((rc = check_tile_count(e, n_captures, n_dop))) return rc;
     if ((rc = ensure_scratch(e, n_captures, e->n_slots, true, n_dop, m_coh ? coh_variants(e, m_coh) : e->nvar))) return rc;
@@ -752,7 +776,7 @@ void finish_pending(acq_engine *e)
     e->pending_out = nullptr;
 }
 
-// acq_search_device and acq_search_aided_device (center_dev != NULL)
+// acq_search_device and acq_search_aided_device (center_dev != NULL); with m_coh > 0 their coherent forms
 int search_device(acq_engine *e, const uint8_t *packed_dev, int n_captures, const int32_t *sel, int n_sel,
                   acq_record *out_dev, void *stream, const int *center_dev = nullptr, int half_width = 0, int m_coh = 0)
 {
@@ -763,7 +787,7 @@ int search_device(acq_engine *e, const uint8_t *packed_dev, int n_captures, cons
     DeviceGuard g(e->device);
     e->last_captures = 0;  // spectra now belong to a search on the caller's stream: acq_refine does not apply
     e->ref_captures = 0;   // ... and acq_refine_device applies once this search is enqueued
-    const int n_dop = m_coh ? coh_dops(e, m_coh) : row_dops(e, center_dev, half_width);
+    const int n_dop = search_dops(e, center_dev, half_width, m_coh);
     if ((rc = set_selection(e, sel, n_sel))) return rc;
     if ((rc = check_tile_count(e, n_captures, n_dop))) return rc;
     if ((rc = ensure_scratch(e, n_captures, e->n_slots, false, n_dop, m_coh ? coh_variants(e, m_coh) : e->nvar))) return rc;
@@ -1072,6 +1096,24 @@ int acq_search_coherent_device(acq_engine *e, const uint8_t *packed_dev, int n_c
     const int rc = check_coherent(e, packed_dev, n_captures, sel, n_sel, m_coh, out_dev);
     if (rc) return rc;
     return search_device(e, packed_dev, n_captures, sel, n_sel, out_dev, stream, nullptr, 0, m_coh);
+}
+
+int acq_search_coherent_aided(acq_engine *e, const uint8_t *packed, int n_captures, const int32_t *sel, int n_sel,
+                              int m_coh, const int32_t *dop_center, int half_width, acq_record *out, acq_cell *grid)
+{
+    int rc = check_coherent_aided_args(e, dop_center, half_width, m_coh);
+    if (rc || (rc = check_coherent(e, packed, n_captures, sel, n_sel, m_coh, out, dop_center, half_width))) return rc;
+    return search_host(e, packed, n_captures, sel, n_sel, out, grid, true, dop_center, half_width, m_coh);
+}
+
+int acq_search_coherent_aided_device(acq_engine *e, const uint8_t *packed_dev, int n_captures, const int32_t *sel,
+                                     int n_sel, int m_coh, const int32_t *dop_center_dev, int half_width,
+                                     acq_record *out_dev, void *stream)
+{
+    int rc = check_coherent_aided_args(e, dop_center_dev, half_width, m_coh);
+    if (rc || (rc = check_coherent(e, packed_dev, n_captures, sel, n_sel, m_coh, out_dev, dop_center_dev, half_width)))
+        return rc;
+    return search_device(e, packed_dev, n_captures, sel, n_sel, out_dev, stream, dop_center_dev, half_width, m_coh);
 }
 
 int acq_submit(acq_engine *e, const uint8_t *packed, int n_captures, const int32_t *sel, int n_sel, acq_record *out)

@@ -565,7 +565,9 @@ struct TileIdx {
     {
         int h;
         if constexpr (PA::kCoh) {   // 1/F-bin steps: integer bin (floored) and sub-bin variant
-            h = p.dop_lo + d;
+            // an aided coherent search (AidedCohSearchArgs): the window and dop_lo..dop_hi in the same 1/F-bin units
+            if constexpr (PA::kAided) h = window_lo(__ldg(p.dop_center + cap * p.n_slots + slot), p.half_width, p.dop_lo, p.dop_hi) + d;
+            else h = p.dop_lo + d;
             const int F = p.nvar;
             dop = (h >= 0 ? h : h - F + 1) / F;
             v = h - F * dop;
@@ -633,8 +635,10 @@ __device__ __forceinline__ size_t d_row(const PA &p, const TileIdx &ti, int b)
     const size_t bv = (size_t)((size_t)ti.cap * p.K + b) * p.nvar + ti.v;
     if (p.n_shift == 1) return bv;
     // the tile's Doppler index h; in an aided search rebuilt from (dop, v), which set_dop formed from the window base
+    // (an aided coherent search: F = nvar steps per bin; unreached, acq_api.cu refuses coherent code_doppler searches)
     int h;
-    if constexpr (PA::kAided) h = ti.dop * (1 + p.half_bin) + ti.v;
+    if constexpr (PA::kAided && PA::kCoh) h = ti.dop * p.nvar + ti.v;
+    else if constexpr (PA::kAided) h = ti.dop * (1 + p.half_bin) + ti.v;
     else h = p.dop_lo + ti.d;
     return bv * p.n_shift + (size_t)(p.smax + code_shift(b, h, p.cd_div));
 }
@@ -2578,8 +2582,10 @@ cudaError_t search_kernels_configure()
         if ((e = cudaFuncSetAttribute(f, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared))) return e;
     if ((e = aided_kernels_configure())) return e;
     using CA = CohSearchArgs;
+    using AC = AidedCohSearchArgs;
     if ((e = cudaFuncSetAttribute(k_search_l1_coh<CA>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)l1_multi_smem_bytes()))) return e;
-    const void *coh[] = {(const void *)k_search_l1_coh<CA>, (const void *)k_coh_variants};
+    if ((e = cudaFuncSetAttribute(k_search_l1_coh<AC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)l1_multi_smem_bytes()))) return e;
+    const void *coh[] = {(const void *)k_search_l1_coh<CA>, (const void *)k_search_l1_coh<AC>, (const void *)k_coh_variants};
     for (const void *f : coh)
         if ((e = cudaFuncSetAttribute(f, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared))) return e;
     return cudaSuccess;
@@ -2808,7 +2814,8 @@ int launch_search_coh(const CohSearchArgs &a_in, int sm_count, cudaStream_t st, 
     if (grid <= 0) return 0;
     CohSearchArgs a = a_in;
     if (!search_claims_tiles(a.n_tiles, grid)) a.tile_ctr = nullptr;
-    launch_k(k_search_l1_coh<CohSearchArgs>, grid, 256, l1_multi_smem_bytes(), st, pdl, a);
+    if (a.dop_center) launch_k(k_search_l1_coh<AidedCohSearchArgs>, grid, 256, l1_multi_smem_bytes(), st, pdl, AidedCohSearchArgs(a));
+    else launch_k(k_search_l1_coh<CohSearchArgs>, grid, 256, l1_multi_smem_bytes(), st, pdl, a);
     return 1;
 }
 

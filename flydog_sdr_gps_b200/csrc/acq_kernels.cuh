@@ -64,6 +64,14 @@ struct CohSearchArgs : SearchArgs {
     CohSearchArgs() = default;
     explicit CohSearchArgs(const SearchArgs &a, int m) : SearchArgs(a), m_coh(m) {}
 };
+// An aided coherent search (acq_search_coherent_aided): k_search_l1_coh over each row's window, with dop_center,
+// half_width and dop_lo..dop_hi all in the coherent grid's 1/F-bin units.  A type of its own, so that the full-range
+// coherent kernel compiles to the code it had without the feature.
+struct AidedCohSearchArgs : CohSearchArgs {
+    static constexpr bool kAided = true;
+    AidedCohSearchArgs() = default;
+    explicit AidedCohSearchArgs(const CohSearchArgs &a) : CohSearchArgs(a) {}
+};
 
 // s(b, h) of acq_params.code_doppler (same integer arithmetic as the oracle's orc_code_shift)
 __host__ __device__ inline int code_shift(int b, int h, int cd_div)

@@ -118,13 +118,18 @@ class CaptureFarm(_Farm):
     each.  Records come back as [n_captures, n_sel] on every rank.
 
     half_width (optional): an aided farm -- every (capture, satellite) row searches only the 2 * half_width + 1 Doppler
-    indices around its own centre (acq_search_aided_device); load() then takes the centres with the captures."""
+    indices around its own centre (acq_search_aided_device); load() then takes the centres with the captures.
 
-    def __init__(self, engine, n_captures, capture_bytes, n_sel, dist=None, device=None, half_width=None):
+    m_coh (optional): a coherent farm -- groups of m_coh blocks added coherently (acq_search_coherent_device); with
+    half_width as well, each row searches its own window of the coherent grid (acq_search_coherent_aided_device), centres
+    and half_width in that grid's 1/F-bin units.  Records keep the shape [n_captures, n_sel]."""
+
+    def __init__(self, engine, n_captures, capture_bytes, n_sel, dist=None, device=None, half_width=None, m_coh=None):
         super().__init__(engine, n_captures, dist, device)
         self.capture_bytes, self.n_sel = capture_bytes, n_sel
         self.per_unit, self.records_shape = n_sel, (n_captures, n_sel)
         self.half_width = half_width
+        self.m_coh = m_coh
         self.h_in = self._empty(self.n_local * capture_bytes, device="cpu", pin=self.pin)
         self.d_in = self._empty(self.n_local * capture_bytes)
         if half_width is not None:   # this rank's Doppler centres, int32 [n_local, n_sel], kept in HBM with the captures
@@ -156,7 +161,13 @@ class CaptureFarm(_Farm):
 
     def search_resident(self):
         """Captures (and, aided, centres) already in HBM (load()); leaves the gathered records in self.d_all.  Asynchronous."""
-        if self.n_local and self.half_width is not None:
+        if self.n_local and self.m_coh is not None and self.half_width is not None:
+            self.eng.search_coherent_aided_device(self.d_in.data_ptr(), self.m_coh, self.d_center.data_ptr(), self.half_width,
+                                                  self.d_rec.data_ptr(), self.n_local, stream_ptr=self._stream_ptr())
+        elif self.n_local and self.m_coh is not None:
+            self.eng.search_coherent_device(self.d_in.data_ptr(), self.m_coh, self.d_rec.data_ptr(), self.n_local,
+                                            stream_ptr=self._stream_ptr())
+        elif self.n_local and self.half_width is not None:
             self.eng.search_aided_device(self.d_in.data_ptr(), self.d_center.data_ptr(), self.half_width, self.d_rec.data_ptr(),
                                          self.n_local, stream_ptr=self._stream_ptr())
         elif self.n_local:

@@ -230,6 +230,25 @@ int acq_search_coherent(acq_engine *e, const uint8_t *packed, int n_captures, co
 int acq_search_coherent_device(acq_engine *e, const uint8_t *packed_dev, int n_captures, const int32_t *sel, int n_sel,
                                int m_coh, acq_record *out_dev, void *stream);
 
+/* Aided coherent search (extension): acq_search_coherent with acq_search_aided's window.  Row r = c*n_sel + s searches
+ * only the W = 2*half_width+1 indices of the coherent grid from lo_r = clamp(dop_center[r] - half_width, M*dop_lo,
+ * M*dop_hi - 2*half_width).  Centres, half_width and the records' dop are in the coherent grid's units (steps of
+ * ACQ_BIN_HZ / F, F = M * (1 + half_bin)), so a coherent record's dop can be passed back as a centre.  W must not exceed
+ * n_dop_c = M*(n_dop - 1) + 1.  The record is Correlate()'s rule over the window, as in acq_search_aided.
+ *   dop_center : HOST, n_captures * n_sel int32 (n_sel = table size when sel is NULL)
+ *   grid       : HOST or NULL; n_captures * n_sel * W cells, cell j of row r = coherent index lo_r + j
+ * Everything else is acq_search_coherent's: the groups and data-bit hypotheses, ACQ_ERR_UNSUPPORTED for E1B rows and
+ * code_doppler engines before any device work, zero records for SBAS rows, and ACQ_ERR_ARG from acq_refine* and
+ * acq_profile* until the next acq_search.  ACQ_ERR_ARG also for a NULL dop_center, half_width < 0 and m_coh outside
+ * 1..ACQ_COH_MAX, reported even with a NULL engine, and for W > n_dop_c.  Synchronous. */
+int acq_search_coherent_aided(acq_engine *e, const uint8_t *packed, int n_captures, const int32_t *sel, int n_sel,
+                              int m_coh, const int32_t *dop_center, int half_width, acq_record *out, acq_cell *grid);
+/* The device-resident form: ordering and validity rules of acq_search_device; dop_center_dev is a DEVICE array read by
+ * the kernels, so it must stay valid until `stream` has passed the search. */
+int acq_search_coherent_aided_device(acq_engine *e, const uint8_t *packed_dev, int n_captures, const int32_t *sel,
+                                     int n_sel, int m_coh, const int32_t *dop_center_dev, int half_width,
+                                     acq_record *out_dev, void *stream);
+
 /* Asynchronous pair over host buffers (the reference yields to other tasks while it computes,
  * gps/search.cpp:479-491): submit enqueues copy-in, search and copy-out on the engine's stream;
  * acq_wait blocks until done, acq_poll returns 1 when done, 0 while running.  The host buffers
