@@ -47,7 +47,7 @@ class CoherentRef:
 
     def for_sat(self, sat):
         """The reference of another satellite on the same capture, sharing its block basebands and spectra."""
-        other = object.__new__(CoherentRef)
+        other = object.__new__(type(self))
         other.__dict__.update(self.__dict__)
         other.sat = sat
         other.C, other.nxt = code_spectra64(self.O, self.sats, sat)
@@ -96,8 +96,3 @@ class CoherentRef:
         lag = P.argmax(axis=1)
         noise = P.mean(axis=1)
         return hs, peak, noise, peak / noise, lag, P
-
-
-def best_cell(snr):
-    """Correlate's pick: the largest snr, the lowest index on ties."""
-    return int(np.argmax(snr))

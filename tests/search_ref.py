@@ -94,6 +94,7 @@ class Worst:
     def __init__(self, label=""):
         self.label = label
         self.peak = self.noise = self.snr = self.profile = 0.0
+        self.dop = self.code = self.fine_peak = 0.0   # refinement (refine_ref.check_fine): bins, FS samples, relative
         self.lag_ties = self.dop_ties = 0
 
     def rel(self, field, got, want):
@@ -103,20 +104,23 @@ class Worst:
 
     def __str__(self):
         return ("precision [%s]: max rel. error peak %.1e noise %.1e snr %.1e, profile %.1e of sqrt(P m + m^2); "
-                "%d lag and %d Doppler ties" % (self.label, self.peak, self.noise, self.snr, self.profile,
-                                                 self.lag_ties, self.dop_ties))
+                "refinement: dop %.1e bin, code_fs %.1e FS samples, peak %.1e; %d lag and %d Doppler ties"
+                % (self.label, self.peak, self.noise, self.snr, self.profile, self.dop, self.code, self.fine_peak,
+                   self.lag_ties, self.dop_ties))
 
 
-def check_cells(got, ref, worst, what=""):
-    """got: CELL_DTYPE cells of one row at ref's Doppler indices; ref: SearchRef.cells.  Peak, noise and snr within
-    their tolerances; a lag other than the reference's first argmax only where the reference's P there is within
-    PEAK_RTOL of the peak.  Cells whose reference P is all zero (an SBAS row) are skipped."""
+def check_cells(got, ref, worst, what="", margin=1.0):
+    """got: CELL_DTYPE cells of one row at ref's Doppler indices; ref: SearchRef.cells (or CoherentRef.cells).  Peak,
+    noise and snr within their tolerances (divided by margin); a lag other than the reference's first argmax only where
+    the reference's P there is within PEAK_RTOL of the peak.  Cells whose reference P is all zero (an SBAS row) are
+    skipped."""
     hs, peak, noise, snr, lag, P = ref
     got = np.asarray(got).reshape(-1)
     assert got.size == hs.size, (what, got.size, hs.size)
     on = noise > 0
     g = got[on]
     for f, want, tol in (("peak", peak[on], PEAK_RTOL), ("noise", noise[on], NOISE_RTOL), ("snr", snr[on], SNR_RTOL)):
+        tol = tol / margin
         e = worst.rel(f, g[f], want)
         assert e <= tol, "%s: %s rel. error %.2e > %.0e at h = %s" % (
             what, f, e, tol, hs[on][np.argmax(np.abs(g[f] / want - 1))])

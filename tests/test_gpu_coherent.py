@@ -8,7 +8,8 @@ import flydog_sdr_gps_b200 as F
 from flydog_sdr_gps_b200 import synth
 from flydog_sdr_gps_b200 import sats as S
 
-from coherent_ref import CoherentRef, best_cell, grid_h
+from coherent_ref import CoherentRef, grid_h
+from search_ref import Worst, check_cells, check_record
 
 pytestmark = pytest.mark.gpu
 BIN = F.BIN_HZ
@@ -46,18 +47,12 @@ def test_m1_is_acq_search_grid(gpu_required, name):
     assert g1.tobytes() == g0.tobytes()
 
 
-# fp32 against fp64: the search forms P from 16384-point float32 FFTs (about 14 roundings deep per value), a float32
-# rotation and M complex additions; relative errors of a power are a few 1e-6 against the largest power of the row.
-# 1e-4 on peak, noise and snr keeps a tenfold margin over that and is far below anything a wrong phase or hypothesis
-# would do (the in-phase test below: 10 % at M = 5 for the wrong sign of the smallest term).
-RTOL = 1e-4
-
-
 @pytest.mark.parametrize("m_coh,groups,half_bin", [(m, g, hb) for m in (2, 3, 4, 5) for g in (1, 2) for hb in (0, 1)])
 def test_against_reference(gpu_required, oracle, m_coh, groups, half_bin):
-    """Cells of two satellites (one with a signal, one without) against the float64 reference: peak, noise, snr within
-    RTOL; lag where the reference's power at the search's lag is not within RTOL of its peak; the record's dop where the
-    reference's runner-up cell is not within RTOL of its best snr."""
+    """Cells and records of two satellites (one with a signal, one without) against the float64 reference at
+    search_ref's tolerances (check_cells, check_record): peak, noise and snr; the lag wherever the reference's power at
+    the search's lag is not within PEAK_RTOL of its peak; the record's dop wherever the reference's runner-up is not
+    within SNR_RTOL of its best snr."""
     K = m_coh * groups
     nav = S.navstar()
     kw = dict(k_noncoh=K, half_bin=half_bin, dop_lo=-4 * (1 + half_bin), dop_hi=3 * (1 + half_bin))
@@ -68,19 +63,14 @@ def test_against_reference(gpu_required, oracle, m_coh, groups, half_bin):
     with F.AcqEngine(nav, F.default_params(**kw)) as eng:
         rec, grid = eng.search_coherent(cap, m_coh, sel=sel, want_grid=True)
         p = eng.params
+    worst = Worst("coherent M = %d, %d groups, half_bin %d" % (m_coh, groups, half_bin))
     for s, sat in enumerate(sel):
-        hs, peak, noise, snr, lag, P = CoherentRef(oracle, p, cap, nav, int(sat)).cells(m_coh)
-        g = grid[0, s]
-        assert np.array_equal(hs, grid_h(p, m_coh)) and g.size == hs.size
-        np.testing.assert_allclose(g["peak"], peak, rtol=RTOL)
-        np.testing.assert_allclose(g["noise"], noise, rtol=RTOL)
-        np.testing.assert_allclose(g["snr"], snr, rtol=RTOL)
-        at_lag = P[np.arange(hs.size), g["lag"]]
-        assert np.all((g["lag"] == lag) | (at_lag >= peak * (1 - RTOL)))
-        b = best_cell(snr)
-        runner = np.sort(snr)[-2]
-        if runner < snr[b] * (1 - RTOL):
-            assert rec[0, s]["dop"] == hs[b] and rec[0, s]["lag"] == lag[b]
+        ref = CoherentRef(oracle, p, cap, nav, int(sat)).cells(m_coh)
+        assert np.array_equal(ref[0], grid_h(p, m_coh))
+        what = "sat %d" % sat
+        check_cells(grid[0, s], ref, worst, what)
+        check_record(rec[0, s], ref, worst, what)
+    print(worst)
     assert rec[0, 0]["dop"] == h_sig   # the signal row finds its cell
 
 

@@ -10,6 +10,7 @@ from flydog_sdr_gps_b200 import _lib, synth
 from flydog_sdr_gps_b200 import sats as S
 
 from coherent_ref import CoherentRef
+from search_ref import Worst
 from test_gpu_coherent_sweep import check_cells, check_record
 
 pytestmark = pytest.mark.gpu
@@ -166,7 +167,7 @@ def test_m1_is_acq_search_aided(gpu_required, kw):
 @pytest.mark.parametrize("m_coh,groups,half_bin", [(2, 2, 0), (3, 1, 1), (4, 2, 1), (5, 1, 0)])
 def test_windows_against_reference(gpu_required, oracle, m_coh, groups, half_bin):
     """Windowed rows (a signal row and a noise row, one window at the range's edge) against the float64 reference with
-    test_gpu_coherent.py::test_against_reference's RTOL 1e-4 rules; each record against the reference's window pick."""
+    search_ref's tolerances (test_gpu_coherent_sweep.check_cells); each record against the reference's window pick."""
     K = m_coh * groups
     nav = S.navstar()
     kw = dict(k_noncoh=K, half_bin=half_bin, dop_lo=-4 * (1 + half_bin), dop_hi=3 * (1 + half_bin))
@@ -181,11 +182,13 @@ def test_windows_against_reference(gpu_required, oracle, m_coh, groups, half_bin
         p = eng.params
     clo, chi = coh_range(p, m_coh)
     base = CoherentRef(oracle, p, cap, nav, 9)
+    worst = Worst("aided coherent M = %d, %d groups, half_bin %d" % (m_coh, groups, half_bin))
     for s, sat in enumerate(sel):
         lo = window_lo(centers[0, s], hw, clo, chi)
         hs_w = np.arange(lo, lo + 2 * hw + 1)
-        hs, snr = check_cells(grid[0, s], base.for_sat(int(sat)), m_coh, hs=hs_w)
+        hs, snr = check_cells(grid[0, s], base.for_sat(int(sat)), m_coh, hs=hs_w, worst=worst, what="sat %d" % sat)
         check_record(rec[0, s], grid[0, s], hs, snr)
+    print(worst)
     assert rec[0, 0]["dop"] == h_sig   # the signal row finds its cell inside its window
 
 

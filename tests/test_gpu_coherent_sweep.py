@@ -9,8 +9,9 @@ import flydog_sdr_gps_b200 as F
 from flydog_sdr_gps_b200 import synth
 from flydog_sdr_gps_b200 import sats as S
 
+import search_ref
 from coherent_ref import CoherentRef, grid_h
-from test_gpu_coherent import RTOL
+from search_ref import SNR_RTOL, Worst
 from test_gpu_limits import SPLIT_CAPTURES, SPLIT_DISTINCT, SPLIT_K, SPLIT_PAST, SPLIT_STRADDLE, split_batch
 
 pytestmark = pytest.mark.gpu
@@ -23,31 +24,31 @@ def _table():
     return S.navstar() + [(120, 145, 0o1106, S.SBAS)] + S.qzss()
 
 
-def check_cells(g, ref, m_coh, hs=None):
-    """GPU cells g (at the Doppler indices hs, default the whole row) against the reference with test_against_reference's
-    rules: peak, noise and snr within RTOL (0/0 = NaN cells of a zero code row on both sides); the lag wherever the
-    reference's power at the GPU's lag is not within RTOL of its peak.  Returns the reference's (hs, snr)."""
+def check_cells(g, ref, m_coh, hs=None, worst=None, what=""):
+    """GPU cells g (at the Doppler indices hs, default the whole row) against the reference at search_ref's tolerances
+    (search_ref.check_cells: peak, noise, snr, and the lag wherever the reference's power at the GPU's lag is not
+    within PEAK_RTOL of its peak); the cells of a zero code row are 0 / 0 = NaN on both sides.  Returns the
+    reference's (hs, snr)."""
     with np.errstate(invalid="ignore", divide="ignore"):
-        hs, peak, noise, snr, lag, P = ref.cells(m_coh, hs=hs)
+        cells = ref.cells(m_coh, hs=hs)
+    hs, peak, noise, snr = cells[:4]
     assert g.size == hs.size
-    np.testing.assert_allclose(g["peak"], peak, rtol=RTOL)
-    np.testing.assert_allclose(g["noise"], noise, rtol=RTOL)
-    np.testing.assert_allclose(g["snr"], snr, rtol=RTOL)
-    at_lag = P[np.arange(hs.size), g["lag"]]
-    assert np.all((g["lag"] == lag) | (at_lag >= peak * (1 - RTOL)))
+    search_ref.check_cells(g, cells, Worst() if worst is None else worst, what)
+    zero = ~(noise > 0)
+    assert (g["peak"][zero] == 0).all() and (g["noise"][zero] == 0).all() and np.isnan(g["snr"][zero]).all(), what
     return hs, snr
 
 
 def check_record(r, g, hs, snr):
     """The record of a whole row: the cell of the best snr (lowest index on ties) wherever the reference's runner-up is
-    not within RTOL of its best; a row whose snr never exceeds 0 keeps {dop 0, lag 0}."""
+    not within SNR_RTOL of its best; a row whose snr never exceeds 0 keeps {dop 0, lag 0}."""
     s = np.where(np.isfinite(snr), snr, -np.inf)
     if not s.max() > 0:
         assert (r["dop"], r["lag"]) == (0, 0)
         return
     b = int(np.argmax(s))
     runner = np.sort(s)[-2] if s.size > 1 else -np.inf
-    if runner < s[b] * (1 - RTOL):
+    if runner < s[b] * (1 - SNR_RTOL):
         assert r["dop"] == hs[b] and r["lag"] == g["lag"][b] and r["peak"] == g["peak"][b], (r, hs[b])
 
 
@@ -110,6 +111,7 @@ def test_coherent_sweep(gpu_required, oracle, seed):
         rec, grid = eng.search_coherent(np.concatenate(caps), M, sel=sel, want_grid=True)
         p = eng.params
     assert rec.shape == (len(caps), len(sel)) and grid.shape[2] == M * (kw["dop_hi"] - kw["dop_lo"]) + 1
+    worst = Worst("coherent sweep seed %d" % seed)
     for c, cap in enumerate(caps):
         base = CoherentRef(oracle, p, cap, table, int(sel[0]))
         seen = {}
@@ -120,9 +122,10 @@ def test_coherent_sweep(gpu_required, oracle, seed):
                 assert grid[c, i].tobytes() == grid[c, j].tobytes() and rec[c, i].tobytes() == rec[c, j].tobytes()
                 continue
             seen[sat] = i
-            hs, snr = check_cells(grid[c, i], base.for_sat(sat), M)
+            hs, snr = check_cells(grid[c, i], base.for_sat(sat), M, worst=worst, what="capture %d sat %d" % (c, sat))
             assert np.array_equal(hs, grid_h(p, M))
             check_record(rec[c, i], grid[c, i], hs, snr)
+    print(worst)
 
 
 # ---------------------------------------------------------------- many tiles per persistent CTA
@@ -148,9 +151,11 @@ def test_many_tiles_per_cta(gpu_required, oracle):
     for i, j in ((0, 3), (2, 4), (1, 5)):
         assert rec[i].tobytes() == rec[j].tobytes() and grid[i].tobytes() == grid[j].tobytes(), (i, j)
     assert alone_r[0].tobytes() == rec[0].tobytes() and alone_g[0].tobytes() == grid[0].tobytes()
+    worst = Worst("coherent, many tiles per CTA")
     for ci, cap, s in ((0, a, 1), (2, c, 7), (1, b, 0)):   # rows 4, 22 and 1: each the strongest signal of its capture
-        hs, snr = check_cells(grid[ci, s], CoherentRef(oracle, p, cap, nav, int(sel[s])), M)
+        hs, snr = check_cells(grid[ci, s], CoherentRef(oracle, p, cap, nav, int(sel[s])), M, worst=worst)
         check_record(rec[ci, s], grid[ci, s], hs, snr)
+    print(worst)
     assert rec[0, 1]["dop"] == 26 and rec[2, 7]["dop"] == -79 and rec[1, 0]["dop"] == 77, rec[:3, [1, 7, 0]]
 
 
@@ -175,10 +180,12 @@ def test_data_bit_edges(gpu_required, oracle, m_coh):
     with F.AcqEngine(nav, F.default_params(k_noncoh=K, dop_lo=-3, dop_hi=3)) as eng:
         rec, grid = eng.search_coherent(np.concatenate(caps), M, sel=[3], want_grid=True)
         p = eng.params
+    worst = Worst("coherent data-bit edges, M = %d" % M)
     for i, cap in enumerate(caps):
-        hs, snr = check_cells(grid[i, 0], CoherentRef(oracle, p, cap, nav, 3), M)
+        hs, snr = check_cells(grid[i, 0], CoherentRef(oracle, p, cap, nav, 3), M, worst=worst, what="capture %d" % i)
         check_record(rec[i, 0], grid[i, 0], hs, snr)
         assert (rec[i, 0]["dop"], rec[i, 0]["lag"]) == (h, 1250), (i, rec[i, 0])
+    print(worst)
     for i in range(1, M):   # edges on block boundaries
         assert 0.85 <= rec[i, 0]["peak"] / rec[0, 0]["peak"] <= 1.15, (i, rec[i, 0], rec[0, 0])
 
@@ -199,12 +206,14 @@ def test_maximum_span(gpu_required, oracle):
     n = M * 4096 + 1
     assert grid.shape == (1, 2, n)
     h0 = M * kw["dop_lo"]
+    worst = Worst("coherent span +-2048, M = 5")
     for s, h_sig in ((0, top), (1, bottom)):
         g = grid[0, s]
         j = np.unique(np.concatenate([np.arange(5), np.arange(n - 5, n), np.arange(h_sig - h0 - 3, h_sig - h0 + 4)]))
-        check_cells(g[j], CoherentRef(oracle, p, caps, nav, int(sel[s])), M, hs=h0 + j)
+        check_cells(g[j], CoherentRef(oracle, p, caps, nav, int(sel[s])), M, hs=h0 + j, worst=worst)
         b = int(np.argmax(g["snr"]))
         assert rec[0, s]["dop"] == h0 + b == h_sig and rec[0, s]["lag"] == g["lag"][b] == 1250, (s, rec[0, s], b)
+    print(worst)
 
 
 # ---------------------------------------------------------------- the launch split of k_coh_variants
@@ -229,8 +238,10 @@ def test_launch_split_of_the_variants(gpu_required, oracle):
     rb = rec.view(np.uint8).reshape(SPLIT_CAPTURES, -1)
     gb = grid.view(np.uint8).reshape(SPLIT_CAPTURES, -1)
     assert np.array_equal(rb, rb[idx]) and np.array_equal(gb, gb[idx])
+    worst = Worst("coherent launch split")
     for c in (SPLIT_STRADDLE, SPLIT_PAST):
         base = CoherentRef(oracle, p, caps[c], nav, int(sel[0]))
         for s, sat in enumerate(sel):
-            hs, snr = check_cells(grid[c, s], base.for_sat(int(sat)), 3)
+            hs, snr = check_cells(grid[c, s], base.for_sat(int(sat)), 3, worst=worst)
             check_record(rec[c, s], grid[c, s], hs, snr)
+    print(worst)

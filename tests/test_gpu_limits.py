@@ -1,7 +1,8 @@
 """GPU suite (-m gpu) at the limits acq_create accepts: the Doppler span of 2048 bins either side (the margin Q of the
 extended code rows), K = 255 non-coherent blocks, code-Doppler compensation at its 33 shifted copies per spectrum, and a
 batch of more than 32 768 block rows (the front end's launch split).  Each case against the CPU oracle on the same
-bytes: records, the whole per-Doppler table, acq_refine against oracle.refine and acq_profile against orc_profile."""
+bytes: records, the whole per-Doppler table, acq_refine against oracle.refine and the float64 RefineRef
+(tests/refine_ref.py), and acq_profile against orc_profile."""
 import numpy as np
 import pytest
 
@@ -11,6 +12,8 @@ from flydog_sdr_gps_b200 import sats as S
 
 from parity import RTOL, Margins, compare_records
 from profile_ref import circular_distance, code_shift, orc_profile, peak2_of
+from refine_ref import RefineRef, check_fine
+from search_ref import Worst
 from test_gpu_parity import _compare_fine
 
 pytestmark = pytest.mark.gpu
@@ -38,12 +41,16 @@ def _search_vs_oracle(eng, oracle, table, kw, cap, sel, label):
 
 def _refine_vs_oracle(eng, oracle, table, kw, cap, rec, rows=None):
     """acq_refine of the last search's records against oracle.refine of the same records (test_gpu_parity's
-    tolerances), over `rows` (default: all)."""
+    tolerances) and against the float64 RefineRef (refine_ref's bound), over `rows` (default: all)."""
     fine = eng.refine(rec)
-    ofine = oracle.refine(cap, table, rec[0], params=oracle.default_params(**kw))
+    oprm = oracle.default_params(**kw)
+    ofine = oracle.refine(cap, table, rec[0], params=oprm)
     rows = np.arange(rec.shape[1]) if rows is None else np.asarray(rows)
     if rows.size:
         _compare_fine(fine[0][rows], ofine[rows], rec[0][rows])
+        worst = Worst("refine at the limits")
+        check_fine(fine[0][rows], rec[0][rows], RefineRef(oracle, oprm, cap, table), worst)
+        print(worst)
     return fine
 
 

@@ -1,7 +1,8 @@
-"""GPU suite (-m gpu) of the precision tier: every non-coherent search kernel's cells, records, lag profiles and
-second-peak rows against the float64 reference (tests/search_ref.py) at the precision fp32 reaches, some 100 times
-tighter than parity.RTOL.  Each case asserts, through acq_plan_launch, that it runs the kernel it is named after; where
-the kernel follows from the total tile count, the whole search runs and a subset of rows is compared."""
+"""GPU suite (-m gpu) of the precision tier: every non-coherent search kernel's cells, records, lag profiles,
+second-peak rows and refinements (k_refine) against the float64 references (tests/search_ref.py, tests/refine_ref.py)
+at the precision fp32 reaches, some 100 times tighter than parity.RTOL.  Each case asserts, through acq_plan_launch,
+that it runs the kernel it is named after; where the kernel follows from the total tile count, the whole search runs and
+a subset of rows is compared.  test_refine_edges refines records placed where no search puts them."""
 import ctypes as C
 
 import numpy as np
@@ -11,9 +12,9 @@ import flydog_sdr_gps_b200 as F
 from flydog_sdr_gps_b200 import _lib, scenarios, synth
 from flydog_sdr_gps_b200 import sats as S
 
-from profile_ref import circular_distance, peak2_of
-from search_ref import (NOISE_RTOL, PEAK_RTOL, PROFILE_TAU, SearchRef, Worst, check_cells, check_profile,
-                        check_record)
+from profile_ref import LAGS_E1B, LAGS_L1, circular_distance, peak2_of
+from refine_ref import RefineRef, check_fine
+from search_ref import NOISE_RTOL, PEAK_RTOL, PROFILE_TAU, Worst, check_cells, check_profile, check_record
 
 pytestmark = pytest.mark.gpu
 
@@ -117,8 +118,9 @@ def test_search_and_profile_at_fp32_precision(gpu_required, oracle, name):
             assert eng.launch_count - n0 == 4
         pk, prof = eng.profile(rec, excl=EXCL, want_profile=True)
         off = eng.profile_offsets(len(caps), sel)
+        fine = eng.refine(rec)
     oprm = oracle.default_params(**kw)
-    refs = [SearchRef(oracle, oprm, cap, table) for cap in caps]
+    refs = [RefineRef(oracle, oprm, cap, table) for cap in caps]
     n_sel = rec.shape[1]
     worst = Worst(name)
     for c, s in compared:
@@ -132,4 +134,61 @@ def test_search_and_profile_at_fp32_precision(gpu_required, oracle, name):
         i = c * n_sel + s
         check_profile(prof[off[i]:off[i + 1]], P, worst, what)
         check_peak2(pk[c, s], P, int(r["lag"]), what)
+        check_fine(fine[c, s], r, refs[c], worst, what)
+    print(worst)
+
+
+# test_refine_edges: three captures of a K = 2, half-bin engine over -9..8 half-bins on the reference table.  Rows: a C/A
+# row with a signal (3), a C/A row without one (20), an E1B row with a signal (44) and the last row of the table (E1B
+# 58, whose negative bins read the zero row after the table in the reference wrap).
+EDGE_SEL = np.array([3, 20, 44, 58], np.int32)
+EDGE_KW = dict(k_noncoh=2, half_bin=1, dop_lo=-9, dop_hi=8)
+
+
+def _edge_records(rec, n_sel, j):
+    """Placement j of the records: the search's records with (dop, lag) set per slot to the j-th pair of the cross
+    product of dop_lo, dop_lo + 1, dop_hi - 1, dop_hi, the record's dop with lag 0, 1, L - 2, L - 1 and the record's lag
+    (slot s starts s pairs further on, so every capture and slot meets every pair)."""
+    out = rec.copy()
+    lo, hi = EDGE_KW["dop_lo"], EDGE_KW["dop_hi"]
+    for c in range(out.shape[0]):
+        for s in range(n_sel):
+            r = out[c, s]
+            L = LAGS_E1B if S.reference_table()[int(r["sat"])][3] == S.E1B else LAGS_L1
+            dops = [lo, lo + 1, hi - 1, hi, int(rec[c, s]["dop"])]
+            lags = [0, 1, L - 2, L - 1, int(rec[c, s]["lag"])]
+            k = (j + s + 7 * c) % 25
+            r["dop"], r["lag"] = dops[k // 5], lags[k % 5]
+    return out
+
+
+def test_refine_edges(gpu_required, oracle):
+    """acq_refine accepts any record that passes its checks: records at dop_lo and dop_hi and the odd and even half-bin
+    indices next to them (d +- 1 one bin past the range), lag 0 (lag n - 1 wraps to N - 1), lags L - 2 and L - 1 of C/A
+    and E1B rows, a row without a signal (den small, delta ill-conditioned or clamped), the last table row in the
+    reference wrap, and rows of the second and third captures -- every one against RefineRef, peak against the
+    reference's sum of |r|^2 at that cell.  acq_refine_device of the same records gives the same bytes."""
+    import torch
+    table = S.reference_table()
+    sig = [[(3, 4001, 3.3 * BIN, 48, 1.0), (44, 30003, -4.2 * BIN, 49, 0.4)],
+           [(3, 16000, -4.4 * BIN, 47, 2.0), (44, 100, 3.9 * BIN, 48, 1.1)],
+           [(3, 0, 0.6 * BIN, 46, 0.3), (44, 65000, -0.2 * BIN, 48, 2.5)]]
+    caps = [synth.make_capture(1300 + c, 2, table, sig[c]) for c in range(3)]
+    oprm = oracle.default_params(**EDGE_KW)
+    refs = [RefineRef(oracle, oprm, cap, table) for cap in caps]
+    worst = Worst("refine edges")
+    with F.AcqEngine(table, F.default_params(**EDGE_KW)) as eng:
+        rec = eng.search(np.concatenate(caps), sel=EDGE_SEL)
+        for j in range(25):
+            placed = _edge_records(rec, len(EDGE_SEL), j)
+            fine = eng.refine(placed)
+            assert (fine["ca_shift"] >= 0).all(), fine
+            d_rec = torch.from_numpy(placed.reshape(-1).view(np.uint8).copy()).cuda()
+            d_out = torch.zeros(fine.nbytes, dtype=torch.uint8, device="cuda")
+            torch.cuda.synchronize()
+            eng.refine_device(d_rec.data_ptr(), d_out.data_ptr(), placed.size)
+            torch.cuda.synchronize()
+            assert d_out.cpu().numpy().tobytes() == fine.tobytes(), j
+            for c in range(len(caps)):
+                check_fine(fine[c], placed[c], refs[c], worst, "placement %d capture %d" % (j, c))
     print(worst)
