@@ -10,6 +10,7 @@
 
 #include <algorithm>
 #include <cstdarg>
+#include <memory>
 #include <numeric>
 
 #include "acq_geom.h"
@@ -85,6 +86,88 @@ void ca_code_bits(int t1, int t2, uint32_t *words)
     }
 }
 
+using namespace acq;
+
+// Owner of device memory, freed with the owner.  alloc() replaces the contents by n uninitialised elements.
+template <typename T>
+struct DevBuf {
+    T *p = nullptr;
+    size_t cap = 0;   // elements; 0 while p is NULL
+    DevBuf() = default;
+    DevBuf(const DevBuf &) = delete;
+    DevBuf &operator=(const DevBuf &) = delete;
+    ~DevBuf() { reset(); }
+    operator T *() const { return p; }
+    void reset()
+    {
+        if (p) cudaFree(p);
+        p = nullptr;
+        cap = 0;
+    }
+    cudaError_t alloc(size_t n)
+    {
+        reset();
+        const cudaError_t ce = cudaMalloc(&p, n * sizeof(T));
+        if (ce == cudaSuccess) cap = n;
+        return ce;
+    }
+};
+
+// Owner of pinned host memory (cudaHostAlloc with Flags); mapped memory is zeroed and its device address kept in dev.
+template <typename T, unsigned Flags>
+struct PinnedBuf {
+    T *p = nullptr, *dev = nullptr;
+    size_t cap = 0;
+    PinnedBuf() = default;
+    PinnedBuf(const PinnedBuf &) = delete;
+    PinnedBuf &operator=(const PinnedBuf &) = delete;
+    ~PinnedBuf() { reset(); }
+    void reset()
+    {
+        if (p) cudaFreeHost(p);
+        p = dev = nullptr;
+        cap = 0;
+    }
+    cudaError_t alloc(size_t n)
+    {
+        reset();
+        cudaError_t ce = cudaHostAlloc(&p, n * sizeof(T), Flags);
+        if (ce == cudaSuccess && (Flags & cudaHostAllocMapped)) {
+            memset(p, 0, n * sizeof(T));
+            ce = cudaHostGetDevicePointer(&dev, p, 0);
+        }
+        if (ce == cudaSuccess) cap = n;
+        return ce;
+    }
+};
+
+// b = a device copy of v (left empty if the copy fails)
+template <typename T>
+cudaError_t upload(DevBuf<T> &b, const std::vector<T> &v)
+{
+    cudaError_t ce = b.alloc(v.size());
+    if (ce == cudaSuccess && (ce = cudaMemcpy(b.p, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice)) != cudaSuccess)
+        b.reset();
+    return ce;
+}
+
+// Rows first..F-1 of the sub-bin rotation table [F][16384]: row v = exp(-2 pi i (v / F) n / N), double precision rounded
+// once.  The angle is pi (a n) / (b N) with a / b = 2 v / F in lowest terms, so that the row v = F / 2 of an even F is
+// formed by the same operations as the half-bin table (F = 2, row 1: pi n / N) and rounds to the same floats.
+std::vector<float2> rotation_table(int F, int first)
+{
+    const double pi = 3.14159265358979323846264338327950288;
+    std::vector<float2> rot((size_t)(F - first) * kN);
+    for (int v = first; v < F; v++) {
+        const int g = std::gcd(2 * v, F), a = 2 * v / g, b = F / g;
+        for (int n = 0; n < kN; n++) {
+            const double ang = pi * (double)((long long)a * n) / (double)((long long)b * kN);
+            rot[(size_t)(v - first) * kN + n] = make_float2((float)cos(ang), (float)(-sin(ang)));
+        }
+    }
+    return rot;
+}
+
 }  // namespace
 
 struct acq_engine {
@@ -100,7 +183,8 @@ struct acq_engine {
     bool pending = false;       // acq_submit outstanding
     int pending_rows = 0;       // ... whose records still sit in h_records (copied to pending_out by acq_poll/acq_wait)
     acq_record *pending_out = nullptr;
-    // device-path ordering: an event behind the last acq_search_device; whatever touches the shared scratch next waits for it
+    // device-path ordering: an event behind the last device-path work on another stream; whatever touches the shared
+    // scratch next waits for it (wait_scratch / hold_scratch)
     cudaEvent_t dev_done = nullptr;
     bool dev_pending = false;
     int64_t launches = 0;
@@ -108,66 +192,80 @@ struct acq_engine {
     cudaEvent_t prof[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
 
     // persistent device data
-    float2 *d_tables = nullptr, *d_rot = nullptr, *d_C = nullptr, *d_Ep = nullptr;
+    DevBuf<float2> d_tables, d_rot, d_C, d_Ep;
     // per-call scratch (grown on demand)
-    size_t cap_blocks = 0 /* spectrum rows */, cap_cells = 0, cap_rows = 0, cap_packed = 0;
-    uint8_t *d_packed = nullptr;
-    float2 *d_x2 = nullptr, *d_Dp = nullptr;
-    acq_cell *d_cells = nullptr;
-    acq_record *d_records = nullptr;
-    unsigned *d_tile_ctr = nullptr;    // [4] claim counters [0,1] and done counters [2,3] of the C/A and the E1B search launch (SearchArgs::tile_ctr); zero between launches
-    unsigned *d_ctas_done = nullptr;   // finished search CTAs of a small search (folded best-Doppler pick); zero between searches
-    unsigned epoch = 0;                // search counter: value of the completion word
+    DevBuf<uint8_t> d_packed;
+    DevBuf<float2> d_x2, d_Dp;   // [spectrum rows][kN] each
+    DevBuf<acq_cell> d_cells;
+    DevBuf<acq_record> d_records;
+    DevBuf<unsigned> d_tile_ctr;    // [4] claim counters [0,1] and done counters [2,3] of the C/A and the E1B search launch (SearchArgs::tile_ctr); zero between launches
+    DevBuf<unsigned> d_ctas_done;   // finished search CTAs of a small search (folded best-Doppler pick); zero between searches
+    unsigned epoch = 0;             // search counter: value of the completion word
     // host path: pinned staging of small captures; records and the completion word in mapped pinned memory,
-    // written by the search kernels themselves
-    uint8_t *h_packed = nullptr;
-    size_t cap_h_packed = 0;
-    acq_record *h_records = nullptr, *dh_records = nullptr;  // host / device address of the same mapped buffer
-    size_t cap_h_records = 0;
-    unsigned *h_flag = nullptr, *dh_flag = nullptr;
+    // written by the search kernels themselves.  h_records is sized for the tagged form a polling host reads (32 B);
+    // the plain 24-byte form fits too.
+    PinnedBuf<uint8_t, cudaHostAllocDefault> h_packed;
+    PinnedBuf<acq_record_tagged, cudaHostAllocMapped> h_records;
+    PinnedBuf<unsigned, cudaHostAllocMapped> h_flag;
     // selection: work list [n_slots] (C/A entries first, then E1B) and slot -> table index
     std::vector<int32_t> sel_cache;
     int sel_kind = -1;  // -1 none, 0 whole table, 1 one satellite, 2 uploaded list
     int n_l1 = 0, n_e1b = 0, n_slots = 0;
     const int2 *cur_work = nullptr;
     const int *cur_slot_sat = nullptr;
-    int2 *d_work_full = nullptr, *d_work_single = nullptr, *d_work = nullptr;   // whole table / (s, 0) per s / uploaded
-    int *d_sat_full = nullptr, *d_slot_sat = nullptr;                            // identity / uploaded
+    DevBuf<int2> d_work_full, d_work_single, d_work;   // whole table / (s, 0) per s / uploaded
+    DevBuf<int> d_sat_full, d_slot_sat;                // identity / uploaded
     int full_n_l1 = 0;
-    size_t cap_slots = 0;
-    // refinement (acq_refine): satellite types on the device, record/output scratch, shape of the last host-path search
-    int *d_sat_type = nullptr;
-    acq_record *d_ref_rec = nullptr;
-    acq_fine *d_fine = nullptr;
-    size_t cap_ref_rec = 0, cap_fine = 0;
-    int last_captures = 0;  // 0: no search whose spectra are still on the device
-    // shape of the most recent search of either path (acq_refine_device): captures (0: none whose spectra are still on
-    // the device), slots, and its slot -> satellite map on the device
-    int ref_captures = 0, ref_slots = 0;
-    const int *ref_slot_sat = nullptr;
-    int ref_n_l1 = 0, ref_n_e1b = 0;   // ... and its C/A and E1B slot counts (acq_profile_device)
-    // peak-quality profile (acq_profile): row output scratch of the host form (its lag profiles get a buffer per call)
-    acq_peak2 *d_peak2 = nullptr;
-    size_t cap_peak2 = 0;
+    // refinement and profile: satellite types on the device, record/output scratch of the host forms (acq_profile's lag
+    // profiles get a buffer per call)
+    DevBuf<int> d_sat_type;
+    DevBuf<acq_record> d_ref_rec;
+    DevBuf<acq_fine> d_fine;
+    DevBuf<acq_peak2> d_peak2;
+    // The most recent search whose spectra are still on the device (captures 0: none), which refinement and profile read:
+    // its slots, device slot -> satellite map and C/A and E1B slot counts.  host: a host-path search, whose records
+    // acq_refine and acq_profile may take (the current selection is then its selection).  A coherent search leaves none.
+    struct LastSearch {
+        int captures = 0, slots = 0, n_l1 = 0, n_e1b = 0;
+        const int *slot_sat = nullptr;
+        bool host = false;
+    } last;
     // aided host search (acq_search_aided): Doppler centres staged in pinned memory, copied to the device with the capture
-    int32_t *h_center = nullptr;
-    size_t cap_h_center = 0;
-    int *d_center = nullptr;
-    size_t cap_center = 0;
+    PinnedBuf<int32_t, cudaHostAllocDefault> h_center;
+    DevBuf<int> d_center;
     // coherent search (acq_search_coherent): sub-bin rotation table [F][16384] of each m_coh, built on first use
-    float2 *d_rot_coh[ACQ_COH_MAX + 1] = {};
+    DevBuf<float2> d_rot_coh[ACQ_COH_MAX + 1];
+
+    // Runs under the engine's device (acq_destroy, acq_create): the work in flight ends before the members free their memory.
+    ~acq_engine()
+    {
+        if (stream) cudaStreamSynchronize(stream);
+        if (dev_pending && dev_done) cudaEventSynchronize(dev_done);
+        for (cudaEvent_t ev : prof)
+            if (ev) cudaEventDestroy(ev);
+        if (done) cudaEventDestroy(done);
+        if (dev_done) cudaEventDestroy(dev_done);
+        if (stream) cudaStreamDestroy(stream);
+    }
 };
 
 namespace {
 
-using namespace acq;
+// What one search call asks for: the engine's whole Doppler range or, aided, a window of W = 2 half_width + 1 cells around
+// each row's centre; non-coherent sums or, coherent, groups of M = m_coh blocks on the 1/F-bin grid.
+struct SearchMode {
+    bool aided, coherent;
+    const int32_t *center;   // aided: one Doppler centre per row (host or device memory, as the entry point)
+    int half_width, m_coh;
+    int dop_scale() const { return coherent ? m_coh : 1; }   // dop_lo / dop_hi of the grid searched, in its units
+    int variants(const acq_engine *e) const { return coherent ? m_coh * (1 + e->prm.half_bin) : e->nvar; }   // per block
+    int full_dops(const acq_engine *e) const { return dop_scale() * (e->n_dop - 1) + 1; }   // n_dop, or n_dop_c
+    int dops(const acq_engine *e) const { return aided ? 2 * half_width + 1 : full_dops(e); }   // cells per row
+};
+constexpr SearchMode kFullRange{false, false, nullptr, 0, 0};
 
-// Build-time switches of the experiment variants (tools/build_variants.py); the product library defines none of
-// them and reads no environment variable.
-//   ACQ_FORCE_E1B_KERNEL=1|2 one-CTA / cluster form of the E1B search regardless of the tile count
-#ifndef ACQ_FORCE_E1B_KERNEL
-#define ACQ_FORCE_E1B_KERNEL 0
-#endif
+// Build-time switch of an experiment variant (tools/build_variants.py); the product library defines none and reads no
+// environment variable.
 //   ACQ_ARG_INPUT=1|0        a search of ONE 1-bit block: the capture travels as the front end's kernel argument (1) or by
 //                            the staging buffer and a copy node like every other search (0, variant "argin0")
 #ifndef ACQ_ARG_INPUT
@@ -184,49 +282,8 @@ constexpr int kHostRecordRowsMax = 256;          // records (24 B each: single P
 constexpr int kFoldPickRowsMax = acq::kPickSmallRowsMax;
 static_assert(kHostRecordRowsMax <= kFoldPickRowsMax, "the completion word is raised by k_pick_small");
 
-int free_engine(acq_engine *e)
-{
-    if (!e) return ACQ_OK;
-    DeviceGuard g(e->device);
-    if (e->stream) cudaStreamSynchronize(e->stream);
-    if (e->dev_pending && e->dev_done) cudaEventSynchronize(e->dev_done);
-    cudaFree(e->d_tables);
-    cudaFree(e->d_rot);
-    cudaFree(e->d_C);
-    cudaFree(e->d_Ep);
-    cudaFree(e->d_packed);
-    cudaFree(e->d_x2);
-    cudaFree(e->d_Dp);
-    cudaFree(e->d_cells);
-    cudaFree(e->d_records);
-    cudaFree(e->d_ctas_done);
-    cudaFree(e->d_tile_ctr);
-    cudaFree(e->d_work_full);
-    cudaFree(e->d_work_single);
-    cudaFree(e->d_work);
-    cudaFree(e->d_sat_full);
-    cudaFree(e->d_slot_sat);
-    cudaFree(e->d_sat_type);
-    cudaFree(e->d_ref_rec);
-    cudaFree(e->d_fine);
-    cudaFree(e->d_peak2);
-    cudaFree(e->d_center);
-    for (float2 *r : e->d_rot_coh) cudaFree(r);
-    if (e->h_center) cudaFreeHost(e->h_center);
-    if (e->h_packed) cudaFreeHost(e->h_packed);
-    if (e->h_records) cudaFreeHost(e->h_records);
-    if (e->h_flag) cudaFreeHost(e->h_flag);
-    if (e->done) cudaEventDestroy(e->done);
-    if (e->dev_done) cudaEventDestroy(e->dev_done);
-    for (cudaEvent_t ev : e->prof)
-        if (ev) cudaEventDestroy(ev);
-    if (e->stream) cudaStreamDestroy(e->stream);
-    delete e;
-    return ACQ_OK;
-}
-
 // Everything that is about to touch the shared scratch from the host (reallocation, synchronous copies) first
-// drains the engine stream and the last device-path search.
+// drains the engine stream and the last device-path work.
 int drain(acq_engine *e)
 {
     CU(cudaStreamSynchronize(e->stream));
@@ -237,72 +294,66 @@ int drain(acq_engine *e)
     return ACQ_OK;
 }
 
-template <typename T>
-int grow(acq_engine *e, T *&ptr, size_t &cap, size_t need_elems, bool zero = false)
+// b holds at least `need` elements: only a buffer that grows drains the engine first
+template <class Buf>
+int grow(acq_engine *e, Buf &b, size_t need)
 {
-    if (need_elems <= cap && ptr) return ACQ_OK;
+    if (need <= b.cap) return ACQ_OK;
     int rc = drain(e);
     if (rc) return rc;
-    if (ptr) CU(cudaFree(ptr));
-    ptr = nullptr;
-    cap = 0;
-    CU(cudaMalloc(&ptr, need_elems * sizeof(T)));
-    if (zero) CU(cudaMemset(ptr, 0, need_elems * sizeof(T)));
-    cap = need_elems;
+    CU(b.alloc(need));
     return ACQ_OK;
 }
 
-// n_dop: Doppler cells per row of this search (the engine's range, the window of an aided search, or the 1/M-bin grid of
-// a coherent one); nvar: spectrum variants per block (e->nvar, or F of a coherent search)
-int ensure_scratch(acq_engine *e, int n_captures, int n_slots, bool host_path, int n_dop, int nvar)
+// Device-path ordering.  Work about to use the engine's scratch on `st` waits for the last device-path work on another
+// stream (a no-op on the stream that recorded it) and, with engine_too, for what the engine stream has queued ...
+int wait_scratch(acq_engine *e, cudaStream_t st, bool engine_too)
 {
-    const size_t blocks = (size_t)n_captures * e->prm.k_noncoh;
-    const size_t spectra = blocks * nvar * e->n_shift;   // rows of x2 and of the capture spectra
-    if (spectra > e->cap_blocks || !e->d_x2) {
-        int rc = drain(e);  // changing scratch under an in-flight search is not allowed
-        if (rc) return rc;
-        if (e->d_x2) CU(cudaFree(e->d_x2));
-        if (e->d_Dp) CU(cudaFree(e->d_Dp));
-        e->d_x2 = e->d_Dp = nullptr;
-        e->cap_blocks = 0;
-        CU(cudaMalloc(&e->d_x2, spectra * kN * sizeof(float2)));
-        CU(cudaMalloc(&e->d_Dp, spectra * kN * sizeof(float2)));
-        e->cap_blocks = spectra;
+    if (e->dev_pending) CU(cudaStreamWaitEvent(st, e->dev_done, 0));
+    if (engine_too && st != e->stream) {
+        CU(cudaEventRecord(e->dev_done, e->stream));
+        CU(cudaStreamWaitEvent(st, e->dev_done, 0));
     }
-    const size_t rows = (size_t)n_captures * n_slots;
-    int rc;
-    if ((rc = grow(e, e->d_cells, e->cap_cells, rows * n_dop))) return rc;
-    if (!host_path) return ACQ_OK;
-    const size_t bytes = blocks * e->block_bytes;
-    if ((rc = grow(e, e->d_packed, e->cap_packed, bytes))) return rc;
-    if (bytes <= kStagePackedMax && bytes > e->cap_h_packed) {
-        if ((rc = drain(e))) return rc;
-        if (e->h_packed) CU(cudaFreeHost(e->h_packed));
-        e->h_packed = nullptr;
-        e->cap_h_packed = 0;
-        CU(cudaHostAlloc(&e->h_packed, bytes, cudaHostAllocDefault));
-        e->cap_h_packed = bytes;
-    }
-    if (rows <= (size_t)kHostRecordRowsMax) {
-        if (rows > e->cap_h_records) {
-            if ((rc = drain(e))) return rc;
-            if (e->h_records) CU(cudaFreeHost(e->h_records));
-            e->h_records = e->dh_records = nullptr;
-            e->cap_h_records = 0;
-            // sized for the tagged form a polling host reads (acq_record_tagged, 32 B); the plain 24-byte form fits too
-            CU(cudaHostAlloc(&e->h_records, rows * sizeof(acq_record_tagged), cudaHostAllocMapped));
-            memset(e->h_records, 0, rows * sizeof(acq_record_tagged));
-            CU(cudaHostGetDevicePointer(&e->dh_records, e->h_records, 0));
-            e->cap_h_records = rows;
-        }
-        return ACQ_OK;
-    }
-    return grow(e, e->d_records, e->cap_rows, rows);
+    return ACQ_OK;
 }
 
-// Split the selection into the 1 ms-window (Navstar/QZSS/SBAS) and E1B work lists.  The whole table and single
-// satellites (what the literal SearchTask loop asks for, one satellite per capture) use lists built at acq_create;
-// any other list is uploaded, which drains the engine first.
+// ... and once it is enqueued on a stream other than the engine's, whatever uses the scratch next (any stream, or the
+// host) waits for it.
+int hold_scratch(acq_engine *e, cudaStream_t st)
+{
+    if (st != e->stream) {
+        CU(cudaEventRecord(e->dev_done, st));
+        e->dev_pending = true;
+    }
+    return ACQ_OK;
+}
+
+// Scratch of a search of n_captures over the current selection in mode m; host_path: also the staging and record buffers
+int ensure_scratch(acq_engine *e, int n_captures, bool host_path, const SearchMode &m)
+{
+    const size_t blocks = (size_t)n_captures * e->prm.k_noncoh;
+    const size_t spectra = blocks * m.variants(e) * e->n_shift * kN;   // x2 and the capture spectra
+    if (spectra > e->d_x2.cap || spectra > e->d_Dp.cap) {
+        int rc = drain(e);  // changing scratch under an in-flight search is not allowed
+        if (rc) return rc;
+        CU(e->d_x2.alloc(spectra));
+        CU(e->d_Dp.alloc(spectra));
+    }
+    if (m.coherent && !e->d_rot_coh[m.m_coh]) CU(upload(e->d_rot_coh[m.m_coh], rotation_table(m.variants(e), 0)));
+    const size_t rows = (size_t)n_captures * e->n_slots;
+    int rc;
+    if ((rc = grow(e, e->d_cells, rows * m.dops(e)))) return rc;
+    if (!host_path) return ACQ_OK;
+    const size_t bytes = blocks * e->block_bytes;
+    if ((rc = grow(e, e->d_packed, bytes))) return rc;
+    if (bytes <= kStagePackedMax && (rc = grow(e, e->h_packed, bytes))) return rc;
+    if (m.aided && ((rc = grow(e, e->d_center, rows)) || (rc = grow(e, e->h_center, rows)))) return rc;
+    return rows <= (size_t)kHostRecordRowsMax ? grow(e, e->h_records, rows) : grow(e, e->d_records, rows);
+}
+
+// Split the selection (checked by check_search) into the 1 ms-window (Navstar/QZSS/SBAS) and E1B work lists.  The whole
+// table and single satellites (what the literal SearchTask loop asks for, one satellite per capture) use lists built at
+// acq_create; any other list is uploaded, which drains the engine first.
 int set_selection(acq_engine *e, const int32_t *sel, int n_sel)
 {
     const int n_sats = (int)e->sats.size();
@@ -319,10 +370,6 @@ int set_selection(acq_engine *e, const int32_t *sel, int n_sel)
         e->n_slots = n_sats;
         return ACQ_OK;
     }
-    if (n_sel <= 0) return fail(ACQ_ERR_ARG, "n_sel must be > 0 when sel is given");
-    for (int i = 0; i < n_sel; i++)
-        if (sel[i] < 0 || sel[i] >= n_sats)
-            return fail(ACQ_ERR_ARG, "satellite index %d outside the table (0..%d)", sel[i], n_sats - 1);
     if (n_sel == 1) {
         const int sat = sel[0];
         e->sel_cache.assign(1, sat);
@@ -352,15 +399,9 @@ int set_selection(acq_engine *e, const int32_t *sel, int n_sel)
     int rc = drain(e);  // the lists may still be read by a search in flight; the copies below are synchronous
     if (rc) return rc;
     e->sel_kind = -1;
-    if ((size_t)n_sel > e->cap_slots) {
-        if (e->d_work) CU(cudaFree(e->d_work));
-        if (e->d_slot_sat) CU(cudaFree(e->d_slot_sat));
-        e->d_work = nullptr;
-        e->d_slot_sat = nullptr;
-        e->cap_slots = 0;
-        CU(cudaMalloc(&e->d_work, (size_t)n_sel * sizeof(int2)));
-        CU(cudaMalloc(&e->d_slot_sat, (size_t)n_sel * sizeof(int)));
-        e->cap_slots = (size_t)n_sel;
+    if ((size_t)n_sel > e->d_work.cap || (size_t)n_sel > e->d_slot_sat.cap) {
+        CU(e->d_work.alloc(n_sel));
+        CU(e->d_slot_sat.alloc(n_sel));
     }
     CU(cudaMemcpy(e->d_work, work.data(), work.size() * sizeof(int2), cudaMemcpyHostToDevice));
     CU(cudaMemcpy(e->d_slot_sat, sel, (size_t)n_sel * sizeof(int), cudaMemcpyHostToDevice));
@@ -374,100 +415,75 @@ int set_selection(acq_engine *e, const int32_t *sel, int n_sel)
     return ACQ_OK;
 }
 
-// Doppler cells per row: the engine's whole range, or the window of an aided search (center != NULL)
-int row_dops(const acq_engine *e, const void *center, int half_width) { return center ? 2 * half_width + 1 : e->n_dop; }
+// Largest Doppler range an engine can have: |index| <= 4094 half-bins (acq_create: at most 2048 bins either side).
+constexpr int kMaxHalfWidth = 4094;
 
-// Coherent search of M = m_coh blocks per group: n_dop_c = M (n_dop - 1) + 1 cells per row (1/M of the engine's Doppler
-// step), F = M (1 + half_bin) spectrum variants per block
-int coh_dops(const acq_engine *e, int m_coh) { return m_coh * (e->n_dop - 1) + 1; }
-int coh_variants(const acq_engine *e, int m_coh) { return m_coh * (1 + e->prm.half_bin); }
-// Doppler cells per row of any search: a window (center != NULL) of either grid, else the coherent or the engine's range
-int search_dops(const acq_engine *e, const void *center, int half_width, int m_coh)
+// The checks of one search call, before anything touches the device.  Those that need no engine come first, so that they
+// are reported whatever the engine.  ACQ_ERR_ARG for the argument errors; ACQ_ERR_UNSUPPORTED for what the coherent
+// search does not cover (E1B rows, code-Doppler engines, more than 2^24 capture spectra) and for searches above the tile
+// bound: a search kernel launch indexes its tiles with 32 bits (and four units per tile with 64).
+int check_search(acq_engine *e, const SearchMode &m, const void *packed, int n_captures, const int32_t *sel, int n_sel,
+                 const void *out, bool device)
 {
-    return (m_coh && !center) ? coh_dops(e, m_coh) : row_dops(e, center, half_width);
-}
-
-// Rotation table of the sub-bin variants, [F][16384]: row v = exp(-2 pi i (v / F) n / N), double precision rounded once.
-// The angle is pi (a n) / (b N) with a / b = 2 v / F in lowest terms, so that the row v = F / 2 of an even F is formed by
-// the same operations as the half-bin table of acq_create (pi n / N) and rounds to the same floats.
-int ensure_coh_rot(acq_engine *e, int m_coh)
-{
-    if (e->d_rot_coh[m_coh]) return ACQ_OK;
-    const int F = coh_variants(e, m_coh);
-    const double pi = 3.14159265358979323846264338327950288;
-    std::vector<float2> rot((size_t)F * kN);
-    for (int v = 0; v < F; v++) {
-        const int g = std::gcd(2 * v, F), a = 2 * v / g, b = F / g;
-        for (int n = 0; n < kN; n++) {
-            const double ang = pi * (double)((long long)a * n) / (double)((long long)b * kN);
-            rot[(size_t)v * kN + n] = make_float2((float)cos(ang), (float)(-sin(ang)));
-        }
-    }
-    float2 *d = nullptr;
-    CU(cudaMalloc(&d, rot.size() * sizeof(float2)));
-    const cudaError_t ce = cudaMemcpy(d, rot.data(), rot.size() * sizeof(float2), cudaMemcpyHostToDevice);
-    if (ce != cudaSuccess) {
-        cudaFree(d);
-        return fail(ACQ_ERR_CUDA, "coherent rotation table: %s", cudaGetErrorString(ce));
-    }
-    e->d_rot_coh[m_coh] = d;
-    return ACQ_OK;
-}
-
-int check_search_args(acq_engine *e, const void *packed, int n_captures, const void *out);
-
-// The arguments of a coherent search, checked before anything touches the device: ACQ_ERR_ARG for the argument errors,
-// ACQ_ERR_UNSUPPORTED for what the coherent search does not cover (E1B rows, code-Doppler engines, searches above the
-// tile and spectrum-row bounds).  center != NULL: an aided coherent search, whose rows hold W = 2 half_width + 1 cells
-// (W <= n_dop_c) rather than n_dop_c; check_coherent_aided_args has checked what needs no engine.
-int check_coherent(acq_engine *e, const void *packed, int n_captures, const int32_t *sel, int n_sel, int m_coh,
-                   const void *out, const int32_t *center = nullptr, int half_width = 0)
-{
+    const int hw = m.half_width;
+    if (m.aided && !m.center) return fail(ACQ_ERR_ARG, "dop_center is NULL");
+    if (m.aided && hw < 0) return fail(ACQ_ERR_ARG, "half_width must be >= 0 (got %d)", hw);
+    if (m.coherent && (m.m_coh < 1 || m.m_coh > ACQ_COH_MAX))
+        return fail(ACQ_ERR_ARG, "m_coh=%d outside 1..%d", m.m_coh, ACQ_COH_MAX);
+    if (m.aided && hw > (m.coherent ? ACQ_COH_MAX : 1) * kMaxHalfWidth)
+        return fail(ACQ_ERR_ARG, "Doppler window W = 2*half_width+1 with half_width %d exceeds n_dop%s of any engine", hw,
+                    m.coherent ? "_c" : "");
     if (!e) return fail(ACQ_ERR_ARG, "engine is NULL");
-    if (m_coh < 1 || m_coh > ACQ_COH_MAX) return fail(ACQ_ERR_ARG, "m_coh=%d outside 1..%d", m_coh, ACQ_COH_MAX);
-    int rc = check_search_args(e, packed, n_captures, out);
-    if (rc) return rc;
-    if (e->prm.k_noncoh % m_coh)
-        return fail(ACQ_ERR_ARG, "k_noncoh=%d is not a multiple of m_coh=%d", e->prm.k_noncoh, m_coh);
-    if (center && half_width > (coh_dops(e, m_coh) - 1) / 2)
-        return fail(ACQ_ERR_ARG, "Doppler window W = 2*half_width+1 with half_width %d exceeds n_dop_c = %d", half_width,
-                    coh_dops(e, m_coh));
+    const int full = m.full_dops(e), K = e->prm.k_noncoh;
+    if (m.aided && 2 * hw + 1 > full) {
+        if (m.coherent)
+            return fail(ACQ_ERR_ARG, "Doppler window W = 2*half_width+1 with half_width %d exceeds n_dop_c = %d", hw, full);
+        return fail(ACQ_ERR_ARG, "Doppler window W = 2*half_width+1 = %d exceeds n_dop = %d", 2 * hw + 1, full);
+    }
+    if (!packed || !out) return fail(ACQ_ERR_ARG, "packed/out must not be NULL");
+    if (n_captures <= 0) return fail(ACQ_ERR_ARG, "n_captures must be > 0 (got %d)", n_captures);
+    if ((long long)n_captures * K * e->n_shift > (1 << 24)) return fail(ACQ_ERR_ARG, "too many capture blocks");
+    if (e->pending) return fail(ACQ_ERR_ARG, "a submitted search is still pending: call acq_wait first");
+    if (device && ((uintptr_t)packed & 15) != 0)
+        return fail(ACQ_ERR_ARG, "packed_dev must be 16-byte aligned (the front end stages it with bulk async copies)");
+    // A non-coherent search forgets the last search from here on, also when it is refused below; a refused coherent
+    // search leaves it.
+    if (!m.coherent) e->last = {};
+    if (m.coherent && K % m.m_coh) return fail(ACQ_ERR_ARG, "k_noncoh=%d is not a multiple of m_coh=%d", K, m.m_coh);
     const int n_sats = (int)e->sats.size();
     if (sel && n_sel <= 0) return fail(ACQ_ERR_ARG, "n_sel must be > 0 when sel is given");
     const int n_slots = sel ? n_sel : n_sats;
-    for (int i = 0; i < n_slots; i++) {
-        const int s = sel ? sel[i] : i;
-        if (s < 0 || s >= n_sats) return fail(ACQ_ERR_ARG, "satellite index %d outside the table (0..%d)", s, n_sats - 1);
+    for (int i = 0; sel && i < n_sel; i++)
+        if (sel[i] < 0 || sel[i] >= n_sats)
+            return fail(ACQ_ERR_ARG, "satellite index %d outside the table (0..%d)", sel[i], n_sats - 1);
+    if (m.coherent) {
+        if (e->prm.code_doppler)
+            return fail(ACQ_ERR_UNSUPPORTED, "coherent search of a code_doppler engine is not implemented");
+        for (int i = 0; i < n_slots; i++)
+            if (e->sats[sel ? sel[i] : i].type == ACQ_E1B)
+                return fail(ACQ_ERR_UNSUPPORTED, "coherent search of E1B rows is not implemented (satellite %d): E1B "
+                            "symbols drift against the block edges", sel ? sel[i] : i);
+        if ((long long)n_captures * K * m.variants(e) > (1 << 24))
+            return fail(ACQ_ERR_UNSUPPORTED, "coherent search too large for one call (more than 2^24 capture spectra): split the captures");
     }
-    if (e->prm.code_doppler)
-        return fail(ACQ_ERR_UNSUPPORTED, "coherent search of a code_doppler engine is not implemented");
-    for (int i = 0; i < n_slots; i++)
-        if (e->sats[sel ? sel[i] : i].type == ACQ_E1B)
-            return fail(ACQ_ERR_UNSUPPORTED, "coherent search of E1B rows is not implemented (satellite %d): E1B symbols "
-                        "drift against the block edges", sel ? sel[i] : i);
-    if ((long long)n_captures * e->prm.k_noncoh * coh_variants(e, m_coh) > (1 << 24))
-        return fail(ACQ_ERR_UNSUPPORTED, "coherent search too large for one call (more than 2^24 capture spectra): split the captures");
-    const int n_dop = center ? 2 * half_width + 1 : coh_dops(e, m_coh);
-    if ((double)n_captures * (double)n_slots * (double)n_dop > (double)acq::kMaxTilesPerLaunch)
-        return fail(ACQ_ERR_UNSUPPORTED, "coherent search too large for one call (more than 2^31 - 1 tiles): split the captures");
+    if ((double)n_captures * (double)n_slots * (double)m.dops(e) > (double)acq::kMaxTilesPerLaunch)
+        return fail(ACQ_ERR_UNSUPPORTED, "%ssearch too large for one call (more than 2^31 - 1 tiles): split the captures",
+                    m.coherent ? "coherent " : "");
     return ACQ_OK;
 }
 
 // Enqueue front end + forward FFT + search (which ends in the best-Doppler pick) on `st` for captures already on the
-// device.  records_dev: where the kernels write the records (device memory, or the device alias of mapped host memory);
-// flag_dev: mapped completion word, or NULL.  center_dev: the rows' Doppler centres on the device (an aided search), or
-// NULL for the whole range.  m_coh > 0: a coherent search (acq_search_coherent) of M = m_coh blocks per group, with
-// center_dev its aided form (acq_search_coherent_aided: centres and half_width in the coherent grid's units).
-int enqueue_search(acq_engine *e, const uint8_t *packed_dev, int n_captures, acq_record *records_dev, unsigned *flag_dev,
-                   cudaStream_t st, const uint8_t *packed_host_arg = nullptr, const int *center_dev = nullptr,
-                   int half_width = 0, int m_coh = 0)
+// device, in mode m with m.center on the device.  records_dev: where the kernels write the records (device memory, or the
+// device alias of mapped host memory); flag_dev: mapped completion word, or NULL.
+int enqueue_search(acq_engine *e, const SearchMode &m, const uint8_t *packed_dev, int n_captures, acq_record *records_dev,
+                   unsigned *flag_dev, cudaStream_t st, const uint8_t *packed_host_arg)
 {
     const int K = e->prm.k_noncoh;
-    const int n_dop = search_dops(e, center_dev, half_width, m_coh);
-    const int nvar = m_coh ? coh_variants(e, m_coh) : e->nvar;
+    const int n_dop = m.dops(e), nvar = m.variants(e);
     const int blocks = n_captures * K;
     const bool prof = e->profiling;
-    if (e->dev_pending) CU(cudaStreamWaitEvent(st, e->dev_done, 0));  // a no-op on the stream that recorded it
+    int rc = wait_scratch(e, st, false);
+    if (rc) return rc;
     // Programmatic dependent launch between the kernels of a search: a gain where the search is a few waves of tiles
     // (single captures: 85 -> 77 us for the reference's 32-PRN cold start) and, since every kernel of the chain asks for
     // the same shared-memory carveout (search_kernels_configure), a small one on long searches too (K = 20: 3.453 ->
@@ -484,9 +500,9 @@ int enqueue_search(acq_engine *e, const uint8_t *packed_dev, int n_captures, acq
     } else {
         // a coherent search: k_front_end writes variant 0 (and with F = 2 variant 1, from row 1 of the table, which equals
         // the half-bin table), k_coh_variants the others
-        const float2 *rot = m_coh ? e->d_rot_coh[m_coh] + kN : e->d_rot;
+        const float2 *rot = m.coherent ? e->d_rot_coh[m.m_coh] + kN : e->d_rot;
         e->launches += launch_front_end(packed_dev, e->d_x2, rot, blocks, nvar, K, e->sample_bits, e->n_shift, e->smax, st);
-        if (nvar > 2) e->launches += launch_coh_variants(e->d_x2, e->d_rot_coh[m_coh], blocks, nvar, K, st);
+        if (nvar > 2) e->launches += launch_coh_variants(e->d_x2, e->d_rot_coh[m.m_coh], blocks, nvar, K, st);
     }
     if (prof) CU(cudaEventRecord(e->prof[1], st));
     e->launches += launch_fwd_fft(e->d_x2, e->d_Dp, e->d_tables, blocks * nvar * e->n_shift, true, e->sm_count, st, pdl);
@@ -498,10 +514,10 @@ int enqueue_search(acq_engine *e, const uint8_t *packed_dev, int n_captures, acq
     a.cells = e->d_cells;
     a.n_slots = e->n_slots;
     a.n_dop = n_dop;
-    a.dop_lo = e->prm.dop_lo * (m_coh ? m_coh : 1);
-    a.dop_center = center_dev;
-    a.half_width = half_width;
-    a.dop_hi = e->prm.dop_hi * (m_coh ? m_coh : 1);
+    a.dop_lo = e->prm.dop_lo * m.dop_scale();
+    a.dop_center = m.center;
+    a.half_width = m.half_width;
+    a.dop_hi = e->prm.dop_hi * m.dop_scale();
     a.half_bin = e->prm.half_bin;
     a.K = K;
     a.nvar = nvar;
@@ -513,28 +529,19 @@ int enqueue_search(acq_engine *e, const uint8_t *packed_dev, int n_captures, acq
     const int n_rows = n_captures * e->n_slots;
     const bool fold = n_rows <= kFoldPickRowsMax;
     const long long tiles_l1 = (long long)n_captures * e->n_l1 * n_dop, tiles_e1b = (long long)n_captures * e->n_e1b * n_dop;
-    // Cluster/DSMEM form of the E1B search when every tile can have a cluster of its own (one wave: 9 us per tile
-    // against 12.5 us for the one-CTA form, measured) or when forced (variant builds).  With more tiles than that the
-    // one-CTA-per-tile forms (k_search_e1b, k_search_e1b_multi for non-coherent sums) have ~2.9x the throughput.
-    const bool e1b_cluster = ACQ_FORCE_E1B_KERNEL == 2 || (ACQ_FORCE_E1B_KERNEL == 0 && tiles_e1b <= e->sm_count / 4);
+    const int kind_l1 = m.coherent ? kSearchL1Coh : search_kind_l1(K, e->prm.half_bin);
     a.ctas_done = e->d_ctas_done;
-    a.ctas_total = fold ? (unsigned)((m_coh ? coh_grid_ctas(tiles_l1, e->sm_count)
-                                            : search_grid_ctas(tiles_l1, search_kind_l1(K, e->prm.half_bin), e->sm_count)) +
-                                     search_grid_ctas(tiles_e1b, e1b_cluster ? kSearchE1bCluster : kSearchE1b, e->sm_count))
+    a.ctas_total = fold ? (unsigned)(search_grid_ctas(tiles_l1, kind_l1, e->sm_count) +
+                                     search_grid_ctas(tiles_e1b, search_kind_e1b(tiles_e1b, e->sm_count), e->sm_count))
                         : 0u;
     a.wait_prior = 1;
-    if (m_coh && e->n_l1 > 0) {   // the selection holds no E1B row (check_coherent)
+    if (e->n_l1 > 0) {   // a coherent search has no E1B row (check_search)
         a.work = e->cur_work;
         a.n_work = e->n_l1;
         a.n_tiles = tiles_l1;
         a.tile_ctr = e->d_tile_ctr;
-        e->launches += launch_search_coh(CohSearchArgs(a, m_coh), e->sm_count, st, pdl);
-    } else if (e->n_l1 > 0) {
-        a.work = e->cur_work;
-        a.n_work = e->n_l1;
-        a.n_tiles = tiles_l1;
-        a.tile_ctr = e->d_tile_ctr;
-        e->launches += launch_search(a, false, e->sm_count, st, pdl);
+        e->launches += m.coherent ? launch_search_coh(CohSearchArgs(a, m.m_coh), e->sm_count, st, pdl)
+                                  : launch_search(a, false, e->sm_count, st, pdl);
         // The C/A kernel raises its launch-dependents trigger only after its own wait for the forward FFT, so an E1B
         // launch chained to it by programmatic dependent launch starts with the capture spectra complete: it does
         // not wait again, and its CTAs move in as the C/A kernel's last CTAs retire (the two write disjoint rows, and
@@ -546,11 +553,10 @@ int enqueue_search(acq_engine *e, const uint8_t *packed_dev, int n_captures, acq
         a.n_work = e->n_e1b;
         a.n_tiles = tiles_e1b;
         a.tile_ctr = e->d_tile_ctr + 1;
-        if (e1b_cluster) e->launches += launch_search_e1b_cluster(a, e->sm_count, st, pdl);
-        else e->launches += launch_search(a, true, e->sm_count, st, pdl);
+        e->launches += launch_search(a, true, e->sm_count, st, pdl);
     }
     if (prof) CU(cudaEventRecord(e->prof[3], st));
-    const PickDop pd{a.dop_lo, center_dev, half_width, a.dop_hi};
+    const PickDop pd{a.dop_lo, m.center, m.half_width, a.dop_hi};
     if (fold)
         e->launches += launch_pick_small(e->d_cells, e->cur_slot_sat, records_dev, e->d_ctas_done, a.ctas_total, flag_dev,
                                          e->epoch, n_rows, e->n_slots, n_dop, pd, st, pdl);
@@ -564,66 +570,20 @@ int enqueue_search(acq_engine *e, const uint8_t *packed_dev, int n_captures, acq
     return ACQ_OK;
 }
 
-int check_search_args(acq_engine *e, const void *packed, int n_captures, const void *out)
-{
-    if (!e) return fail(ACQ_ERR_ARG, "engine is NULL");
-    if (!packed || !out) return fail(ACQ_ERR_ARG, "packed/out must not be NULL");
-    if (n_captures <= 0) return fail(ACQ_ERR_ARG, "n_captures must be > 0 (got %d)", n_captures);
-    if ((long long)n_captures * e->prm.k_noncoh * e->n_shift > (1 << 24)) return fail(ACQ_ERR_ARG, "too many capture blocks");
-    if (e->pending) return fail(ACQ_ERR_ARG, "a submitted search is still pending: call acq_wait first");
-    return ACQ_OK;
-}
-
-// after set_selection: a search kernel launch indexes its tiles with 32 bits (and four units per tile with 64)
-int check_tile_count(acq_engine *e, int n_captures, int n_dop)
-{
-    if ((double)n_captures * (double)e->n_slots * (double)n_dop > (double)acq::kMaxTilesPerLaunch)
-        return fail(ACQ_ERR_UNSUPPORTED, "search too large for one call (more than 2^31 - 1 tiles): split the captures");
-    return ACQ_OK;
-}
-
-// Largest Doppler range an engine can have: |index| <= 4094 half-bins (acq_create: at most 2048 bins either side).
-constexpr int kMaxHalfWidth = 4094;
-
-// Arguments of an aided search that need no engine come first, so that they are reported whatever the engine.
-int check_aided_args(acq_engine *e, const int32_t *dop_center, int half_width)
-{
-    if (!dop_center) return fail(ACQ_ERR_ARG, "dop_center is NULL");
-    if (half_width < 0) return fail(ACQ_ERR_ARG, "half_width must be >= 0 (got %d)", half_width);
-    if (half_width > kMaxHalfWidth)
-        return fail(ACQ_ERR_ARG, "Doppler window W = 2*half_width+1 with half_width %d exceeds n_dop of any engine", half_width);
-    if (!e) return fail(ACQ_ERR_ARG, "engine is NULL");
-    if (2 * half_width + 1 > e->n_dop)
-        return fail(ACQ_ERR_ARG, "Doppler window W = 2*half_width+1 = %d exceeds n_dop = %d", 2 * half_width + 1, e->n_dop);
-    return ACQ_OK;
-}
-
-// Arguments of an aided coherent search that need no engine come first, as in check_aided_args.
-int check_coherent_aided_args(acq_engine *e, const int32_t *dop_center, int half_width, int m_coh)
-{
-    if (!dop_center) return fail(ACQ_ERR_ARG, "dop_center is NULL");
-    if (half_width < 0) return fail(ACQ_ERR_ARG, "half_width must be >= 0 (got %d)", half_width);
-    if (m_coh < 1 || m_coh > ACQ_COH_MAX) return fail(ACQ_ERR_ARG, "m_coh=%d outside 1..%d", m_coh, ACQ_COH_MAX);
-    if (half_width > ACQ_COH_MAX * kMaxHalfWidth)
-        return fail(ACQ_ERR_ARG, "Doppler window W = 2*half_width+1 with half_width %d exceeds n_dop_c of any engine", half_width);
-    if (!e) return fail(ACQ_ERR_ARG, "engine is NULL");
-    return ACQ_OK;
-}
-
 // Wait for a host-polled search and collect its records: k_pick_small writes every record into mapped memory as two
 // 16-byte halves that each end in the search's epoch (acq_record_tagged), so a half whose tag matches has arrived whole.
 // The stream is queried now and then so that a failed launch cannot hang the caller; the mapped word *h_flag is only
 // ever written to report that the pick gave up (0xffffffff).
 int poll_records(acq_engine *e, acq_record *out, size_t rows)
 {
-    const volatile acq_record_tagged *h = reinterpret_cast<const volatile acq_record_tagged *>(e->h_records);
+    const volatile acq_record_tagged *h = e->h_records.p;
     const unsigned epoch = e->epoch;
     unsigned spins = 0;
     for (size_t i = 0; i < rows; i++) {
         while (h[i].tag0 != epoch || h[i].tag1 != epoch) {
             if ((++spins & 0x3ff) == 0) {
-                if (*(volatile unsigned *)e->h_flag == 0xffffffffu) {
-                    *e->h_flag = 0;
+                if (*(volatile unsigned *)e->h_flag.p == 0xffffffffu) {
+                    *e->h_flag.p = 0;
                     return fail(ACQ_ERR_CUDA, "search kernels did not complete (best-Doppler pick timed out)");
                 }
                 const cudaError_t q = cudaStreamQuery(e->stream);
@@ -645,25 +605,112 @@ int poll_records(acq_engine *e, acq_record *out, size_t rows)
     return ACQ_OK;
 }
 
-// After a search of either path is enqueued: the shape acq_refine_device and acq_profile_device check their call and
-// their records against.
-void set_refine_shape(acq_engine *e, int n_captures)
+// Host path.  center (HOST, one per row) of an aided mode is staged through pinned memory.
+int search_host(acq_engine *e, const SearchMode &m, const uint8_t *packed, int n_captures, const int32_t *sel, int n_sel,
+                acq_record *out, acq_cell *grid, bool sync)
 {
-    e->ref_captures = n_captures;
-    e->ref_slots = e->n_slots;
-    e->ref_slot_sat = e->cur_slot_sat;
-    e->ref_n_l1 = e->n_l1;
-    e->ref_n_e1b = e->n_e1b;
+    int rc = check_search(e, m, packed, n_captures, sel, n_sel, out, false);
+    if (rc) return rc;
+    DeviceGuard g(e->device);
+    e->last = {};  // until this search is enqueued, there are no spectra refinement or profile could use
+    if ((rc = set_selection(e, sel, n_sel)) || (rc = ensure_scratch(e, n_captures, true, m))) return rc;
+    const int n_dop = m.dops(e);
+    const size_t bytes = (size_t)n_captures * e->prm.k_noncoh * e->block_bytes;
+    const size_t rows = (size_t)n_captures * e->n_slots;
+    const bool host_records = rows <= (size_t)kHostRecordRowsMax;
+    const long long tiles_total = (long long)rows * n_dop * e->prm.k_noncoh;
+    const bool poll = host_records && sync && !grid && !e->profiling && tiles_total <= 64LL * e->sm_count;
+    // The reference's own search -- one 1-bit block (gps/search.cpp:389-411) -- hands its 8 KiB to the front end as a
+    // kernel argument: the launch carries the bytes, nothing is staged or copied ahead of the first kernel.
+    const bool as_arg = ACQ_ARG_INPUT && !m.coherent && n_captures == 1 && e->prm.k_noncoh == 1 && e->sample_bits == 1 &&
+                        bytes == (size_t)ACQ_BLOCK_BYTES;
+    const uint8_t *src = packed;
+    if (!as_arg) {
+        if (bytes <= kStagePackedMax) {
+            memcpy(e->h_packed.p, packed, bytes);
+            src = e->h_packed.p;
+        }
+        CU(cudaMemcpyAsync(e->d_packed, src, bytes, cudaMemcpyHostToDevice, e->stream));
+    }
+    SearchMode dm = m;
+    if (m.aided) {   // from pinned memory: an asynchronous copy node ahead of the front end, even when the capture rides as an argument
+        memcpy(e->h_center.p, m.center, rows * sizeof(int32_t));
+        CU(cudaMemcpyAsync(e->d_center, e->h_center.p, rows * sizeof(int32_t), cudaMemcpyHostToDevice, e->stream));
+        dm.center = e->d_center;
+    }
+    acq_record *records_dev = host_records ? reinterpret_cast<acq_record *>(e->h_records.dev) : e->d_records.p;
+    if ((rc = enqueue_search(e, dm, e->d_packed, n_captures, records_dev, poll ? e->h_flag.dev : nullptr, e->stream,
+                             as_arg ? packed : nullptr)))
+        return rc;
+    if (!m.coherent) e->last = {n_captures, e->n_slots, e->n_l1, e->n_e1b, e->cur_slot_sat, true};
+    if (!host_records) CU(cudaMemcpyAsync(out, e->d_records, rows * sizeof(acq_record), cudaMemcpyDeviceToHost, e->stream));
+    if (grid)
+        CU(cudaMemcpyAsync(grid, e->d_cells, rows * n_dop * sizeof(acq_cell), cudaMemcpyDeviceToHost, e->stream));
+    if (!sync) {
+        CU(cudaEventRecord(e->done, e->stream));
+        e->pending = true;
+        e->pending_rows = host_records ? (int)rows : 0;
+        e->pending_out = out;
+        return ACQ_OK;
+    }
+    if (poll) {
+        if ((rc = poll_records(e, out, rows))) return rc;
+    } else {
+        CU(cudaStreamSynchronize(e->stream));
+        if (host_records) memcpy(out, e->h_records.p, rows * sizeof(acq_record));
+    }
+    e->dev_pending = false;  // this search was ordered behind the last device-path work, so that is complete too
+    return ACQ_OK;
 }
 
-int enqueue_refine(acq_engine *e, const acq_record *rec_dev, int n_records, int flags, acq_fine *out_dev,
-                   const int *slot_sat, int n_slots, cudaStream_t st)
+// completion of an acq_submit: records that the kernels left in the mapped buffer go to the caller's array
+void finish_pending(acq_engine *e)
 {
-    e->launches += launch_refine(e->d_Dp, e->d_Ep, rec_dev, e->d_sat_type, slot_sat, out_dev, n_records, n_slots,
-                                 e->prm.k_noncoh, e->nvar, e->prm.half_bin, e->ext_len, e->Q, e->n_shift, e->smax,
-                                 e->cd_div, (int)e->sats.size(), e->prm.dop_lo, e->prm.dop_hi, e->prm.thr_l1,
-                                 e->prm.thr_e1b, flags, st);
-    CU(cudaGetLastError());
+    if (e->pending_rows > 0 && e->pending_out)
+        memcpy(e->pending_out, e->h_records.p, (size_t)e->pending_rows * sizeof(acq_record));
+    e->pending = false;
+    e->pending_rows = 0;
+    e->pending_out = nullptr;
+}
+
+// Device path: packed_dev, out_dev and the centres of an aided mode are the caller's device arrays
+int search_device(acq_engine *e, const SearchMode &m, const uint8_t *packed_dev, int n_captures, const int32_t *sel,
+                  int n_sel, acq_record *out_dev, void *stream)
+{
+    int rc = check_search(e, m, packed_dev, n_captures, sel, n_sel, out_dev, true);
+    if (rc) return rc;
+    DeviceGuard g(e->device);
+    e->last = {};  // refinement and profile apply once this search is enqueued
+    if ((rc = set_selection(e, sel, n_sel)) || (rc = ensure_scratch(e, n_captures, false, m))) return rc;
+    cudaStream_t st = stream ? (cudaStream_t)stream : e->stream;
+    if ((rc = enqueue_search(e, m, packed_dev, n_captures, out_dev, nullptr, st, nullptr))) return rc;
+    if (!m.coherent) e->last = {n_captures, e->n_slots, e->n_l1, e->n_e1b, e->cur_slot_sat, false};
+    return hold_scratch(e, st);
+}
+
+// The checks of acq_refine* and acq_profile* (`what`) against the last search, after those of their own arguments.
+// The host forms take the records of a host-path search and check each one here; the device forms leave that to the
+// kernels, which write a marker row for a record that fails.
+int check_records(acq_engine *e, const acq_record *rec, int n_records, bool device, const char *what)
+{
+    if (e->pending) return fail(ACQ_ERR_ARG, "a submitted search is still pending: call acq_wait first");
+    if (device && e->last.captures <= 0)
+        return fail(ACQ_ERR_ARG, "no search whose spectra are still on the device to %s", what);
+    if (!device && (e->last.captures <= 0 || !e->last.host))
+        return fail(ACQ_ERR_ARG, "no completed host-path search to %s", what);
+    const long long rows = (long long)e->last.captures * e->last.slots;
+    if (n_records != rows) return fail(ACQ_ERR_ARG, "n_records=%d but the last search produced %lld records", n_records, rows);
+    if (device) return ACQ_OK;
+    for (int i = 0; i < n_records; i++) {
+        const acq_record &r = rec[i];
+        if (r.sat != e->sel_cache[i % e->last.slots])
+            return fail(ACQ_ERR_ARG, "record %d: sat %d is not the satellite searched in that slot", i, r.sat);
+        const int L = (e->sats[r.sat].type == ACQ_E1B) ? ACQ_LAGS_E1B : ACQ_LAGS_L1;
+        if (r.lag < 0 || r.lag >= L) return fail(ACQ_ERR_ARG, "record %d: lag %d outside 0..%d", i, r.lag, L - 1);
+        // a row that never exceeded snr 0 carries dop 0 (k_best_dop), which may lie outside an asymmetric range
+        if ((r.dop < e->prm.dop_lo || r.dop > e->prm.dop_hi) && !(r.dop == 0 && r.snr == 0.0f))
+            return fail(ACQ_ERR_ARG, "record %d: Doppler index %d outside %d..%d", i, r.dop, e->prm.dop_lo, e->prm.dop_hi);
+    }
     return ACQ_OK;
 }
 
@@ -679,126 +726,54 @@ int check_excl(int excl, int n_l1)
 // Lag-vector floats of one capture's rows (acq_b200.h: L per slot)
 size_t profile_capture_len(int n_l1, int n_e1b) { return (size_t)n_l1 * ACQ_LAGS_L1 + (size_t)n_e1b * ACQ_LAGS_E1B; }
 
-int enqueue_profile(acq_engine *e, const acq_record *rec_dev, int n_records, int flags, int excl, acq_peak2 *out_dev,
-                    float *profile_dev, const int *slot_sat, int n_slots, int n_l1, int n_e1b, cudaStream_t st)
+// The arguments refinement and profile share: the spectra and shape of the last search, the records and the flags
+template <class A>
+A last_search_args(const acq_engine *e, const acq_record *rec_dev, int flags)
 {
-    e->launches += launch_profile(e->d_Dp, e->d_Ep, e->d_tables, rec_dev, e->d_sat_type, slot_sat, out_dev, profile_dev,
-                                  n_records, n_slots, n_l1, n_e1b, e->prm.k_noncoh, e->nvar, e->prm.half_bin, e->ext_len, e->Q,
-                                  e->n_shift, e->smax, e->cd_div, (int)e->sats.size(), e->prm.dop_lo, e->prm.dop_hi,
-                                  e->prm.thr_l1, e->prm.thr_e1b, flags, excl, st);
+    A a{};
+    a.Dp = e->d_Dp;
+    a.Ep = e->d_Ep;
+    a.rec = rec_dev;
+    a.sat_type = e->d_sat_type;
+    a.slot_sat = e->last.slot_sat;
+    a.n_slots = e->last.slots;
+    a.K = e->prm.k_noncoh;
+    a.nvar = e->nvar;
+    a.half_bin = e->prm.half_bin;
+    a.ext_len = e->ext_len;
+    a.Q = e->Q;
+    a.n_shift = e->n_shift;
+    a.smax = e->smax;
+    a.cd_div = e->cd_div;
+    a.n_sats = (int)e->sats.size();
+    a.dop_lo = e->prm.dop_lo;
+    a.dop_hi = e->prm.dop_hi;
+    a.flags = flags;
+    a.thr_l1 = e->prm.thr_l1;
+    a.thr_e1b = e->prm.thr_e1b;
+    return a;
+}
+
+int enqueue_refine(acq_engine *e, const acq_record *rec_dev, int n_records, int flags, acq_fine *out_dev, cudaStream_t st)
+{
+    RefineArgs a = last_search_args<RefineArgs>(e, rec_dev, flags);
+    a.out = out_dev;
+    e->launches += launch_refine(a, n_records, st);
     CU(cudaGetLastError());
     return ACQ_OK;
 }
 
-// center (HOST, one per row) and half_width: an aided search (acq_search_aided), or NULL for the whole range
-// m_coh > 0: a coherent search (acq_search_coherent, or with center acq_search_coherent_aided), its arguments already
-// checked by check_coherent
-int search_host(acq_engine *e, const uint8_t *packed, int n_captures, const int32_t *sel, int n_sel, acq_record *out,
-                acq_cell *grid, bool sync, const int32_t *center = nullptr, int half_width = 0, int m_coh = 0)
+int enqueue_profile(acq_engine *e, const acq_record *rec_dev, int n_records, int flags, int excl, acq_peak2 *out_dev,
+                    float *profile_dev, cudaStream_t st)
 {
-    int rc = check_search_args(e, packed, n_captures, out);
-    if (rc) return rc;
-    DeviceGuard g(e->device);
-    e->last_captures = 0;  // until this search is enqueued, there are no spectra acq_refine could use
-    e->ref_captures = 0;
-    const int n_dop = search_dops(e, center, half_width, m_coh);
-    if ((rc = set_selection(e, sel, n_sel))) return rc;
-    if ((rc = check_tile_count(e, n_captures, n_dop))) return rc;
-    if ((rc = ensure_scratch(e, n_captures, e->n_slots, true, n_dop, m_coh ? coh_variants(e, m_coh) : e->nvar))) return rc;
-    if (m_coh && (rc = ensure_coh_rot(e, m_coh))) return rc;
-    const size_t bytes = (size_t)n_captures * e->prm.k_noncoh * e->block_bytes;
-    const size_t rows = (size_t)n_captures * e->n_slots;
-    if (center) {
-        if ((rc = grow(e, e->d_center, e->cap_center, rows))) return rc;
-        if (rows > e->cap_h_center) {
-            if ((rc = drain(e))) return rc;
-            if (e->h_center) CU(cudaFreeHost(e->h_center));
-            e->h_center = nullptr;
-            e->cap_h_center = 0;
-            CU(cudaHostAlloc(&e->h_center, rows * sizeof(int32_t), cudaHostAllocDefault));
-            e->cap_h_center = rows;
-        }
-    }
-    const bool host_records = rows <= (size_t)kHostRecordRowsMax;
-    const long long tiles_total = (long long)rows * n_dop * e->prm.k_noncoh;
-    const bool poll = host_records && sync && !grid && !e->profiling && tiles_total <= 64LL * e->sm_count;
-    // The reference's own search -- one 1-bit block (gps/search.cpp:389-411) -- hands its 8 KiB to the front end as a
-    // kernel argument: the launch carries the bytes, nothing is staged or copied ahead of the first kernel.
-    const bool as_arg = ACQ_ARG_INPUT && !m_coh && n_captures == 1 && e->prm.k_noncoh == 1 && e->sample_bits == 1 &&
-                        bytes == (size_t)ACQ_BLOCK_BYTES;
-    const uint8_t *src = packed;
-    if (!as_arg) {
-        if (bytes <= kStagePackedMax) {
-            memcpy(e->h_packed, packed, bytes);
-            src = e->h_packed;
-        }
-        CU(cudaMemcpyAsync(e->d_packed, src, bytes, cudaMemcpyHostToDevice, e->stream));
-    }
-    if (center) {   // from pinned memory: an asynchronous copy node ahead of the front end, even when the capture rides as an argument
-        memcpy(e->h_center, center, rows * sizeof(int32_t));
-        CU(cudaMemcpyAsync(e->d_center, e->h_center, rows * sizeof(int32_t), cudaMemcpyHostToDevice, e->stream));
-    }
-    if ((rc = enqueue_search(e, e->d_packed, n_captures, host_records ? e->dh_records : e->d_records,
-                             poll ? e->dh_flag : nullptr, e->stream, as_arg ? packed : nullptr, center ? e->d_center : nullptr,
-                             half_width, m_coh)))
-        return rc;
-    if (!m_coh) {   // a coherent search leaves spectra that refinement and profile cannot read
-        e->last_captures = n_captures;
-        set_refine_shape(e, n_captures);
-    }
-    if (!host_records) CU(cudaMemcpyAsync(out, e->d_records, rows * sizeof(acq_record), cudaMemcpyDeviceToHost, e->stream));
-    if (grid)
-        CU(cudaMemcpyAsync(grid, e->d_cells, rows * n_dop * sizeof(acq_cell), cudaMemcpyDeviceToHost, e->stream));
-    if (!sync) {
-        CU(cudaEventRecord(e->done, e->stream));
-        e->pending = true;
-        e->pending_rows = host_records ? (int)rows : 0;
-        e->pending_out = out;
-        return ACQ_OK;
-    }
-    if (poll) {
-        if ((rc = poll_records(e, out, rows))) return rc;
-    } else {
-        CU(cudaStreamSynchronize(e->stream));
-        if (host_records) memcpy(out, e->h_records, rows * sizeof(acq_record));
-    }
-    e->dev_pending = false;  // this search was ordered behind the last device-path search, so that one is complete too
-    return ACQ_OK;
-}
-
-// completion of an acq_submit: records that the kernels left in the mapped buffer go to the caller's array
-void finish_pending(acq_engine *e)
-{
-    if (e->pending_rows > 0 && e->pending_out)
-        memcpy(e->pending_out, e->h_records, (size_t)e->pending_rows * sizeof(acq_record));
-    e->pending = false;
-    e->pending_rows = 0;
-    e->pending_out = nullptr;
-}
-
-// acq_search_device and acq_search_aided_device (center_dev != NULL); with m_coh > 0 their coherent forms
-int search_device(acq_engine *e, const uint8_t *packed_dev, int n_captures, const int32_t *sel, int n_sel,
-                  acq_record *out_dev, void *stream, const int *center_dev = nullptr, int half_width = 0, int m_coh = 0)
-{
-    int rc = check_search_args(e, packed_dev, n_captures, out_dev);
-    if (rc) return rc;
-    if (((uintptr_t)packed_dev & 15) != 0)
-        return fail(ACQ_ERR_ARG, "packed_dev must be 16-byte aligned (the front end stages it with bulk async copies)");
-    DeviceGuard g(e->device);
-    e->last_captures = 0;  // spectra now belong to a search on the caller's stream: acq_refine does not apply
-    e->ref_captures = 0;   // ... and acq_refine_device applies once this search is enqueued
-    const int n_dop = search_dops(e, center_dev, half_width, m_coh);
-    if ((rc = set_selection(e, sel, n_sel))) return rc;
-    if ((rc = check_tile_count(e, n_captures, n_dop))) return rc;
-    if ((rc = ensure_scratch(e, n_captures, e->n_slots, false, n_dop, m_coh ? coh_variants(e, m_coh) : e->nvar))) return rc;
-    if (m_coh && (rc = ensure_coh_rot(e, m_coh))) return rc;
-    cudaStream_t st = stream ? (cudaStream_t)stream : e->stream;
-    if ((rc = enqueue_search(e, packed_dev, n_captures, out_dev, nullptr, st, nullptr, center_dev, half_width, m_coh))) return rc;
-    if (!m_coh) set_refine_shape(e, n_captures);
-    if (st != e->stream) {  // whatever uses the engine's scratch next (any stream, or the host) waits for this search
-        CU(cudaEventRecord(e->dev_done, st));
-        e->dev_pending = true;
-    }
+    ProfileArgs a = last_search_args<ProfileArgs>(e, rec_dev, flags);
+    a.tables = e->d_tables;
+    a.out = out_dev;
+    a.profile = profile_dev;
+    a.n_e1b_slots = e->last.n_e1b;
+    a.excl = excl;
+    e->launches += launch_profile(a, n_records, e->last.n_l1, st);
+    CU(cudaGetLastError());
     return ACQ_OK;
 }
 
@@ -891,7 +866,7 @@ int acq_create(acq_engine **out, const acq_params *params, const acq_sat *sats, 
                     prop.major, prop.minor);
 
     DeviceGuard g(device);
-    acq_engine *e = new acq_engine;
+    std::unique_ptr<acq_engine> e(new acq_engine);   // freed on every error return below
     e->device = device;
     e->sm_count = prop.multiProcessorCount;
     e->sm_clock_khz = prop.clockRate;
@@ -907,28 +882,16 @@ int acq_create(acq_engine **out, const acq_params *params, const acq_sat *sats, 
     e->Q = max_bins / 4 + 2;
     e->ext_len = kSub + 2 * e->Q;
 
-#define CUE(call)                                                                                   \
-    do {                                                                                            \
-        cudaError_t _e = (call);                                                                    \
-        if (_e != cudaSuccess) {                                                                    \
-            fail(ACQ_ERR_CUDA, "%s:%d %s: %s", __FILE__, __LINE__, #call, cudaGetErrorString(_e)); \
-            free_engine(e);                                                                         \
-            return ACQ_ERR_CUDA;                                                                    \
-        }                                                                                           \
-    } while (0)
-
-    CUE(cudaStreamCreateWithFlags(&e->stream, cudaStreamNonBlocking));
-    CUE(cudaEventCreateWithFlags(&e->done, cudaEventDisableTiming));
-    CUE(cudaEventCreateWithFlags(&e->dev_done, cudaEventDisableTiming));
-    CUE(search_kernels_configure());
+    CU(cudaStreamCreateWithFlags(&e->stream, cudaStreamNonBlocking));
+    CU(cudaEventCreateWithFlags(&e->done, cudaEventDisableTiming));
+    CU(cudaEventCreateWithFlags(&e->dev_done, cudaEventDisableTiming));
+    CU(search_kernels_configure());
     // completion counter of small searches, mapped completion word
-    CUE(cudaMalloc(&e->d_ctas_done, sizeof(unsigned)));
-    CUE(cudaMemset(e->d_ctas_done, 0, sizeof(unsigned)));
-    CUE(cudaMalloc(&e->d_tile_ctr, 4 * sizeof(unsigned)));
-    CUE(cudaMemset(e->d_tile_ctr, 0, 4 * sizeof(unsigned)));
-    CUE(cudaHostAlloc(&e->h_flag, sizeof(unsigned), cudaHostAllocMapped));
-    *e->h_flag = 0;
-    CUE(cudaHostGetDevicePointer(&e->dh_flag, e->h_flag, 0));
+    CU(e->d_ctas_done.alloc(1));
+    CU(cudaMemset(e->d_ctas_done, 0, sizeof(unsigned)));
+    CU(e->d_tile_ctr.alloc(4));
+    CU(cudaMemset(e->d_tile_ctr, 0, 4 * sizeof(unsigned)));
+    CU(e->h_flag.alloc(1));
     {   // work lists that need no upload: the whole table (C/A rows first, then E1B) and every single satellite
         std::vector<int2> full, single(n_sats);
         std::vector<int> ident(n_sats);
@@ -943,12 +906,9 @@ int acq_create(acq_engine **out, const acq_params *params, const acq_sat *sats, 
             single[i] = make_int2(i, 0);
             ident[i] = i;
         }
-        CUE(cudaMalloc(&e->d_work_full, n_sats * sizeof(int2)));
-        CUE(cudaMalloc(&e->d_work_single, n_sats * sizeof(int2)));
-        CUE(cudaMalloc(&e->d_sat_full, n_sats * sizeof(int)));
-        CUE(cudaMemcpy(e->d_work_full, full.data(), n_sats * sizeof(int2), cudaMemcpyHostToDevice));
-        CUE(cudaMemcpy(e->d_work_single, single.data(), n_sats * sizeof(int2), cudaMemcpyHostToDevice));
-        CUE(cudaMemcpy(e->d_sat_full, ident.data(), n_sats * sizeof(int), cudaMemcpyHostToDevice));
+        CU(upload(e->d_work_full, full));
+        CU(upload(e->d_work_single, single));
+        CU(upload(e->d_sat_full, ident));
     }
 
     // ---- twiddle tables, constants (double precision on the host, rounded once)
@@ -979,25 +939,14 @@ int acq_create(acq_engine **out, const acq_params *params, const acq_sat *sats, 
     float hb[17];
     for (int i = 0; i < 16; i++) hb[i] = (float)taps_even[i];
     hb[16] = (float)0.500009;
-    CUE(launch_tables_init(cC, hb));
-    CUE(cudaMalloc(&e->d_tables, tables.size() * sizeof(float2)));
-    CUE(cudaMemcpy(e->d_tables, tables.data(), tables.size() * sizeof(float2), cudaMemcpyHostToDevice));
+    CU(launch_tables_init(cC, hb));
+    CU(upload(e->d_tables, tables));
     {
         std::vector<int> types(n_sats);
         for (int i = 0; i < n_sats; i++) types[i] = sats[i].type;
-        CUE(cudaMalloc(&e->d_sat_type, n_sats * sizeof(int)));
-        CUE(cudaMemcpy(e->d_sat_type, types.data(), n_sats * sizeof(int), cudaMemcpyHostToDevice));
+        CU(upload(e->d_sat_type, types));
     }
-    if (e->nvar == 2) {
-        const double pi = 3.14159265358979323846264338327950288;
-        std::vector<float2> rot(kN);
-        for (int n = 0; n < kN; n++) {
-            const double a = pi * (double)n / (double)kN;
-            rot[n] = make_float2((float)cos(a), (float)(-sin(a)));
-        }
-        CUE(cudaMalloc(&e->d_rot, kN * sizeof(float2)));
-        CUE(cudaMemcpy(e->d_rot, rot.data(), kN * sizeof(float2), cudaMemcpyHostToDevice));
-    }
+    if (e->nvar == 2) CU(upload(e->d_rot, rotation_table(2, 1)));   // the half-bin rotation exp(-i pi n / N)
 
     // ---- code spectra (replaces the loops at gps/search.cpp:243-346)
     std::vector<uint32_t> chips((size_t)n_sats * 128);
@@ -1015,110 +964,93 @@ int acq_create(acq_engine **out, const acq_params *params, const acq_sat *sats, 
             codelen_boc[2 * i + 1] = 0;
         }
     }
-    uint32_t *d_chips = nullptr;
-    int *d_clb = nullptr;
-    float2 *d_x1 = nullptr, *d_x2 = nullptr;
-    cudaError_t ce = cudaSuccess;
-    do {
-        if ((ce = cudaMalloc(&d_chips, chips.size() * sizeof(uint32_t)))) break;
-        if ((ce = cudaMalloc(&d_clb, codelen_boc.size() * sizeof(int)))) break;
-        if ((ce = cudaMalloc(&d_x1, (size_t)n_sats * 32768 * sizeof(float2)))) break;
-        if ((ce = cudaMalloc(&d_x2, (size_t)n_sats * kN * sizeof(float2)))) break;
-        if ((ce = cudaMalloc(&e->d_C, (size_t)n_sats * kN * sizeof(float2)))) break;
-        if ((ce = cudaMalloc(&e->d_Ep, (size_t)n_sats * 4 * e->ext_len * sizeof(float2)))) break;
-        if ((ce = cudaMemcpy(d_chips, chips.data(), chips.size() * sizeof(uint32_t), cudaMemcpyHostToDevice))) break;
-        if ((ce = cudaMemcpy(d_clb, codelen_boc.data(), codelen_boc.size() * sizeof(int), cudaMemcpyHostToDevice)))
-            break;
-        e->launches += launch_hb1_code(d_chips, d_clb, d_x1, n_sats, e->stream);
-        e->launches += launch_hb2(d_x1, d_x2, nullptr, n_sats, 1, 1, e->stream);
-        e->launches += launch_fwd_fft(d_x2, e->d_C, e->d_tables, n_sats, false, e->sm_count, e->stream);
-        e->launches += launch_build_ext(e->d_C, e->d_Ep, n_sats, e->Q, e->ext_len, prm.wrap_mode, e->stream);
-        if ((ce = cudaGetLastError())) break;
-        ce = cudaStreamSynchronize(e->stream);
-    } while (0);
-    cudaFree(d_chips);
-    cudaFree(d_clb);
-    cudaFree(d_x1);
-    cudaFree(d_x2);
-    CUE(ce);
-#undef CUE
-    *out = e;
+    DevBuf<uint32_t> d_chips;
+    DevBuf<int> d_clb;
+    DevBuf<float2> d_x1, d_x2;
+    CU(upload(d_chips, chips));
+    CU(upload(d_clb, codelen_boc));
+    CU(d_x1.alloc((size_t)n_sats * 32768));
+    CU(d_x2.alloc((size_t)n_sats * kN));
+    CU(e->d_C.alloc((size_t)n_sats * kN));
+    CU(e->d_Ep.alloc((size_t)n_sats * 4 * e->ext_len));
+    e->launches += launch_hb1_code(d_chips, d_clb, d_x1, n_sats, e->stream);
+    e->launches += launch_hb2(d_x1, d_x2, nullptr, n_sats, 1, 1, e->stream);
+    e->launches += launch_fwd_fft(d_x2, e->d_C, e->d_tables, n_sats, false, e->sm_count, e->stream);
+    e->launches += launch_build_ext(e->d_C, e->d_Ep, n_sats, e->Q, e->ext_len, prm.wrap_mode, e->stream);
+    CU(cudaGetLastError());
+    CU(cudaStreamSynchronize(e->stream));
+    *out = e.release();
     return ACQ_OK;
 }
 
-int acq_destroy(acq_engine *e) { return free_engine(e); }
+int acq_destroy(acq_engine *e)
+{
+    if (e) {
+        DeviceGuard g(e->device);   // the engine's memory is freed under its own device
+        delete e;
+    }
+    return ACQ_OK;
+}
 
 int acq_search(acq_engine *e, const uint8_t *packed, int n_captures, const int32_t *sel, int n_sel, acq_record *out)
 {
-    return search_host(e, packed, n_captures, sel, n_sel, out, nullptr, true);
+    return search_host(e, kFullRange, packed, n_captures, sel, n_sel, out, nullptr, true);
 }
 
 int acq_search_grid(acq_engine *e, const uint8_t *packed, int n_captures, const int32_t *sel, int n_sel,
                     acq_record *out, acq_cell *grid)
 {
     if (!grid) return fail(ACQ_ERR_ARG, "grid is NULL");
-    return search_host(e, packed, n_captures, sel, n_sel, out, grid, true);
+    return search_host(e, kFullRange, packed, n_captures, sel, n_sel, out, grid, true);
 }
 
 int acq_search_aided(acq_engine *e, const uint8_t *packed, int n_captures, const int32_t *sel, int n_sel,
                      const int32_t *dop_center, int half_width, acq_record *out, acq_cell *grid)
 {
-    const int rc = check_aided_args(e, dop_center, half_width);
-    if (rc) return rc;
-    return search_host(e, packed, n_captures, sel, n_sel, out, grid, true, dop_center, half_width);
+    return search_host(e, {true, false, dop_center, half_width, 0}, packed, n_captures, sel, n_sel, out, grid, true);
 }
 
 int acq_search_device(acq_engine *e, const uint8_t *packed_dev, int n_captures, const int32_t *sel, int n_sel,
                       acq_record *out_dev, void *stream)
 {
-    return search_device(e, packed_dev, n_captures, sel, n_sel, out_dev, stream);
+    return search_device(e, kFullRange, packed_dev, n_captures, sel, n_sel, out_dev, stream);
 }
 
 int acq_search_aided_device(acq_engine *e, const uint8_t *packed_dev, int n_captures, const int32_t *sel, int n_sel,
                             const int32_t *dop_center_dev, int half_width, acq_record *out_dev, void *stream)
 {
-    const int rc = check_aided_args(e, dop_center_dev, half_width);
-    if (rc) return rc;
-    return search_device(e, packed_dev, n_captures, sel, n_sel, out_dev, stream, dop_center_dev, half_width);
+    return search_device(e, {true, false, dop_center_dev, half_width, 0}, packed_dev, n_captures, sel, n_sel, out_dev, stream);
 }
 
 int acq_search_coherent(acq_engine *e, const uint8_t *packed, int n_captures, const int32_t *sel, int n_sel, int m_coh,
                         acq_record *out, acq_cell *grid)
 {
-    const int rc = check_coherent(e, packed, n_captures, sel, n_sel, m_coh, out);
-    if (rc) return rc;
-    return search_host(e, packed, n_captures, sel, n_sel, out, grid, true, nullptr, 0, m_coh);
+    return search_host(e, {false, true, nullptr, 0, m_coh}, packed, n_captures, sel, n_sel, out, grid, true);
 }
 
 int acq_search_coherent_device(acq_engine *e, const uint8_t *packed_dev, int n_captures, const int32_t *sel, int n_sel,
                                int m_coh, acq_record *out_dev, void *stream)
 {
-    const int rc = check_coherent(e, packed_dev, n_captures, sel, n_sel, m_coh, out_dev);
-    if (rc) return rc;
-    return search_device(e, packed_dev, n_captures, sel, n_sel, out_dev, stream, nullptr, 0, m_coh);
+    return search_device(e, {false, true, nullptr, 0, m_coh}, packed_dev, n_captures, sel, n_sel, out_dev, stream);
 }
 
 int acq_search_coherent_aided(acq_engine *e, const uint8_t *packed, int n_captures, const int32_t *sel, int n_sel,
                               int m_coh, const int32_t *dop_center, int half_width, acq_record *out, acq_cell *grid)
 {
-    int rc = check_coherent_aided_args(e, dop_center, half_width, m_coh);
-    if (rc || (rc = check_coherent(e, packed, n_captures, sel, n_sel, m_coh, out, dop_center, half_width))) return rc;
-    return search_host(e, packed, n_captures, sel, n_sel, out, grid, true, dop_center, half_width, m_coh);
+    return search_host(e, {true, true, dop_center, half_width, m_coh}, packed, n_captures, sel, n_sel, out, grid, true);
 }
 
 int acq_search_coherent_aided_device(acq_engine *e, const uint8_t *packed_dev, int n_captures, const int32_t *sel,
                                      int n_sel, int m_coh, const int32_t *dop_center_dev, int half_width,
                                      acq_record *out_dev, void *stream)
 {
-    int rc = check_coherent_aided_args(e, dop_center_dev, half_width, m_coh);
-    if (rc || (rc = check_coherent(e, packed_dev, n_captures, sel, n_sel, m_coh, out_dev, dop_center_dev, half_width)))
-        return rc;
-    return search_device(e, packed_dev, n_captures, sel, n_sel, out_dev, stream, dop_center_dev, half_width, m_coh);
+    return search_device(e, {true, true, dop_center_dev, half_width, m_coh}, packed_dev, n_captures, sel, n_sel, out_dev,
+                         stream);
 }
 
 int acq_submit(acq_engine *e, const uint8_t *packed, int n_captures, const int32_t *sel, int n_sel, acq_record *out)
 {
-    return search_host(e, packed, n_captures, sel, n_sel, out, nullptr, false);
+    return search_host(e, kFullRange, packed, n_captures, sel, n_sel, out, nullptr, false);
 }
 
 int acq_poll(acq_engine *e)
@@ -1154,28 +1086,13 @@ int acq_refine(acq_engine *e, const acq_record *rec, int n_records, acq_fine *ou
 {
     if (!e) return fail(ACQ_ERR_ARG, "engine is NULL");
     if (!rec || !out) return fail(ACQ_ERR_ARG, "rec/out must not be NULL");
-    if (e->pending) return fail(ACQ_ERR_ARG, "a submitted search is still pending: call acq_wait first");
-    if (e->last_captures <= 0) return fail(ACQ_ERR_ARG, "no completed host-path search to refine");
-    const long long rows = (long long)e->last_captures * e->n_slots;
-    if (n_records != rows)
-        return fail(ACQ_ERR_ARG, "n_records=%d but the last search produced %lld records", n_records, rows);
-    for (int i = 0; i < n_records; i++) {
-        const acq_record &r = rec[i];
-        if (r.sat != e->sel_cache[i % e->n_slots])
-            return fail(ACQ_ERR_ARG, "record %d: sat %d is not the satellite searched in that slot", i, r.sat);
-        const int L = (e->sats[r.sat].type == ACQ_E1B) ? ACQ_LAGS_E1B : ACQ_LAGS_L1;
-        if (r.lag < 0 || r.lag >= L) return fail(ACQ_ERR_ARG, "record %d: lag %d outside 0..%d", i, r.lag, L - 1);
-        // a row that never exceeded snr 0 carries dop 0 (k_best_dop), which may lie outside an asymmetric range
-        if ((r.dop < e->prm.dop_lo || r.dop > e->prm.dop_hi) && !(r.dop == 0 && r.snr == 0.0f))
-            return fail(ACQ_ERR_ARG, "record %d: Doppler index %d outside %d..%d", i, r.dop, e->prm.dop_lo, e->prm.dop_hi);
-    }
-    DeviceGuard g(e->device);
-    int rc = grow(e, e->d_ref_rec, e->cap_ref_rec, (size_t)n_records);
+    int rc = check_records(e, rec, n_records, false, "refine");
     if (rc) return rc;
-    if ((rc = grow(e, e->d_fine, e->cap_fine, (size_t)n_records))) return rc;
+    DeviceGuard g(e->device);
+    if ((rc = grow(e, e->d_ref_rec, (size_t)n_records)) || (rc = grow(e, e->d_fine, (size_t)n_records))) return rc;
     CU(cudaMemcpyAsync(e->d_ref_rec, rec, (size_t)n_records * sizeof(acq_record), cudaMemcpyHostToDevice, e->stream));
     // the records are checked above, so the kernel's own checks pass every row
-    if ((rc = enqueue_refine(e, e->d_ref_rec, n_records, 0, e->d_fine, e->cur_slot_sat, e->n_slots, e->stream))) return rc;
+    if ((rc = enqueue_refine(e, e->d_ref_rec, n_records, 0, e->d_fine, e->stream))) return rc;
     CU(cudaMemcpyAsync(out, e->d_fine, (size_t)n_records * sizeof(acq_fine), cudaMemcpyDeviceToHost, e->stream));
     CU(cudaStreamSynchronize(e->stream));
     return ACQ_OK;
@@ -1186,29 +1103,15 @@ int acq_refine_device(acq_engine *e, const acq_record *rec_dev, int n_records, i
     if (!e) return fail(ACQ_ERR_ARG, "engine is NULL");
     if (!rec_dev || !out_dev) return fail(ACQ_ERR_ARG, "rec_dev/out_dev must not be NULL");
     if (flags & ~ACQ_REFINE_DETECTED) return fail(ACQ_ERR_ARG, "unknown flag bits 0x%x", (unsigned)(flags & ~ACQ_REFINE_DETECTED));
-    if (e->ref_captures <= 0) return fail(ACQ_ERR_ARG, "no search whose spectra are still on the device to refine");
-    if (e->pending) return fail(ACQ_ERR_ARG, "a submitted search is still pending: call acq_wait first");
-    const long long rows = (long long)e->ref_captures * e->ref_slots;
-    if (n_records != rows)
-        return fail(ACQ_ERR_ARG, "n_records=%d but the last search produced %lld records", n_records, rows);
+    int rc = check_records(e, rec_dev, n_records, true, "refine");
+    if (rc) return rc;
     if (((uintptr_t)out_dev & 15) != 0) return fail(ACQ_ERR_ARG, "out_dev must be 16-byte aligned (one 16-byte store per row)");
     if (((uintptr_t)rec_dev & 3) != 0) return fail(ACQ_ERR_ARG, "rec_dev must be 4-byte aligned");
     DeviceGuard g(e->device);
     cudaStream_t st = stream ? (cudaStream_t)stream : e->stream;
-    // after the search that left the spectra: a device-path search on another stream is behind dev_done, anything
-    // else on the engine stream
-    if (e->dev_pending) CU(cudaStreamWaitEvent(st, e->dev_done, 0));
-    if (st != e->stream) {
-        CU(cudaEventRecord(e->dev_done, e->stream));
-        CU(cudaStreamWaitEvent(st, e->dev_done, 0));
-    }
-    int rc = enqueue_refine(e, rec_dev, n_records, flags, out_dev, e->ref_slot_sat, e->ref_slots, st);
-    if (rc) return rc;
-    if (st != e->stream) {  // the next search overwrites the spectra: whatever touches the scratch next waits for this
-        CU(cudaEventRecord(e->dev_done, st));
-        e->dev_pending = true;
-    }
-    return ACQ_OK;
+    // after the search that left the spectra (on any stream), before the next search overwrites them
+    if ((rc = wait_scratch(e, st, true)) || (rc = enqueue_refine(e, rec_dev, n_records, flags, out_dev, st))) return rc;
+    return hold_scratch(e, st);
 }
 
 int acq_profile(acq_engine *e, const acq_record *rec, int n_records, int excl, acq_peak2 *out, float *profile)
@@ -1216,26 +1119,11 @@ int acq_profile(acq_engine *e, const acq_record *rec, int n_records, int excl, a
     if (!e) return fail(ACQ_ERR_ARG, "engine is NULL");
     if (!rec || !out) return fail(ACQ_ERR_ARG, "rec/out must not be NULL");
     if (excl < 0) return fail(ACQ_ERR_ARG, "excl must be >= 0 (got %d)", excl);
-    if (e->pending) return fail(ACQ_ERR_ARG, "a submitted search is still pending: call acq_wait first");
-    if (e->last_captures <= 0) return fail(ACQ_ERR_ARG, "no completed host-path search to profile");
-    const long long rows = (long long)e->last_captures * e->n_slots;
-    if (n_records != rows)
-        return fail(ACQ_ERR_ARG, "n_records=%d but the last search produced %lld records", n_records, rows);
-    int rc = check_excl(excl, e->n_l1);
-    if (rc) return rc;
-    for (int i = 0; i < n_records; i++) {   // acq_refine's checks
-        const acq_record &r = rec[i];
-        if (r.sat != e->sel_cache[i % e->n_slots])
-            return fail(ACQ_ERR_ARG, "record %d: sat %d is not the satellite searched in that slot", i, r.sat);
-        const int L = (e->sats[r.sat].type == ACQ_E1B) ? ACQ_LAGS_E1B : ACQ_LAGS_L1;
-        if (r.lag < 0 || r.lag >= L) return fail(ACQ_ERR_ARG, "record %d: lag %d outside 0..%d", i, r.lag, L - 1);
-        if ((r.dop < e->prm.dop_lo || r.dop > e->prm.dop_hi) && !(r.dop == 0 && r.snr == 0.0f))
-            return fail(ACQ_ERR_ARG, "record %d: Doppler index %d outside %d..%d", i, r.dop, e->prm.dop_lo, e->prm.dop_hi);
-    }
+    int rc = check_records(e, rec, n_records, false, "profile");
+    if (rc || (rc = check_excl(excl, e->last.n_l1))) return rc;
     DeviceGuard g(e->device);
-    const size_t n_prof = (size_t)e->last_captures * profile_capture_len(e->n_l1, e->n_e1b);
-    if ((rc = grow(e, e->d_ref_rec, e->cap_ref_rec, (size_t)n_records))) return rc;
-    if ((rc = grow(e, e->d_peak2, e->cap_peak2, (size_t)n_records))) return rc;
+    const size_t n_prof = (size_t)e->last.captures * profile_capture_len(e->last.n_l1, e->last.n_e1b);
+    if ((rc = grow(e, e->d_ref_rec, (size_t)n_records)) || (rc = grow(e, e->d_peak2, (size_t)n_records))) return rc;
     // The lag profiles (512 MiB for a 1024-capture C/A search) live only for this call: the engine keeps no buffer of
     // that size.  The buffer is freed after the engine stream has passed every use of it, on the error paths too.
     struct CallBuffer {
@@ -1252,9 +1140,7 @@ int acq_profile(acq_engine *e, const acq_record *rec, int n_records, int excl, a
     if (profile) CU(cudaMalloc(&d_prof.p, n_prof * sizeof(float)));
     CU(cudaMemcpyAsync(e->d_ref_rec, rec, (size_t)n_records * sizeof(acq_record), cudaMemcpyHostToDevice, e->stream));
     // the records are checked above, so the kernel's own checks pass every row
-    if ((rc = enqueue_profile(e, e->d_ref_rec, n_records, 0, excl, e->d_peak2, d_prof.p,
-                              e->cur_slot_sat, e->n_slots, e->n_l1, e->n_e1b, e->stream)))
-        return rc;
+    if ((rc = enqueue_profile(e, e->d_ref_rec, n_records, 0, excl, e->d_peak2, d_prof.p, e->stream))) return rc;
     CU(cudaMemcpyAsync(out, e->d_peak2, (size_t)n_records * sizeof(acq_peak2), cudaMemcpyDeviceToHost, e->stream));
     if (profile) CU(cudaMemcpyAsync(profile, d_prof.p, n_prof * sizeof(float), cudaMemcpyDeviceToHost, e->stream));
     CU(cudaStreamSynchronize(e->stream));
@@ -1268,32 +1154,17 @@ int acq_profile_device(acq_engine *e, const acq_record *rec_dev, int n_records, 
     if (!rec_dev || !out_dev) return fail(ACQ_ERR_ARG, "rec_dev/out_dev must not be NULL");
     if (flags & ~ACQ_PROFILE_DETECTED) return fail(ACQ_ERR_ARG, "unknown flag bits 0x%x", (unsigned)(flags & ~ACQ_PROFILE_DETECTED));
     if (excl < 0) return fail(ACQ_ERR_ARG, "excl must be >= 0 (got %d)", excl);
-    if (e->ref_captures <= 0) return fail(ACQ_ERR_ARG, "no search whose spectra are still on the device to profile");
-    if (e->pending) return fail(ACQ_ERR_ARG, "a submitted search is still pending: call acq_wait first");
-    const long long rows = (long long)e->ref_captures * e->ref_slots;
-    if (n_records != rows)
-        return fail(ACQ_ERR_ARG, "n_records=%d but the last search produced %lld records", n_records, rows);
-    int rc = check_excl(excl, e->ref_n_l1);
-    if (rc) return rc;
+    int rc = check_records(e, rec_dev, n_records, true, "profile");
+    if (rc || (rc = check_excl(excl, e->last.n_l1))) return rc;
     if (((uintptr_t)out_dev & 15) != 0) return fail(ACQ_ERR_ARG, "out_dev must be 16-byte aligned (one 16-byte store per row)");
     if (((uintptr_t)rec_dev & 3) != 0) return fail(ACQ_ERR_ARG, "rec_dev must be 4-byte aligned");
     if (((uintptr_t)profile_dev & 3) != 0) return fail(ACQ_ERR_ARG, "profile_dev must be 4-byte aligned");
     DeviceGuard g(e->device);
     cudaStream_t st = stream ? (cudaStream_t)stream : e->stream;
     // ordered as acq_refine_device: after the search that left the spectra, before the next one
-    if (e->dev_pending) CU(cudaStreamWaitEvent(st, e->dev_done, 0));
-    if (st != e->stream) {
-        CU(cudaEventRecord(e->dev_done, e->stream));
-        CU(cudaStreamWaitEvent(st, e->dev_done, 0));
-    }
-    if ((rc = enqueue_profile(e, rec_dev, n_records, flags, excl, out_dev, profile_dev, e->ref_slot_sat, e->ref_slots,
-                              e->ref_n_l1, e->ref_n_e1b, st)))
+    if ((rc = wait_scratch(e, st, true)) || (rc = enqueue_profile(e, rec_dev, n_records, flags, excl, out_dev, profile_dev, st)))
         return rc;
-    if (st != e->stream) {
-        CU(cudaEventRecord(e->dev_done, st));
-        e->dev_pending = true;
-    }
-    return ACQ_OK;
+    return hold_scratch(e, st);
 }
 
 int acq_detected(const acq_engine *e, const acq_record *r)
@@ -1318,42 +1189,22 @@ int acq_get_capture_spectrum(acq_engine *e, const uint8_t *packed, int half_rot,
     if (half_rot != 0 && half_rot != 1) return fail(ACQ_ERR_ARG, "half_rot must be 0 or 1");
     if (e->pending) return fail(ACQ_ERR_ARG, "a submitted search is still pending");
     DeviceGuard g(e->device);
-    uint8_t *d_pk = nullptr;
-    float2 *d_x2 = nullptr, *d_D = nullptr, *d_rot = nullptr;
-    std::vector<float2> rot;
-    int rc = ACQ_OK;
-    cudaError_t ce = cudaSuccess;
-    do {
-        if ((ce = cudaMalloc(&d_pk, e->block_bytes))) break;
-        if ((ce = cudaMalloc(&d_x2, 2 * kN * sizeof(float2)))) break;
-        if ((ce = cudaMalloc(&d_D, kN * sizeof(float2)))) break;
-        if ((ce = cudaMemcpy(d_pk, packed, e->block_bytes, cudaMemcpyHostToDevice))) break;
-        const float2 *rotp = e->d_rot;
-        if (half_rot && !rotp) {
-            const double pi = 3.14159265358979323846264338327950288;
-            rot.resize(kN);
-            for (int n = 0; n < kN; n++) {
-                const double a = pi * (double)n / (double)kN;
-                rot[n] = make_float2((float)cos(a), (float)(-sin(a)));
-            }
-            if ((ce = cudaMalloc(&d_rot, kN * sizeof(float2)))) break;
-            if ((ce = cudaMemcpy(d_rot, rot.data(), kN * sizeof(float2), cudaMemcpyHostToDevice))) break;
-            rotp = d_rot;
-        }
-        e->launches += launch_front_end(d_pk, d_x2, rotp, 1, half_rot ? 2 : 1, 1, e->sample_bits, 1, 0, e->stream);
-        const float2 *sel_x2 = d_x2 + (half_rot ? kN : 0);
-        e->launches += launch_fwd_fft(sel_x2, d_D, e->d_tables, 1, false, e->sm_count, e->stream);
-        if ((ce = cudaGetLastError())) break;
-        if ((ce = cudaStreamSynchronize(e->stream))) break;
-        if (x2 && (ce = cudaMemcpy(x2, sel_x2, kN * sizeof(float2), cudaMemcpyDeviceToHost))) break;
-        if (D && (ce = cudaMemcpy(D, d_D, kN * sizeof(float2), cudaMemcpyDeviceToHost))) break;
-    } while (0);
-    cudaFree(d_pk);
-    cudaFree(d_x2);
-    cudaFree(d_D);
-    cudaFree(d_rot);
-    if (ce != cudaSuccess) rc = fail(ACQ_ERR_CUDA, "acq_get_capture_spectrum: %s", cudaGetErrorString(ce));
-    return rc;
+    DevBuf<uint8_t> d_pk;
+    DevBuf<float2> d_x2, d_D, d_rot;
+    CU(d_pk.alloc(e->block_bytes));
+    CU(d_x2.alloc(2 * kN));
+    CU(d_D.alloc(kN));
+    CU(cudaMemcpy(d_pk, packed, e->block_bytes, cudaMemcpyHostToDevice));
+    if (half_rot && !e->d_rot) CU(upload(d_rot, rotation_table(2, 1)));
+    const float2 *rotp = e->d_rot ? e->d_rot : d_rot;
+    e->launches += launch_front_end(d_pk, d_x2, rotp, 1, half_rot ? 2 : 1, 1, e->sample_bits, 1, 0, e->stream);
+    const float2 *sel_x2 = d_x2 + (half_rot ? kN : 0);
+    e->launches += launch_fwd_fft(sel_x2, d_D, e->d_tables, 1, false, e->sm_count, e->stream);
+    CU(cudaGetLastError());
+    CU(cudaStreamSynchronize(e->stream));
+    if (x2) CU(cudaMemcpy(x2, sel_x2, kN * sizeof(float2), cudaMemcpyDeviceToHost));
+    if (D) CU(cudaMemcpy(D, d_D, kN * sizeof(float2), cudaMemcpyDeviceToHost));
+    return ACQ_OK;
 }
 
 int acq_n_sats(const acq_engine *e) { return e ? (int)e->sats.size() : fail(ACQ_ERR_ARG, "engine is NULL"); }
@@ -1372,9 +1223,7 @@ int acq_plan_launch(int k_noncoh, int half_bin, int e1b, int64_t n_tiles, int sm
     if (!out || k_noncoh < 1 || sm_count < 1 || n_tiles < 1 || n_tiles > acq::kMaxTilesPerLaunch)
         return fail(ACQ_ERR_ARG, "acq_plan_launch: bad argument");
     memset(out, 0, sizeof *out);
-    int kind;
-    if (e1b) kind = (ACQ_FORCE_E1B_KERNEL == 2 || (ACQ_FORCE_E1B_KERNEL == 0 && n_tiles <= sm_count / 4)) ? acq::kSearchE1bCluster : acq::kSearchE1b;
-    else kind = acq::search_kind_l1(k_noncoh, half_bin);
+    const int kind = e1b ? acq::search_kind_e1b(n_tiles, sm_count) : acq::search_kind_l1(k_noncoh, half_bin);
     out->kernel = kind;
     out->grid = acq::search_grid_ctas(n_tiles, kind, sm_count);
     out->claims = kind != acq::kSearchE1bCluster && acq::search_claims_tiles(n_tiles, out->grid);

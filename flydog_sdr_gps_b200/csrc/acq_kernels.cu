@@ -13,6 +13,7 @@
 // The half-band stages use explicit round-to-nearest mul/add in the reference's summation order
 // (no FMA contraction), so the FFT inputs are bit-identical to the reference's x86 build.
 #include <cooperative_groups.h>
+#include <type_traits>
 
 #include "acq_fft.cuh"
 #include "acq_kernels.cuh"
@@ -2151,18 +2152,6 @@ __global__ void __launch_bounds__(256, 2) k_search_e1b_ldg(const SearchArgs p)
 // a CTA whose record fails one, or that ACQ_REFINE_DETECTED skips, writes a marker row and exits before any load of
 // the spectra (a uniform branch: every thread reads the same record).
 // ---------------------------------------------------------------------------------------------
-struct RefineArgs {
-    const float2 *Dp;
-    const float2 *Ep;
-    const acq_record *rec;   // [n_rows], row = cap * n_slots + slot
-    const int *sat_type;     // [n_sats]
-    const int *slot_sat;     // [n_slots] satellite searched in each slot
-    acq_fine *out;
-    int n_slots, K, nvar, half_bin, ext_len, Q, n_shift, smax, cd_div;
-    int n_sats, dop_lo, dop_hi, flags;
-    float thr_l1, thr_e1b;
-};
-
 __global__ void __launch_bounds__(256) k_refine(const RefineArgs p)
 {
     __shared__ float red[8][10];
@@ -2322,20 +2311,6 @@ __device__ __forceinline__ int record_marker(const acq_record &rc, const int *sl
     }
     return marker;
 }
-
-struct ProfileArgs {
-    const float2 *Dp;
-    const float2 *Ep;
-    const float2 *tables;
-    const acq_record *rec;   // [n_rows], row = cap * n_slots + slot
-    const int *sat_type;     // [n_sats]
-    const int *slot_sat;     // [n_slots] satellite searched in each slot
-    acq_peak2 *out;
-    float *profile;          // NULL, or the packed lag vectors (acq_b200.h)
-    int n_slots, n_e1b_slots, K, nvar, half_bin, ext_len, Q, n_shift, smax, cd_div;
-    int n_sats, dop_lo, dop_hi, flags, excl;
-    float thr_l1, thr_e1b;
-};
 
 constexpr size_t kProfileRedBytes = 64 * sizeof(float);                 // reduction slots, the record's power, TMEM slot
 constexpr size_t kProfilePsBytes = sizeof(float) * 64 * 256;            // E1B, K > 1: running block sums [64][256]
@@ -2519,46 +2494,68 @@ static size_t search_l1_smem_bytes() { return fft_smem4_bytes() + 64 * sizeof(fl
 static size_t search_e1b_smem_bytes() { return e1b_smem_bytes(); }
 static size_t search_e1b_cluster_smem_bytes() { return fft_smem3_bytes() + 2 * sizeof(float2) * kSub + 64 * sizeof(float); }
 static size_t fwd_smem_bytes() { return fft_smem3_bytes() + kZBytes; }
+#ifdef ACQ_VARIANT_E1B_LDG
+static size_t search_e1b_ldg_smem_bytes() { return fft_smem3_bytes() + 64 * sizeof(float); }
+#endif
 
-// The search kernels of an aided search (AidedSearchArgs): the product forms only, with the shared-memory size and carveout
-// of their full-range instantiations.
-static cudaError_t aided_kernels_configure()
+// The search kernel of argument type PA for a launch of `kind` with K > 1 (multi) or K = 1, and its dynamic shared
+// memory.  launch_search_as launches what it returns and configure_search_kernels configures what it returns for every
+// (kind, multi), so every search kernel a launch can pick is configured.
+template <class PA>
+struct SearchKernel {
+    void (*f)(PA);
+    size_t smem;
+};
+template <class PA>
+static SearchKernel<PA> search_kernel(int kind, bool multi)
 {
-    using A = AidedSearchArgs;
-    const void *k[] = {(const void *)k_search_l1<false, A>, (const void *)k_search_l1_multi<A>, (const void *)k_search_l1_cr<A>,
-                       (const void *)k_search_e1b<A>, (const void *)k_search_e1b_multi<A>, (const void *)k_search_e1b_cluster<false, A>,
-                       (const void *)k_search_e1b_cluster<true, A>};
-    const int smem[] = {(int)search_l1_smem_bytes(), (int)l1_multi_smem_bytes(), (int)l1_multi_smem_bytes(), (int)search_e1b_smem_bytes(),
-                        (int)e1b_multi_smem_bytes(), (int)search_e1b_cluster_smem_bytes(), (int)search_e1b_cluster_smem_bytes()};
-    cudaError_t e;
-    for (int i = 0; i < 7; i++) {
-        if ((e = cudaFuncSetAttribute(k[i], cudaFuncAttributeMaxDynamicSharedMemorySize, smem[i]))) return e;
-        if ((e = cudaFuncSetAttribute(k[i], cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared))) return e;
+    if constexpr (PA::kCoh) {
+        return {k_search_l1_coh<PA>, l1_multi_smem_bytes()};
+    } else {
+        switch (kind) {
+        case kSearchE1bCluster:
+            return {multi ? k_search_e1b_cluster<true, PA> : k_search_e1b_cluster<false, PA>, search_e1b_cluster_smem_bytes()};
+        case kSearchE1b:
+            if (multi) return {k_search_e1b_multi<PA>, e1b_multi_smem_bytes()};
+            return {k_search_e1b<PA>, search_e1b_smem_bytes()};
+        case kSearchL1Multi: return {k_search_l1_multi<PA>, l1_multi_smem_bytes()};
+        case kSearchL1Cr: return {k_search_l1_cr<PA>, l1_multi_smem_bytes()};
+        default:
+#ifdef ACQ_VARIANT_L1_MULTI_TW   // the K > 1 form that keeps the stage-B twiddles (not the code run) in tensor memory
+            if constexpr (std::is_same_v<PA, SearchArgs>)
+                if (multi) return {k_search_l1<true, PA>, search_l1_smem_bytes()};
+#endif
+            if (multi) return {k_search_l1_multi<PA>, l1_multi_smem_bytes()};
+            return {k_search_l1<false, PA>, search_l1_smem_bytes()};
+        }
     }
-    return cudaSuccess;
+}
+
+template <class PA>
+static cudaError_t configure_search_kernels()
+{
+    cudaError_t e = cudaSuccess;
+    for (int kind : {kSearchL1, kSearchL1Multi, kSearchL1Cr, kSearchE1b, kSearchE1bCluster})
+        for (bool multi : {false, true}) {
+            const SearchKernel<PA> k = search_kernel<PA>(kind, multi);
+            if ((e = cudaFuncSetAttribute(k.f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k.smem)) ||
+                (e = cudaFuncSetAttribute(k.f, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared)))
+                return e;
+        }
+    return e;
 }
 
 cudaError_t search_kernels_configure()
 {
-    using S = SearchArgs;
     cudaError_t e;
-    const int l1 = (int)search_l1_smem_bytes(), e1 = (int)search_e1b_smem_bytes(), fw = (int)fwd_smem_bytes();
-    if ((e = cudaFuncSetAttribute(k_search_l1<false, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, l1))) return e;
-#ifdef ACQ_VARIANT_L1_MULTI_TW
-    if ((e = cudaFuncSetAttribute(k_search_l1<true, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, l1))) return e;
-#endif
-    if ((e = cudaFuncSetAttribute(k_search_l1_multi<S>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)l1_multi_smem_bytes()))) return e;
-    if ((e = cudaFuncSetAttribute(k_search_l1_cr<S>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)l1_multi_smem_bytes()))) return e;
-    if ((e = cudaFuncSetAttribute(k_search_e1b<S>, cudaFuncAttributeMaxDynamicSharedMemorySize, e1))) return e;
-    if ((e = cudaFuncSetAttribute(k_search_e1b_multi<S>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)e1b_multi_smem_bytes()))) return e;
+    if ((e = configure_search_kernels<SearchArgs>()) || (e = configure_search_kernels<AidedSearchArgs>()) ||
+        (e = configure_search_kernels<CohSearchArgs>()) || (e = configure_search_kernels<AidedCohSearchArgs>()))
+        return e;
 #ifdef ACQ_VARIANT_E1B_LDG
-    const int e1g = (int)(fft_smem3_bytes() + 64 * sizeof(float));
-    if ((e = cudaFuncSetAttribute(k_search_e1b_ldg, cudaFuncAttributeMaxDynamicSharedMemorySize, e1g))) return e;
+    if ((e = cudaFuncSetAttribute(k_search_e1b_ldg, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)search_e1b_ldg_smem_bytes())))
+        return e;
 #endif
-    const int ec = (int)search_e1b_cluster_smem_bytes();
-    if ((e = cudaFuncSetAttribute(k_search_e1b_cluster<false, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, ec))) return e;
-    if ((e = cudaFuncSetAttribute(k_search_e1b_cluster<true, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, ec))) return e;
-    const int fc = (int)(fft_smem3_bytes() + 2 * sizeof(float2) * kSub);
+    const int fw = (int)fwd_smem_bytes(), fc = (int)(fft_smem3_bytes() + 2 * sizeof(float2) * kSub);
     if ((e = cudaFuncSetAttribute(k_fwd_fft_cluster<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, fc))) return e;
     if ((e = cudaFuncSetAttribute(k_fwd_fft_cluster<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, fc))) return e;
     if ((e = cudaFuncSetAttribute(k_fwd_fft<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, fw))) return e;
@@ -2569,24 +2566,12 @@ cudaError_t search_kernels_configure()
     // its SMs at the 196 KiB split and the E1B kernel (2 x 103.8 KiB) at 228 KiB, and an SM changes its split only when
     // it is empty: in a GPS + Galileo search the E1B CTAs -- launched to move in as the C/A CTAs retire -- entered no SM
     // before BOTH its C/A CTAs had gone (trace: first E1B CTA at 54.8 us although half the C/A CTAs leave by 50 us).
+    // (the search kernels: configure_search_kernels)
     const void *chain[] = {(const void *)k_front_end<false>, (const void *)k_front_end<true>, (const void *)k_front_end_arg,
                            (const void *)k_fwd_fft<true>, (const void *)k_fwd_fft<false>, (const void *)k_fwd_fft_cluster<true>,
-                           (const void *)k_fwd_fft_cluster<false>, (const void *)k_search_l1<false, S>,
-#ifdef ACQ_VARIANT_L1_MULTI_TW
-                           (const void *)k_search_l1<true, S>,
-#endif
-                           (const void *)k_search_l1_cr<S>, (const void *)k_search_l1_multi<S>, (const void *)k_search_e1b<S>,
-                           (const void *)k_search_e1b_multi<S>, (const void *)k_search_e1b_cluster<false, S>,
-                           (const void *)k_search_e1b_cluster<true, S>, (const void *)k_pick_small, (const void *)k_best_dop};
+                           (const void *)k_fwd_fft_cluster<false>, (const void *)k_coh_variants, (const void *)k_pick_small,
+                           (const void *)k_best_dop};
     for (const void *f : chain)
-        if ((e = cudaFuncSetAttribute(f, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared))) return e;
-    if ((e = aided_kernels_configure())) return e;
-    using CA = CohSearchArgs;
-    using AC = AidedCohSearchArgs;
-    if ((e = cudaFuncSetAttribute(k_search_l1_coh<CA>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)l1_multi_smem_bytes()))) return e;
-    if ((e = cudaFuncSetAttribute(k_search_l1_coh<AC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)l1_multi_smem_bytes()))) return e;
-    const void *coh[] = {(const void *)k_search_l1_coh<CA>, (const void *)k_search_l1_coh<AC>, (const void *)k_coh_variants};
-    for (const void *f : coh)
         if ((e = cudaFuncSetAttribute(f, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared))) return e;
     return cudaSuccess;
 }
@@ -2686,6 +2671,18 @@ int search_kind_l1(int K, int half_bin)
     return kSearchL1Cr;
 }
 
+// Which E1B search kernel: the cluster/DSMEM form when every tile can have a cluster of its own (one wave: 9 us per tile
+// against 12.5 us for the one-CTA form, measured).  With more tiles than that the one-CTA-per-tile forms (k_search_e1b,
+// k_search_e1b_multi for non-coherent sums) have ~2.9x the throughput.
+#ifndef ACQ_FORCE_E1B_KERNEL
+#define ACQ_FORCE_E1B_KERNEL 0   // variants e1b_cta / e1b_cluster: 1 = always the one-CTA form, 2 = always the cluster form
+#endif
+int search_kind_e1b(long long n_tiles, int sm_count)
+{
+    if (ACQ_FORCE_E1B_KERNEL) return ACQ_FORCE_E1B_KERNEL == 2 ? kSearchE1bCluster : kSearchE1b;
+    return n_tiles <= sm_count / 4 ? kSearchE1bCluster : kSearchE1b;
+}
+
 // Claimed tiles or the static stride?  Claiming evens out the two CTAs of an SM and the SMs among themselves, at the price
 // of a greedy tail: once the counter runs dry every CTA still finishes its tile, up to a whole tile time with the SM half
 // empty.  Over many rounds that is noise against what the balance wins (13.7 rounds of E1B tiles: 201.6 -> 190.5 us through
@@ -2737,57 +2734,38 @@ int search_grid_ctas(long long n_tiles, int kind, int sm_count)
     }
     long long cap = (long long)sm_count * 2;  // two persistent CTAs per SM
     if (kind == kSearchE1bCluster) cap = sm_count / 4;
+    if (kind == kSearchL1Coh) cap = sm_count;  // one per SM (512 tensor-memory columns each)
     return (int)(n_tiles < cap ? n_tiles : cap);
 }
 
-// The aided instantiations of the product search kernels (launch_search with SearchArgs::dop_center set).
-static int launch_search_aided(const AidedSearchArgs &a, int kind, int grid, bool e1b, int sm_count, cudaStream_t st, bool pdl)
+template <class PA>
+static int launch_search_as(PA a, int kind, int sm_count, cudaStream_t st, bool pdl)
 {
-    using A = AidedSearchArgs;
-    if (e1b) {
-        if (a.K > 1) launch_k(k_search_e1b_multi<A>, grid, 256, e1b_multi_smem_bytes(), st, pdl, a);
-        else launch_k(k_search_e1b<A>, grid, 256, search_e1b_smem_bytes(), st, pdl, a);
-    } else if (a.K > 1) {
-        launch_k(k_search_l1_multi<A>, grid, 256, l1_multi_smem_bytes(), st, pdl, a);
-    } else if (kind == kSearchL1Cr) {
-        AidedSearchArgs c = a;
-        search_chunks(c.n_tiles, 2 * sm_count, &c.ck_n16, &c.ck_n4);
-        launch_k(k_search_l1_cr<A>, grid, 256, l1_multi_smem_bytes(), st, pdl, c);
-    } else {
-        launch_k(k_search_l1<false, A>, grid, 256, search_l1_smem_bytes(), st, pdl, a);
-    }
+    const int grid = search_grid_ctas(a.n_tiles, kind, sm_count);
+    if (grid <= 0) return 0;
+    if (!search_claims_tiles(a.n_tiles, grid)) a.tile_ctr = nullptr;   // few rounds: static stride
+    if (kind == kSearchL1Cr) search_chunks(a.n_tiles, 2 * sm_count, &a.ck_n16, &a.ck_n4);
+    SearchKernel<PA> k = search_kernel<PA>(kind, a.K > 1);
+#ifdef ACQ_VARIANT_E1B_LDG   // one-CTA E1B search with its operands straight from L2, full-range searches only
+    if constexpr (std::is_same_v<PA, SearchArgs>)
+        if (kind == kSearchE1b) k = {k_search_e1b_ldg, search_e1b_ldg_smem_bytes()};
+#endif
+    // the cluster form runs a cluster of four CTAs per tile
+    launch_k(k.f, kind == kSearchE1bCluster ? 4 * grid : grid, 256, k.smem, st, pdl, a);
     return 1;
 }
 
-int launch_search(const SearchArgs &a_in, bool e1b, int sm_count, cudaStream_t st, bool pdl)
+int launch_search(const SearchArgs &a, bool e1b, int sm_count, cudaStream_t st, bool pdl)
 {
-    const int kind = e1b ? kSearchE1b : search_kind_l1(a_in.K, a_in.half_bin);
-    const int grid = search_grid_ctas(a_in.n_tiles, kind, sm_count);
-    if (grid <= 0) return 0;
-    SearchArgs a = a_in;
-    if (!search_claims_tiles(a.n_tiles, grid)) a.tile_ctr = nullptr;   // few rounds: static stride
-    if (a.dop_center) return launch_search_aided(AidedSearchArgs(a), kind, grid, e1b, sm_count, st, pdl);
-    using S = SearchArgs;
-    if (e1b) {
-#ifdef ACQ_VARIANT_E1B_LDG
-        launch_k(k_search_e1b_ldg, grid, 256, fft_smem3_bytes() + 64 * sizeof(float), st, pdl, a);
-#else
-        if (a.K > 1) launch_k(k_search_e1b_multi<S>, grid, 256, e1b_multi_smem_bytes(), st, pdl, a);
-        else launch_k(k_search_e1b<S>, grid, 256, search_e1b_smem_bytes(), st, pdl, a);
-#endif
-        return 1;
-    }
-#ifdef ACQ_VARIANT_L1_MULTI_TW   // the K > 1 form that keeps the stage-B twiddles (not the code run) in tensor memory
-    launch_k(a.K > 1 ? k_search_l1<true, S> : k_search_l1<false, S>, grid, 256, search_l1_smem_bytes(), st, pdl, a);
-#else
-    if (a.K > 1) launch_k(k_search_l1_multi<S>, grid, 256, l1_multi_smem_bytes(), st, pdl, a);
-    else if (kind == kSearchL1Cr) {
-        search_chunks(a.n_tiles, 2 * sm_count, &a.ck_n16, &a.ck_n4);
-        launch_k(k_search_l1_cr<S>, grid, 256, l1_multi_smem_bytes(), st, pdl, a);
-    }
-    else launch_k(k_search_l1<false, S>, grid, 256, search_l1_smem_bytes(), st, pdl, a);
-#endif
-    return 1;
+    const int kind = e1b ? search_kind_e1b(a.n_tiles, sm_count) : search_kind_l1(a.K, a.half_bin);
+    if (a.dop_center) return launch_search_as(AidedSearchArgs(a), kind, sm_count, st, pdl);
+    return launch_search_as(a, kind, sm_count, st, pdl);
+}
+
+int launch_search_coh(const CohSearchArgs &a, int sm_count, cudaStream_t st, bool pdl)
+{
+    if (a.dop_center) return launch_search_as(AidedCohSearchArgs(a), kSearchL1Coh, sm_count, st, pdl);
+    return launch_search_as(a, kSearchL1Coh, sm_count, st, pdl);
 }
 
 int launch_coh_variants(float2 *x2, const float2 *rot, int n_rows, int F, int K, cudaStream_t st)
@@ -2801,64 +2779,23 @@ int launch_coh_variants(float2 *x2, const float2 *rot, int n_rows, int F, int K,
     return launched;
 }
 
-// one persistent CTA per SM (512 tensor-memory columns each); tiles claimed from a counter from ACQ_DYN_MIN_ROUNDS rounds
-int coh_grid_ctas(long long n_tiles, int sm_count)
-{
-    if (n_tiles <= 0 || n_tiles > kMaxTilesPerLaunch) return 0;
-    return (int)(n_tiles < sm_count ? n_tiles : sm_count);
-}
-
-int launch_search_coh(const CohSearchArgs &a_in, int sm_count, cudaStream_t st, bool pdl)
-{
-    const int grid = coh_grid_ctas(a_in.n_tiles, sm_count);
-    if (grid <= 0) return 0;
-    CohSearchArgs a = a_in;
-    if (!search_claims_tiles(a.n_tiles, grid)) a.tile_ctr = nullptr;
-    if (a.dop_center) launch_k(k_search_l1_coh<AidedCohSearchArgs>, grid, 256, l1_multi_smem_bytes(), st, pdl, AidedCohSearchArgs(a));
-    else launch_k(k_search_l1_coh<CohSearchArgs>, grid, 256, l1_multi_smem_bytes(), st, pdl, a);
-    return 1;
-}
-
-int launch_search_e1b_cluster(const SearchArgs &a, int sm_count, cudaStream_t st, bool pdl)
-{
-    const int n_clusters = search_grid_ctas(a.n_tiles, kSearchE1bCluster, sm_count);
-    if (n_clusters <= 0) return 0;
-    if (a.dop_center)
-        launch_k(a.K > 1 ? k_search_e1b_cluster<true, AidedSearchArgs> : k_search_e1b_cluster<false, AidedSearchArgs>, 4 * n_clusters,
-                 256, search_e1b_cluster_smem_bytes(), st, pdl, AidedSearchArgs(a));
-    else
-        launch_k(a.K > 1 ? k_search_e1b_cluster<true, SearchArgs> : k_search_e1b_cluster<false, SearchArgs>, 4 * n_clusters, 256,
-                 search_e1b_cluster_smem_bytes(), st, pdl, a);
-    return 1;
-}
-
-int launch_refine(const float2 *Dp, const float2 *Ep, const acq_record *rec, const int *sat_type, const int *slot_sat,
-                  acq_fine *out, int n_rows, int n_slots, int K, int nvar, int half_bin, int ext_len, int Q, int n_shift,
-                  int smax, int cd_div, int n_sats, int dop_lo, int dop_hi, float thr_l1, float thr_e1b, int flags,
-                  cudaStream_t st)
+int launch_refine(const RefineArgs &a, int n_rows, cudaStream_t st)
 {
     if (n_rows <= 0) return 0;
-    RefineArgs a{Dp, Ep, rec, sat_type, slot_sat, out, n_slots, K, nvar, half_bin, ext_len, Q, n_shift, smax, cd_div,
-                 n_sats, dop_lo, dop_hi, flags, thr_l1, thr_e1b};
     k_refine<<<n_rows, 256, 0, st>>>(a);
     return 1;
 }
 
-int launch_profile(const float2 *Dp, const float2 *Ep, const float2 *tables, const acq_record *rec, const int *sat_type,
-                   const int *slot_sat, acq_peak2 *out, float *profile, int n_rows, int n_slots, int n_l1_slots,
-                   int n_e1b_slots, int K, int nvar, int half_bin, int ext_len, int Q, int n_shift, int smax, int cd_div,
-                   int n_sats, int dop_lo, int dop_hi, float thr_l1, float thr_e1b, int flags, int excl, cudaStream_t st)
+int launch_profile(const ProfileArgs &a, int n_rows, int n_l1_slots, cudaStream_t st)
 {
     if (n_rows <= 0) return 0;
-    ProfileArgs a{Dp, Ep, tables, rec, sat_type, slot_sat, out, profile, n_slots, n_e1b_slots, K, nvar, half_bin, ext_len, Q,
-                  n_shift, smax, cd_div, n_sats, dop_lo, dop_hi, flags, excl, thr_l1, thr_e1b};
     int n = 0;
     if (n_l1_slots > 0) {
-        k_profile<false><<<n_rows, 256, profile_smem_bytes(false, K), st>>>(a);
+        k_profile<false><<<n_rows, 256, profile_smem_bytes(false, a.K), st>>>(a);
         n++;
     }
-    if (n_e1b_slots > 0) {
-        k_profile<true><<<n_rows, 256, profile_smem_bytes(true, K), st>>>(a);
+    if (a.n_e1b_slots > 0) {
+        k_profile<true><<<n_rows, 256, profile_smem_bytes(true, a.K), st>>>(a);
         n++;
     }
     return n;

@@ -108,13 +108,13 @@ int launch_hb2(const float2 *x1, float2 *x2, const float2 *rot, int n_rows, int 
 int launch_fwd_fft(const float2 *x2, float2 *out, const float2 *tables, int n_rows, bool polyphase, int sm_count,
                    cudaStream_t st, bool pdl = false);
 int launch_build_ext(const float2 *C, float2 *Ep, int n_sats, int Q, int ext_len, int wrap_mode, cudaStream_t st);
+// the C/A (e1b false) or E1B rows of a search; the kernel is search_kind_l1's or search_kind_e1b's, in the instantiation
+// of the aided search when a.dop_center is set
 int launch_search(const SearchArgs &a, bool e1b, int sm_count, cudaStream_t st, bool pdl = false);
-int launch_search_e1b_cluster(const SearchArgs &a, int sm_count, cudaStream_t st, bool pdl = false);
 // Coherent search (acq_search_coherent): the sub-bin variants 1..F-1 of every block row of x2 (layout [row][F][16384]),
 // formed from variant 0 with the host-built table rot ([F][16384]); then the C/A search kernel k_search_l1_coh, one CTA
-// per SM, with grid coh_grid_ctas() (what SearchArgs::ctas_total counts).
+// per SM (kind kSearchL1Coh).
 int launch_coh_variants(float2 *x2, const float2 *rot, int n_rows, int F, int K, cudaStream_t st);
-int coh_grid_ctas(long long n_tiles, int sm_count);
 int launch_search_coh(const CohSearchArgs &a, int sm_count, cudaStream_t st, bool pdl = false);
 // Doppler indices of the cell rows a best-Doppler pick reads: cell d of row r is index dop_lo + d, or, with
 // dop_center (an aided search), window_lo(dop_center[r], half_width, dop_lo, dop_hi) + d.
@@ -133,8 +133,10 @@ int launch_pick_small(const acq_cell *cells, const int *slot_sat, acq_record *ou
                       bool pdl = false);
 // CTAs of a search launch that store cells (what SearchArgs::ctas_total sums over the launches of one search)
 // Search kernel kinds, reported as acq_launch_plan.kernel: the values are ABI (4 and 5 named kernels since removed)
-enum { kSearchL1 = 0, kSearchE1b = 1, kSearchE1bCluster = 2, kSearchL1Multi = 3, kSearchL1Cr = 6 };
+// (kSearchL1Coh, k_search_l1_coh, is never reported: acq_plan_launch covers the non-coherent searches)
+enum { kSearchL1 = 0, kSearchE1b = 1, kSearchE1bCluster = 2, kSearchL1Multi = 3, kSearchL1Cr = 6, kSearchL1Coh = 7 };
 int search_kind_l1(int K, int half_bin);   // which C/A search kernel (and so which grid) a search uses
+int search_kind_e1b(long long n_tiles, int sm_count);   // ... and which E1B search kernel
 constexpr int kPickSmallRowsMax = 256;  // rows k_pick_small stages in shared memory
 // A record as k_pick_small hands it to a POLLING host (mapped pinned memory): two 16-byte halves, each carrying the
 // search's epoch in its last word.  Each half arrives by one 16-byte store, so a host that sees the epoch in a half has
@@ -155,17 +157,35 @@ void search_chunk_lengths(int *big, int *mid);
 // refinement of the records of the most recent search (one CTA per record).  Each CTA checks its record against the
 // search's shape (slot_sat, n_sats, dop_lo..dop_hi) and writes a marker row for one that fails (ca_shift -2) or, with
 // ACQ_REFINE_DETECTED in flags, for one below its satellite type's threshold (ca_shift -1)
-int launch_refine(const float2 *Dp, const float2 *Ep, const acq_record *rec, const int *sat_type, const int *slot_sat,
-                  acq_fine *out, int n_rows, int n_slots, int K, int nvar, int half_bin, int ext_len, int Q, int n_shift,
-                  int smax, int cd_div, int n_sats, int dop_lo, int dop_hi, float thr_l1, float thr_e1b, int flags,
-                  cudaStream_t st);
+struct RefineArgs {
+    const float2 *Dp;
+    const float2 *Ep;
+    const acq_record *rec;   // [n_rows], row = cap * n_slots + slot
+    const int *sat_type;     // [n_sats]
+    const int *slot_sat;     // [n_slots] satellite searched in each slot
+    acq_fine *out;
+    int n_slots, K, nvar, half_bin, ext_len, Q, n_shift, smax, cd_div;
+    int n_sats, dop_lo, dop_hi, flags;
+    float thr_l1, thr_e1b;
+};
+int launch_refine(const RefineArgs &a, int n_rows, cudaStream_t st);
 // peak-quality profile of the records of the most recent search (acq_profile): one CTA per record in each of two
 // launches, the C/A rows (n_l1_slots > 0) and the E1B rows (n_e1b_slots > 0).  Record checks and markers (lag2 -2 / -1
-// with ACQ_PROFILE_DETECTED in flags) as launch_refine; profile NULL or the packed lag vectors of acq_b200.h
-int launch_profile(const float2 *Dp, const float2 *Ep, const float2 *tables, const acq_record *rec, const int *sat_type,
-                   const int *slot_sat, acq_peak2 *out, float *profile, int n_rows, int n_slots, int n_l1_slots,
-                   int n_e1b_slots, int K, int nvar, int half_bin, int ext_len, int Q, int n_shift, int smax, int cd_div,
-                   int n_sats, int dop_lo, int dop_hi, float thr_l1, float thr_e1b, int flags, int excl, cudaStream_t st);
+// with ACQ_PROFILE_DETECTED in flags) as launch_refine
+struct ProfileArgs {
+    const float2 *Dp;
+    const float2 *Ep;
+    const float2 *tables;
+    const acq_record *rec;   // [n_rows], row = cap * n_slots + slot
+    const int *sat_type;     // [n_sats]
+    const int *slot_sat;     // [n_slots] satellite searched in each slot
+    acq_peak2 *out;
+    float *profile;          // NULL, or the packed lag vectors (acq_b200.h)
+    int n_slots, n_e1b_slots, K, nvar, half_bin, ext_len, Q, n_shift, smax, cd_div;
+    int n_sats, dop_lo, dop_hi, flags, excl;
+    float thr_l1, thr_e1b;
+};
+int launch_profile(const ProfileArgs &a, int n_rows, int n_l1_slots, cudaStream_t st);
 cudaError_t search_kernels_configure();
 
 }  // namespace acq
