@@ -43,6 +43,10 @@ _SIGNATURES = [
     ("acq_refine_device", C.c_int, [_P, _P, C.c_int, C.c_int, _P, _P]),
     ("acq_profile", C.c_int, [_P, _P, C.c_int, C.c_int, _P, _P]),
     ("acq_profile_device", C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, _P, _P, _P]),
+    ("acq_refine_coherent", C.c_int, [_P, _P, C.c_int, _P]),
+    ("acq_refine_coherent_device", C.c_int, [_P, _P, C.c_int, C.c_float, _P, _P]),
+    ("acq_profile_coherent", C.c_int, [_P, _P, C.c_int, C.c_int, _P, _P]),
+    ("acq_profile_coherent_device", C.c_int, [_P, _P, C.c_int, C.c_float, C.c_int, _P, _P, _P]),
     ("acq_detected", C.c_int, [_P, _P]),
     ("acq_get_code_spectrum", C.c_int, [_P, C.c_int, _P]),
     ("acq_get_capture_spectrum", C.c_int, [_P, _P, C.c_int, _P, _P]),

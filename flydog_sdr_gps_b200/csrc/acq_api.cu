@@ -12,6 +12,7 @@
 #include <cstdarg>
 #include <memory>
 #include <numeric>
+#include <type_traits>
 
 #include "acq_geom.h"
 #include "acq_kernels.cuh"
@@ -224,12 +225,15 @@ struct acq_engine {
     DevBuf<acq_peak2> d_peak2;
     // The most recent search whose spectra are still on the device (captures 0: none), which refinement and profile read:
     // its slots, device slot -> satellite map and C/A and E1B slot counts.  host: a host-path search, whose records
-    // acq_refine and acq_profile may take (the current selection is then its selection).  A coherent search leaves none.
+    // acq_refine and acq_profile may take (the current selection is then its selection).  A coherent search leaves none
+    // there: its shape goes to last_coh (m_coh > 0), which only acq_refine_coherent* and acq_profile_coherent* read.  A
+    // search clears both when it starts.
     struct LastSearch {
         int captures = 0, slots = 0, n_l1 = 0, n_e1b = 0;
         const int *slot_sat = nullptr;
         bool host = false;
-    } last;
+        int m_coh = 0;   // coherent: M; the spectra hold F = M (1 + half_bin) variants per block
+    } last, last_coh;
     // aided host search (acq_search_aided): Doppler centres staged in pinned memory, copied to the device with the capture
     PinnedBuf<int32_t, cudaHostAllocDefault> h_center;
     DevBuf<int> d_center;
@@ -446,9 +450,9 @@ int check_search(acq_engine *e, const SearchMode &m, const void *packed, int n_c
     if (e->pending) return fail(ACQ_ERR_ARG, "a submitted search is still pending: call acq_wait first");
     if (device && ((uintptr_t)packed & 15) != 0)
         return fail(ACQ_ERR_ARG, "packed_dev must be 16-byte aligned (the front end stages it with bulk async copies)");
-    // A non-coherent search forgets the last search from here on, also when it is refused below; a refused coherent
-    // search leaves it.
-    if (!m.coherent) e->last = {};
+    // A non-coherent search forgets the last search (of either kind) from here on, also when it is refused below; a
+    // refused coherent search leaves it.
+    if (!m.coherent) e->last = e->last_coh = {};
     if (m.coherent && K % m.m_coh) return fail(ACQ_ERR_ARG, "k_noncoh=%d is not a multiple of m_coh=%d", K, m.m_coh);
     const int n_sats = (int)e->sats.size();
     if (sel && n_sel <= 0) return fail(ACQ_ERR_ARG, "n_sel must be > 0 when sel is given");
@@ -612,7 +616,7 @@ int search_host(acq_engine *e, const SearchMode &m, const uint8_t *packed, int n
     int rc = check_search(e, m, packed, n_captures, sel, n_sel, out, false);
     if (rc) return rc;
     DeviceGuard g(e->device);
-    e->last = {};  // until this search is enqueued, there are no spectra refinement or profile could use
+    e->last = e->last_coh = {};  // until this search is enqueued, there are no spectra refinement or profile could use
     if ((rc = set_selection(e, sel, n_sel)) || (rc = ensure_scratch(e, n_captures, true, m))) return rc;
     const int n_dop = m.dops(e);
     const size_t bytes = (size_t)n_captures * e->prm.k_noncoh * e->block_bytes;
@@ -643,6 +647,7 @@ int search_host(acq_engine *e, const SearchMode &m, const uint8_t *packed, int n
                              as_arg ? packed : nullptr)))
         return rc;
     if (!m.coherent) e->last = {n_captures, e->n_slots, e->n_l1, e->n_e1b, e->cur_slot_sat, true};
+    else e->last_coh = {n_captures, e->n_slots, e->n_l1, e->n_e1b, e->cur_slot_sat, true, m.m_coh};
     if (!host_records) CU(cudaMemcpyAsync(out, e->d_records, rows * sizeof(acq_record), cudaMemcpyDeviceToHost, e->stream));
     if (grid)
         CU(cudaMemcpyAsync(grid, e->d_cells, rows * n_dop * sizeof(acq_cell), cudaMemcpyDeviceToHost, e->stream));
@@ -680,36 +685,45 @@ int search_device(acq_engine *e, const SearchMode &m, const uint8_t *packed_dev,
     int rc = check_search(e, m, packed_dev, n_captures, sel, n_sel, out_dev, true);
     if (rc) return rc;
     DeviceGuard g(e->device);
-    e->last = {};  // refinement and profile apply once this search is enqueued
+    e->last = e->last_coh = {};  // refinement and profile apply once this search is enqueued
     if ((rc = set_selection(e, sel, n_sel)) || (rc = ensure_scratch(e, n_captures, false, m))) return rc;
     cudaStream_t st = stream ? (cudaStream_t)stream : e->stream;
     if ((rc = enqueue_search(e, m, packed_dev, n_captures, out_dev, nullptr, st, nullptr))) return rc;
     if (!m.coherent) e->last = {n_captures, e->n_slots, e->n_l1, e->n_e1b, e->cur_slot_sat, false};
+    else e->last_coh = {n_captures, e->n_slots, e->n_l1, e->n_e1b, e->cur_slot_sat, false, m.m_coh};
     return hold_scratch(e, st);
 }
 
+// The search acq_refine* and acq_profile* apply to (last), or acq_refine_coherent* and acq_profile_coherent* (last_coh)
+const acq_engine::LastSearch &last_of(const acq_engine *e, bool coherent) { return coherent ? e->last_coh : e->last; }
+
 // The checks of acq_refine* and acq_profile* (`what`) against the last search, after those of their own arguments.
 // The host forms take the records of a host-path search and check each one here; the device forms leave that to the
-// kernels, which write a marker row for a record that fails.
-int check_records(acq_engine *e, const acq_record *rec, int n_records, bool device, const char *what)
+// kernels, which write a marker row for a record that fails.  coherent: the checks of the coherent forms, against the
+// last coherent search, whose records' Doppler indices run over M dop_lo .. M dop_hi.
+int check_records(acq_engine *e, const acq_record *rec, int n_records, bool device, bool coherent, const char *what)
 {
     if (e->pending) return fail(ACQ_ERR_ARG, "a submitted search is still pending: call acq_wait first");
-    if (device && e->last.captures <= 0)
-        return fail(ACQ_ERR_ARG, "no search whose spectra are still on the device to %s", what);
-    if (!device && (e->last.captures <= 0 || !e->last.host))
-        return fail(ACQ_ERR_ARG, "no completed host-path search to %s", what);
-    const long long rows = (long long)e->last.captures * e->last.slots;
-    if (n_records != rows) return fail(ACQ_ERR_ARG, "n_records=%d but the last search produced %lld records", n_records, rows);
+    const acq_engine::LastSearch &ls = last_of(e, coherent);
+    const char *kind = coherent ? "coherent " : "";
+    if (device && ls.captures <= 0)
+        return fail(ACQ_ERR_ARG, "no %ssearch whose spectra are still on the device to %s", kind, what);
+    if (!device && (ls.captures <= 0 || !ls.host))
+        return fail(ACQ_ERR_ARG, "no completed host-path %ssearch to %s", kind, what);
+    const long long rows = (long long)ls.captures * ls.slots;
+    if (n_records != rows)
+        return fail(ACQ_ERR_ARG, "n_records=%d but the last %ssearch produced %lld records", n_records, kind, rows);
     if (device) return ACQ_OK;
+    const int M = coherent ? ls.m_coh : 1, lo = M * e->prm.dop_lo, hi = M * e->prm.dop_hi;
     for (int i = 0; i < n_records; i++) {
         const acq_record &r = rec[i];
-        if (r.sat != e->sel_cache[i % e->last.slots])
+        if (r.sat != e->sel_cache[i % ls.slots])
             return fail(ACQ_ERR_ARG, "record %d: sat %d is not the satellite searched in that slot", i, r.sat);
         const int L = (e->sats[r.sat].type == ACQ_E1B) ? ACQ_LAGS_E1B : ACQ_LAGS_L1;
         if (r.lag < 0 || r.lag >= L) return fail(ACQ_ERR_ARG, "record %d: lag %d outside 0..%d", i, r.lag, L - 1);
         // a row that never exceeded snr 0 carries dop 0 (k_best_dop), which may lie outside an asymmetric range
-        if ((r.dop < e->prm.dop_lo || r.dop > e->prm.dop_hi) && !(r.dop == 0 && r.snr == 0.0f))
-            return fail(ACQ_ERR_ARG, "record %d: Doppler index %d outside %d..%d", i, r.dop, e->prm.dop_lo, e->prm.dop_hi);
+        if ((r.dop < lo || r.dop > hi) && !(r.dop == 0 && r.snr == 0.0f))
+            return fail(ACQ_ERR_ARG, "record %d: Doppler index %d outside %d..%d", i, r.dop, lo, hi);
     }
     return ACQ_OK;
 }
@@ -726,19 +740,23 @@ int check_excl(int excl, int n_l1)
 // Lag-vector floats of one capture's rows (acq_b200.h: L per slot)
 size_t profile_capture_len(int n_l1, int n_e1b) { return (size_t)n_l1 * ACQ_LAGS_L1 + (size_t)n_e1b * ACQ_LAGS_E1B; }
 
-// The arguments refinement and profile share: the spectra and shape of the last search, the records and the flags
+// The arguments refinement and profile share: the spectra and shape of the last search (coherent: the last coherent
+// search, its F variants per block and its M times finer Doppler range), the records and the flags.  A coherent form's
+// min_snr is the threshold of its DETECTED flag (set when min_snr > 0).
 template <class A>
-A last_search_args(const acq_engine *e, const acq_record *rec_dev, int flags)
+A last_search_args(const acq_engine *e, bool coherent, const acq_record *rec_dev, int flags, float min_snr)
 {
+    const acq_engine::LastSearch &ls = last_of(e, coherent);
+    const int M = coherent ? ls.m_coh : 1;
     A a{};
     a.Dp = e->d_Dp;
     a.Ep = e->d_Ep;
     a.rec = rec_dev;
     a.sat_type = e->d_sat_type;
-    a.slot_sat = e->last.slot_sat;
-    a.n_slots = e->last.slots;
+    a.slot_sat = ls.slot_sat;
+    a.n_slots = ls.slots;
     a.K = e->prm.k_noncoh;
-    a.nvar = e->nvar;
+    a.nvar = coherent ? M * (1 + e->prm.half_bin) : e->nvar;
     a.half_bin = e->prm.half_bin;
     a.ext_len = e->ext_len;
     a.Q = e->Q;
@@ -746,34 +764,142 @@ A last_search_args(const acq_engine *e, const acq_record *rec_dev, int flags)
     a.smax = e->smax;
     a.cd_div = e->cd_div;
     a.n_sats = (int)e->sats.size();
-    a.dop_lo = e->prm.dop_lo;
-    a.dop_hi = e->prm.dop_hi;
+    a.dop_lo = M * e->prm.dop_lo;
+    a.dop_hi = M * e->prm.dop_hi;
     a.flags = flags;
-    a.thr_l1 = e->prm.thr_l1;
-    a.thr_e1b = e->prm.thr_e1b;
+    a.thr_l1 = coherent ? min_snr : e->prm.thr_l1;
+    a.thr_e1b = coherent ? min_snr : e->prm.thr_e1b;
+    if constexpr (std::is_base_of_v<RefineCohArgs, A> || std::is_base_of_v<ProfileCohArgs, A>) a.m_coh = M;
     return a;
 }
 
-int enqueue_refine(acq_engine *e, const acq_record *rec_dev, int n_records, int flags, acq_fine *out_dev, cudaStream_t st)
+int enqueue_refine(acq_engine *e, bool coherent, const acq_record *rec_dev, int n_records, int flags, float min_snr,
+                   acq_fine *out_dev, cudaStream_t st)
 {
-    RefineArgs a = last_search_args<RefineArgs>(e, rec_dev, flags);
-    a.out = out_dev;
-    e->launches += launch_refine(a, n_records, st);
+    if (coherent) {
+        RefineCohArgs a = last_search_args<RefineCohArgs>(e, true, rec_dev, flags, min_snr);
+        a.out = out_dev;
+        e->launches += launch_refine_coh(a, n_records, st);
+    } else {
+        RefineArgs a = last_search_args<RefineArgs>(e, false, rec_dev, flags, 0.0f);
+        a.out = out_dev;
+        e->launches += launch_refine(a, n_records, st);
+    }
     CU(cudaGetLastError());
     return ACQ_OK;
 }
 
-int enqueue_profile(acq_engine *e, const acq_record *rec_dev, int n_records, int flags, int excl, acq_peak2 *out_dev,
-                    float *profile_dev, cudaStream_t st)
+template <class A>
+A profile_args(const acq_engine *e, bool coherent, const acq_record *rec_dev, int flags, float min_snr, int excl,
+               acq_peak2 *out_dev, float *profile_dev)
 {
-    ProfileArgs a = last_search_args<ProfileArgs>(e, rec_dev, flags);
+    A a = last_search_args<A>(e, coherent, rec_dev, flags, min_snr);
     a.tables = e->d_tables;
     a.out = out_dev;
     a.profile = profile_dev;
-    a.n_e1b_slots = e->last.n_e1b;
+    a.n_e1b_slots = last_of(e, coherent).n_e1b;
     a.excl = excl;
-    e->launches += launch_profile(a, n_records, e->last.n_l1, st);
+    return a;
+}
+
+int enqueue_profile(acq_engine *e, bool coherent, const acq_record *rec_dev, int n_records, int flags, float min_snr,
+                    int excl, acq_peak2 *out_dev, float *profile_dev, cudaStream_t st)
+{
+    if (coherent)   // a coherent search has C/A rows only (check_search)
+        e->launches += launch_profile_coh(
+            profile_args<ProfileCohArgs>(e, true, rec_dev, flags, min_snr, excl, out_dev, profile_dev), n_records, st);
+    else
+        e->launches += launch_profile(profile_args<ProfileArgs>(e, false, rec_dev, flags, 0.0f, excl, out_dev, profile_dev),
+                                      n_records, e->last.n_l1, st);
     CU(cudaGetLastError());
+    return ACQ_OK;
+}
+
+// acq_refine / acq_refine_coherent after their argument checks: the records go to the device, are refined on the engine
+// stream and come back.  The records are checked here, so the kernel's own checks pass every row.
+int refine_host(acq_engine *e, bool coherent, const acq_record *rec, int n_records, acq_fine *out)
+{
+    int rc = check_records(e, rec, n_records, false, coherent, "refine");
+    if (rc) return rc;
+    DeviceGuard g(e->device);
+    if ((rc = grow(e, e->d_ref_rec, (size_t)n_records)) || (rc = grow(e, e->d_fine, (size_t)n_records))) return rc;
+    CU(cudaMemcpyAsync(e->d_ref_rec, rec, (size_t)n_records * sizeof(acq_record), cudaMemcpyHostToDevice, e->stream));
+    if ((rc = enqueue_refine(e, coherent, e->d_ref_rec, n_records, 0, 0.0f, e->d_fine, e->stream))) return rc;
+    CU(cudaMemcpyAsync(out, e->d_fine, (size_t)n_records * sizeof(acq_fine), cudaMemcpyDeviceToHost, e->stream));
+    CU(cudaStreamSynchronize(e->stream));
+    return ACQ_OK;
+}
+
+// acq_refine_device / acq_refine_coherent_device after their argument checks
+int refine_device(acq_engine *e, bool coherent, const acq_record *rec_dev, int n_records, int flags, float min_snr,
+                  acq_fine *out_dev, void *stream)
+{
+    int rc = check_records(e, rec_dev, n_records, true, coherent, "refine");
+    if (rc) return rc;
+    if (((uintptr_t)out_dev & 15) != 0) return fail(ACQ_ERR_ARG, "out_dev must be 16-byte aligned (one 16-byte store per row)");
+    if (((uintptr_t)rec_dev & 3) != 0) return fail(ACQ_ERR_ARG, "rec_dev must be 4-byte aligned");
+    DeviceGuard g(e->device);
+    cudaStream_t st = stream ? (cudaStream_t)stream : e->stream;
+    // after the search that left the spectra (on any stream), before the next search overwrites them
+    if ((rc = wait_scratch(e, st, true)) || (rc = enqueue_refine(e, coherent, rec_dev, n_records, flags, min_snr, out_dev, st)))
+        return rc;
+    return hold_scratch(e, st);
+}
+
+// acq_profile / acq_profile_coherent after their argument checks (excl >= 0)
+int profile_host(acq_engine *e, bool coherent, const acq_record *rec, int n_records, int excl, acq_peak2 *out, float *profile)
+{
+    int rc = check_records(e, rec, n_records, false, coherent, "profile");
+    const acq_engine::LastSearch &ls = last_of(e, coherent);
+    if (rc || (rc = check_excl(excl, ls.n_l1))) return rc;
+    DeviceGuard g(e->device);
+    const size_t n_prof = (size_t)ls.captures * profile_capture_len(ls.n_l1, ls.n_e1b);
+    if ((rc = grow(e, e->d_ref_rec, (size_t)n_records)) || (rc = grow(e, e->d_peak2, (size_t)n_records))) return rc;
+    // The lag profiles (512 MiB for a 1024-capture C/A search) live only for this call: the engine keeps no buffer of
+    // that size.  The buffer is freed after the engine stream has passed every use of it, on the error paths too.
+    struct CallBuffer {
+        cudaStream_t st;
+        float *p = nullptr;
+        ~CallBuffer()
+        {
+            if (p) {
+                cudaStreamSynchronize(st);
+                cudaFree(p);
+            }
+        }
+    } d_prof{e->stream};
+    if (profile) CU(cudaMalloc(&d_prof.p, n_prof * sizeof(float)));
+    CU(cudaMemcpyAsync(e->d_ref_rec, rec, (size_t)n_records * sizeof(acq_record), cudaMemcpyHostToDevice, e->stream));
+    // the records are checked above, so the kernel's own checks pass every row
+    if ((rc = enqueue_profile(e, coherent, e->d_ref_rec, n_records, 0, 0.0f, excl, e->d_peak2, d_prof.p, e->stream))) return rc;
+    CU(cudaMemcpyAsync(out, e->d_peak2, (size_t)n_records * sizeof(acq_peak2), cudaMemcpyDeviceToHost, e->stream));
+    if (profile) CU(cudaMemcpyAsync(profile, d_prof.p, n_prof * sizeof(float), cudaMemcpyDeviceToHost, e->stream));
+    CU(cudaStreamSynchronize(e->stream));
+    return ACQ_OK;
+}
+
+// acq_profile_device / acq_profile_coherent_device after their argument checks (excl >= 0)
+int profile_device(acq_engine *e, bool coherent, const acq_record *rec_dev, int n_records, int flags, float min_snr, int excl,
+                   acq_peak2 *out_dev, float *profile_dev, void *stream)
+{
+    int rc = check_records(e, rec_dev, n_records, true, coherent, "profile");
+    if (rc || (rc = check_excl(excl, last_of(e, coherent).n_l1))) return rc;
+    if (((uintptr_t)out_dev & 15) != 0) return fail(ACQ_ERR_ARG, "out_dev must be 16-byte aligned (one 16-byte store per row)");
+    if (((uintptr_t)rec_dev & 3) != 0) return fail(ACQ_ERR_ARG, "rec_dev must be 4-byte aligned");
+    if (((uintptr_t)profile_dev & 3) != 0) return fail(ACQ_ERR_ARG, "profile_dev must be 4-byte aligned");
+    DeviceGuard g(e->device);
+    cudaStream_t st = stream ? (cudaStream_t)stream : e->stream;
+    // ordered as acq_refine_device: after the search that left the spectra, before the next one
+    if ((rc = wait_scratch(e, st, true)) ||
+        (rc = enqueue_profile(e, coherent, rec_dev, n_records, flags, min_snr, excl, out_dev, profile_dev, st)))
+        return rc;
+    return hold_scratch(e, st);
+}
+
+// min_snr of the coherent device forms: a NaN would skip every row without saying so
+int check_min_snr(float min_snr)
+{
+    if (std::isnan(min_snr)) return fail(ACQ_ERR_ARG, "min_snr is NaN");
     return ACQ_OK;
 }
 
@@ -1086,16 +1212,7 @@ int acq_refine(acq_engine *e, const acq_record *rec, int n_records, acq_fine *ou
 {
     if (!e) return fail(ACQ_ERR_ARG, "engine is NULL");
     if (!rec || !out) return fail(ACQ_ERR_ARG, "rec/out must not be NULL");
-    int rc = check_records(e, rec, n_records, false, "refine");
-    if (rc) return rc;
-    DeviceGuard g(e->device);
-    if ((rc = grow(e, e->d_ref_rec, (size_t)n_records)) || (rc = grow(e, e->d_fine, (size_t)n_records))) return rc;
-    CU(cudaMemcpyAsync(e->d_ref_rec, rec, (size_t)n_records * sizeof(acq_record), cudaMemcpyHostToDevice, e->stream));
-    // the records are checked above, so the kernel's own checks pass every row
-    if ((rc = enqueue_refine(e, e->d_ref_rec, n_records, 0, e->d_fine, e->stream))) return rc;
-    CU(cudaMemcpyAsync(out, e->d_fine, (size_t)n_records * sizeof(acq_fine), cudaMemcpyDeviceToHost, e->stream));
-    CU(cudaStreamSynchronize(e->stream));
-    return ACQ_OK;
+    return refine_host(e, false, rec, n_records, out);
 }
 
 int acq_refine_device(acq_engine *e, const acq_record *rec_dev, int n_records, int flags, acq_fine *out_dev, void *stream)
@@ -1103,15 +1220,24 @@ int acq_refine_device(acq_engine *e, const acq_record *rec_dev, int n_records, i
     if (!e) return fail(ACQ_ERR_ARG, "engine is NULL");
     if (!rec_dev || !out_dev) return fail(ACQ_ERR_ARG, "rec_dev/out_dev must not be NULL");
     if (flags & ~ACQ_REFINE_DETECTED) return fail(ACQ_ERR_ARG, "unknown flag bits 0x%x", (unsigned)(flags & ~ACQ_REFINE_DETECTED));
-    int rc = check_records(e, rec_dev, n_records, true, "refine");
+    return refine_device(e, false, rec_dev, n_records, flags, 0.0f, out_dev, stream);
+}
+
+int acq_refine_coherent(acq_engine *e, const acq_record *rec, int n_records, acq_fine *out)
+{
+    if (!e) return fail(ACQ_ERR_ARG, "engine is NULL");
+    if (!rec || !out) return fail(ACQ_ERR_ARG, "rec/out must not be NULL");
+    return refine_host(e, true, rec, n_records, out);
+}
+
+int acq_refine_coherent_device(acq_engine *e, const acq_record *rec_dev, int n_records, float min_snr, acq_fine *out_dev,
+                               void *stream)
+{
+    if (!e) return fail(ACQ_ERR_ARG, "engine is NULL");
+    if (!rec_dev || !out_dev) return fail(ACQ_ERR_ARG, "rec_dev/out_dev must not be NULL");
+    int rc = check_min_snr(min_snr);
     if (rc) return rc;
-    if (((uintptr_t)out_dev & 15) != 0) return fail(ACQ_ERR_ARG, "out_dev must be 16-byte aligned (one 16-byte store per row)");
-    if (((uintptr_t)rec_dev & 3) != 0) return fail(ACQ_ERR_ARG, "rec_dev must be 4-byte aligned");
-    DeviceGuard g(e->device);
-    cudaStream_t st = stream ? (cudaStream_t)stream : e->stream;
-    // after the search that left the spectra (on any stream), before the next search overwrites them
-    if ((rc = wait_scratch(e, st, true)) || (rc = enqueue_refine(e, rec_dev, n_records, flags, out_dev, st))) return rc;
-    return hold_scratch(e, st);
+    return refine_device(e, true, rec_dev, n_records, min_snr > 0.0f ? ACQ_REFINE_DETECTED : 0, min_snr, out_dev, stream);
 }
 
 int acq_profile(acq_engine *e, const acq_record *rec, int n_records, int excl, acq_peak2 *out, float *profile)
@@ -1119,32 +1245,7 @@ int acq_profile(acq_engine *e, const acq_record *rec, int n_records, int excl, a
     if (!e) return fail(ACQ_ERR_ARG, "engine is NULL");
     if (!rec || !out) return fail(ACQ_ERR_ARG, "rec/out must not be NULL");
     if (excl < 0) return fail(ACQ_ERR_ARG, "excl must be >= 0 (got %d)", excl);
-    int rc = check_records(e, rec, n_records, false, "profile");
-    if (rc || (rc = check_excl(excl, e->last.n_l1))) return rc;
-    DeviceGuard g(e->device);
-    const size_t n_prof = (size_t)e->last.captures * profile_capture_len(e->last.n_l1, e->last.n_e1b);
-    if ((rc = grow(e, e->d_ref_rec, (size_t)n_records)) || (rc = grow(e, e->d_peak2, (size_t)n_records))) return rc;
-    // The lag profiles (512 MiB for a 1024-capture C/A search) live only for this call: the engine keeps no buffer of
-    // that size.  The buffer is freed after the engine stream has passed every use of it, on the error paths too.
-    struct CallBuffer {
-        cudaStream_t st;
-        float *p = nullptr;
-        ~CallBuffer()
-        {
-            if (p) {
-                cudaStreamSynchronize(st);
-                cudaFree(p);
-            }
-        }
-    } d_prof{e->stream};
-    if (profile) CU(cudaMalloc(&d_prof.p, n_prof * sizeof(float)));
-    CU(cudaMemcpyAsync(e->d_ref_rec, rec, (size_t)n_records * sizeof(acq_record), cudaMemcpyHostToDevice, e->stream));
-    // the records are checked above, so the kernel's own checks pass every row
-    if ((rc = enqueue_profile(e, e->d_ref_rec, n_records, 0, excl, e->d_peak2, d_prof.p, e->stream))) return rc;
-    CU(cudaMemcpyAsync(out, e->d_peak2, (size_t)n_records * sizeof(acq_peak2), cudaMemcpyDeviceToHost, e->stream));
-    if (profile) CU(cudaMemcpyAsync(profile, d_prof.p, n_prof * sizeof(float), cudaMemcpyDeviceToHost, e->stream));
-    CU(cudaStreamSynchronize(e->stream));
-    return ACQ_OK;
+    return profile_host(e, false, rec, n_records, excl, out, profile);
 }
 
 int acq_profile_device(acq_engine *e, const acq_record *rec_dev, int n_records, int flags, int excl, acq_peak2 *out_dev,
@@ -1154,17 +1255,27 @@ int acq_profile_device(acq_engine *e, const acq_record *rec_dev, int n_records, 
     if (!rec_dev || !out_dev) return fail(ACQ_ERR_ARG, "rec_dev/out_dev must not be NULL");
     if (flags & ~ACQ_PROFILE_DETECTED) return fail(ACQ_ERR_ARG, "unknown flag bits 0x%x", (unsigned)(flags & ~ACQ_PROFILE_DETECTED));
     if (excl < 0) return fail(ACQ_ERR_ARG, "excl must be >= 0 (got %d)", excl);
-    int rc = check_records(e, rec_dev, n_records, true, "profile");
-    if (rc || (rc = check_excl(excl, e->last.n_l1))) return rc;
-    if (((uintptr_t)out_dev & 15) != 0) return fail(ACQ_ERR_ARG, "out_dev must be 16-byte aligned (one 16-byte store per row)");
-    if (((uintptr_t)rec_dev & 3) != 0) return fail(ACQ_ERR_ARG, "rec_dev must be 4-byte aligned");
-    if (((uintptr_t)profile_dev & 3) != 0) return fail(ACQ_ERR_ARG, "profile_dev must be 4-byte aligned");
-    DeviceGuard g(e->device);
-    cudaStream_t st = stream ? (cudaStream_t)stream : e->stream;
-    // ordered as acq_refine_device: after the search that left the spectra, before the next one
-    if ((rc = wait_scratch(e, st, true)) || (rc = enqueue_profile(e, rec_dev, n_records, flags, excl, out_dev, profile_dev, st)))
-        return rc;
-    return hold_scratch(e, st);
+    return profile_device(e, false, rec_dev, n_records, flags, 0.0f, excl, out_dev, profile_dev, stream);
+}
+
+int acq_profile_coherent(acq_engine *e, const acq_record *rec, int n_records, int excl, acq_peak2 *out, float *profile)
+{
+    if (!e) return fail(ACQ_ERR_ARG, "engine is NULL");
+    if (!rec || !out) return fail(ACQ_ERR_ARG, "rec/out must not be NULL");
+    if (excl < 0) return fail(ACQ_ERR_ARG, "excl must be >= 0 (got %d)", excl);
+    return profile_host(e, true, rec, n_records, excl, out, profile);
+}
+
+int acq_profile_coherent_device(acq_engine *e, const acq_record *rec_dev, int n_records, float min_snr, int excl,
+                                acq_peak2 *out_dev, float *profile_dev, void *stream)
+{
+    if (!e) return fail(ACQ_ERR_ARG, "engine is NULL");
+    if (!rec_dev || !out_dev) return fail(ACQ_ERR_ARG, "rec_dev/out_dev must not be NULL");
+    int rc = check_min_snr(min_snr);
+    if (rc) return rc;
+    if (excl < 0) return fail(ACQ_ERR_ARG, "excl must be >= 0 (got %d)", excl);
+    return profile_device(e, true, rec_dev, n_records, min_snr > 0.0f ? ACQ_PROFILE_DETECTED : 0, min_snr, excl, out_dev,
+                          profile_dev, stream);
 }
 
 int acq_detected(const acq_engine *e, const acq_record *r)

@@ -2470,6 +2470,315 @@ __global__ void __launch_bounds__(256, E1B ? 1 : 2) k_profile(const ProfileArgs 
 }
 
 // ---------------------------------------------------------------------------------------------
+// K8.  Hand-off of coherent records (acq_profile_coherent*, acq_refine_coherent*).  A coherent record's dop is an index h
+// of the 1/F-bin grid (F = M (1 + half_bin)): code row d = floor(h / F), spectrum variant v = h - F d of every block
+// (the spectra the coherent search left in HBM, [cap][block][F][k2][4096]).  Group g holds blocks b = g M + j, and block
+// j >= 1 enters the group's sum rotated by theta_j = 2 pi j (v N - 16 d F) / (F N), the phase k_search_l1_coh uses.
+// Records are checked with record_marker on the coherent range M dop_lo .. M dop_hi; the caller's min_snr arrives as
+// thr_l1 with the DETECTED flag.
+// ---------------------------------------------------------------------------------------------
+constexpr int kCohPrefixCols = 4 * 32;   // TMEM columns of one thread's prefixes S_1..S_{M-1} (16 complex each)
+
+// k_profile_coh: the row at the record's h, built as k_profile<false> builds a row (variant v of each block times code
+// row d, subfft4096_inv3, the running cfma combine), then k_search_l1_coh's group logic verbatim: S_j = T saved before
+// each fold T = cfma(acc, w, T), the per-lag max of |T|^2 and |2 S_s - T|^2 in the search's order, P summed over the
+// groups.  So P is bitwise the vector the search reduced: the profile at the record's lag is acq_record.peak and its
+// first maximum is the record's lag; at M = 1 this is k_profile<false> step for step.  The prefixes live in tensor memory
+// as in the search (256 columns per CTA: threads t and t + 128 share lanes).
+__global__ void __launch_bounds__(256, 1) k_profile_coh(const ProfileCohArgs p)
+{
+    extern __shared__ __align__(1024) unsigned char smem[];
+    constexpr int L = ACQ_LAGS_L1;
+    const int row = blockIdx.x, t = threadIdx.x;
+    const int slot = row % p.n_slots, cap = row / p.n_slots;
+    const acq_record rc = p.rec[row];
+    const int marker = record_marker(rc, p.slot_sat, slot, p.sat_type, p.n_sats, p.dop_lo, p.dop_hi,
+                                     (p.flags & ACQ_PROFILE_DETECTED) != 0, p.thr_l1, p.thr_e1b);
+    float *prof = p.profile ? p.profile + (size_t)row * L : nullptr;   // every row of a coherent search is C/A
+    if (marker != 0) {   // uniform: every thread read the same record
+        const float nan = __int_as_float(0x7fc00000);   // quiet NaN
+        if (t == 0) {
+            acq_peak2 o;
+            o.peak2 = o.ratio = o.noise_ex = nan;
+            o.lag2 = marker;
+            p.out[row] = o;
+        }
+        if (prof)
+            for (int n = t; n < L; n += 256) prof[n] = nan;
+        return;
+    }
+    const FftSmem3 s = fft_smem3_carve(smem);
+    float *red_f = reinterpret_cast<float *>(smem + fft_smem3_bytes());   // [16] warp partials, [16] record's power, [48] TMEM slot
+    int *red_i = reinterpret_cast<int *>(red_f + 32);                     // [8]
+    float *pk = red_f + 16;
+    load_t2(s, p.tables, t);
+    const uint32_t tmem_base = tmem_alloc_cta<2 * kCohPrefixCols>(reinterpret_cast<uint32_t *>(red_f + 48), t);
+    const uint32_t s_taddr = tmem_base + tmem_lane_base(t) + (uint32_t)((t >> 7) * kCohPrefixCols);   // [s - 1][16 complex]
+    const float2 *base = p.tables + kT2Elems + t;
+    const int M = p.m_coh, F = p.nvar, FN = F * kN;
+    const int dop = (rc.dop >= 0 ? rc.dop : rc.dop - F + 1) / F;
+    const int v = rc.dop - F * dop;
+    int step = (v * kN - 16 * dop * F) % FN;   // theta_j in units of 1 / (F N) cycle: j * step mod F N
+    if (step < 0) step += FN;
+    Peak best;
+    best.p = -1.0f;   // every power (>= 0) wins over it
+    best.n = 0x7fffffff;
+    best.sum = 0.0f;
+    int buf = 0, j = 0, ph = 0;
+    float P[16];
+    float2 T[16];
+    for (int b = 0; b < p.K; b++) {
+        const float2 *D = p.Dp + ((size_t)((size_t)cap * p.K + b) * F + v) * kN;
+        float2 x[16], acc[16];
+#pragma unroll 1
+        for (int k2 = 0; k2 < 4; k2++) {
+            {   // x[a] = conj(data[k]) * code[k - dop], k = 1024 a + 4 t + k2
+                const int r = (k2 - dop) & 3;
+                const int q = (k2 - dop - r) >> 2;
+                const float2 *Dk = D + k2 * kSub + t;
+                const float2 *Ek = p.Ep + (size_t)(rc.sat * 4 + r) * p.ext_len + p.Q + q + t;
+#pragma unroll
+                for (int a = 0; a < 16; a++) x[a] = cmul_conj_a(__ldg(Dk + 256 * a), __ldg(Ek + 256 * a));
+            }
+            subfft4096_inv3(x, k2, __ldg(base + k2 * 256), buf, s, t);
+            buf ^= 1;
+            if (k2 == 0) {
+#pragma unroll
+                for (int n2 = 0; n2 < 16; n2++) acc[n2] = x[r16(n2)];
+            } else {
+#pragma unroll
+                for (int n2 = 0; n2 < 16; n2++) acc[n2] = cfma(x[r16(n2)], c_cC[k2][n2], acc[n2]);
+            }
+        }
+        if (j == 0) {
+#pragma unroll
+            for (int n2 = 0; n2 < 16; n2++) T[n2] = acc[n2];
+        } else {   // S_j = T, then T += exp(i theta_j) r'_b
+            tmem_st16(s_taddr + 32 * (j - 1), T);
+            tmem_wait_st();
+            float sn, cs;
+            sincospif(__fdiv_rn((float)(2 * ph), (float)FN), &sn, &cs);
+            const float2 w = make_float2(cs, sn);
+#pragma unroll
+            for (int n2 = 0; n2 < 16; n2++) T[n2] = cfma(acc[n2], w, T[n2]);
+        }
+        if (j == M - 1) {   // end of the group: best data-bit hypothesis per lag
+            float pg[16];
+#pragma unroll
+            for (int n2 = 0; n2 < 16; n2++) pg[n2] = cpower(T[n2]);
+            for (int e = 1; e < M; e++) {
+                float2 S[16];
+                tmem_ld16(s_taddr + 32 * (e - 1), S);
+                tmem_wait_ld();
+#pragma unroll
+                for (int n2 = 0; n2 < 16; n2++)
+                    pg[n2] = fmaxf(pg[n2], cpower(make_float2(2.0f * S[n2].x - T[n2].x, 2.0f * S[n2].y - T[n2].y)));
+            }
+#pragma unroll
+            for (int n2 = 0; n2 < 16; n2++) P[n2] = (b == M - 1) ? pg[n2] : (P[n2] + pg[n2]);
+            j = 0;
+            ph = 0;
+        } else {
+            j++;
+            ph += step;
+            if (ph >= FN) ph -= FN;
+        }
+    }
+#pragma unroll
+    for (int n2 = 0; n2 < 16; n2++) {
+        const int n = lag_of3(t, n2);
+        if (n < L) profile_visit(n, P[n2], rc.lag, p.excl, L, best, pk, prof);
+    }
+    const Peak tot = block_reduce_peak(best, red_f, red_i, t);   // its barrier also publishes *pk
+    if (t == 0) {
+        acq_peak2 o;
+        o.peak2 = tot.p;
+        o.lag2 = tot.n;
+        o.ratio = __fdiv_rn(*pk, tot.p);
+        o.noise_ex = __fdiv_rn(tot.sum, (float)(L - 2 * p.excl - 1));
+        p.out[row] = o;
+    }
+    tmem_free_cta<2 * kCohPrefixCols>(tmem_base, t);
+}
+
+// k_refine_coh: k_refine's five correlation sums per block -- (h - H, n), (h, n - 1), (h, n), (h, n + 1), (h + H, n) with
+// H = 1 + half_bin, one bin of the group's DFT (ACQ_BIN_HZ / M) -- where each Doppler point reads its own spectrum variant
+// and code row, (d', v') = split(h +- H, F).  Thread 0 folds block j of a group into each point's group sum rotated by
+// that point's theta_j (the search's arithmetic), keeps the prefixes, and at the group's end applies the data-bit
+// hypothesis that is the first maximum at the centre point (h, n) -- "no edge", then s = 1..M-1, the search's rule -- to
+// all five sums.  A code row shifted by d' puts e^{+j 2 pi d' n_b / N} on a block's sum at lag n_b = n + 16 b; theta_j
+// removes the 16 j d' part, so the group sum carries that of its first block, n_b0 = n + 16 g M, and the outer points
+// are put back on the centre's phase by e^{-+j 2 pi (d' - d) n_b0 / N} (the spectrum variants rotate at the undelayed
+// sample index, k_coh_variants, and add no lag-dependent phase).  Then k_refine's estimator on the group sums: num / den
+// and early / late summed over the groups, dop_hz = (h / F + delta / M) ACQ_BIN_HZ = (h + H delta) ACQ_BIN_HZ / F, peak
+// = sum over the groups of |X_g(h, n)|^2.  At M = 1 every step is k_refine's operation in k_refine's order (no rotation,
+// the three variants are one, d' = d -+ 1): the same bytes.
+__global__ void __launch_bounds__(256) k_refine_coh(const RefineCohArgs p)
+{
+    __shared__ float red[8][10];
+    __shared__ float2 pre[5][ACQ_COH_MAX - 1];   // thread 0: prefixes S_s of the five group sums
+    const int row = blockIdx.x, t = threadIdx.x;
+    const acq_record rc = p.rec[row];
+    const int cap = row / p.n_slots;
+    const int marker = record_marker(rc, p.slot_sat, row % p.n_slots, p.sat_type, p.n_sats, p.dop_lo, p.dop_hi,
+                                     (p.flags & ACQ_REFINE_DETECTED) != 0, p.thr_l1, p.thr_e1b);
+    if (marker != 0) {
+        if (t == 0) {
+            acq_fine o;
+            o.dop_hz = o.code_fs = __int_as_float(0x7fc00000);   // quiet NaN
+            o.peak = 0.0f;
+            o.ca_shift = marker;
+            p.out[row] = o;
+        }
+        return;
+    }
+    const int M = p.m_coh, F = p.nvar, H = F / M, FN = F * kN;
+    const int n = rc.lag;
+    int dd[3], vv[3], step[3], ph[3];   // Doppler points h - H, h, h + H: code row, variant, theta step, phase
+#pragma unroll
+    for (int i = 0; i < 3; i++) {
+        const int hh = rc.dop + (i - 1) * H;
+        dd[i] = (hh >= 0 ? hh : hh - F + 1) / F;
+        vv[i] = hh - F * dd[i];
+        step[i] = (vv[i] * kN - 16 * dd[i] * F) % FN;
+        if (step[i] < 0) step[i] += FN;
+        ph[i] = 0;
+    }
+    float num = 0.0f, den = 0.0f, early = 0.0f, late = 0.0f, peak = 0.0f;  // thread 0 only
+    float2 T[5];                                                           // thread 0 only: the group sums
+    for (int b = 0; b < p.K; b++) {
+        const int j = b % M;
+        const size_t blk = ((size_t)cap * p.K + b) * F;
+        const float2 *Dm = p.Dp + (blk + vv[0]) * kN, *D0 = p.Dp + (blk + vv[1]) * kN, *Dp = p.Dp + (blk + vv[2]) * kN;
+        float2 acc[5];
+#pragma unroll
+        for (int i = 0; i < 5; i++) acc[i] = make_float2(0.0f, 0.0f);
+        for (int k2 = 0; k2 < 4; k2++) {
+            const float2 *Er[3];
+#pragma unroll
+            for (int i = 0; i < 3; i++) {  // code rows of the three Doppler points
+                const int r = (k2 - dd[i]) & 3;
+                const int q = (k2 - dd[i] - r) >> 2;
+                Er[i] = p.Ep + (size_t)(rc.sat * 4 + r) * p.ext_len + p.Q + q;
+            }
+            for (int k1 = t; k1 < kSub; k1 += 256) {
+                const int k = 4 * k1 + k2;
+                float sn, cs, s1, c1;
+                sincospif((float)((k * n) & (kN - 1)) * (1.0f / 8192.0f), &sn, &cs);  // e^{+j 2 pi k n / N}
+                sincospif((float)k * (1.0f / 8192.0f), &s1, &c1);                      // e^{+j 2 pi k / N}
+                const float2 w0 = make_float2(cs, sn), wk = make_float2(c1, s1);
+                const float2 pm = cmul(cmul_conj_a(Dm[k2 * kSub + k1], Er[0][k1]), w0);
+                const float2 pc = cmul(cmul_conj_a(D0[k2 * kSub + k1], Er[1][k1]), w0);
+                const float2 pp = cmul(cmul_conj_a(Dp[k2 * kSub + k1], Er[2][k1]), w0);
+                acc[0] = cadd(acc[0], pm);
+                acc[1] = cadd(acc[1], cmul(pc, make_float2(c1, -s1)));  // lag n-1
+                acc[2] = cadd(acc[2], pc);
+                acc[3] = cadd(acc[3], cmul(pc, wk));                    // lag n+1
+                acc[4] = cadd(acc[4], pp);
+            }
+        }
+        // CTA reduction of the five complex sums
+#pragma unroll
+        for (int i = 0; i < 5; i++) {
+#pragma unroll
+            for (int off = 16; off > 0; off >>= 1) {
+                acc[i].x += __shfl_xor_sync(0xffffffffu, acc[i].x, off);
+                acc[i].y += __shfl_xor_sync(0xffffffffu, acc[i].y, off);
+            }
+        }
+        __syncthreads();  // red[] of the previous block has been consumed
+        if ((t & 31) == 0) {
+#pragma unroll
+            for (int i = 0; i < 5; i++) {
+                red[t >> 5][2 * i] = acc[i].x;
+                red[t >> 5][2 * i + 1] = acc[i].y;
+            }
+        }
+        __syncthreads();
+        if (t == 0) {
+            float2 R[5];
+#pragma unroll
+            for (int i = 0; i < 5; i++) {
+                R[i] = make_float2(0.0f, 0.0f);
+                for (int w = 0; w < 8; w++) R[i].x += red[w][2 * i], R[i].y += red[w][2 * i + 1];
+            }
+            if (j == 0) {
+#pragma unroll
+                for (int i = 0; i < 5; i++) T[i] = R[i];
+            } else {   // S_j = T, then T += exp(i theta_j) R, theta_j of each point's own (d', v')
+                float2 w[3];
+#pragma unroll
+                for (int i = 0; i < 3; i++) {
+                    float sn, cs;
+                    sincospif(__fdiv_rn((float)(2 * ph[i]), (float)FN), &sn, &cs);
+                    w[i] = make_float2(cs, sn);
+                }
+#pragma unroll
+                for (int i = 0; i < 5; i++) {
+                    pre[i][j - 1] = T[i];
+                    T[i] = cfma(R[i], w[i == 0 ? 0 : (i == 4 ? 2 : 1)], T[i]);
+                }
+            }
+            if (j == M - 1) {
+                // the data-bit hypothesis of the centre point: first maximum of |T|^2, |2 S_s - T|^2 (s = 1..M-1)
+                float pb = cpower(T[2]);
+                int sb = 0;
+                for (int e = 1; e < M; e++) {
+                    const float2 S = pre[2][e - 1];
+                    const float pw = cpower(make_float2(2.0f * S.x - T[2].x, 2.0f * S.y - T[2].y));
+                    if (pw > pb) pb = pw, sb = e;
+                }
+                float2 X[5];
+#pragma unroll
+                for (int i = 0; i < 5; i++) {
+                    X[i] = T[i];
+                    if (sb) {   // blocks before the edge +1, from it on -1: 2 S_s - T
+                        const float2 S = pre[i][sb - 1];
+                        X[i] = make_float2(2.0f * S.x - T[i].x, 2.0f * S.y - T[i].y);
+                    }
+                }
+                float sn, cs;
+                // e^{+j 2 pi n_b0 / N}, n_b0 = n + 16 g M: the lag of the group's first block in the undelayed block
+                sincospif((float)((n + 16 * (b - j)) & (kN - 1)) * (1.0f / 8192.0f), &sn, &cs);
+                const float2 Xm = dd[0] != dd[1] ? cmul(X[0], make_float2(cs, sn)) : X[0];
+                const float2 Xp = dd[2] != dd[1] ? cmul(X[4], make_float2(cs, -sn)) : X[4];
+                const float2 X0 = X[2];
+                const float2 a = csub(Xm, Xp);
+                const float2 g = csub(csub(cadd(X0, X0), Xm), Xp);
+                num += a.x * g.x + a.y * g.y;
+                den += g.x * g.x + g.y * g.y;
+                early += X[1].x * X[2].x + X[1].y * X[2].y;
+                late += X[3].x * X[2].x + X[3].y * X[2].y;
+                peak += X[2].x * X[2].x + X[2].y * X[2].y;
+#pragma unroll
+                for (int i = 0; i < 3; i++) ph[i] = 0;
+            } else {
+#pragma unroll
+                for (int i = 0; i < 3; i++) {
+                    ph[i] += step[i];
+                    if (ph[i] >= FN) ph[i] -= FN;
+                }
+            }
+        }
+    }
+    if (t == 0) {
+        float delta = den > 0.0f ? num / den : 0.0f;
+        delta = fminf(1.0f, fmaxf(-1.0f, delta));
+        float eps = (early + late) > 0.0f ? 3.0f * (late - early) / (early + late) : 0.0f;
+        eps = fminf(1.0f, fmaxf(-1.0f, eps));
+        constexpr int L = ACQ_LAGS_L1;
+        acq_fine o;
+        o.dop_hz = (__fdiv_rn((float)rc.dop, (float)F) + __fdiv_rn(delta, (float)M)) * (float)ACQ_BIN_HZ;
+        o.code_fs = (float)ACQ_DECIM * ((float)n + eps);
+        o.peak = peak;
+        int cs = (int)lrintf(o.code_fs) % (L * ACQ_DECIM);
+        if (cs < 0) cs += L * ACQ_DECIM;
+        o.ca_shift = cs;
+        p.out[row] = o;
+    }
+}
+
+// ---------------------------------------------------------------------------------------------
 // launchers
 // ---------------------------------------------------------------------------------------------
 // Launch with (pdl) or without programmatic stream serialization: with it the grid may become resident while the
@@ -2562,6 +2871,7 @@ cudaError_t search_kernels_configure()
     if ((e = cudaFuncSetAttribute(k_fwd_fft<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, fw))) return e;
     if ((e = cudaFuncSetAttribute(k_profile<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)profile_smem_bytes(false, 1)))) return e;
     if ((e = cudaFuncSetAttribute(k_profile<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)profile_smem_bytes(true, 2)))) return e;
+    if ((e = cudaFuncSetAttribute(k_profile_coh, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)profile_smem_bytes(false, 1)))) return e;
     // One shared-memory carveout for every kernel of a search.  Left to the driver, the C/A kernel (2 x 96.3 KiB) runs
     // its SMs at the 196 KiB split and the E1B kernel (2 x 103.8 KiB) at 228 KiB, and an SM changes its split only when
     // it is empty: in a GPS + Galileo search the E1B CTAs -- launched to move in as the C/A CTAs retire -- entered no SM
@@ -2799,6 +3109,20 @@ int launch_profile(const ProfileArgs &a, int n_rows, int n_l1_slots, cudaStream_
         n++;
     }
     return n;
+}
+
+int launch_refine_coh(const RefineCohArgs &a, int n_rows, cudaStream_t st)
+{
+    if (n_rows <= 0) return 0;
+    k_refine_coh<<<n_rows, 256, 0, st>>>(a);
+    return 1;
+}
+
+int launch_profile_coh(const ProfileCohArgs &a, int n_rows, cudaStream_t st)
+{
+    if (n_rows <= 0) return 0;
+    k_profile_coh<<<n_rows, 256, profile_smem_bytes(false, a.K), st>>>(a);
+    return 1;
 }
 
 #ifdef ACQ_TRACE

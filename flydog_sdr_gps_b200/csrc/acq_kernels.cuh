@@ -186,6 +186,19 @@ struct ProfileArgs {
     float thr_l1, thr_e1b;
 };
 int launch_profile(const ProfileArgs &a, int n_rows, int n_l1_slots, cudaStream_t st);
+// Refinement and profile of the records of a coherent search (acq_refine_coherent*, acq_profile_coherent*): k_refine_coh
+// and k_profile_coh, one CTA per record.  The inherited fields describe the coherent search: nvar = F = m_coh (1 +
+// half_bin) spectrum variants per block, dop_lo..dop_hi = m_coh times the engine's range (the record's 1/F-bin grid),
+// n_shift = 1.  A row is skipped (marker -1) when flags has the DETECTED bit and its snr is not >= thr_l1 (the caller's
+// min_snr); every row is C/A.
+struct RefineCohArgs : RefineArgs {
+    int m_coh;
+};
+struct ProfileCohArgs : ProfileArgs {
+    int m_coh;
+};
+int launch_refine_coh(const RefineCohArgs &a, int n_rows, cudaStream_t st);
+int launch_profile_coh(const ProfileCohArgs &a, int n_rows, cudaStream_t st);
 cudaError_t search_kernels_configure();
 
 }  // namespace acq

@@ -311,6 +311,38 @@ class AcqEngine:
         _check(self._L.acq_profile_device(self._h, rec_dev, int(n), flags, int(excl), out_dev, profile_dev, stream_ptr),
                self._L)
 
+    # ---- hand-off of a coherent search's records (the most recent search, when it was coherent)
+    def refine_coherent(self, records):
+        """acq_refine_coherent: refinement of the records of the most recent host-path coherent search -- FINE_DTYPE
+        array of the same shape (Doppler in Hz interpolated between the 1/F-bin grid points, code phase in FS samples)."""
+        r = np.ascontiguousarray(records, RECORD_DTYPE)
+        out = np.zeros(r.shape, FINE_DTYPE)
+        _check(self._L.acq_refine_coherent(self._h, r.ctypes.data, r.size, out.ctypes.data), self._L)
+        return out
+
+    def refine_coherent_device(self, rec_dev, out_dev, n, min_snr=0.0, stream_ptr=None):
+        """acq_refine_coherent_device: rec_dev (acq_record) / out_dev (acq_fine, 16-byte aligned) are device pointers
+        (ints) of the n rows of the most recent coherent search of either path.  Rows with snr < min_snr are marked
+        (ca_shift -1), not refined; min_snr <= 0 refines every row.  Enqueues on stream_ptr (None = engine stream)."""
+        _check(self._L.acq_refine_coherent_device(self._h, rec_dev, int(n), float(min_snr), out_dev, stream_ptr), self._L)
+
+    def profile_coherent(self, records, excl=4, want_profile=False):
+        """acq_profile_coherent: peak quality of the records of the most recent host-path coherent search -- PEAK2_DTYPE
+        array of the same shape; want_profile: also the lag vectors, float32 [n_records * LAGS_L1]."""
+        r = np.ascontiguousarray(records, RECORD_DTYPE)
+        out = np.zeros(r.shape, PEAK2_DTYPE)
+        prof = np.zeros(r.size * LAGS_L1, np.float32) if want_profile else None
+        _check(self._L.acq_profile_coherent(self._h, r.ctypes.data, r.size, int(excl), out.ctypes.data,
+                                            prof.ctypes.data if want_profile and prof.size else None), self._L)
+        return (out, prof) if want_profile else out
+
+    def profile_coherent_device(self, rec_dev, out_dev, n, excl=4, min_snr=0.0, profile_dev=None, stream_ptr=None):
+        """acq_profile_coherent_device: rec_dev / out_dev (acq_peak2, 16-byte aligned) / profile_dev (float32 [n *
+        LAGS_L1], or None) are device pointers (ints) of the n rows of the most recent coherent search of either path.
+        Rows with snr < min_snr are marked (lag2 -1); min_snr <= 0 evaluates every row.  Enqueues on stream_ptr."""
+        _check(self._L.acq_profile_coherent_device(self._h, rec_dev, int(n), float(min_snr), int(excl), out_dev,
+                                                   profile_dev, stream_ptr), self._L)
+
     def detected(self, records):
         """Detection rule of SearchTask (search.cpp:549,591) applied to a record array."""
         r = np.asarray(records)

@@ -12,7 +12,8 @@ all_gather_into_tensor of the 24-byte records over NCCL, device->host copy of th
 is the same without the two copies (captures already in HBM, records left there).  `refine` / `refine_resident` do the
 same for the hand-off refinement of those records (acq_refine_device on each rank, then the 16-byte fine records gathered
 the same way), and `profile` / `profile_resident` for their peak quality (acq_profile_device, 16-byte acq_peak2 rows; the
-lag profiles themselves stay on each rank).
+lag profiles themselves stay on each rank).  A coherent CaptureFarm (m_coh) hands its records off with `refine_coherent`
+/ `profile_coherent` (acq_refine_coherent_device, acq_profile_coherent_device) over the same buffers and gather.
 
 `engine` is an AcqEngine.  The CPU suite exercises the same classes under gloo with a stand-in whose
 `search_device(...)`, `refine_device(...)` and `profile_device(...)` run the oracle on CPU tensors; nothing in this module computes a search itself.
@@ -64,15 +65,39 @@ class _Farm:
         parts = [host_bytes[r * slot: r * slot + self.counts[r] * per_unit * size] for r in range(self.world)]
         return np.concatenate(parts).view(dtype)
 
-    def refine_resident(self, detected_only=True):
-        """Hand-off refinement of the local records of the last search_resident() (acq_refine_device on the current torch
-        stream) into a local fine buffer padded like d_rec, then the same padded gather; returns the gathered 16-byte
-        fine records.  detected_only: undetected rows carry the marker ca_shift = -1 instead of values.  Asynchronous."""
+    def _fine_buffers(self):
         if self.d_fine is None:   # allocated on first use: a farm that never refines keeps no fine buffers
             n = self.max_local * self.per_unit * FINE
             self.d_fine = self._empty(n)
             self.d_fine_all = self._empty(self.world * n) if self.world > 1 else self.d_fine
             self.h_fine_all = self._empty(self.d_fine_all.numel(), device="cpu", pin=self.pin)
+
+    def _pk_buffers(self):
+        if self.d_pk is None:   # allocated on first use, as the fine buffers
+            n = self.max_local * self.per_unit * PEAK2
+            self.d_pk = self._empty(n)
+            self.d_pk_all = self._empty(self.world * n) if self.world > 1 else self.d_pk
+            self.h_pk_all = self._empty(self.d_pk_all.numel(), device="cpu", pin=self.pin)
+
+    def _fine_out(self):
+        """Copy the gathered fine records out and wait: FINE_DTYPE shaped like the records."""
+        self.h_fine_all.copy_(self.d_fine_all, non_blocking=True)
+        if self.device.type == "cuda":
+            self.torch.cuda.current_stream().synchronize()
+        return self._unpad(self.h_fine_all.numpy(), self.per_unit, FINE_DTYPE).reshape(self.records_shape)
+
+    def _pk_out(self):
+        """Copy the gathered acq_peak2 rows out and wait: PEAK2_DTYPE shaped like the records."""
+        self.h_pk_all.copy_(self.d_pk_all, non_blocking=True)
+        if self.device.type == "cuda":
+            self.torch.cuda.current_stream().synchronize()
+        return self._unpad(self.h_pk_all.numpy(), self.per_unit, PEAK2_DTYPE).reshape(self.records_shape)
+
+    def refine_resident(self, detected_only=True):
+        """Hand-off refinement of the local records of the last search_resident() (acq_refine_device on the current torch
+        stream) into a local fine buffer padded like d_rec, then the same padded gather; returns the gathered 16-byte
+        fine records.  detected_only: undetected rows carry the marker ca_shift = -1 instead of values.  Asynchronous."""
+        self._fine_buffers()
         if self.n_local:
             self.eng.refine_device(self.d_rec.data_ptr(), self.d_fine.data_ptr(), self.n_local * self.per_unit,
                                    detected_only=detected_only, stream_ptr=self._stream_ptr())
@@ -83,20 +108,13 @@ class _Farm:
         """refine_resident, copy out, wait.  Returns a FINE_DTYPE array shaped like search()'s records (numpy view of the
         pinned result buffer: valid until the next refine)."""
         self.refine_resident(detected_only)
-        self.h_fine_all.copy_(self.d_fine_all, non_blocking=True)
-        if self.device.type == "cuda":
-            self.torch.cuda.current_stream().synchronize()
-        return self._unpad(self.h_fine_all.numpy(), self.per_unit, FINE_DTYPE).reshape(self.records_shape)
+        return self._fine_out()
 
     def profile_resident(self, excl=4, detected_only=True):
         """Peak quality of the local records of the last search_resident() (acq_profile_device on the current torch
         stream, no lag profiles) into a local buffer padded like d_rec, then the same padded gather; returns the gathered
         16-byte acq_peak2 rows.  detected_only: undetected rows carry the marker lag2 = -1.  Asynchronous."""
-        if self.d_pk is None:   # allocated on first use, as the fine buffers
-            n = self.max_local * self.per_unit * PEAK2
-            self.d_pk = self._empty(n)
-            self.d_pk_all = self._empty(self.world * n) if self.world > 1 else self.d_pk
-            self.h_pk_all = self._empty(self.d_pk_all.numel(), device="cpu", pin=self.pin)
+        self._pk_buffers()
         if self.n_local:
             self.eng.profile_device(self.d_rec.data_ptr(), self.d_pk.data_ptr(), self.n_local * self.per_unit, excl=excl,
                                     detected_only=detected_only, stream_ptr=self._stream_ptr())
@@ -107,10 +125,7 @@ class _Farm:
         """profile_resident, copy out, wait.  Returns a PEAK2_DTYPE array shaped like search()'s records (numpy view of
         the pinned result buffer: valid until the next profile)."""
         self.profile_resident(excl, detected_only)
-        self.h_pk_all.copy_(self.d_pk_all, non_blocking=True)
-        if self.device.type == "cuda":
-            self.torch.cuda.current_stream().synchronize()
-        return self._unpad(self.h_pk_all.numpy(), self.per_unit, PEAK2_DTYPE).reshape(self.records_shape)
+        return self._pk_out()
 
 
 class CaptureFarm(_Farm):
@@ -185,6 +200,44 @@ class CaptureFarm(_Farm):
         if self.device.type == "cuda":
             self.torch.cuda.current_stream().synchronize()
         return self._unpad(self.h_all.numpy(), self.n_sel).reshape(self.n_units, self.n_sel)
+
+    # ---- hand-off of a coherent farm's records: the same buffers and gather as refine() / profile()
+    def _need_coherent(self):
+        if self.m_coh is None:
+            raise ValueError("refine_coherent / profile_coherent need a farm created with m_coh (a coherent search)")
+
+    def refine_coherent_resident(self, min_snr=0.0):
+        """acq_refine_coherent_device of the local records of the last search_resident() on the current torch stream, then
+        the padded gather; returns the gathered 16-byte fine records.  Rows with snr < min_snr carry ca_shift = -1
+        (min_snr <= 0: every row is refined).  Asynchronous."""
+        self._need_coherent()
+        self._fine_buffers()
+        if self.n_local:
+            self.eng.refine_coherent_device(self.d_rec.data_ptr(), self.d_fine.data_ptr(), self.n_local * self.per_unit,
+                                            min_snr=min_snr, stream_ptr=self._stream_ptr())
+        self._gather(self.d_fine_all, self.d_fine)
+        return self.d_fine_all
+
+    def refine_coherent(self, min_snr=0.0):
+        """refine_coherent_resident, copy out, wait: FINE_DTYPE [n_captures, n_sel] (valid until the next refine)."""
+        self.refine_coherent_resident(min_snr)
+        return self._fine_out()
+
+    def profile_coherent_resident(self, excl=4, min_snr=0.0):
+        """acq_profile_coherent_device of the local records of the last search_resident() (no lag profiles), then the
+        padded gather; returns the gathered acq_peak2 rows.  Rows with snr < min_snr carry lag2 = -1.  Asynchronous."""
+        self._need_coherent()
+        self._pk_buffers()
+        if self.n_local:
+            self.eng.profile_coherent_device(self.d_rec.data_ptr(), self.d_pk.data_ptr(), self.n_local * self.per_unit,
+                                             excl=excl, min_snr=min_snr, stream_ptr=self._stream_ptr())
+        self._gather(self.d_pk_all, self.d_pk)
+        return self.d_pk_all
+
+    def profile_coherent(self, excl=4, min_snr=0.0):
+        """profile_coherent_resident, copy out, wait: PEAK2_DTYPE [n_captures, n_sel] (valid until the next profile)."""
+        self.profile_coherent_resident(excl, min_snr)
+        return self._pk_out()
 
     @property
     def h2d_bytes(self):

@@ -221,7 +221,8 @@ int acq_search_aided_device(acq_engine *e, const uint8_t *packed_dev, int n_capt
  * last one 4 ms code period and drift 16 samples per block against the block edges), an engine with code_doppler = 1, a
  * search of more than 2^31 - 1 (capture, satellite, cell) tiles or 2^24 capture spectra (F per block).  SBAS rows give
  * the records of acq_search.  A coherent search leaves no spectra acq_refine, acq_refine_device, acq_profile or
- * acq_profile_device could use: they return ACQ_ERR_ARG until the next acq_search. */
+ * acq_profile_device could use: they return ACQ_ERR_ARG until the next acq_search.  Its records are refined and
+ * profiled by acq_refine_coherent* and acq_profile_coherent* instead. */
 #define ACQ_COH_MAX 5
 int acq_search_coherent(acq_engine *e, const uint8_t *packed, int n_captures, const int32_t *sel, int n_sel, int m_coh,
                         acq_record *out, acq_cell *grid);
@@ -238,8 +239,8 @@ int acq_search_coherent_device(acq_engine *e, const uint8_t *packed_dev, int n_c
  *   dop_center : HOST, n_captures * n_sel int32 (n_sel = table size when sel is NULL)
  *   grid       : HOST or NULL; n_captures * n_sel * W cells, cell j of row r = coherent index lo_r + j
  * Everything else is acq_search_coherent's: the groups and data-bit hypotheses, ACQ_ERR_UNSUPPORTED for E1B rows and
- * code_doppler engines before any device work, zero records for SBAS rows, and ACQ_ERR_ARG from acq_refine* and
- * acq_profile* until the next acq_search.  ACQ_ERR_ARG also for a NULL dop_center, half_width < 0 and m_coh outside
+ * code_doppler engines before any device work, zero records for SBAS rows, ACQ_ERR_ARG from acq_refine* and
+ * acq_profile* until the next acq_search, and acq_refine_coherent* / acq_profile_coherent* for its records.  ACQ_ERR_ARG also for a NULL dop_center, half_width < 0 and m_coh outside
  * 1..ACQ_COH_MAX, reported even with a NULL engine, and for W > n_dop_c.  Synchronous. */
 int acq_search_coherent_aided(acq_engine *e, const uint8_t *packed, int n_captures, const int32_t *sel, int n_sel,
                               int m_coh, const int32_t *dop_center, int half_width, acq_record *out, acq_cell *grid);
@@ -338,6 +339,42 @@ int acq_profile(acq_engine *e, const acq_record *rec, int n_records, int excl, a
 #define ACQ_PROFILE_DETECTED 1
 int acq_profile_device(acq_engine *e, const acq_record *rec_dev, int n_records, int flags, int excl, acq_peak2 *out_dev,
                        float *profile_dev, void *stream);
+
+/* Hand-off of a coherent detection (extension): refinement and peak quality of the records of the MOST RECENT search
+ * when that search was coherent (acq_search_coherent*, full or aided).  The host forms take the records of a host-path
+ * coherent search (acq_search_coherent, acq_search_coherent_aided), the device forms those of a coherent search of either
+ * path.  After a non-coherent search (or none) all four return ACQ_ERR_ARG, as acq_refine* and acq_profile* do after a
+ * coherent one.  Rows, ordering, alignment, the per-record checks and markers, and the ACQ_ERR_ARG cases follow
+ * acq_refine / acq_refine_device / acq_profile / acq_profile_device, with two changes: a record's dop is an index of
+ * the coherent grid, checked against M*dop_lo .. M*dop_hi (dop 0 with snr 0 is still accepted), and the device forms
+ * take min_snr in place of the DETECTED flag.
+ *   min_snr : rows whose snr is not >= min_snr are skipped and marked (ca_shift -1, lag2 -1); min_snr <= 0 evaluates
+ *             every row.  ACQ_ERR_ARG for a NaN.  (acq_detected's thr_l1 does not carry over to a coherent snr.)
+ * Coherent searches have no E1B rows, so every profile row is ACQ_LAGS_L1 floats (row i at i * ACQ_LAGS_L1).
+ *
+ * acq_profile_coherent: the row at the record's index h = dop, formed as the coherent search formed it -- code row
+ * d = floor(h / F), spectrum variant v = h - F d of each block, every group's blocks added with the search's phases
+ * theta_j, the per-lag maximum over the data-bit hypotheses, the groups' powers summed -- with the search's operations in
+ * its order.  So the profile at the record's lag equals acq_record.peak to the bit and the profile's first maximum is
+ * the record's lag; peak2, lag2, ratio and noise_ex are acq_profile's reduction of that vector.  With M = 1 the rows
+ * (and profiles) are acq_profile's after acq_search of the same bytes.
+ *
+ * acq_refine_coherent: the refinement of acq_refine on the group sums.  In each group of M blocks the correlation is
+ * summed coherently at five points around the record -- Doppler indices h - H, h, h + H at its lag and lags lag-1,
+ * lag+1 at h, with H = 1 + half_bin: one bin of the group's DFT, ACQ_BIN_HZ / M -- each block rotated by the search's
+ * phase and signed by the data-bit hypothesis that is largest at (h, lag) (the search's rule, applied to all five).
+ * The three-point Doppler interpolation and the early/late code phase are then formed over the groups as acq_refine
+ * forms them over the blocks:
+ *   dop_hz  = (h + H * delta) * ACQ_BIN_HZ / F,  F = M * (1 + half_bin), |delta| <= 1
+ *   code_fs = ACQ_DECIM * (lag + eps), ca_shift as acq_refine
+ *   peak    = the sum over the groups of |group sum at (h, lag)|^2, the record's peak to fp32 precision
+ * With M = 1 the rows are acq_refine's after acq_search of the same bytes. */
+int acq_refine_coherent(acq_engine *e, const acq_record *rec, int n_records, acq_fine *out);
+int acq_refine_coherent_device(acq_engine *e, const acq_record *rec_dev, int n_records, float min_snr,
+                               acq_fine *out_dev, void *stream);
+int acq_profile_coherent(acq_engine *e, const acq_record *rec, int n_records, int excl, acq_peak2 *out, float *profile);
+int acq_profile_coherent_device(acq_engine *e, const acq_record *rec_dev, int n_records, float min_snr, int excl,
+                                acq_peak2 *out_dev, float *profile_dev, void *stream);
 
 /* Detection rule of SearchTask (gps/search.cpp:549,591): snr >= threshold of the sat's type. */
 int acq_detected(const acq_engine *e, const acq_record *r);
