@@ -12,7 +12,6 @@
 #include <cstdarg>
 #include <memory>
 #include <numeric>
-#include <type_traits>
 
 #include "acq_geom.h"
 #include "acq_kernels.cuh"
@@ -740,12 +739,13 @@ int check_excl(int excl, int n_l1)
 // Lag-vector floats of one capture's rows (acq_b200.h: L per slot)
 size_t profile_capture_len(int n_l1, int n_e1b) { return (size_t)n_l1 * ACQ_LAGS_L1 + (size_t)n_e1b * ACQ_LAGS_E1B; }
 
-// The arguments refinement and profile share: the spectra and shape of the last search (coherent: the last coherent
-// search, its F variants per block and its M times finer Doppler range), the records and the flags.  A coherent form's
-// min_snr is the threshold of its DETECTED flag (set when min_snr > 0).
+// The arguments refinement and profile share: the spectra and shape of the last search (A::kCoh: the last coherent search,
+// its F variants per block and its M times finer Doppler range), the records and the flags.  A coherent form's min_snr is
+// the threshold of its DETECTED flag (set when min_snr > 0).
 template <class A>
-A last_search_args(const acq_engine *e, bool coherent, const acq_record *rec_dev, int flags, float min_snr)
+A last_search_args(const acq_engine *e, const acq_record *rec_dev, int flags, float min_snr)
 {
+    constexpr bool coherent = A::kCoh;
     const acq_engine::LastSearch &ls = last_of(e, coherent);
     const int M = coherent ? ls.m_coh : 1;
     A a{};
@@ -769,48 +769,36 @@ A last_search_args(const acq_engine *e, bool coherent, const acq_record *rec_dev
     a.flags = flags;
     a.thr_l1 = coherent ? min_snr : e->prm.thr_l1;
     a.thr_e1b = coherent ? min_snr : e->prm.thr_e1b;
-    if constexpr (std::is_base_of_v<RefineCohArgs, A> || std::is_base_of_v<ProfileCohArgs, A>) a.m_coh = M;
+    if constexpr (coherent) a.m_coh = M;
     return a;
 }
 
 int enqueue_refine(acq_engine *e, bool coherent, const acq_record *rec_dev, int n_records, int flags, float min_snr,
                    acq_fine *out_dev, cudaStream_t st)
 {
-    if (coherent) {
-        RefineCohArgs a = last_search_args<RefineCohArgs>(e, true, rec_dev, flags, min_snr);
+    auto launch = [&](auto a) {
         a.out = out_dev;
-        e->launches += launch_refine_coh(a, n_records, st);
-    } else {
-        RefineArgs a = last_search_args<RefineArgs>(e, false, rec_dev, flags, 0.0f);
-        a.out = out_dev;
-        e->launches += launch_refine(a, n_records, st);
-    }
+        return launch_refine(a, n_records, st);
+    };
+    e->launches += coherent ? launch(last_search_args<RefineCohArgs>(e, rec_dev, flags, min_snr))
+                            : launch(last_search_args<RefineArgs>(e, rec_dev, flags, min_snr));
     CU(cudaGetLastError());
     return ACQ_OK;
-}
-
-template <class A>
-A profile_args(const acq_engine *e, bool coherent, const acq_record *rec_dev, int flags, float min_snr, int excl,
-               acq_peak2 *out_dev, float *profile_dev)
-{
-    A a = last_search_args<A>(e, coherent, rec_dev, flags, min_snr);
-    a.tables = e->d_tables;
-    a.out = out_dev;
-    a.profile = profile_dev;
-    a.n_e1b_slots = last_of(e, coherent).n_e1b;
-    a.excl = excl;
-    return a;
 }
 
 int enqueue_profile(acq_engine *e, bool coherent, const acq_record *rec_dev, int n_records, int flags, float min_snr,
                     int excl, acq_peak2 *out_dev, float *profile_dev, cudaStream_t st)
 {
-    if (coherent)   // a coherent search has C/A rows only (check_search)
-        e->launches += launch_profile_coh(
-            profile_args<ProfileCohArgs>(e, true, rec_dev, flags, min_snr, excl, out_dev, profile_dev), n_records, st);
-    else
-        e->launches += launch_profile(profile_args<ProfileArgs>(e, false, rec_dev, flags, 0.0f, excl, out_dev, profile_dev),
-                                      n_records, e->last.n_l1, st);
+    auto launch = [&](auto a) {
+        a.tables = e->d_tables;
+        a.out = out_dev;
+        a.profile = profile_dev;
+        a.n_e1b_slots = last_of(e, coherent).n_e1b;   // 0 after a coherent search (C/A rows only, check_search)
+        a.excl = excl;
+        return launch_profile(a, n_records, st);
+    };
+    e->launches += coherent ? launch(last_search_args<ProfileCohArgs>(e, rec_dev, flags, min_snr))
+                            : launch(last_search_args<ProfileArgs>(e, rec_dev, flags, min_snr));
     CU(cudaGetLastError());
     return ACQ_OK;
 }

@@ -2136,165 +2136,24 @@ __global__ void __launch_bounds__(256, 2) k_search_e1b_ldg(const SearchArgs p)
 #endif  // ACQ_VARIANT_E1B_LDG
 
 // ---------------------------------------------------------------------------------------------
-// K6.  Acquisition refinement for the hand-off to tracking (SURVEY 8(f) rank 4).  The search reports the code phase
-// in /DECIM samples and the Doppler in bins of 249.76 Hz (search.cpp:574-575); the tracking loops then need a 5 s
-// settle to pull in the LO (gps/channel.cpp:345-372) because +-125 Hz exceeds the Costas pull-in range.  For each
-// record this kernel evaluates the correlation r_d[n] = sum_k conj(D[k]) C[k-d] e^{+j 2 pi k n / N} (the very sum
-// the inverse FFT computes, search.cpp:471-481) at five points around the peak -- (d-1, n) (d, n-1) (d, n)
-// (d, n+1) (d+1, n) -- straight from the spectra the search left in HBM, and forms
-//   Doppler: delta = Re[(Xm - Xp) conj(2 X0 - Xm - Xp)] / |2 X0 - Xm - Xp|^2   (three-bin interpolation of a
-//            rectangular-window DFT; X_d = r_d[n] e^{-j 2 pi d n / N} puts the three bins on a common phase),
-//   code   : eps = slope (l - e) / (l + e),  e/l = Re(r[n-+1] conj(r[n]))       (early-minus-late over the
-//            correlation triangle: 4 samples per chip -> slope 3; BOC(1,1) main peak -> slope 1/3),
-// each summed over the K blocks.  One CTA per record; thread t owns k1 = t + 256 i for all four residues.
-// The records may come from device memory the host never saw (acq_refine_device), so each CTA checks its own record
-// first -- the checks of acq_refine, in the same order, the satellite's range before sat_type is indexed with it -- and
-// a CTA whose record fails one, or that ACQ_REFINE_DETECTED skips, writes a marker row and exits before any load of
-// the spectra (a uniform branch: every thread reads the same record).
+// K6.  Hand-off to tracking: refinement (k_refine: acq_refine*, acq_refine_coherent*) and peak quality (k_profile:
+// acq_profile*, acq_profile_coherent*) of the records of the most recent search, one 256-thread CTA per record, straight
+// from the spectra the search left in HBM.  Each kernel has an instance for the records of a non-coherent search
+// (RefineArgs / ProfileArgs) and one for those of a coherent search (RefineCohArgs / ProfileCohArgs, kCoh).  The
+// non-coherent instance is the coherent arithmetic with M the constant 1, so it compiles none of the group code.
+//   A record's dop is an index h of the 1/F-bin grid, F = nvar spectrum variants per block (1 + half_bin; coherent: M (1 +
+// half_bin)): code row d = floor(h / F), variant v = h - F d.  Block b of that Doppler index is spectrum row ((cap K + b)
+// nvar + v) n_shift + smax + cshift (d_row's rule; cshift: the code-Doppler copy, non-coherent only), which the front end
+// delayed by 16 b + cshift samples so that lag n lines up across blocks.  Coherent groups hold blocks b = g M + j; block
+// j >= 1 enters its group's sum rotated by theta_j = 2 pi j (v N - 16 d F) / (F N), the phase k_search_l1_coh uses.
+//   The records may come from device memory the host never saw (the _device forms), so each CTA first checks its own
+// record (record_marker) and a CTA whose record fails a check, or that the DETECTED flag skips, writes a marker row and
+// exits before any load of the spectra (a uniform branch: every thread reads the same record).  A coherent record is
+// checked on the range M dop_lo .. M dop_hi, and the caller's min_snr arrives as thr_l1 with the DETECTED flag.
 // ---------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256) k_refine(const RefineArgs p)
-{
-    __shared__ float red[8][10];
-    const int row = blockIdx.x, t = threadIdx.x;
-    const acq_record rc = p.rec[row];
-    const int cap = row / p.n_slots;
-    // the record checks of acq_refine, made here on a record the host may never have seen; record_marker (k_profile)
-    // restates them and must stay in step with this copy and with the host forms
-    int marker = 0;   // -2: the record fails a check, -1: skipped below the detection threshold
-    bool e1b = false;
-    if (rc.sat < 0 || rc.sat >= p.n_sats || rc.sat != p.slot_sat[row % p.n_slots]) {
-        marker = -2;
-    } else {
-        e1b = p.sat_type[rc.sat] == ACQ_E1B;
-        const int L = e1b ? ACQ_LAGS_E1B : ACQ_LAGS_L1;
-        if (rc.lag < 0 || rc.lag >= L) marker = -2;
-        // a row that never exceeded snr 0 carries dop 0 (k_best_dop), which may lie outside an asymmetric range
-        else if ((rc.dop < p.dop_lo || rc.dop > p.dop_hi) && !(rc.dop == 0 && rc.snr == 0.0f)) marker = -2;
-        else if ((p.flags & ACQ_REFINE_DETECTED) && !(rc.snr >= (e1b ? p.thr_e1b : p.thr_l1))) marker = -1;
-    }
-    if (marker != 0) {
-        if (t == 0) {
-            acq_fine o;
-            o.dop_hz = o.code_fs = __int_as_float(0x7fc00000);   // quiet NaN
-            o.peak = 0.0f;
-            o.ca_shift = marker;
-            p.out[row] = o;
-        }
-        return;
-    }
-    const int v = p.half_bin ? (rc.dop & 1) : 0;
-    const int dop = p.half_bin ? ((rc.dop - v) >> 1) : rc.dop;
-    const int n = rc.lag;
-    float num = 0.0f, den = 0.0f, early = 0.0f, late = 0.0f, peak = 0.0f;  // thread 0 only
-    for (int b = 0; b < p.K; b++) {
-        // the copy of block b the search read at this record's Doppler index (code-Doppler compensation), delayed
-        // by 16 b + cshift samples in the front end
-        const int cshift = p.n_shift > 1 ? code_shift(b, rc.dop, p.cd_div) : 0;
-        const float2 *D = p.Dp + (((size_t)((size_t)cap * p.K + b) * p.nvar + v) * p.n_shift + (p.smax + cshift)) * kN;
-        float2 acc[5];
-#pragma unroll
-        for (int j = 0; j < 5; j++) acc[j] = make_float2(0.0f, 0.0f);
-        for (int k2 = 0; k2 < 4; k2++) {
-            const float2 *Er[3];
-#pragma unroll
-            for (int j = 0; j < 3; j++) {  // code rows for Doppler dop-1, dop, dop+1
-                const int dd = dop - 1 + j;
-                const int r = (k2 - dd) & 3;
-                const int q = (k2 - dd - r) >> 2;
-                Er[j] = p.Ep + (size_t)(rc.sat * 4 + r) * p.ext_len + p.Q + q;
-            }
-            for (int k1 = t; k1 < kSub; k1 += 256) {
-                const int k = 4 * k1 + k2;
-                const float2 d = D[k2 * kSub + k1];
-                float sn, cs, s1, c1;
-                sincospif((float)((k * n) & (kN - 1)) * (1.0f / 8192.0f), &sn, &cs);  // e^{+j 2 pi k n / N}
-                sincospif((float)k * (1.0f / 8192.0f), &s1, &c1);                      // e^{+j 2 pi k / N}
-                const float2 w0 = make_float2(cs, sn), wk = make_float2(c1, s1);
-                const float2 pm = cmul(cmul_conj_a(d, Er[0][k1]), w0);
-                const float2 pc = cmul(cmul_conj_a(d, Er[1][k1]), w0);
-                const float2 pp = cmul(cmul_conj_a(d, Er[2][k1]), w0);
-                acc[0] = cadd(acc[0], pm);
-                acc[1] = cadd(acc[1], cmul(pc, make_float2(c1, -s1)));  // lag n-1
-                acc[2] = cadd(acc[2], pc);
-                acc[3] = cadd(acc[3], cmul(pc, wk));                    // lag n+1
-                acc[4] = cadd(acc[4], pp);
-            }
-        }
-        // CTA reduction of the five complex sums
-#pragma unroll
-        for (int j = 0; j < 5; j++) {
-#pragma unroll
-            for (int off = 16; off > 0; off >>= 1) {
-                acc[j].x += __shfl_xor_sync(0xffffffffu, acc[j].x, off);
-                acc[j].y += __shfl_xor_sync(0xffffffffu, acc[j].y, off);
-            }
-        }
-        __syncthreads();  // red[] of the previous block has been consumed
-        if ((t & 31) == 0) {
-#pragma unroll
-            for (int j = 0; j < 5; j++) {
-                red[t >> 5][2 * j] = acc[j].x;
-                red[t >> 5][2 * j + 1] = acc[j].y;
-            }
-        }
-        __syncthreads();
-        if (t == 0) {
-            float2 R[5];
-#pragma unroll
-            for (int j = 0; j < 5; j++) {
-                R[j] = make_float2(0.0f, 0.0f);
-                for (int w = 0; w < 8; w++) R[j].x += red[w][2 * j], R[j].y += red[w][2 * j + 1];
-            }
-            float sn, cs;
-            // w1 = e^{+j 2 pi n_b / N}, n_b = n + 16 b: the front end delayed block b by 16 b samples, so lag n of
-            // its spectrum is lag n + 16 b of the block itself -- the lag the Doppler phase term refers to
-            sincospif((float)((n + 16 * b + cshift) & (kN - 1)) * (1.0f / 8192.0f), &sn, &cs);
-            const float2 Xm = cmul(R[0], make_float2(cs, sn)), Xp = cmul(R[4], make_float2(cs, -sn)), X0 = R[2];
-            const float2 a = csub(Xm, Xp);
-            const float2 g = csub(csub(cadd(X0, X0), Xm), Xp);
-            num += a.x * g.x + a.y * g.y;
-            den += g.x * g.x + g.y * g.y;
-            early += R[1].x * R[2].x + R[1].y * R[2].y;
-            late += R[3].x * R[2].x + R[3].y * R[2].y;
-            peak += R[2].x * R[2].x + R[2].y * R[2].y;
-        }
-    }
-    if (t == 0) {
-        float delta = den > 0.0f ? num / den : 0.0f;
-        delta = fminf(1.0f, fmaxf(-1.0f, delta));
-        float eps = (early + late) > 0.0f ? (e1b ? (1.0f / 3.0f) : 3.0f) * (late - early) / (early + late) : 0.0f;
-        eps = fminf(1.0f, fmaxf(-1.0f, eps));
-        const int L = e1b ? ACQ_LAGS_E1B : ACQ_LAGS_L1;
-        acq_fine o;
-        o.dop_hz = ((p.half_bin ? 0.5f * (float)rc.dop : (float)rc.dop) + delta) * (float)ACQ_BIN_HZ;
-        o.code_fs = (float)ACQ_DECIM * ((float)n + eps);
-        o.peak = peak;
-        int cs = (int)lrintf(o.code_fs) % (L * ACQ_DECIM);
-        if (cs < 0) cs += L * ACQ_DECIM;
-        o.ca_shift = cs;
-        p.out[row] = o;
-    }
-}
-
-// ---------------------------------------------------------------------------------------------
-// K7.  Peak-quality profile of searched rows (acq_profile / acq_profile_device).  For each record the row is evaluated at
-// the record's Doppler index, exactly as the search evaluated it: the product of the capture spectrum the search left
-// in HBM (the same half-bin spectrum and code-Doppler copy, d_row's rule) with the extended code row (the same wrap),
-// four sub-FFTs of 4096 points per block, the search's radix-4 combine -- the running accumulation of the C/A kernels,
-// the parked-residue butterfly of the E1B kernels -- and the block powers summed in block order.  Every step is the
-// search kernels' own arithmetic in their order (subfft4096_inv3 computes what subfft4096_inv4 / inv4s compute), so
-// the power at every lag is bitwise the one the search reduced: the profile at the record's lag is acq_record.peak and
-// the first maximum of the profile is the record's lag.  Then one pass over the lags forms the largest power outside
-// the main lobe (circular distance > excl, the lowest lag on ties), the mean power there, and the profile row.
-// One CTA per row; E1B parks three residues in tensor memory as k_search_e1b does and, for K > 1, keeps the 64 running
-// block sums of a thread in a thread-private 64 KiB shared-memory array (the C/A sums stay in registers).  The two
-// types are two instantiations launched over the same rows: a CTA whose slot is of the other type exits at once.
-// Records are checked in the kernel with k_refine's checks and markers (lag2 = -2 / -1).
-// ---------------------------------------------------------------------------------------------
-// k_refine's checks of a record the host never saw, in the same order (k_refine keeps its own copy of them, so that its
-// code does not change; the host forms make the same checks in acq_refine / acq_profile): 0 if the record passes, -2 if
-// it fails one (the satellite's range is checked before sat_type is indexed with it), -1 if `detected_only` and it is
-// below its type's threshold.
+// The checks of the host forms (check_records), in their order, on a record the host may never have seen: 0 if the record
+// passes, -2 if it fails one (the satellite's range is checked before sat_type is indexed with it), -1 if `detected_only`
+// and it is below its type's threshold.
 __device__ __forceinline__ int record_marker(const acq_record &rc, const int *slot_sat, int slot, const int *sat_type, int n_sats,
                                              int dop_lo, int dop_hi, bool detected_only, float thr_l1, float thr_e1b)
 {
@@ -2312,311 +2171,49 @@ __device__ __forceinline__ int record_marker(const acq_record &rc, const int *sl
     return marker;
 }
 
-constexpr size_t kProfileRedBytes = 64 * sizeof(float);                 // reduction slots, the record's power, TMEM slot
-constexpr size_t kProfilePsBytes = sizeof(float) * 64 * 256;            // E1B, K > 1: running block sums [64][256]
-__host__ __device__ constexpr size_t profile_smem_bytes(bool e1b, int K)
+// Code row d = floor(h / F) of Doppler index h.  F = 1 + half_bin of a non-coherent search floors by a shift: a division
+// there moved k_refine's loads behind its twiddle arithmetic (+28 % time) and cost k_profile<E1B> a spill.
+template <class A>
+__device__ __forceinline__ int code_row(const A &p, int h)
 {
-    return fft_smem3_bytes() + kProfileRedBytes + (e1b && K > 1 ? kProfilePsBytes : 0);
+    if constexpr (A::kCoh) return (h >= 0 ? h : h - p.nvar + 1) / p.nvar;
+    else return h >> p.half_bin;
 }
 
-// One lag of the final powers: the record's power, the running maximum / sum outside the main lobe, the profile.
-__device__ __forceinline__ void profile_visit(int n, float pw, int lag, int excl, int L, Peak &best, float *pk, float *prof)
+// Block b's spectrum at variant v and code-Doppler copy cshift: row ((cap K + b) nvar + v) n_shift + smax + cshift (d_row's
+// rule).  A coherent search has one copy per spectrum (code_doppler engines are refused), so n_shift = 1 folds in there.
+template <class A>
+__device__ __forceinline__ const float2 *spectrum_row(const A &p, int cap, int b, int v, int cshift)
 {
-    if (n == lag) *pk = pw;
-    int d = n - lag;
-    d = d < 0 ? -d : d;
-    d = min(d, L - d);
-    if (d > excl) peak_merge(best, pw, n, pw);   // strict > or the lower lag on equal power
-    if (prof) prof[n] = pw;
+    const int n_shift = A::kCoh ? 1 : p.n_shift, smax = A::kCoh ? 0 : p.smax;
+    return p.Dp + (((size_t)((size_t)cap * p.K + b) * p.nvar + v) * n_shift + (smax + cshift)) * kN;
 }
 
-template <bool E1B>
-__global__ void __launch_bounds__(256, E1B ? 1 : 2) k_profile(const ProfileArgs p)
-{
-    extern __shared__ __align__(1024) unsigned char smem[];
-    constexpr int L = E1B ? ACQ_LAGS_E1B : ACQ_LAGS_L1;
-    const int row = blockIdx.x, t = threadIdx.x;
-    const int slot = row % p.n_slots, cap = row / p.n_slots;
-    if ((p.sat_type[p.slot_sat[slot]] == ACQ_E1B) != E1B) return;   // a row of the other launch
-    const acq_record rc = p.rec[row];
-    const int marker = record_marker(rc, p.slot_sat, slot, p.sat_type, p.n_sats, p.dop_lo, p.dop_hi,
-                                     (p.flags & ACQ_PROFILE_DETECTED) != 0, p.thr_l1, p.thr_e1b);
-    float *prof = nullptr;
-    if (p.profile) {   // row offset: the L of every earlier slot of this capture (uniform loop: every thread counts)
-        int e1b_before = 0;
-        for (int s0 = 0; s0 < slot; s0 += 256) {
-            const int s = s0 + t;
-            e1b_before += __syncthreads_count(s < slot && p.sat_type[p.slot_sat[s]] == ACQ_E1B);
-        }
-        const size_t cap_len = (size_t)p.n_slots * ACQ_LAGS_L1 + (size_t)p.n_e1b_slots * (ACQ_LAGS_E1B - ACQ_LAGS_L1);
-        prof = p.profile + (size_t)cap * cap_len + (size_t)slot * ACQ_LAGS_L1 + (size_t)e1b_before * (ACQ_LAGS_E1B - ACQ_LAGS_L1);
-    }
-    if (marker != 0) {   // uniform: every thread read the same record
-        const float nan = __int_as_float(0x7fc00000);   // quiet NaN
-        if (t == 0) {
-            acq_peak2 o;
-            o.peak2 = o.ratio = o.noise_ex = nan;
-            o.lag2 = marker;
-            p.out[row] = o;
-        }
-        if (prof)
-            for (int n = t; n < L; n += 256) prof[n] = nan;
-        return;
-    }
-    const FftSmem3 s = fft_smem3_carve(smem);
-    float *red_f = reinterpret_cast<float *>(smem + fft_smem3_bytes());   // [16] warp partials, [16] record's power, [48] TMEM slot
-    int *red_i = reinterpret_cast<int *>(red_f + 32);                     // [8]
-    float *pk = red_f + 16;
-    float *Pt = reinterpret_cast<float *>(smem + fft_smem3_bytes() + kProfileRedBytes) + t;   // E1B, K > 1: [64][256]
-    load_t2(s, p.tables, t);
-    uint32_t tmem_base = 0, zaddr = 0;
-    if constexpr (E1B) {   // this thread's TMEM: lane 32*(warp%4) + (t%32), columns [96*(warp/4), +96): [k2][n2] parked
-        tmem_base = tmem_alloc_cta<kE1bTmemCols>(reinterpret_cast<uint32_t *>(red_f + 48), t);
-        zaddr = tmem_base + tmem_lane_base(t) + (uint32_t)((t >> 7) * 96);
-    }
-    const float2 *base = p.tables + kT2Elems + t;
-    const int v = p.half_bin ? (rc.dop & 1) : 0;
-    const int dop = p.half_bin ? ((rc.dop - v) >> 1) : rc.dop;
-    Peak best;
-    best.p = -1.0f;   // every power (>= 0) wins over it
-    best.n = 0x7fffffff;
-    best.sum = 0.0f;
-    int buf = 0;
-    float P[16];   // C/A: block sums of this thread's lags lag_of3(t, n2)
-    for (int b = 0; b < p.K; b++) {
-        // the copy of block b the search read at this Doppler index (d_row): delayed by 16 b (+ the code-Doppler shift)
-        // samples in the front end, so lag n lines up across blocks
-        const int cshift = p.n_shift > 1 ? code_shift(b, rc.dop, p.cd_div) : 0;
-        const float2 *D = p.Dp + (((size_t)((size_t)cap * p.K + b) * p.nvar + v) * p.n_shift + (p.smax + cshift)) * kN;
-        float2 x[16], acc[16];
-#pragma unroll 1
-        for (int k2 = 0; k2 < 4; k2++) {
-            {   // x[a] = conj(data[k]) * code[k - dop], k = 1024 a + 4 t + k2   (search.cpp:471; load_products)
-                const int r = (k2 - dop) & 3;
-                const int q = (k2 - dop - r) >> 2;
-                const float2 *Dk = D + k2 * kSub + t;
-                const float2 *Ek = p.Ep + (size_t)(rc.sat * 4 + r) * p.ext_len + p.Q + q + t;
-#pragma unroll
-                for (int a = 0; a < 16; a++) x[a] = cmul_conj_a(__ldg(Dk + 256 * a), __ldg(Ek + 256 * a));
-            }
-            subfft4096_inv3(x, k2, __ldg(base + k2 * 256), buf, s, t);
-            buf ^= 1;
-            if constexpr (E1B) {
-                if (k2 < 3) {
-                    float2 z[16];
-#pragma unroll
-                    for (int n2 = 0; n2 < 16; n2++) z[n2] = (k2 == 0) ? x[r16(n2)] : cmul(x[r16(n2)], c_cC[k2][n2]);
-                    tmem_st16(zaddr + 32 * k2, z);
-                    tmem_wait_st();
-                }
-            } else {   // lags 0..4095 only: m = 0 of the radix-4 combine, accumulated as in k_search_l1
-                if (k2 == 0) {
-#pragma unroll
-                    for (int n2 = 0; n2 < 16; n2++) acc[n2] = x[r16(n2)];
-                } else {
-#pragma unroll
-                    for (int n2 = 0; n2 < 16; n2++) acc[n2] = cfma(x[r16(n2)], c_cC[k2][n2], acc[n2]);
-                }
-            }
-        }
-        const bool last = b + 1 == p.K;
-        if constexpr (E1B) {   // radix-4 combine over k2 (k_search_e1b / k_search_e1b_multi), lags lag_of3(t, n2) + 4096 m
-#pragma unroll
-            for (int c4 = 0; c4 < 4; c4++) {
-                float2 za[4], zb[4], zc[4];
-                tmem_ld4(zaddr + 0 * 32 + 8 * c4, za);
-                tmem_ld4(zaddr + 1 * 32 + 8 * c4, zb);
-                tmem_ld4(zaddr + 2 * 32 + 8 * c4, zc);
-                tmem_wait_ld();
-#pragma unroll
-                for (int i = 0; i < 4; i++) {
-                    const int n2 = 4 * c4 + i;
-                    float2 z0 = za[i], z1 = zb[i], z2 = zc[i];
-                    float2 z3 = cmul(x[r16(n2)], c_cC[3][n2]);
-                    radix4_inv(z0, z1, z2, z3);  // z_m = sum_k2 z_k2 * j^{k2*m}
-                    const float2 zz[4] = {z0, z1, z2, z3};
-#pragma unroll
-                    for (int m = 0; m < 4; m++) {
-                        float pw = cpower(zz[m]);
-                        if (b > 0) pw = Pt[(4 * n2 + m) * 256] + pw;
-                        if (!last) Pt[(4 * n2 + m) * 256] = pw;
-                        const int n = lag_of3(t, n2) + 4096 * m;
-                        if (last && n < L) profile_visit(n, pw, rc.lag, p.excl, L, best, pk, prof);
-                    }
-                }
-            }
-        } else {
-#pragma unroll
-            for (int n2 = 0; n2 < 16; n2++) P[n2] = (b == 0) ? cpower(acc[n2]) : (P[n2] + cpower(acc[n2]));
-        }
-    }
-    if constexpr (!E1B) {
-#pragma unroll
-        for (int n2 = 0; n2 < 16; n2++) {
-            const int n = lag_of3(t, n2);
-            if (n < L) profile_visit(n, P[n2], rc.lag, p.excl, L, best, pk, prof);
-        }
-    }
-    const Peak tot = block_reduce_peak(best, red_f, red_i, t);   // its barrier also publishes *pk
-    if (t == 0) {
-        acq_peak2 o;
-        o.peak2 = tot.p;
-        o.lag2 = tot.n;
-        o.ratio = __fdiv_rn(*pk, tot.p);
-        o.noise_ex = __fdiv_rn(tot.sum, (float)(L - 2 * p.excl - 1));
-        p.out[row] = o;
-    }
-    if constexpr (E1B) tmem_free_cta<kE1bTmemCols>(tmem_base, t);
-}
-
-// ---------------------------------------------------------------------------------------------
-// K8.  Hand-off of coherent records (acq_profile_coherent*, acq_refine_coherent*).  A coherent record's dop is an index h
-// of the 1/F-bin grid (F = M (1 + half_bin)): code row d = floor(h / F), spectrum variant v = h - F d of every block
-// (the spectra the coherent search left in HBM, [cap][block][F][k2][4096]).  Group g holds blocks b = g M + j, and block
-// j >= 1 enters the group's sum rotated by theta_j = 2 pi j (v N - 16 d F) / (F N), the phase k_search_l1_coh uses.
-// Records are checked with record_marker on the coherent range M dop_lo .. M dop_hi; the caller's min_snr arrives as
-// thr_l1 with the DETECTED flag.
-// ---------------------------------------------------------------------------------------------
-constexpr int kCohPrefixCols = 4 * 32;   // TMEM columns of one thread's prefixes S_1..S_{M-1} (16 complex each)
-
-// k_profile_coh: the row at the record's h, built as k_profile<false> builds a row (variant v of each block times code
-// row d, subfft4096_inv3, the running cfma combine), then k_search_l1_coh's group logic verbatim: S_j = T saved before
-// each fold T = cfma(acc, w, T), the per-lag max of |T|^2 and |2 S_s - T|^2 in the search's order, P summed over the
-// groups.  So P is bitwise the vector the search reduced: the profile at the record's lag is acq_record.peak and its
-// first maximum is the record's lag; at M = 1 this is k_profile<false> step for step.  The prefixes live in tensor memory
-// as in the search (256 columns per CTA: threads t and t + 128 share lanes).
-__global__ void __launch_bounds__(256, 1) k_profile_coh(const ProfileCohArgs p)
-{
-    extern __shared__ __align__(1024) unsigned char smem[];
-    constexpr int L = ACQ_LAGS_L1;
-    const int row = blockIdx.x, t = threadIdx.x;
-    const int slot = row % p.n_slots, cap = row / p.n_slots;
-    const acq_record rc = p.rec[row];
-    const int marker = record_marker(rc, p.slot_sat, slot, p.sat_type, p.n_sats, p.dop_lo, p.dop_hi,
-                                     (p.flags & ACQ_PROFILE_DETECTED) != 0, p.thr_l1, p.thr_e1b);
-    float *prof = p.profile ? p.profile + (size_t)row * L : nullptr;   // every row of a coherent search is C/A
-    if (marker != 0) {   // uniform: every thread read the same record
-        const float nan = __int_as_float(0x7fc00000);   // quiet NaN
-        if (t == 0) {
-            acq_peak2 o;
-            o.peak2 = o.ratio = o.noise_ex = nan;
-            o.lag2 = marker;
-            p.out[row] = o;
-        }
-        if (prof)
-            for (int n = t; n < L; n += 256) prof[n] = nan;
-        return;
-    }
-    const FftSmem3 s = fft_smem3_carve(smem);
-    float *red_f = reinterpret_cast<float *>(smem + fft_smem3_bytes());   // [16] warp partials, [16] record's power, [48] TMEM slot
-    int *red_i = reinterpret_cast<int *>(red_f + 32);                     // [8]
-    float *pk = red_f + 16;
-    load_t2(s, p.tables, t);
-    const uint32_t tmem_base = tmem_alloc_cta<2 * kCohPrefixCols>(reinterpret_cast<uint32_t *>(red_f + 48), t);
-    const uint32_t s_taddr = tmem_base + tmem_lane_base(t) + (uint32_t)((t >> 7) * kCohPrefixCols);   // [s - 1][16 complex]
-    const float2 *base = p.tables + kT2Elems + t;
-    const int M = p.m_coh, F = p.nvar, FN = F * kN;
-    const int dop = (rc.dop >= 0 ? rc.dop : rc.dop - F + 1) / F;
-    const int v = rc.dop - F * dop;
-    int step = (v * kN - 16 * dop * F) % FN;   // theta_j in units of 1 / (F N) cycle: j * step mod F N
-    if (step < 0) step += FN;
-    Peak best;
-    best.p = -1.0f;   // every power (>= 0) wins over it
-    best.n = 0x7fffffff;
-    best.sum = 0.0f;
-    int buf = 0, j = 0, ph = 0;
-    float P[16];
-    float2 T[16];
-    for (int b = 0; b < p.K; b++) {
-        const float2 *D = p.Dp + ((size_t)((size_t)cap * p.K + b) * F + v) * kN;
-        float2 x[16], acc[16];
-#pragma unroll 1
-        for (int k2 = 0; k2 < 4; k2++) {
-            {   // x[a] = conj(data[k]) * code[k - dop], k = 1024 a + 4 t + k2
-                const int r = (k2 - dop) & 3;
-                const int q = (k2 - dop - r) >> 2;
-                const float2 *Dk = D + k2 * kSub + t;
-                const float2 *Ek = p.Ep + (size_t)(rc.sat * 4 + r) * p.ext_len + p.Q + q + t;
-#pragma unroll
-                for (int a = 0; a < 16; a++) x[a] = cmul_conj_a(__ldg(Dk + 256 * a), __ldg(Ek + 256 * a));
-            }
-            subfft4096_inv3(x, k2, __ldg(base + k2 * 256), buf, s, t);
-            buf ^= 1;
-            if (k2 == 0) {
-#pragma unroll
-                for (int n2 = 0; n2 < 16; n2++) acc[n2] = x[r16(n2)];
-            } else {
-#pragma unroll
-                for (int n2 = 0; n2 < 16; n2++) acc[n2] = cfma(x[r16(n2)], c_cC[k2][n2], acc[n2]);
-            }
-        }
-        if (j == 0) {
-#pragma unroll
-            for (int n2 = 0; n2 < 16; n2++) T[n2] = acc[n2];
-        } else {   // S_j = T, then T += exp(i theta_j) r'_b
-            tmem_st16(s_taddr + 32 * (j - 1), T);
-            tmem_wait_st();
-            float sn, cs;
-            sincospif(__fdiv_rn((float)(2 * ph), (float)FN), &sn, &cs);
-            const float2 w = make_float2(cs, sn);
-#pragma unroll
-            for (int n2 = 0; n2 < 16; n2++) T[n2] = cfma(acc[n2], w, T[n2]);
-        }
-        if (j == M - 1) {   // end of the group: best data-bit hypothesis per lag
-            float pg[16];
-#pragma unroll
-            for (int n2 = 0; n2 < 16; n2++) pg[n2] = cpower(T[n2]);
-            for (int e = 1; e < M; e++) {
-                float2 S[16];
-                tmem_ld16(s_taddr + 32 * (e - 1), S);
-                tmem_wait_ld();
-#pragma unroll
-                for (int n2 = 0; n2 < 16; n2++)
-                    pg[n2] = fmaxf(pg[n2], cpower(make_float2(2.0f * S[n2].x - T[n2].x, 2.0f * S[n2].y - T[n2].y)));
-            }
-#pragma unroll
-            for (int n2 = 0; n2 < 16; n2++) P[n2] = (b == M - 1) ? pg[n2] : (P[n2] + pg[n2]);
-            j = 0;
-            ph = 0;
-        } else {
-            j++;
-            ph += step;
-            if (ph >= FN) ph -= FN;
-        }
-    }
-#pragma unroll
-    for (int n2 = 0; n2 < 16; n2++) {
-        const int n = lag_of3(t, n2);
-        if (n < L) profile_visit(n, P[n2], rc.lag, p.excl, L, best, pk, prof);
-    }
-    const Peak tot = block_reduce_peak(best, red_f, red_i, t);   // its barrier also publishes *pk
-    if (t == 0) {
-        acq_peak2 o;
-        o.peak2 = tot.p;
-        o.lag2 = tot.n;
-        o.ratio = __fdiv_rn(*pk, tot.p);
-        o.noise_ex = __fdiv_rn(tot.sum, (float)(L - 2 * p.excl - 1));
-        p.out[row] = o;
-    }
-    tmem_free_cta<2 * kCohPrefixCols>(tmem_base, t);
-}
-
-// k_refine_coh: k_refine's five correlation sums per block -- (h - H, n), (h, n - 1), (h, n), (h, n + 1), (h + H, n) with
-// H = 1 + half_bin, one bin of the group's DFT (ACQ_BIN_HZ / M) -- where each Doppler point reads its own spectrum variant
-// and code row, (d', v') = split(h +- H, F).  Thread 0 folds block j of a group into each point's group sum rotated by
-// that point's theta_j (the search's arithmetic), keeps the prefixes, and at the group's end applies the data-bit
+// k_refine (SURVEY 8(f) rank 4).  The search reports the code phase in /DECIM samples and the Doppler in bins of 249.76 Hz
+// (search.cpp:574-575); the tracking loops then need a 5 s settle to pull in the LO (gps/channel.cpp:345-372) because
+// +-125 Hz exceeds the Costas pull-in range.  For each record this kernel evaluates the correlation
+// r_h[n] = sum_k conj(D[k]) C[k-d] e^{+j 2 pi k n / N} (the very sum the inverse FFT computes, search.cpp:471-481) at five
+// points around the peak -- (h - H, n) (h, n - 1) (h, n) (h, n + 1) (h + H, n), H = F / M: one bin of the group's DFT
+// (ACQ_BIN_HZ / M) -- each Doppler point at its own (d', v') = split(h +- H), so at M > 1 it reads its own spectrum
+// variant and code row (at M = 1 the three points share v and d' = d -+ 1).  Thread 0 folds block j of a group into each
+// point's group sum rotated by that point's theta_j, keeps the prefixes, and at the group's end applies the data-bit
 // hypothesis that is the first maximum at the centre point (h, n) -- "no edge", then s = 1..M-1, the search's rule -- to
-// all five sums.  A code row shifted by d' puts e^{+j 2 pi d' n_b / N} on a block's sum at lag n_b = n + 16 b; theta_j
-// removes the 16 j d' part, so the group sum carries that of its first block, n_b0 = n + 16 g M, and the outer points
-// are put back on the centre's phase by e^{-+j 2 pi (d' - d) n_b0 / N} (the spectrum variants rotate at the undelayed
-// sample index, k_coh_variants, and add no lag-dependent phase).  Then k_refine's estimator on the group sums: num / den
-// and early / late summed over the groups, dop_hz = (h / F + delta / M) ACQ_BIN_HZ = (h + H delta) ACQ_BIN_HZ / F, peak
-// = sum over the groups of |X_g(h, n)|^2.  At M = 1 every step is k_refine's operation in k_refine's order (no rotation,
-// the three variants are one, d' = d -+ 1): the same bytes.
-__global__ void __launch_bounds__(256) k_refine_coh(const RefineCohArgs p)
+// all five sums.  A code row shifted by d' puts e^{+j 2 pi d' n_b / N} on a block's sum at lag n_b = n + 16 b + cshift;
+// theta_j removes the 16 j d' part, so a group sum carries that of its first block, n_b0 = n + 16 (b - j) + cshift, and
+// the outer points are put back on the centre's phase by e^{-+j 2 pi (d' - d) n_b0 / N} where d' != d (the spectrum
+// variants rotate at the undelayed sample index, k_coh_variants, and add no lag-dependent phase).  Then, summed over the
+// groups:
+//   Doppler: delta = Re[(Xm - Xp) conj(2 X0 - Xm - Xp)] / |2 X0 - Xm - Xp|^2   (three-bin interpolation of a
+//            rectangular-window DFT), dop_hz = (h / F + delta / M) ACQ_BIN_HZ,
+//   code   : eps = slope (l - e) / (l + e),  e/l = Re(X[n-+1] conj(X[n]))       (early-minus-late over the
+//            correlation triangle: 4 samples per chip -> slope 3; BOC(1,1) main peak -> slope 1/3),
+//   peak   : sum of |X(h, n)|^2.
+// Thread t owns k1 = t + 256 i for all four residues.
+template <class RA>
+__global__ void __launch_bounds__(256) k_refine(const RA p)
 {
     __shared__ float red[8][10];
-    __shared__ float2 pre[5][ACQ_COH_MAX - 1];   // thread 0: prefixes S_s of the five group sums
+    __shared__ float2 pre[5][ACQ_COH_MAX - 1];   // coherent, thread 0: prefixes S_s of the five group sums
     const int row = blockIdx.x, t = threadIdx.x;
     const acq_record rc = p.rec[row];
     const int cap = row / p.n_slots;
@@ -2632,13 +2229,17 @@ __global__ void __launch_bounds__(256) k_refine_coh(const RefineCohArgs p)
         }
         return;
     }
-    const int M = p.m_coh, F = p.nvar, H = F / M, FN = F * kN;
+    // every row of a coherent search is C/A (reading its type moved the coherent instance's loads: +5 % time)
+    const bool e1b = !RA::kCoh && p.sat_type[rc.sat] == ACQ_E1B;
+    int M = 1;
+    if constexpr (RA::kCoh) M = p.m_coh;
+    const int F = p.nvar, H = F / M, FN = F * kN;
     const int n = rc.lag;
     int dd[3], vv[3], step[3], ph[3];   // Doppler points h - H, h, h + H: code row, variant, theta step, phase
 #pragma unroll
     for (int i = 0; i < 3; i++) {
         const int hh = rc.dop + (i - 1) * H;
-        dd[i] = (hh >= 0 ? hh : hh - F + 1) / F;
+        dd[i] = code_row(p, hh);
         vv[i] = hh - F * dd[i];
         step[i] = (vv[i] * kN - 16 * dd[i] * F) % FN;
         if (step[i] < 0) step[i] += FN;
@@ -2648,8 +2249,10 @@ __global__ void __launch_bounds__(256) k_refine_coh(const RefineCohArgs p)
     float2 T[5];                                                           // thread 0 only: the group sums
     for (int b = 0; b < p.K; b++) {
         const int j = b % M;
-        const size_t blk = ((size_t)cap * p.K + b) * F;
-        const float2 *Dm = p.Dp + (blk + vv[0]) * kN, *D0 = p.Dp + (blk + vv[1]) * kN, *Dp = p.Dp + (blk + vv[2]) * kN;
+        const int cshift = !RA::kCoh && p.n_shift > 1 ? code_shift(b, rc.dop, p.cd_div) : 0;
+        const float2 *D0 = spectrum_row(p, cap, b, vv[1], cshift);
+        const float2 *Dm = RA::kCoh ? spectrum_row(p, cap, b, vv[0], 0) : D0;
+        const float2 *Dp = RA::kCoh ? spectrum_row(p, cap, b, vv[2], 0) : D0;
         float2 acc[5];
 #pragma unroll
         for (int i = 0; i < 5; i++) acc[i] = make_float2(0.0f, 0.0f);
@@ -2738,10 +2341,9 @@ __global__ void __launch_bounds__(256) k_refine_coh(const RefineCohArgs p)
                     }
                 }
                 float sn, cs;
-                // e^{+j 2 pi n_b0 / N}, n_b0 = n + 16 g M: the lag of the group's first block in the undelayed block
-                sincospif((float)((n + 16 * (b - j)) & (kN - 1)) * (1.0f / 8192.0f), &sn, &cs);
-                const float2 Xm = dd[0] != dd[1] ? cmul(X[0], make_float2(cs, sn)) : X[0];
-                const float2 Xp = dd[2] != dd[1] ? cmul(X[4], make_float2(cs, -sn)) : X[4];
+                sincospif((float)((n + 16 * (b - j) + cshift) & (kN - 1)) * (1.0f / 8192.0f), &sn, &cs);
+                const float2 Xm = !RA::kCoh || dd[0] != dd[1] ? cmul(X[0], make_float2(cs, sn)) : X[0];
+                const float2 Xp = !RA::kCoh || dd[2] != dd[1] ? cmul(X[4], make_float2(cs, -sn)) : X[4];
                 const float2 X0 = X[2];
                 const float2 a = csub(Xm, Xp);
                 const float2 g = csub(csub(cadd(X0, X0), Xm), Xp);
@@ -2764,11 +2366,13 @@ __global__ void __launch_bounds__(256) k_refine_coh(const RefineCohArgs p)
     if (t == 0) {
         float delta = den > 0.0f ? num / den : 0.0f;
         delta = fminf(1.0f, fmaxf(-1.0f, delta));
-        float eps = (early + late) > 0.0f ? 3.0f * (late - early) / (early + late) : 0.0f;
+        float eps = (early + late) > 0.0f ? (e1b ? (1.0f / 3.0f) : 3.0f) * (late - early) / (early + late) : 0.0f;
         eps = fminf(1.0f, fmaxf(-1.0f, eps));
-        constexpr int L = ACQ_LAGS_L1;
+        const int L = e1b ? ACQ_LAGS_E1B : ACQ_LAGS_L1;
+        // h / F + delta / M; at F = 1 + half_bin and M = 1 the same value without two divisions on every CTA's tail
+        const float h_bins = RA::kCoh ? __fdiv_rn((float)rc.dop, (float)F) : (p.half_bin ? 0.5f : 1.0f) * (float)rc.dop;
         acq_fine o;
-        o.dop_hz = (__fdiv_rn((float)rc.dop, (float)F) + __fdiv_rn(delta, (float)M)) * (float)ACQ_BIN_HZ;
+        o.dop_hz = (h_bins + (RA::kCoh ? __fdiv_rn(delta, (float)M) : delta)) * (float)ACQ_BIN_HZ;
         o.code_fs = (float)ACQ_DECIM * ((float)n + eps);
         o.peak = peak;
         int cs = (int)lrintf(o.code_fs) % (L * ACQ_DECIM);
@@ -2776,6 +2380,230 @@ __global__ void __launch_bounds__(256) k_refine_coh(const RefineCohArgs p)
         o.ca_shift = cs;
         p.out[row] = o;
     }
+}
+
+// k_profile.  Each record's row is evaluated once more at the record's Doppler index, exactly as the search evaluated it:
+// the product of the capture spectrum the search read (variant v, the code-Doppler copy) with the extended code row d
+// (the same wrap), four sub-FFTs of 4096 points per block, the search's radix-4 combine -- the running accumulation of
+// the C/A kernels, the parked-residue butterfly of the E1B kernels -- and the block powers summed in block order, or for a
+// coherent search k_search_l1_coh's group step (coh_fold).  Every step is the search kernels' own arithmetic in their
+// order (subfft4096_inv3 computes what subfft4096_inv4 / inv4s compute), so the power at every lag is bitwise the one
+// the search reduced: the profile at the record's lag is acq_record.peak and the first maximum of the profile is the
+// record's lag.  Then one pass over the lags forms the largest power outside the main lobe (circular distance > excl,
+// the lowest lag on ties), the mean power there, and the profile row.
+// E1B parks three residues in tensor memory as k_search_e1b does and, for K > 1, keeps the 64 running block sums of a
+// thread in a thread-private 64 KiB shared-memory array (the C/A sums stay in registers); the coherent instance keeps the
+// group prefixes in tensor memory as the search does (256 columns per CTA: threads t and t + 128 share lanes).  C/A and
+// E1B rows of a non-coherent search are two instances launched over the same rows: a CTA whose slot is of the other type
+// exits at once.  Every row of a coherent search is C/A.
+constexpr size_t kProfileRedBytes = 64 * sizeof(float);                 // reduction slots, the record's power, TMEM slot
+constexpr size_t kProfilePsBytes = sizeof(float) * 64 * 256;            // E1B, K > 1: running block sums [64][256]
+__host__ __device__ constexpr size_t profile_smem_bytes(bool e1b, int K)
+{
+    return fft_smem3_bytes() + kProfileRedBytes + (e1b && K > 1 ? kProfilePsBytes : 0);
+}
+constexpr int kCohPrefixCols = 4 * 32;   // TMEM columns of one thread's prefixes S_1..S_{M-1} (16 complex each)
+
+// One lag of the final powers: the record's power, the running maximum / sum outside the main lobe, the profile.
+__device__ __forceinline__ void profile_visit(int n, float pw, int lag, int excl, int L, Peak &best, float *pk, float *prof)
+{
+    if (n == lag) *pk = pw;
+    int d = n - lag;
+    d = d < 0 ? -d : d;
+    d = min(d, L - d);
+    if (d > excl) peak_merge(best, pw, n, pw);   // strict > or the lower lag on equal power
+    if (prof) prof[n] = pw;
+}
+
+// k_search_l1_coh's group step, in its operations and order: block b, the j-th of its group, with this thread's 16 lag
+// values acc.  S_j = T is parked in tensor memory at s_taddr + 32 (j - 1) before T += exp(i theta_j) acc, theta_j =
+// 2 pi ph / (F N); at the group's end the best data-bit hypothesis of each lag goes into P, and j / ph advance by one
+// block (ph by the record's theta step).  At M = 1 it is P = b == 0 ? |acc|^2 : P + |acc|^2.
+__device__ __forceinline__ void coh_fold(const float2 (&acc)[16], float2 (&T)[16], float (&P)[16], int &j, int &ph, int b,
+                                         int M, int step, int FN, uint32_t s_taddr)
+{
+    if (j == 0) {
+#pragma unroll
+        for (int n2 = 0; n2 < 16; n2++) T[n2] = acc[n2];
+    } else {   // S_j = T, then T += exp(i theta_j) r'_b
+        tmem_st16(s_taddr + 32 * (j - 1), T);
+        tmem_wait_st();
+        float sn, cs;
+        sincospif(__fdiv_rn((float)(2 * ph), (float)FN), &sn, &cs);
+        const float2 w = make_float2(cs, sn);
+#pragma unroll
+        for (int n2 = 0; n2 < 16; n2++) T[n2] = cfma(acc[n2], w, T[n2]);
+    }
+    if (j == M - 1) {   // end of the group: best data-bit hypothesis per lag
+        float pg[16];
+#pragma unroll
+        for (int n2 = 0; n2 < 16; n2++) pg[n2] = cpower(T[n2]);
+        for (int e = 1; e < M; e++) {
+            float2 S[16];
+            tmem_ld16(s_taddr + 32 * (e - 1), S);
+            tmem_wait_ld();
+#pragma unroll
+            for (int n2 = 0; n2 < 16; n2++)
+                pg[n2] = fmaxf(pg[n2], cpower(make_float2(2.0f * S[n2].x - T[n2].x, 2.0f * S[n2].y - T[n2].y)));
+        }
+#pragma unroll
+        for (int n2 = 0; n2 < 16; n2++) P[n2] = (b == M - 1) ? pg[n2] : (P[n2] + pg[n2]);
+        j = 0;
+        ph = 0;
+    } else {
+        j++;
+        ph += step;
+        if (ph >= FN) ph -= FN;
+    }
+}
+
+template <class PA, bool E1B>
+__global__ void __launch_bounds__(256, E1B || PA::kCoh ? 1 : 2) k_profile(const PA p)
+{
+    extern __shared__ __align__(1024) unsigned char smem[];
+    constexpr int L = E1B ? ACQ_LAGS_E1B : ACQ_LAGS_L1;
+    constexpr int kTmemCols = E1B ? kE1bTmemCols : (PA::kCoh ? 2 * kCohPrefixCols : 0);
+    const int row = blockIdx.x, t = threadIdx.x;
+    const int slot = row % p.n_slots, cap = row / p.n_slots;
+    if (!PA::kCoh && (p.sat_type[p.slot_sat[slot]] == ACQ_E1B) != E1B) return;   // a row of the other launch
+    const acq_record rc = p.rec[row];
+    const int marker = record_marker(rc, p.slot_sat, slot, p.sat_type, p.n_sats, p.dop_lo, p.dop_hi,
+                                     (p.flags & ACQ_PROFILE_DETECTED) != 0, p.thr_l1, p.thr_e1b);
+    float *prof = nullptr;
+    if (p.profile) {
+        if constexpr (PA::kCoh) {
+            prof = p.profile + (size_t)row * L;
+        } else {   // row offset: the L of every earlier slot of this capture (uniform loop: every thread counts)
+            int e1b_before = 0;
+            for (int s0 = 0; s0 < slot; s0 += 256) {
+                const int s = s0 + t;
+                e1b_before += __syncthreads_count(s < slot && p.sat_type[p.slot_sat[s]] == ACQ_E1B);
+            }
+            const size_t cap_len = (size_t)p.n_slots * ACQ_LAGS_L1 + (size_t)p.n_e1b_slots * (ACQ_LAGS_E1B - ACQ_LAGS_L1);
+            prof = p.profile + (size_t)cap * cap_len + (size_t)slot * ACQ_LAGS_L1 + (size_t)e1b_before * (ACQ_LAGS_E1B - ACQ_LAGS_L1);
+        }
+    }
+    if (marker != 0) {   // uniform: every thread read the same record
+        const float nan = __int_as_float(0x7fc00000);   // quiet NaN
+        if (t == 0) {
+            acq_peak2 o;
+            o.peak2 = o.ratio = o.noise_ex = nan;
+            o.lag2 = marker;
+            p.out[row] = o;
+        }
+        if (prof)
+            for (int n = t; n < L; n += 256) prof[n] = nan;
+        return;
+    }
+    const FftSmem3 s = fft_smem3_carve(smem);
+    float *red_f = reinterpret_cast<float *>(smem + fft_smem3_bytes());   // [16] warp partials, [16] record's power, [48] TMEM slot
+    int *red_i = reinterpret_cast<int *>(red_f + 32);                     // [8]
+    float *pk = red_f + 16;
+    float *Pt = reinterpret_cast<float *>(smem + fft_smem3_bytes() + kProfileRedBytes) + t;   // E1B, K > 1: [64][256]
+    load_t2(s, p.tables, t);
+    // this thread's TMEM: lane 32*(warp%4) + (t%32); E1B: columns [96*(warp/4), +96), [k2][n2] parked; coherent: columns
+    // [kCohPrefixCols*(warp/4), +kCohPrefixCols), [s - 1][16 complex]
+    uint32_t tmem_base = 0, taddr = 0;
+    if constexpr (kTmemCols > 0) {
+        tmem_base = tmem_alloc_cta<kTmemCols>(reinterpret_cast<uint32_t *>(red_f + 48), t);
+        taddr = tmem_base + tmem_lane_base(t) + (uint32_t)((t >> 7) * (E1B ? 96 : kCohPrefixCols));
+    }
+    const float2 *base = p.tables + kT2Elems + t;
+    int M = 1;
+    if constexpr (PA::kCoh) M = p.m_coh;
+    const int F = p.nvar, FN = F * kN;
+    const int dop = code_row(p, rc.dop);
+    const int v = rc.dop - F * dop;
+    int step = (v * kN - 16 * dop * F) % FN;   // theta_j in units of 1 / (F N) cycle: j * step mod F N
+    if (step < 0) step += FN;
+    Peak best;
+    best.p = -1.0f;   // every power (>= 0) wins over it
+    best.n = 0x7fffffff;
+    best.sum = 0.0f;
+    int buf = 0, j = 0, ph = 0;
+    float P[16];    // C/A: block (group) sums of this thread's lags lag_of3(t, n2)
+    float2 T[16];   // C/A: the running group sum
+    for (int b = 0; b < p.K; b++) {
+        const int cshift = !PA::kCoh && p.n_shift > 1 ? code_shift(b, rc.dop, p.cd_div) : 0;
+        const float2 *D = spectrum_row(p, cap, b, v, cshift);
+        float2 x[16], acc[16];
+#pragma unroll 1
+        for (int k2 = 0; k2 < 4; k2++) {
+            {   // x[a] = conj(data[k]) * code[k - dop], k = 1024 a + 4 t + k2   (search.cpp:471; load_products)
+                const int r = (k2 - dop) & 3;
+                const int q = (k2 - dop - r) >> 2;
+                const float2 *Dk = D + k2 * kSub + t;
+                const float2 *Ek = p.Ep + (size_t)(rc.sat * 4 + r) * p.ext_len + p.Q + q + t;
+#pragma unroll
+                for (int a = 0; a < 16; a++) x[a] = cmul_conj_a(__ldg(Dk + 256 * a), __ldg(Ek + 256 * a));
+            }
+            subfft4096_inv3(x, k2, __ldg(base + k2 * 256), buf, s, t);
+            buf ^= 1;
+            if constexpr (E1B) {
+                if (k2 < 3) {
+                    float2 z[16];
+#pragma unroll
+                    for (int n2 = 0; n2 < 16; n2++) z[n2] = (k2 == 0) ? x[r16(n2)] : cmul(x[r16(n2)], c_cC[k2][n2]);
+                    tmem_st16(taddr + 32 * k2, z);
+                    tmem_wait_st();
+                }
+            } else {   // lags 0..4095 only: m = 0 of the radix-4 combine, accumulated as in k_search_l1
+                if (k2 == 0) {
+#pragma unroll
+                    for (int n2 = 0; n2 < 16; n2++) acc[n2] = x[r16(n2)];
+                } else {
+#pragma unroll
+                    for (int n2 = 0; n2 < 16; n2++) acc[n2] = cfma(x[r16(n2)], c_cC[k2][n2], acc[n2]);
+                }
+            }
+        }
+        const bool last = b + 1 == p.K;
+        if constexpr (E1B) {   // radix-4 combine over k2 (k_search_e1b / k_search_e1b_multi), lags lag_of3(t, n2) + 4096 m
+#pragma unroll
+            for (int c4 = 0; c4 < 4; c4++) {
+                float2 za[4], zb[4], zc[4];
+                tmem_ld4(taddr + 0 * 32 + 8 * c4, za);
+                tmem_ld4(taddr + 1 * 32 + 8 * c4, zb);
+                tmem_ld4(taddr + 2 * 32 + 8 * c4, zc);
+                tmem_wait_ld();
+#pragma unroll
+                for (int i = 0; i < 4; i++) {
+                    const int n2 = 4 * c4 + i;
+                    float2 z0 = za[i], z1 = zb[i], z2 = zc[i];
+                    float2 z3 = cmul(x[r16(n2)], c_cC[3][n2]);
+                    radix4_inv(z0, z1, z2, z3);  // z_m = sum_k2 z_k2 * j^{k2*m}
+                    const float2 zz[4] = {z0, z1, z2, z3};
+#pragma unroll
+                    for (int m = 0; m < 4; m++) {
+                        float pw = cpower(zz[m]);
+                        if (b > 0) pw = Pt[(4 * n2 + m) * 256] + pw;
+                        if (!last) Pt[(4 * n2 + m) * 256] = pw;
+                        const int n = lag_of3(t, n2) + 4096 * m;
+                        if (last && n < L) profile_visit(n, pw, rc.lag, p.excl, L, best, pk, prof);
+                    }
+                }
+            }
+        } else {
+            coh_fold(acc, T, P, j, ph, b, M, step, FN, taddr);
+        }
+    }
+    if constexpr (!E1B) {
+#pragma unroll
+        for (int n2 = 0; n2 < 16; n2++) {
+            const int n = lag_of3(t, n2);
+            if (n < L) profile_visit(n, P[n2], rc.lag, p.excl, L, best, pk, prof);
+        }
+    }
+    const Peak tot = block_reduce_peak(best, red_f, red_i, t);   // its barrier also publishes *pk
+    if (t == 0) {
+        acq_peak2 o;
+        o.peak2 = tot.p;
+        o.lag2 = tot.n;
+        o.ratio = __fdiv_rn(*pk, tot.p);
+        o.noise_ex = __fdiv_rn(tot.sum, (float)(L - 2 * p.excl - 1));
+        p.out[row] = o;
+    }
+    if constexpr (kTmemCols > 0) tmem_free_cta<kTmemCols>(tmem_base, t);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -2869,9 +2697,9 @@ cudaError_t search_kernels_configure()
     if ((e = cudaFuncSetAttribute(k_fwd_fft_cluster<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, fc))) return e;
     if ((e = cudaFuncSetAttribute(k_fwd_fft<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, fw))) return e;
     if ((e = cudaFuncSetAttribute(k_fwd_fft<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, fw))) return e;
-    if ((e = cudaFuncSetAttribute(k_profile<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)profile_smem_bytes(false, 1)))) return e;
-    if ((e = cudaFuncSetAttribute(k_profile<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)profile_smem_bytes(true, 2)))) return e;
-    if ((e = cudaFuncSetAttribute(k_profile_coh, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)profile_smem_bytes(false, 1)))) return e;
+    if ((e = cudaFuncSetAttribute(k_profile<ProfileArgs, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)profile_smem_bytes(false, 1)))) return e;
+    if ((e = cudaFuncSetAttribute(k_profile<ProfileArgs, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)profile_smem_bytes(true, 2)))) return e;
+    if ((e = cudaFuncSetAttribute(k_profile<ProfileCohArgs, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)profile_smem_bytes(false, 1)))) return e;
     // One shared-memory carveout for every kernel of a search.  Left to the driver, the C/A kernel (2 x 96.3 KiB) runs
     // its SMs at the 196 KiB split and the E1B kernel (2 x 103.8 KiB) at 228 KiB, and an SM changes its split only when
     // it is empty: in a GPS + Galileo search the E1B CTAs -- launched to move in as the C/A CTAs retire -- entered no SM
@@ -3089,41 +2917,35 @@ int launch_coh_variants(float2 *x2, const float2 *rot, int n_rows, int F, int K,
     return launched;
 }
 
-int launch_refine(const RefineArgs &a, int n_rows, cudaStream_t st)
+template <class RA>
+int launch_refine(const RA &a, int n_rows, cudaStream_t st)
 {
     if (n_rows <= 0) return 0;
-    k_refine<<<n_rows, 256, 0, st>>>(a);
+    k_refine<RA><<<n_rows, 256, 0, st>>>(a);
     return 1;
 }
+template int launch_refine(const RefineArgs &, int, cudaStream_t);
+template int launch_refine(const RefineCohArgs &, int, cudaStream_t);
 
-int launch_profile(const ProfileArgs &a, int n_rows, int n_l1_slots, cudaStream_t st)
+template <class PA>
+int launch_profile(const PA &a, int n_rows, cudaStream_t st)
 {
     if (n_rows <= 0) return 0;
     int n = 0;
-    if (n_l1_slots > 0) {
-        k_profile<false><<<n_rows, 256, profile_smem_bytes(false, a.K), st>>>(a);
+    if (a.n_slots > a.n_e1b_slots) {
+        k_profile<PA, false><<<n_rows, 256, profile_smem_bytes(false, a.K), st>>>(a);
         n++;
     }
-    if (a.n_e1b_slots > 0) {
-        k_profile<true><<<n_rows, 256, profile_smem_bytes(true, a.K), st>>>(a);
-        n++;
+    if constexpr (!PA::kCoh) {
+        if (a.n_e1b_slots > 0) {
+            k_profile<PA, true><<<n_rows, 256, profile_smem_bytes(true, a.K), st>>>(a);
+            n++;
+        }
     }
     return n;
 }
-
-int launch_refine_coh(const RefineCohArgs &a, int n_rows, cudaStream_t st)
-{
-    if (n_rows <= 0) return 0;
-    k_refine_coh<<<n_rows, 256, 0, st>>>(a);
-    return 1;
-}
-
-int launch_profile_coh(const ProfileCohArgs &a, int n_rows, cudaStream_t st)
-{
-    if (n_rows <= 0) return 0;
-    k_profile_coh<<<n_rows, 256, profile_smem_bytes(false, a.K), st>>>(a);
-    return 1;
-}
+template int launch_profile(const ProfileArgs &, int, cudaStream_t);
+template int launch_profile(const ProfileCohArgs &, int, cudaStream_t);
 
 #ifdef ACQ_TRACE
 }  // namespace acq

@@ -154,9 +154,10 @@ bool search_claims_tiles(long long n_tiles, int grid);   // tiles claimed from a
 void search_chunks(long long n_tiles, int grid, unsigned *n_big, unsigned *n_mid);
 long long search_chunk_count(long long n_tiles, int grid);
 void search_chunk_lengths(int *big, int *mid);
-// refinement of the records of the most recent search (one CTA per record).  Each CTA checks its record against the
-// search's shape (slot_sat, n_sats, dop_lo..dop_hi) and writes a marker row for one that fails (ca_shift -2) or, with
-// ACQ_REFINE_DETECTED in flags, for one below its satellite type's threshold (ca_shift -1)
+// Refinement (k_refine) and peak-quality profile (k_profile) of the records of the most recent search, one CTA per record.
+// Each CTA checks its record against the search's shape (slot_sat, n_sats, dop_lo..dop_hi) and writes a marker row for one
+// that fails (ca_shift / lag2 -2) or, with ACQ_REFINE_DETECTED / ACQ_PROFILE_DETECTED in flags, for one below its
+// satellite type's threshold (-1).  launch_profile launches the C/A rows and the E1B rows (n_e1b_slots > 0) separately.
 struct RefineArgs {
     const float2 *Dp;
     const float2 *Ep;
@@ -167,11 +168,8 @@ struct RefineArgs {
     int n_slots, K, nvar, half_bin, ext_len, Q, n_shift, smax, cd_div;
     int n_sats, dop_lo, dop_hi, flags;
     float thr_l1, thr_e1b;
+    static constexpr bool kCoh = false;
 };
-int launch_refine(const RefineArgs &a, int n_rows, cudaStream_t st);
-// peak-quality profile of the records of the most recent search (acq_profile): one CTA per record in each of two
-// launches, the C/A rows (n_l1_slots > 0) and the E1B rows (n_e1b_slots > 0).  Record checks and markers (lag2 -2 / -1
-// with ACQ_PROFILE_DETECTED in flags) as launch_refine
 struct ProfileArgs {
     const float2 *Dp;
     const float2 *Ep;
@@ -184,21 +182,25 @@ struct ProfileArgs {
     int n_slots, n_e1b_slots, K, nvar, half_bin, ext_len, Q, n_shift, smax, cd_div;
     int n_sats, dop_lo, dop_hi, flags, excl;
     float thr_l1, thr_e1b;
+    static constexpr bool kCoh = false;
 };
-int launch_profile(const ProfileArgs &a, int n_rows, int n_l1_slots, cudaStream_t st);
-// Refinement and profile of the records of a coherent search (acq_refine_coherent*, acq_profile_coherent*): k_refine_coh
-// and k_profile_coh, one CTA per record.  The inherited fields describe the coherent search: nvar = F = m_coh (1 +
-// half_bin) spectrum variants per block, dop_lo..dop_hi = m_coh times the engine's range (the record's 1/F-bin grid),
-// n_shift = 1.  A row is skipped (marker -1) when flags has the DETECTED bit and its snr is not >= thr_l1 (the caller's
-// min_snr); every row is C/A.
+// The records of a coherent search (acq_refine_coherent*, acq_profile_coherent*).  The inherited fields describe the
+// coherent search: nvar = F = m_coh (1 + half_bin) spectrum variants per block, dop_lo..dop_hi = m_coh times the engine's
+// range (the record's 1/F-bin grid), n_shift = 1.  A row is skipped (marker -1) when flags has the DETECTED bit and its
+// snr is not >= thr_l1 (the caller's min_snr); every row is C/A.
 struct RefineCohArgs : RefineArgs {
+    static constexpr bool kCoh = true;
     int m_coh;
 };
 struct ProfileCohArgs : ProfileArgs {
+    static constexpr bool kCoh = true;
     int m_coh;
 };
-int launch_refine_coh(const RefineCohArgs &a, int n_rows, cudaStream_t st);
-int launch_profile_coh(const ProfileCohArgs &a, int n_rows, cudaStream_t st);
+// RA: RefineArgs or RefineCohArgs; PA: ProfileArgs or ProfileCohArgs
+template <class RA>
+int launch_refine(const RA &a, int n_rows, cudaStream_t st);
+template <class PA>
+int launch_profile(const PA &a, int n_rows, cudaStream_t st);
 cudaError_t search_kernels_configure();
 
 }  // namespace acq
